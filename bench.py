@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (our arm: libuwip.so on N B200s)
   python bench.py --impl reference --gpus N --steps K ...   (CPU arm: the reference's algorithm on host cores)
+  python bench.py ... --dump-outputs DIR                    (also write the last timed step's outputs, see dump_outputs)
 
 A step = one pass of the chain over one batch of `--frames` (default 256) synthetic 3840x2160 bgr8
 frames per GPU (BASELINE.json configs[3]); frames shard across ranks by batch with no collective on
@@ -166,6 +167,28 @@ def cpu_chain_fps(procs, w, h, frames_per_proc=1, first=0):
     return len(jobs) / dt, dt
 
 
+DUMP_SAMPLE = 8 << 20   # output bytes written by --dump-outputs (32 MB as float32) when the batch holds more
+
+
+def dump_outputs(path, d_out, flags):
+    """What the last timed step returned to its caller, as float32 .npy files under `path`: `frames` = the output bytes
+    (the whole (n, H, W, 3) batch, or when it holds more than DUMP_SAMPLE bytes, the bytes at the flat positions
+    np.unique(default_rng(SEED).integers(0, batch size, DUMP_SAMPLE)) in that order) and `frame_flags` = the per-frame
+    flags (1 = the reference's result is a NaN frame)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    flat = d_out.reshape(-1)
+    if flat.numel() <= DUMP_SAMPLE:
+        frames = d_out.cpu().numpy()
+    else:
+        pos = np.unique(np.random.default_rng(SEED).integers(0, flat.numel(), DUMP_SAMPLE))
+        frames = flat[torch.from_numpy(pos).to(flat.device)].cpu().numpy()
+    np.save(os.path.join(path, "frames.npy"), frames.astype(np.float32))
+    np.save(os.path.join(path, "frame_flags.npy"), np.asarray(flags, np.float32))
+
+
 def chain_config(W, H, n):
     """`config` of the bench line: the same dictionary for the CUDA arm and for the reference arm."""
     fbytes = W * H * 3
@@ -279,14 +302,20 @@ def main():
     ap.add_argument("--frames", type=int, default=256, help="frames per GPU per step")
     ap.add_argument("--width", type=int, default=W4K)
     ap.add_argument("--height", type=int, default=H4K)
-    ap.add_argument("--e2e-steps", type=int, default=5)
+    ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of the host-buffer call (default: --steps)")
     ap.add_argument("--stream", type=int, default=0, help="BASELINE configs[4]: one pass over a stream of this many frames, "
                                                            "contiguous frame ranges per rank, per-frame checksums gathered")
     ap.add_argument("--copy-ceiling", action="store_true", help="also time the bare H2D + D2H copies of the e2e step (no kernels)")
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) as DIR/<name>.npy; "
+                                                          "CUDA arm only")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm; the reference arm keeps none")
+    if args.e2e_steps is None:
+        args.e2e_steps = args.steps
     if args.impl == "reference":
         return run_reference(args)
     if args.warmup < 3:
@@ -363,7 +392,10 @@ def main():
         ctx.profile(False)
         sums = ctx.checksum_dev(d_out, min(n, 4), W, H)
         # frames whose result is the reference's NaN frame (S = 0/0 somewhere, SURVEY D9): the chain writes zeros for them
-        nan_frames = int((np.asarray(ctx.last_frame_flags(n)) != 0).sum())
+        flags = np.asarray(ctx.last_frame_flags(n))
+        nan_frames = int((flags != 0).sum())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, d_out, flags)
 
     stream_res = None
     if args.stream > 0:

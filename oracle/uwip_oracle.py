@@ -507,6 +507,13 @@ def golden_frame(key: str) -> np.ndarray:
     return np.random.default_rng(int(seed, 16)).integers(0, 256, (H, W, 3), dtype=np.uint8)
 
 
+def golden_pixels(a: np.ndarray, px: np.ndarray) -> np.ndarray:
+    """Values of an (H, W) or (H, W, C) map at the flat pixel indices `px`: the float maps of tests/golden/dehaze_literal.npz
+    are stored at such a sample of pixels (its `px` key), compared maps are taken there."""
+    a = np.asarray(a)
+    return a.reshape((-1,) + a.shape[2:])[px]
+
+
 def calc_blur(bgr: np.ndarray, aperture: int = 3) -> np.float32:
     """float calcBlur(Mat frame), videostrip.cpp:170-184: the standard deviation of the Laplacian, returned as float."""
     return np.float32(mean_stddev_u8(laplacian3_u8(bgr2gray(bgr), aperture))[1])

@@ -241,16 +241,17 @@ def test_dehaze_golden_literal(ctx):
     z = np.load(os.path.join(GOLD, "dehaze_literal.npz"))
     for name in sorted({k.split("/")[0] for k in z.files}):
         fr = z[name + "/frame"]
+        px = z[name + "/px"]   # the float maps are stored at these pixels
         B, _ = ctx.background_light(fr, 15)
         assert np.abs(B - z[name + "/B"]).max() < 1e-15
         got8, gotf = ctx.bgdehaze(fr, return_float=True)
-        assert np.abs(gotf - z[name + "/out"]).max() < OUT_TOL, name
+        assert np.abs(O.golden_pixels(gotf, px) - z[name + "/out"]).max() < OUT_TOL, name
         ref8 = O._sat_u8_from_rint(z[name + "/out"] * 255).astype(int)
-        assert np.abs(got8.astype(int) - ref8).max() <= 1, name
+        assert np.abs(O.golden_pixels(got8, px).astype(int) - ref8).max() <= 1, name
         if name + "/t_blue" in z.files:
             rb, rg = ctx.refined_transmission(fr)
-            assert (np.abs(rb - z[name + "/t_blue"]) / np.abs(z[name + "/t_blue"])).max() < 1e-5
-            assert (np.abs(rg - z[name + "/t_green"]) / np.abs(z[name + "/t_green"])).max() < 1e-5
+            assert (np.abs(O.golden_pixels(rb, px) - z[name + "/t_blue"]) / np.abs(z[name + "/t_blue"])).max() < 1e-5
+            assert (np.abs(O.golden_pixels(rg, px) - z[name + "/t_green"]) / np.abs(z[name + "/t_green"])).max() < 1e-5
 
 
 def test_dehaze_1080p(ctx):
@@ -305,6 +306,28 @@ def test_chain_batch_matches_single_and_device_path(ctx):
     want = np.stack([O.chain_frame(f) for f in frames])
     assert np.abs(host.astype(int) - want.astype(int)).max() <= 1
     assert (ctx.last_frame_flags(n) == 0).all()
+
+
+def test_bench_dump_outputs_are_the_chain_outputs(ctx, tmp_path):
+    """`bench.py --dump-outputs DIR` writes what its timed chain step returned: the batch is small enough to be written
+    whole, so frames.npy must equal the chain of the same synthetic frames, and frame_flags.npy their flags."""
+    import json
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    W, H, n = 320, 180, 2
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--frames", str(n), "--width", str(W), "--height", str(H),
+                        "--steps", "1", "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600, cwd=root)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 1
+    frames = np.stack([O.synth_frame(0x5EED0004, f, W, H) for f in range(n)])   # bench.py's SEED, rank 0's frames
+    want = ctx.chain(frames)
+    got = np.load(tmp_path / "frames.npy")
+    assert got.dtype == np.float32 and (got == want).all()
+    flags = np.load(tmp_path / "frame_flags.npy")
+    assert flags.dtype == np.float32 and (flags == ctx.last_frame_flags(n)).all()
 
 
 def test_chain_host_schedule(ctx, monkeypatch):

@@ -171,6 +171,34 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["config"] == bench.chain_config(3840, 2160, 256)
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs DIR`: float32 .npy files of what the timed call returned, the whole batch when it is small,
+    otherwise the same seeded sample of positions on every run; at most 64 MB for the default 256-frame 4K batch."""
+    import torch
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+
+    assert 4 * bench.DUMP_SAMPLE + 4 * 256 <= 64 << 20
+    out = np.random.default_rng(2).integers(0, 256, (3, 20, 30, 3), dtype=np.uint8)
+    bench.dump_outputs(str(tmp_path / "a"), torch.from_numpy(out), np.array([0, 1, 0], np.int32))
+    frames, flags = np.load(tmp_path / "a" / "frames.npy"), np.load(tmp_path / "a" / "frame_flags.npy")
+    assert frames.dtype == flags.dtype == np.float32
+    assert (frames == out).all() and flags.tolist() == [0, 1, 0]
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), torch.from_numpy(out), np.zeros(3, np.int32))
+    b, c = np.load(tmp_path / "b" / "frames.npy"), np.load(tmp_path / "c" / "frames.npy")
+    assert b.dtype == np.float32 and 900 < b.size <= 1000 and (b == c).all()
+    pos = np.unique(np.random.default_rng(bench.SEED).integers(0, out.size, 1000))
+    assert (b == out.reshape(-1)[pos]).all()
+    # the reference arm keeps no outputs: asking it for them is an error, not a silent no-op
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path / "r")],
+                       capture_output=True, text=True, timeout=60, cwd=root)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "r").exists()
+
+
 def test_cli_argument_conventions():
     """The CLI shims keep cv::CommandLineParser's `-key=value` convention and the reference's defaults (histretch.cpp:68-74)."""
     from uwimageproc_b200.cli._args import parse
