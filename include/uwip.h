@@ -138,8 +138,8 @@ int uwip_clahe_entropy_sweep_u8(uwip_ctx* ctx, const uint8_t* plane, int width, 
                                 size_t pitch, int tiles, const double* clips, int n_clips,
                                 int flavour, float* entropies);
 /* the whole sweep of aclahe.cpp:160-193 / ACLAHE.py:20-47 in one call: n_frames device planes x n_grids square grids
- * (the reference's 2, 4, 8, 16, 32) x n_clips clip limits -> entropies [n_frames][n_grids][n_clips] (HOST pointer; the
- * 49-point knee search on them stays on the host like the reference's scipy calls).  Synchronises the stream. */
+ * (the reference's 2, 4, 8, 16, 32) x n_clips clip limits -> entropies [n_frames][n_grids][n_clips] (HOST pointer, for a
+ * host-side knee search; uwip_aclahe_params_u8_dev does the whole parameter search on the device).  Synchronises the stream. */
 int uwip_clahe_entropy_sweep_u8_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_frames, int width, int height,
                                     const int* grids, int n_grids, const double* clips, int n_clips,
                                     int flavour, float* entropies);
@@ -150,6 +150,30 @@ int uwip_aclahe_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t src_pitch, uint8_
 int uwip_aclahe_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_frames,
                          int width, int height, double clip, int tiles_x, int tiles_y,
                          int hsv_round);
+
+/* ---- automatic CLAHE parameters: ParametrosACLAHE (ACLAHE.py:9-129) on the device ------------------------------------ */
+/* loop: which sweep of ACLAHE.py:38-47 to run.  REPAIRED evaluates all 50 clip limits per block size (what the code
+ * intends); AS_COMMITTED is the file as it stands (the sweep body lost its indentation, the curves are all zero and the clip
+ * limit degenerates to 0: crowd.png -> (8, 0)). */
+typedef enum uwip_aclahe_loop {
+  UWIP_ACLAHE_LOOP_REPAIRED = 0,
+  UWIP_ACLAHE_LOOP_AS_COMMITTED = 1
+} uwip_aclahe_loop;
+/* For each of n equal-size device planes: GaussianBlur 3x3 -> entropy of CLAHE(blurred, k, c) for k in 2, 4, 8, 16, 32 and
+ * c in 0, 0.5 .. 24.5 -> per block size the knee of the entropy curve (scipy's curve_fit double exponential restated as
+ * MINPACK lmdif, not-a-knot spline, curvature argmax; csrc/aclahe_knee.h) -> CL = max of the five knees (an integer 0..48,
+ * used directly as the clip limit) -> BS = the block size whose entropy of CLAHE(blurred, BS, CL), rounded to float16, is
+ * the last maximum.  d_bs, d_cl: device int32[n].  A plane whose fit fails (the reference raises RuntimeError) gets
+ * BS = CL = -1 and the frame flag UWIP_FRAME_ACLAHE_NOFIT.  Planes too small for a 32 x 32 grid are refused
+ * (UWIP_ERR_INVALID).  Stream ordered, does not synchronise. */
+int uwip_aclahe_params_u8_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_planes, int width, int height, int loop,
+                              int32_t* d_bs, int32_t* d_cl);
+/* automatic aclahe on n device frames: V of each frame -> uwip_aclahe_params_u8_dev -> BGR->HSV, CLAHE on V with the
+ * frame's own (BS, CL), HSV->BGR.  clip and tiles_x x tiles_y are used only for frames whose fit failed.  d_bs, d_cl:
+ * optional device int32[n] outputs (NULL: not returned).  Stream ordered, does not synchronise. */
+int uwip_aclahe_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_frames, int width, int height,
+                              int loop, int hsv_round, double clip, int tiles_x, int tiles_y, int32_t* d_bs,
+                              int32_t* d_cl);
 
 /* ---- modules/bgdehaze ---------------------------------------------------------------------- */
 typedef struct uwip_dehaze_params {
@@ -207,6 +231,12 @@ void uwip_chain_defaults(uwip_chain_params* p);
 /* device resident: n_frames contiguous bgr8 frames in, same out (d_src may equal d_dst). */
 int uwip_chain_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_frames,
                         int width, int height, const uwip_chain_params* p);
+/* the chain with automatic CLAHE parameters: the parameters of each frame are found on the V plane of the frame that
+ * enters CLAHE (the histretch output, as the aclahe CLI does with its input); p->clip and p->tiles_* apply only to frames
+ * whose fit failed (UWIP_FRAME_ACLAHE_NOFIT).  d_bs, d_cl: optional device int32[n] outputs (NULL: not returned).  A frame's
+ * bytes do not depend on the batch it is in. */
+int uwip_chain_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_frames, int width, int height,
+                             const uwip_chain_params* p, int loop, int32_t* d_bs, int32_t* d_cl);
 /* host buffers (pinned memory recommended): H2D, chain, D2H pipelined over sub-batches through two staging buffers per
  * direction; the sub-batch sizes ramp up and down in whole CTA waves (csrc/e2e_schedule.h) so that only a few frames'
  * upload and download are exposed.  The bytes are those of the device-resident call whatever the schedule.  Returns after
@@ -214,11 +244,14 @@ int uwip_chain_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int
 int uwip_chain_bgr8(uwip_ctx* ctx, const uint8_t* src, uint8_t* dst, int n_frames, int width,
                     int height, const uwip_chain_params* p);
 
-/* per-frame status of the LAST uwip_chain_bgr8[_dev] / uwip_bgdehaze_bgr8_dev call on this context
- * (synchronises the stream).  UWIP_FRAME_NAN: the reference's adaptiveExp_map is NaN for the whole
- * frame (S = 0/0 where Yi = Yj = 0, BGDehaze.py:83, spreads through the box filters and the final
- * min-max; SURVEY 8a-D9) - the 8-bit output is then all zeros, exactly what imwrite would store. */
+/* per-frame status bits of the LAST uwip_chain_bgr8[_auto][_dev] / uwip_bgdehaze_bgr8_dev / uwip_aclahe_params_u8_dev /
+ * uwip_aclahe_bgr8_auto_dev call on this context (synchronises the stream).  UWIP_FRAME_NAN: the reference's
+ * adaptiveExp_map is NaN for the whole frame (S = 0/0 where Yi = Yj = 0, BGDehaze.py:83, spreads through the box filters
+ * and the final min-max; SURVEY 8a-D9) - the 8-bit output is then all zeros, exactly what imwrite would store.
+ * UWIP_FRAME_ACLAHE_NOFIT: an automatic-CLAHE call could not fit an entropy curve of the frame (the reference's curve_fit
+ * raises RuntimeError); the frame's BS = CL = -1 and it was processed with the fixed clip limit and grid. */
 #define UWIP_FRAME_NAN 1
+#define UWIP_FRAME_ACLAHE_NOFIT 2
 int uwip_last_frame_flags(uwip_ctx* ctx, int n_frames, int32_t* flags_host);
 
 /* ---- modules/videostrip: calcBlur (SURVEY 8f row N4, the frame-quality gate in front of the chain) */

@@ -68,6 +68,8 @@ SIGNATURES = {
     "uwip_clahe_entropy_sweep_u8_dev": (_i, [_P, _u8p, _i, _i, _i, C.POINTER(_i), _i, C.POINTER(_d), _i, _i, C.POINTER(C.c_float)]),
     "uwip_aclahe_bgr8": (_i, [_P, _u8p, _sz, _u8p, _sz, _i, _i, _d, _i, _i, _i]),
     "uwip_aclahe_bgr8_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, _d, _i, _i, _i]),
+    "uwip_aclahe_params_u8_dev": (_i, [_P, _u8p, _i, _i, _i, _i, _P, _P]),
+    "uwip_aclahe_bgr8_auto_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, _i, _i, _d, _i, _i, _P, _P]),
     "uwip_dehaze_defaults": (None, [C.POINTER(DehazeParams)]),
     "uwip_chain_defaults": (None, [C.POINTER(ChainParams)]),
     "uwip_boxfilter_f64": (_i, [_P, _P, _i, _i, _i, _P]),
@@ -79,6 +81,7 @@ SIGNATURES = {
     "uwip_bgdehaze_bgr8": (_i, [_P, _u8p, _sz, _u8p, _sz, _i, _i, C.POINTER(DehazeParams), _P]),
     "uwip_bgdehaze_bgr8_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, C.POINTER(DehazeParams)]),
     "uwip_chain_bgr8_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, C.POINTER(ChainParams)]),
+    "uwip_chain_bgr8_auto_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, C.POINTER(ChainParams), _i, _P, _P]),
     "uwip_chain_bgr8": (_i, [_P, _u8p, _u8p, _i, _i, _i, C.POINTER(ChainParams)]),
     "uwip_last_frame_flags": (_i, [_P, _i, _P]),
     "uwip_jpeg_info": (_i, [_P, _u8p, _sz, C.POINTER(_i), C.POINTER(_i)]),

@@ -7,6 +7,7 @@ from . import _lib
 from ._lib import ChainParams, DehazeParams, UwipError
 
 HSV_ROUND = {"cv2": 0, "trunc": 1, "rint": 2}
+ACLAHE_LOOP = {"repaired": 0, "as_committed": 1}
 ORDER = {"intended": 0, "literal": 1}
 
 
@@ -238,6 +239,30 @@ class Context:
         self._ck(self.lib.uwip_chain_bgr8(self.h, _ptr(a), _ptr(out), a.shape[0], a.shape[2], a.shape[1], C.byref(p)))
         return out[0] if single else out
 
+    def chain_auto(self, frames, params=None, loop="repaired"):
+        """The chain with automatic CLAHE parameters on a host array: frames uint8 (N, H, W, 3) or (H, W, 3) ->
+        (out of the same shape, BS int32[N], CL int32[N]); BS = CL = -1 where the fit failed (those frames used
+        params' fixed clip and tiles)."""
+        import torch
+
+        a = np.asarray(frames)
+        single = a.ndim == 3
+        if single:
+            a = a[None]
+        if a.dtype != np.uint8 or a.ndim != 4 or a.shape[3] != 3:
+            raise ValueError("expected uint8 (N, H, W, 3)")
+        n, h, w = a.shape[:3]
+        with torch.cuda.device(self.device):
+            d_src = torch.from_numpy(np.ascontiguousarray(a)).to("cuda")
+            d_dst = torch.empty_like(d_src)
+            d_bs = torch.empty(n, dtype=torch.int32, device="cuda")
+            d_cl = torch.empty(n, dtype=torch.int32, device="cuda")
+            torch.cuda.synchronize()
+            self.chain_auto_dev(d_src, d_dst, n, w, h, params, loop, d_bs, d_cl)
+            self.synchronize()
+            out, bs, cl = d_dst.cpu().numpy(), d_bs.cpu().numpy(), d_cl.cpu().numpy()
+        return (out[0] if single else out), bs, cl
+
     def chain_host_ptr(self, src_ptr, dst_ptr, n, width, height, params=None):
         p = params or self.chain_params()
         self._ck(self.lib.uwip_chain_bgr8(self.h, int(src_ptr), int(dst_ptr), n, width, height, C.byref(p)))
@@ -246,6 +271,13 @@ class Context:
     def chain_dev(self, d_src, d_dst, n, width, height, params=None):
         p = params or self.chain_params()
         self._ck(self.lib.uwip_chain_bgr8_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, C.byref(p)))
+
+    def chain_auto_dev(self, d_src, d_dst, n, width, height, params=None, loop="repaired", d_bs=None, d_cl=None):
+        """The chain with the CLAHE clip limit and grid of every frame found on the device (ParametrosACLAHE on the V plane
+        of the histretch output); d_bs, d_cl: optional device int32[n] outputs."""
+        p = params or self.chain_params()
+        self._ck(self.lib.uwip_chain_bgr8_auto_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, C.byref(p), ACLAHE_LOOP[loop],
+                                                   _ptr(d_bs) if d_bs is not None else None, _ptr(d_cl) if d_cl is not None else None))
 
     # ---- JPEG files to and from the device (nvJPEG) ------------------------------------------------
     def jpeg_info(self, data):
@@ -285,7 +317,8 @@ class Context:
         return out[: n.value].tobytes()
 
     def last_frame_flags(self, n):
-        """Per-frame status of the last batched chain / bgdehaze call: 1 = the reference output is NaN (D9)."""
+        """Per-frame status bits of the last batched chain / bgdehaze / automatic-aclahe call: 1 = the reference output is NaN
+        (D9), 2 = the automatic CLAHE fit failed (BS = CL = -1, fixed parameters used)."""
         out = np.empty(n, np.int32)
         self._ck(self.lib.uwip_last_frame_flags(self.h, int(n), _ptr(out)))
         return out
@@ -297,6 +330,25 @@ class Context:
     def aclahe_dev(self, d_src, d_dst, n, width, height, clip=2.0, tiles=(8, 8), hsv_round="cv2"):
         self._ck(self.lib.uwip_aclahe_bgr8_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, float(clip), tiles[0], tiles[1],
                                                HSV_ROUND[hsv_round]))
+
+    def aclahe_params_dev(self, d_planes, n, width, height, loop="repaired", d_bs=None, d_cl=None):
+        """ParametrosACLAHE on n device planes -> (BS, CL) in device int32[n] arrays (torch tensors unless given).  Stream
+        ordered: synchronise (or read the tensors on the context's stream) before using them."""
+        if d_bs is None or d_cl is None:
+            import torch
+
+            d_bs = torch.empty(n, dtype=torch.int32, device="cuda:%d" % self.device) if d_bs is None else d_bs
+            d_cl = torch.empty(n, dtype=torch.int32, device="cuda:%d" % self.device) if d_cl is None else d_cl
+        self._ck(self.lib.uwip_aclahe_params_u8_dev(self.h, _ptr(d_planes), n, width, height, ACLAHE_LOOP[loop], _ptr(d_bs), _ptr(d_cl)))
+        return d_bs, d_cl
+
+    def aclahe_auto_dev(self, d_src, d_dst, n, width, height, loop="repaired", hsv_round="cv2", clip=2.0, tiles=(8, 8), d_bs=None,
+                        d_cl=None):
+        """aclahe with each frame's own automatic (BS, CL); clip and tiles apply to frames whose fit failed."""
+        self._ck(self.lib.uwip_aclahe_bgr8_auto_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, ACLAHE_LOOP[loop],
+                                                    HSV_ROUND[hsv_round], float(clip), int(tiles[0]), int(tiles[1]),
+                                                    _ptr(d_bs) if d_bs is not None else None,
+                                                    _ptr(d_cl) if d_cl is not None else None))
 
     def clahe_dev(self, d_src, d_dst, n, width, height, clip=40.0, tiles=(8, 8)):
         self._ck(self.lib.uwip_clahe_u8_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, float(clip), int(tiles[0]), int(tiles[1])))

@@ -14,7 +14,9 @@ CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 LIB = os.path.join(HERE, "libuwip.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["cabi.cu", "histretch.cu", "clahe.cu", "dehaze.cu", "dehaze_gf1a.cu", "synth.cu", "blurmetric.cu", "jpegio.cu"]
+SOURCES = ["cabi.cu", "histretch.cu", "clahe.cu", "dehaze.cu", "dehaze_gf1a.cu", "synth.cu", "blurmetric.cu", "jpegio.cu", "aclahe_knee.cu"]
+# the knee search restates scipy's double-precision fit: no contraction into FMA
+SOURCE_FLAGS = {"aclahe_knee.cu": ["--fmad=false"]}
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",
@@ -31,7 +33,7 @@ def _nvcc():
 
 
 def _digest():
-    h = hashlib.sha256(" ".join(NVCC_FLAGS).encode())
+    h = hashlib.sha256((" ".join(NVCC_FLAGS) + repr(sorted(SOURCE_FLAGS.items()))).encode())
     paths = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(ROOT, "include", "uwip.h")]
     for p in paths:
         with open(p, "rb") as f:
@@ -50,7 +52,7 @@ def build(force=False, verbose=False):
 
     def cc(src):
         obj = os.path.join(OBJ, src.replace(".cu", ".o"))
-        cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [nvcc] + NVCC_FLAGS + SOURCE_FLAGS.get(src, []) + (["-Xptxas", "-v"] if verbose else []) + ["-c", os.path.join(CSRC, src), "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("nvcc failed for %s:\n%s\n%s" % (src, r.stdout, r.stderr))

@@ -413,6 +413,37 @@ int uwip_aclahe_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t sp, uint8_t* dst,
   return stage_out(ctx, d, dst, dp, w, h, 3);
 }
 
+static int32_t* flags_get(uwip_ctx* ctx, int n);
+
+// BS / CL outputs of the automatic calls: the caller's device arrays or the context's
+static int auto_outputs(uwip_ctx* ctx, int n, int32_t*& d_bs, int32_t*& d_cl) {
+  if (d_bs && d_cl) return UWIP_OK;
+  int32_t* ws = (int32_t*)uwip_slot(ctx, SLOT_AUTO_BSCL, sizeof(int32_t) * 2 * (size_t)n);
+  if (!ws) return UWIP_ERR_NOMEM;
+  if (!d_bs) d_bs = ws;
+  if (!d_cl) d_cl = ws + n;
+  return UWIP_OK;
+}
+
+int uwip_aclahe_params_u8_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int loop, int32_t* d_bs, int32_t* d_cl) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, d_planes && d_bs && d_cl && n > 0 && w > 0 && h > 0, "bad argument");
+  int32_t* flags = flags_get(ctx, n);
+  if (!flags) return UWIP_ERR_NOMEM;
+  UWIP_CHECK(aclahe_params_planes_dev(ctx, d_planes, n, w, h, loop, d_bs, d_cl));
+  return aclahe_nofit_flags(ctx, d_cl, n, flags, false);
+}
+int uwip_aclahe_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, int hsv_round,
+                              double clip, int tx, int ty, int32_t* d_bs, int32_t* d_cl) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, d_src && d_dst && n > 0 && w > 0 && h > 0 && hsv_round >= 0 && hsv_round <= 2, "bad argument");
+  UWIP_CHECK(auto_outputs(ctx, n, d_bs, d_cl));
+  int32_t* flags = flags_get(ctx, n);
+  if (!flags) return UWIP_ERR_NOMEM;
+  UWIP_CHECK(aclahe_frames_auto_dev(ctx, d_src, d_dst, n, w, h, loop, clip, tx, ty, hsv_round, nullptr, nullptr, d_bs, d_cl));
+  return aclahe_nofit_flags(ctx, d_cl, n, flags, false);
+}
+
 // ---- videostrip calcBlur ------------------------------------------------------------------------------
 int uwip_calc_blur_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, int n, int w, int h, int aperture, double* d_mean_std) {
   CTX_GUARD(ctx);
@@ -609,7 +640,23 @@ int uwip_bgdehaze_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, 
 }
 
 // ---- the chain ------------------------------------------------------------------------------------------
-static int chain_sub(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int m, int w, int h, const uwip_chain_params& p, FrameState* fs, int32_t* flags) {
+// automatic CLAHE parameters of a chain call (uwip_chain_bgr8_auto_dev): per-frame outputs of the sub-batch
+struct ChainAuto {
+  int loop;
+  int32_t* d_bs;
+  int32_t* d_cl;
+};
+
+static int chain_aclahe(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int m, int w, int h, const uwip_chain_params& p,
+                        const uint8_t* d_prelut, FrameState* fs, const ChainAuto* au) {
+  if (au)
+    return aclahe_frames_auto_dev(ctx, d_src, d_dst, m, w, h, au->loop, p.clip, p.tiles_x, p.tiles_y, p.hsv_round, d_prelut, fs, au->d_bs,
+                                  au->d_cl);
+  return aclahe_frames_dev(ctx, d_src, d_dst, m, w, h, p.clip, p.tiles_x, p.tiles_y, p.hsv_round, d_prelut, fs);
+}
+
+static int chain_sub(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int m, int w, int h, const uwip_chain_params& p, FrameState* fs, int32_t* flags,
+                     const ChainAuto* au = nullptr) {
   size_t fbytes = (size_t)w * h * 3;
   uint8_t* tmp = (uint8_t*)uwip_slot(ctx, SLOT_TMP_FRAME, fbytes * m);
   if (!tmp) return UWIP_ERR_NOMEM;
@@ -624,12 +671,13 @@ static int chain_sub(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int m,
     if (!d_hist || !d_lut) return UWIP_ERR_NOMEM;
     UWIP_CHECK(k_histogram_frame(ctx, d_src, m, w, h, CH_V, d_hist));
     UWIP_CHECK(k_percentile_lut(ctx, d_hist, m, w, h, p.lo, p.hi, fs, d_lut));
-    UWIP_CHECK(aclahe_frames_dev(ctx, d_src, tmp, m, w, h, p.clip, p.tiles_x, p.tiles_y, p.hsv_round, d_lut, fs));
+    UWIP_CHECK(chain_aclahe(ctx, d_src, tmp, m, w, h, p, d_lut, fs, au));
   } else {
     UWIP_CHECK(histretch_frames_dev(ctx, d_src, tmp, m, w, h, p.channels, p.lo, p.hi, p.order, p.hsv_round));
-    UWIP_CHECK(aclahe_frames_dev(ctx, tmp, tmp, m, w, h, p.clip, p.tiles_x, p.tiles_y, p.hsv_round, nullptr, fs));
+    UWIP_CHECK(chain_aclahe(ctx, tmp, tmp, m, w, h, p, nullptr, fs, au));
   }
-  return dehaze_frames_dev(ctx, tmp, d_dst, m, w, h, p.dehaze, true, fs, nullptr, flags);
+  UWIP_CHECK(dehaze_frames_dev(ctx, tmp, d_dst, m, w, h, p.dehaze, true, fs, nullptr, flags));
+  return au ? aclahe_nofit_flags(ctx, au->d_cl, m, flags, true) : UWIP_OK;
 }
 
 // size every workspace slot a sub-batch of m frames touches (the slots only grow: a later, smaller sub-batch reuses them)
@@ -667,6 +715,27 @@ int uwip_chain_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int
   for (int i = 0; i < n; i += nb) {
     int m = std::min(nb, n - i);
     UWIP_CHECK(chain_sub(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, *p, fs, flags + i));
+  }
+  return UWIP_OK;
+}
+
+int uwip_chain_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, const uwip_chain_params* p, int loop,
+                             int32_t* d_bs, int32_t* d_cl) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, d_src && d_dst, "null pointer");
+  UWIP_CHECK(chain_check(ctx, p, n, w, h));
+  UWIP_REQUIRE(ctx, loop == UWIP_ACLAHE_LOOP_REPAIRED || loop == UWIP_ACLAHE_LOOP_AS_COMMITTED, "bad loop");
+  UWIP_CHECK(aclahe_check_auto_size(ctx, w, h));
+  UWIP_CHECK(auto_outputs(ctx, n, d_bs, d_cl));
+  int nb = sub_batch(ctx, n, w, h);
+  FrameState* fs = frame_state_get(ctx, nb);
+  int32_t* flags = flags_get(ctx, n);
+  if (!fs || !flags) return UWIP_ERR_NOMEM;
+  size_t fbytes = (size_t)w * h * 3;
+  for (int i = 0; i < n; i += nb) {
+    int m = std::min(nb, n - i);
+    ChainAuto au = {loop, d_bs + i, d_cl + i};
+    UWIP_CHECK(chain_sub(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, *p, fs, flags + i, &au));
   }
   return UWIP_OK;
 }

@@ -7,6 +7,8 @@
 // (2) clip + redistribute + block prefix scan -> per-tile LUT, (3) bilinear blend of four tile LUTs,
 // fused with the BGR<->HSV conversions (and, in the chain, with the histretch LUT in front and the
 // dehaze min/max reduction behind).
+#include <cuda_fp16.h>
+
 #include <algorithm>
 #include <vector>
 
@@ -22,7 +24,7 @@ struct TileGeom {
   int tw, th;    // tile size
 };
 
-static TileGeom make_geom(int W, int H, int tx, int ty) {
+__host__ __device__ static TileGeom make_geom(int W, int H, int tx, int ty) {
   TileGeom g;
   g.W = W; g.H = H; g.tx = tx; g.ty = ty;
   if (W % tx == 0 && H % ty == 0) {
@@ -36,6 +38,15 @@ static TileGeom make_geom(int W, int H, int tx, int ty) {
   return g;
 }
 
+// per-frame CLAHE parameters of the automatic path (grid, clip limit in counts, LUT scale), read by the PF instantiations
+// of the three passes below: a CTA works on one frame, so its geometry stays uniform.  The workspaces of the PF passes
+// hold `tpf` tiles per frame (the largest grid of the batch), CTAs beyond their frame's tile count exit.
+struct FrameClahe {
+  TileGeom g;
+  int cl;
+  float lut_scale;
+};
+
 __device__ __forceinline__ int reflect101(int i, int n) {
   if (n == 1) return 0;
   while (i < 0 || i >= n) i = (i < 0) ? -i : 2 * n - 2 - i;
@@ -46,13 +57,18 @@ __device__ __forceinline__ int reflect101(int i, int n) {
 // FRAME=false: src is an 8U plane.  FRAME=true: src is bgr8 and the value is the HSV V channel
 // (max(b,g,r)), optionally pushed through two 256-entry LUTs (trunc / rint flavour chosen by x) =
 // the histretch stretch followed by the HSV->BGR->HSV round trip of its V channel.
-template <bool FRAME>
+template <bool FRAME, bool PF = false>
 __global__ void __launch_bounds__(TH_THREADS) tilehist_kernel(const uint8_t* __restrict__ src, TileGeom g, int splits,
                                                               const uint8_t* __restrict__ prelut2 /*[n][2][256] or null*/,
-                                                              int body_w, uint32_t* __restrict__ hist) {
+                                                              int body_w, uint32_t* __restrict__ hist,
+                                                              const FrameClahe* __restrict__ pf = nullptr, int tpf = 0) {
   __shared__ uint32_t sh[TH_WARPS][256];
   __shared__ uint8_t s_pre[2][256];
   int f = blockIdx.z;
+  if (PF) {
+    g = pf[f].g;
+    if ((int)blockIdx.x >= g.tx * g.ty) return;
+  }
   for (int i = threadIdx.x; i < TH_WARPS * 256; i += TH_THREADS) (&sh[0][0])[i] = 0;
   if (FRAME) {
     s_pre[0][threadIdx.x] = prelut2 ? prelut2[((size_t)f * 2 + 0) * 256 + threadIdx.x] : (uint8_t)threadIdx.x;
@@ -120,7 +136,7 @@ __global__ void __launch_bounds__(TH_THREADS) tilehist_kernel(const uint8_t* __r
   uint32_t s = 0;
 #pragma unroll
   for (int w = 0; w < TH_WARPS; w++) s += sh[w][threadIdx.x];
-  if (s) atomicAdd(&hist[((size_t)f * g.tx * g.ty + tile) * 256 + threadIdx.x], s);
+  if (s) atomicAdd(&hist[((PF ? (size_t)f * tpf : (size_t)f * g.tx * g.ty) + tile) * 256 + threadIdx.x], s);
 }
 
 // ---- pass 2: clip, redistribute, scan, LUT -------------------------------------------------------
@@ -148,14 +164,22 @@ __device__ __forceinline__ uint32_t block_incl_scan_256(uint32_t v, uint32_t* s_
 
 // one block per (tile, frame); `cl` = clip limit in counts (0: no clipping); n_cl > 1 builds LUTs for
 // several clip limits at once (entropy sweep): lut layout [frame][tile][icl][256]
+// PF: one clip limit per frame from pf[frame] (n_cl = 1), `tpf` tiles per frame of which the frame's grid uses the first
+template <bool PF = false>
 __global__ void __launch_bounds__(256) clahe_lut_kernel(const uint32_t* __restrict__ hist, const int* __restrict__ cls, int n_cl,
-                                                        float lut_scale, uint8_t* __restrict__ lut) {
+                                                        float lut_scale, uint8_t* __restrict__ lut,
+                                                        const FrameClahe* __restrict__ pf = nullptr, int tpf = 0) {
   __shared__ uint32_t s_warp[8];
   int t = threadIdx.x;
   size_t tile = blockIdx.x;
+  if (PF) {
+    const FrameClahe& q = pf[blockIdx.x / tpf];
+    if ((int)(blockIdx.x % tpf) >= q.g.tx * q.g.ty) return;
+    lut_scale = q.lut_scale;
+  }
   uint32_t h0 = hist[tile * 256 + t];
   for (int ic = 0; ic < n_cl; ic++) {
-    int cl = cls[ic];
+    int cl = PF ? pf[blockIdx.x / tpf].cl : cls[ic];
     uint32_t h = h0;
     if (cl > 0) {
       uint32_t excess = h > (uint32_t)cl ? h - cl : 0, clipped;
@@ -264,20 +288,22 @@ constexpr int AP_THREADS = 256;
 // and the loop body is four pixels long (the former sixteen-pixel body was 60 KB of code: a third of the warp stalls
 // were instruction fetches).
 constexpr int AP_ROWS = 8;   // rows whose y interpolation is tabulated per block
-template <int MODE, bool PRE>
+template <int MODE, bool PRE, bool PF = false>
 __global__ void __launch_bounds__(AP_THREADS) clahe_apply_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst,
-                                                                 TileGeom g, int rows_per, const uint8_t* __restrict__ lut,
+                                                                 TileGeom gp, int rows_per, const uint8_t* __restrict__ lut,
                                                                  const uint8_t* __restrict__ prelut /*[n][256], PRE only*/,
-                                                                 int body_w, FrameState* fs) {
+                                                                 int body_w, FrameState* fs,
+                                                                 const FrameClahe* __restrict__ pf = nullptr, int tpf = 0) {
   extern __shared__ uint8_t s_lut[];  // [3][tx][256] when it fits
   __shared__ uint8_t s_pre[256];
   __shared__ int s_sdiv[256], s_hdiv[256];
   __shared__ Interp s_iy[AP_ROWS];
   __shared__ __align__(16) float s_sec[48];
   int f = blockIdx.y;
+  const TileGeom g = PF ? pf[f].g : gp;
   int y0 = blockIdx.x * rows_per, y1 = min(y0 + rows_per, g.H);
   float inv_tw = __fdiv_rn(1.0f, (float)g.tw), inv_th = __fdiv_rn(1.0f, (float)g.th);
-  const uint8_t* flut = lut + (size_t)f * g.tx * g.ty * 256;
+  const uint8_t* flut = lut + (PF ? (size_t)f * tpf : (size_t)f * g.tx * g.ty) * 256;
   // tile rows needed by this band
   int ty_lo = interp_coord(y0, inv_th, g.ty).t1;
   int ty_hi = interp_coord(y1 - 1, inv_th, g.ty).t2;
@@ -448,7 +474,7 @@ static int clahe_common(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int
   int cl = clip_count(clip, g.tw * g.th);
   UWIP_CUDA(ctx, cudaMemcpyAsync(d_cl, &cl, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   float lut_scale = 255.0f / (float)(g.tw * g.th);
-  UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel, (unsigned)ntile, 256, 0, d_th, d_cl, 1, lut_scale, d_tl);
+  UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel<false>, (unsigned)ntile, 256, 0, d_th, d_cl, 1, lut_scale, d_tl);
   int rows_per = 8;
   while (rows_per > 1 && (long long)cdiv(h, rows_per) * n < (long long)ctx->sm_count * 4) rows_per /= 2;
   dim3 grid3(cdiv(h, rows_per), n);
@@ -557,19 +583,25 @@ __global__ void __launch_bounds__(SW_THREADS, 2) sweep_cell_kernel(const uint8_t
     if (s_hist[i]) atomicAdd(&oh[i], s_hist[i]);
 }
 
-// n planes x n_grids square grids x n_clips clip limits -> entropies [n][n_grids][n_clips] (host pointer)
-int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, const int* grids, int n_grids,
-                                  const double* clips, int n_clips, int flavour, float* entropies_host) {
-  UWIP_REQUIRE(ctx, n >= 1 && w >= 1 && h >= 1, "bad size");
-  UWIP_REQUIRE(ctx, n_clips >= 1 && n_clips <= SW_MAX_CL, "1..64 clip limits per sweep");
-  UWIP_REQUIRE(ctx, n_grids >= 1 && n_grids <= 16, "1..16 grids per sweep");
-  size_t max_tiles = 0;
+static int check_sweep_size(uwip_ctx* ctx, int w, int h, const int* grids, int n_grids) {
   for (int gi = 0; gi < n_grids; gi++) {
     UWIP_REQUIRE(ctx, grids[gi] >= 1 && grids[gi] <= 256, "tile grid out of range");
     TileGeom g = make_geom(w, h, grids[gi], grids[gi]);
     UWIP_REQUIRE(ctx, (g.EW == w || 2 * w - 2 >= g.EW - 1) && (g.EH == h || 2 * h - 2 >= g.EH - 1), "image too small for grid");
-    max_tiles = std::max(max_tiles, (size_t)grids[gi] * grids[gi]);
   }
+  return UWIP_OK;
+}
+
+// n planes x n_grids square grids x n_clips clip limits -> entropies on the device, layout [grid][frame][clip]; the
+// pointer is workspace of the context (valid until the next sweep)
+static int clahe_entropy_sweep_core(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, const int* grids, int n_grids,
+                                    const double* clips, int n_clips, int flavour, float** d_ent_out) {
+  UWIP_REQUIRE(ctx, n >= 1 && w >= 1 && h >= 1, "bad size");
+  UWIP_REQUIRE(ctx, n_clips >= 1 && n_clips <= SW_MAX_CL, "1..64 clip limits per sweep");
+  UWIP_REQUIRE(ctx, n_grids >= 1 && n_grids <= 16, "1..16 grids per sweep");
+  UWIP_CHECK(check_sweep_size(ctx, w, h, grids, n_grids));
+  size_t max_tiles = 0;
+  for (int gi = 0; gi < n_grids; gi++) max_tiles = std::max(max_tiles, (size_t)grids[gi] * grids[gi]);
   uint32_t* d_th = (uint32_t*)uwip_slot(ctx, SLOT_TILEHIST, (size_t)n * max_tiles * 256 * 4);
   uint8_t* d_tl = (uint8_t*)uwip_slot(ctx, SLOT_TILELUT, (size_t)n * max_tiles * 256 * n_clips + 16);
   const size_t hist_bytes = (size_t)n * n_grids * n_clips * 256 * 4, ent_bytes = (size_t)n * n_grids * n_clips * 4;
@@ -597,7 +629,7 @@ int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n,
     dim3 grid1(tiles * tiles, splits, n);
     UWIP_LAUNCH(ctx, "clahe_tilehist", tilehist_kernel<false>, grid1, TH_THREADS, 0, d_planes, g, splits, (const uint8_t*)nullptr, 0, d_th);
     float lut_scale = 255.0f / (float)(g.tw * g.th);
-    UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel, (unsigned)(ntile * n), 256, 0, d_th, d_cl, n_clips, lut_scale, d_tl);
+    UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel<false>, (unsigned)(ntile * n), 256, 0, d_th, d_cl, n_clips, lut_scale, d_tl);
     // bands of rows per cell: enough CTAs to fill the machine, at least 8 rows each
     const int cells = (tiles + 1) * (tiles + 1);
     const int cell_rows = g.th + 6;
@@ -610,6 +642,16 @@ int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n,
     UWIP_LAUNCH(ctx, "clahe_sweep_hist", sweep_cell_kernel, grid3, SW_THREADS, smem, d_planes, g, band_rows, bands, d_tl, n_clips, d_oh_g);
   }
   UWIP_CHECK(k_entropy(ctx, d_oh, n * n_grids * n_clips, w, h, flavour, d_ent));
+  *d_ent_out = d_ent;
+  return UWIP_OK;
+}
+
+// n planes x n_grids square grids x n_clips clip limits -> entropies [n][n_grids][n_clips] (host pointer)
+int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, const int* grids, int n_grids,
+                                  const double* clips, int n_clips, int flavour, float* entropies_host) {
+  float* d_ent = nullptr;
+  UWIP_CHECK(clahe_entropy_sweep_core(ctx, d_planes, n, w, h, grids, n_grids, clips, n_clips, flavour, &d_ent));
+  const size_t ent_bytes = (size_t)n * n_grids * n_clips * 4;
   std::vector<float> tmp((size_t)n * n_grids * n_clips);
   UWIP_CUDA(ctx, cudaMemcpyAsync(tmp.data(), d_ent, ent_bytes, cudaMemcpyDeviceToHost, ctx->stream));
   UWIP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -623,4 +665,194 @@ int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n,
 int clahe_entropy_sweep_dev(uwip_ctx* ctx, const uint8_t* d_plane, int w, int h, int tiles, const double* clips, int n_clips,
                             int flavour, float* entropies_host) {
   return clahe_entropy_sweep_batch_dev(ctx, d_plane, 1, w, h, &tiles, 1, clips, n_clips, flavour, entropies_host);
+}
+
+// ---- automatic CLAHE parameters (ParametrosACLAHE, ACLAHE.py:9-129; SURVEY 8f N1) and CLAHE with per-frame parameters ----
+static const int AUTO_GRIDS[5] = {2, 4, 8, 16, 32};   // ACLAHE.py:21
+constexpr int AUTO_NCL = 50;                          // np.arange(0, 25, 0.5)
+constexpr int AUTO_TPF = 32 * 32;                     // tiles per frame of the PF workspaces: the largest automatic grid
+
+__device__ __forceinline__ int clip_count_dev(double clip, int area) {   // clip_count on the device
+  if (!(clip > 0)) return 0;
+  int cl = (int)(clip * area / 256.0);
+  return cl < 1 ? 1 : cl;
+}
+
+// V plane of n bgr8 frames, optionally through the fused histretch head's two LUTs (the V of the intermediate frame)
+__global__ void vplane_kernel(const uint8_t* __restrict__ src, int w, int h, const uint8_t* __restrict__ prelut2, int body_w,
+                              uint8_t* __restrict__ dst) {
+  const int f = blockIdx.y;
+  const size_t n_px = (size_t)w * h;
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_px; i += (size_t)gridDim.x * blockDim.x) {
+    const uint8_t* p = src + (f * n_px + i) * 3;
+    int v = imax3(p[0], p[1], p[2]);
+    if (prelut2) v = prelut2[((size_t)f * 2 + ((int)(i % w) < body_w ? 0 : 1)) * 256 + v];
+    dst[f * n_px + i] = (uint8_t)v;
+  }
+}
+
+// the CLAHE parameters of grid `grid` at each frame's own clip limit (the block-size pick, ACLAHE.py:102-113)
+__global__ void pick_params_kernel(const int* __restrict__ cl, int n, TileGeom g, FrameClahe* __restrict__ pf) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
+  FrameClahe q;
+  q.g = g;
+  q.cl = clip_count_dev((double)max(cl[f], 0), g.tw * g.th);
+  q.lut_scale = 255.0f / (float)(g.tw * g.th);
+  pf[f] = q;
+}
+
+// BS = the grid whose entropy, rounded to float16, is the last maximum (ACLAHE.py:102, 117-121); -1 with CL for a frame
+// whose fit failed
+__global__ void pick_bs_kernel(const float* __restrict__ ent /*[5][n]*/, int n, const int* __restrict__ cl, int* __restrict__ bs) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
+  int w = 0;
+  float best = 0.f;
+  for (int m = 0; m < 5; m++) {
+    const float e = __half2float(__float2half_rn(ent[(size_t)m * n + f]));
+    if (m == 0 || e >= best) { best = e; w = m; }
+  }
+  const int grids[5] = {2, 4, 8, 16, 32};
+  bs[f] = cl[f] < 0 ? -1 : grids[w];
+}
+
+// per-frame parameters of the CLAHE apply: (BS, CL) or, for a frame whose fit failed, the caller's fixed ones
+__global__ void auto_geom_kernel(const int* __restrict__ bs, const int* __restrict__ cl, int n, int w, int h, FrameClahe fallback,
+                                 FrameClahe* __restrict__ pf) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
+  FrameClahe q = fallback;
+  if (cl[f] >= 0) {
+    q.g = make_geom(w, h, bs[f], bs[f]);
+    q.cl = clip_count_dev((double)cl[f], q.g.tw * q.g.th);
+    q.lut_scale = 255.0f / (float)(q.g.tw * q.g.th);
+  }
+  pf[f] = q;
+}
+
+__global__ void nofit_flags_kernel(const int* __restrict__ cl, int n, int32_t* __restrict__ flags, int keep) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
+  flags[f] = (keep ? flags[f] : 0) | (cl[f] < 0 ? UWIP_FRAME_ACLAHE_NOFIT : 0);
+}
+
+int aclahe_nofit_flags(uwip_ctx* ctx, const int* d_cl, int n, int32_t* d_flags, bool keep) {
+  UWIP_LAUNCH(ctx, "aclahe_flags", nofit_flags_kernel, cdiv(n, 128), 128, 0, d_cl, n, d_flags, keep ? 1 : 0);
+  return UWIP_OK;
+}
+
+int aclahe_check_auto_size(uwip_ctx* ctx, int w, int h) { return check_sweep_size(ctx, w, h, AUTO_GRIDS, 5); }
+
+// ParametrosACLAHE on n equal-size planes: blur -> sweep (5 grids x 50 clip limits) -> knee per grid -> CL = max of the knees
+// -> entropy of CLAHE(blurred, k, CL) per grid -> BS.  loop = 0 repaired, 1 as committed (CL = 0, ACLAHE.py:40-47 as it
+// stands).  Stream ordered; d_bs, d_cl are device int32[n].
+int aclahe_params_planes_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int loop, int* d_bs, int* d_cl) {
+  UWIP_REQUIRE(ctx, n >= 1 && w >= 1 && h >= 1, "bad size");
+  UWIP_REQUIRE(ctx, loop == UWIP_ACLAHE_LOOP_REPAIRED || loop == UWIP_ACLAHE_LOOP_AS_COMMITTED, "bad loop");
+  UWIP_CHECK(aclahe_check_auto_size(ctx, w, h));
+  const size_t n_px = (size_t)w * h;
+  uint8_t* d_blur = (uint8_t*)uwip_slot(ctx, SLOT_ABLUR, (size_t)n * n_px);
+  const size_t pf_bytes = align_up(sizeof(FrameClahe) * 5 * n, 256), ent_bytes = align_up(sizeof(float) * 5 * n, 256);
+  const size_t hist_bytes = (size_t)5 * n * 256 * 4;
+  char* d_ws = (char*)uwip_slot(ctx, SLOT_AUTO, 256 * 8 + pf_bytes + ent_bytes + hist_bytes);
+  if (!d_blur || !d_ws) return UWIP_ERR_NOMEM;
+  double* d_xd = (double*)d_ws;                                 // derivatives of the clip curve [2][49]
+  FrameClahe* d_pf = (FrameClahe*)(d_ws + 256 * 8);             // [5][n]
+  float* d_pent = (float*)(d_ws + 256 * 8 + pf_bytes);          // [5][n]
+  uint32_t* d_ph = (uint32_t*)(d_ws + 256 * 8 + pf_bytes + ent_bytes);   // [5][n][256]
+  UWIP_CHECK(k_blur3(ctx, d_planes, d_blur, w, h, n));
+  if (loop == UWIP_ACLAHE_LOOP_REPAIRED) {
+    double clips[AUTO_NCL];
+    for (int i = 0; i < AUTO_NCL; i++) clips[i] = 0.5 * i;
+    float* d_ent = nullptr;
+    UWIP_CHECK(clahe_entropy_sweep_core(ctx, d_blur, n, w, h, AUTO_GRIDS, 5, clips, AUTO_NCL, 1, &d_ent));
+    UWIP_CHECK(k_aclahe_knees(ctx, d_ent, n, AUTO_NCL, d_xd, d_cl));
+  } else {
+    UWIP_CUDA(ctx, cudaMemsetAsync(d_cl, 0, sizeof(int) * n, ctx->stream));
+  }
+  // block size: the tile-histogram, LUT and sweep passes with one clip limit per frame
+  uint32_t* d_th = (uint32_t*)uwip_slot(ctx, SLOT_TILEHIST, (size_t)n * AUTO_TPF * 256 * 4);
+  uint8_t* d_tl = (uint8_t*)uwip_slot(ctx, SLOT_TILELUT, (size_t)n * AUTO_TPF * 256 + 16);
+  if (!d_th || !d_tl) return UWIP_ERR_NOMEM;
+  UWIP_CUDA(ctx, cudaMemsetAsync(d_ph, 0, hist_bytes, ctx->stream));
+  const size_t smem = (size_t)256 * 8;
+  for (int gi = 0; gi < 5; gi++) {
+    const int tiles = AUTO_GRIDS[gi];
+    const TileGeom g = make_geom(w, h, tiles, tiles);
+    const int ntile = tiles * tiles;
+    FrameClahe* pf = d_pf + (size_t)gi * n;
+    UWIP_LAUNCH(ctx, "aclahe_pick_params", pick_params_kernel, cdiv(n, 128), 128, 0, d_cl, n, g, pf);
+    UWIP_CUDA(ctx, cudaMemsetAsync(d_th, 0, (size_t)n * ntile * 256 * 4, ctx->stream));
+    const int splits = pick_splits(ctx, g, n);
+    UWIP_LAUNCH(ctx, "clahe_tilehist", tilehist_kernel<false>, dim3(ntile, splits, n), TH_THREADS, 0, d_blur, g, splits,
+                (const uint8_t*)nullptr, 0, d_th);
+    UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel<true>, (unsigned)(ntile * n), 256, 0, d_th, (const int*)nullptr, 1, 0.f, d_tl,
+                (const FrameClahe*)pf, ntile);
+    const int cells = (tiles + 1) * (tiles + 1), cell_rows = g.th + 6;
+    int bands = std::max(1, std::min(cdiv(ctx->sm_count * 4, cells * n), cdiv(cell_rows, 8)));
+    const int band_rows = cdiv(cell_rows, bands);
+    bands = cdiv(cell_rows, band_rows);
+    UWIP_LAUNCH(ctx, "clahe_sweep_hist", sweep_cell_kernel, dim3(cells * bands, 1, n), SW_THREADS, smem, d_blur, g, band_rows, bands,
+                d_tl, 1, d_ph + (size_t)gi * n * 256);
+  }
+  UWIP_CHECK(k_entropy(ctx, d_ph, 5 * n, w, h, 1, d_pent));
+  UWIP_LAUNCH(ctx, "aclahe_pick_bs", pick_bs_kernel, cdiv(n, 128), 128, 0, d_pent, n, d_cl, d_bs);
+  return UWIP_OK;
+}
+
+// BGR->HSV, CLAHE on V with each frame's own (BS, CL), HSV->BGR on n frames (optionally behind the fused histretch head and
+// with the dehaze min / max, like aclahe_frames_dev).  The parameters are found on the V plane of the frame that enters CLAHE;
+// frames whose fit fails (CL = -1) get the fixed clip / tx x ty.
+int aclahe_frames_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty,
+                           int hsv_round, const uint8_t* d_prelut, FrameState* fs, int* d_bs, int* d_cl) {
+  UWIP_REQUIRE(ctx, tx >= 1 && ty >= 1 && tx <= 256 && ty <= 256, "tile grid out of range");
+  UWIP_REQUIRE(ctx, w >= 1 && h >= 1 && n >= 1, "bad size");
+  const TileGeom gf = make_geom(w, h, tx, ty);
+  UWIP_REQUIRE(ctx, (gf.EW == w || 2 * w - 2 >= gf.EW - 1 || w == 1) && (gf.EH == h || 2 * h - 2 >= gf.EH - 1 || h == 1),
+               "image too small for this tile grid (reflect-101 padding undefined)");
+  UWIP_CHECK(aclahe_check_auto_size(ctx, w, h));
+  const size_t n_px = (size_t)w * h;
+  const int bw = body_width(w, hsv_round);
+  uint8_t* d_v = (uint8_t*)uwip_slot(ctx, SLOT_APLANE, (size_t)n * n_px);
+  if (!d_v) return UWIP_ERR_NOMEM;
+  uint8_t* d_pre2 = nullptr;
+  if (d_prelut) {
+    d_pre2 = (uint8_t*)uwip_slot(ctx, SLOT_LUT, (size_t)n * 256 * 4) + (size_t)n * 256;  // second half of the LUT slot
+    if (!d_pre2) return UWIP_ERR_NOMEM;
+    UWIP_LAUNCH(ctx, "prelut2", prelut2_kernel, n, 256, 0, d_prelut, d_pre2);
+  }
+  UWIP_LAUNCH(ctx, "aclahe_vplane", vplane_kernel, dim3(std::max(1, std::min(cdiv((int)std::min<size_t>(n_px, 1 << 30), 256), 1024)), n), 256, 0,
+              d_src, w, h, (const uint8_t*)d_pre2, bw, d_v);
+  UWIP_CHECK(aclahe_params_planes_dev(ctx, d_v, n, w, h, loop, d_bs, d_cl));
+  // per-frame geometry in the PF workspace: tpf tiles per frame
+  const int tpf = std::max(AUTO_TPF, tx * ty);
+  char* d_ws = (char*)uwip_slot(ctx, SLOT_AUTO, 0);   // the params call sized it: [2][49] doubles, then FrameClahe[5][n]
+  FrameClahe* d_pf = (FrameClahe*)(d_ws + 256 * 8);   // reuses the pick's [0][n] block, consumed by then in stream order
+  FrameClahe fb;
+  fb.g = gf;
+  fb.cl = clip_count(clip, gf.tw * gf.th);
+  fb.lut_scale = 255.0f / (float)(gf.tw * gf.th);
+  UWIP_LAUNCH(ctx, "aclahe_geom", auto_geom_kernel, cdiv(n, 128), 128, 0, d_bs, d_cl, n, w, h, fb, d_pf);
+  uint32_t* d_th = (uint32_t*)uwip_slot(ctx, SLOT_TILEHIST, (size_t)n * tpf * 256 * 4);
+  uint8_t* d_tl = (uint8_t*)uwip_slot(ctx, SLOT_TILELUT, (size_t)n * tpf * 256 + 16);
+  if (!d_th || !d_tl) return UWIP_ERR_NOMEM;
+  UWIP_CUDA(ctx, cudaMemsetAsync(d_th, 0, (size_t)n * tpf * 256 * 4, ctx->stream));
+  // row splits sized for the coarsest grid (2 x 2: the tallest tiles); finer grids leave the upper splits idle
+  const int splits = pick_splits(ctx, make_geom(w, h, 2, 2), n);
+  UWIP_LAUNCH(ctx, "clahe_tilehist", (tilehist_kernel<true, true>), dim3(tpf, splits, n), TH_THREADS, 0, d_src, gf, splits,
+              (const uint8_t*)d_pre2, bw, d_th, (const FrameClahe*)d_pf, tpf);
+  UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel<true>, (unsigned)((size_t)tpf * n), 256, 0, d_th, (const int*)nullptr, 1, 0.f, d_tl,
+              (const FrameClahe*)d_pf, tpf);
+  int rows_per = 8;
+  while (rows_per > 1 && (long long)cdiv(h, rows_per) * n < (long long)ctx->sm_count * 4) rows_per /= 2;
+  dim3 grid3(cdiv(h, rows_per), n);
+  const size_t smem = (size_t)3 * 32 * 256;   // staged LUT rows of grids up to 32 tiles wide
+  if (d_prelut)
+    UWIP_LAUNCH(ctx, "clahe_apply", (clahe_apply_kernel<1, true, true>), grid3, AP_THREADS, smem, d_src, d_dst, gf, rows_per, d_tl, d_prelut,
+                bw, fs, (const FrameClahe*)d_pf, tpf);
+  else
+    UWIP_LAUNCH(ctx, "clahe_apply", (clahe_apply_kernel<1, false, true>), grid3, AP_THREADS, smem, d_src, d_dst, gf, rows_per, d_tl,
+                d_prelut, bw, fs, (const FrameClahe*)d_pf, tpf);
+  return UWIP_OK;
 }

@@ -83,6 +83,10 @@ enum Slot {
   SLOT_SPLANE,        // dehaze: exposure ratio per pixel (f32)
   SLOT_BLURSUMS,      // calcBlur: per-frame sum and sum of squares of the 8-bit Laplacian (u64 x2)
   SLOT_BLUROUT,       // calcBlur: per-frame mean, stdev (f64 x2)
+  SLOT_APLANE,        // automatic CLAHE: V planes of the frames (u8)
+  SLOT_ABLUR,         // automatic CLAHE: blurred planes (u8)
+  SLOT_AUTO,          // automatic CLAHE: clip-curve derivatives, per-frame parameters, pick histograms and entropies
+  SLOT_AUTO_BSCL,     // automatic CLAHE: BS, CL of the frames when the caller does not ask for them (int32 x2)
 };
 
 const char* uwip_set_err(uwip_ctx* ctx, const char* fmt, ...);
@@ -362,7 +366,7 @@ int k_apply_lut_plane(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n
 int k_apply_lut_frame(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_frames, int w, int h, int channel, const uint8_t* d_lut, bool use_lut, int hsv_round);
 int k_hist_to_float(uwip_ctx* ctx, const uint32_t* d_hist, float* d_out, int n);
 int k_entropy(uwip_ctx* ctx, const uint32_t* d_hist, int n_hists, int w, int h, int flavour, float* d_out);
-int k_blur3(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int w, int h);
+int k_blur3(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int w, int h, int n = 1);   // n planes of w x h
 int histretch_frames_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, const char* channels, int lo, int hi, int order, int hsv_round);
 
 // clahe.cu
@@ -370,6 +374,13 @@ int clahe_planes_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n,
 int aclahe_frames_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, double clip, int tx, int ty, int hsv_round, const uint8_t* d_prelut /*optional per-frame stretch LUT fused in front*/, FrameState* fs_minmax /*optional: accumulate dehaze D0 min/max of the output*/);
 int clahe_entropy_sweep_dev(uwip_ctx* ctx, const uint8_t* d_plane, int w, int h, int tiles, const double* clips, int n_clips, int flavour, float* entropies_host);
 int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, const int* grids, int n_grids, const double* clips, int n_clips, int flavour, float* entropies_host);
+int aclahe_check_auto_size(uwip_ctx* ctx, int w, int h);   // UWIP_ERR_INVALID when a plane is too small for a grid of 2..32
+int aclahe_params_planes_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int loop, int* d_bs, int* d_cl);
+int aclahe_frames_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty, int hsv_round, const uint8_t* d_prelut, FrameState* fs_minmax, int* d_bs, int* d_cl);
+int aclahe_nofit_flags(uwip_ctx* ctx, const int* d_cl, int n, int32_t* d_flags, bool keep);   // flags |= NOFIT where CL < 0
+
+// aclahe_knee.cu
+int k_aclahe_knees(uwip_ctx* ctx, const float* d_ent /*[5][n][n_clips]*/, int n, int n_clips, double* d_xd /*[2][49] scratch*/, int* d_cl);
 
 // dehaze.cu
 struct DehazeDebug {  // optional float64 stage outputs for the stage-wise host API (device pointers)

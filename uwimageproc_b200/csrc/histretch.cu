@@ -521,11 +521,13 @@ int k_entropy(uwip_ctx* ctx, const uint32_t* d_hist, int n_hists, int w, int h, 
   return UWIP_OK;
 }
 
-// GaussianBlur((3,3),0) on 8U: (sum [1 2 1]^T [1 2 1] p + 8) >> 4, reflect-101 border (ACLAHE.py:15)
+// GaussianBlur((3,3),0) on 8U: (sum [1 2 1]^T [1 2 1] p + 8) >> 4, reflect-101 border (ACLAHE.py:15); plane blockIdx.z
 __global__ void blur3_kernel(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, int w, int h) {
   int x = blockIdx.x * blockDim.x + threadIdx.x;
   int y = blockIdx.y * blockDim.y + threadIdx.y;
   if (x >= w || y >= h) return;
+  src += (size_t)blockIdx.z * w * h;
+  dst += (size_t)blockIdx.z * w * h;
   auto rx = [&](int i) { return i < 0 ? -i : (i >= w ? 2 * w - 2 - i : i); };
   auto ry = [&](int i) { return i < 0 ? -i : (i >= h ? 2 * h - 2 - i : i); };
   int xs[3] = {w > 1 ? rx(x - 1) : 0, x, w > 1 ? rx(x + 1) : 0};
@@ -538,8 +540,8 @@ __global__ void blur3_kernel(const uint8_t* __restrict__ src, uint8_t* __restric
     for (int i = 0; i < 3; i++) acc += k[j] * k[i] * src[(size_t)ys[j] * w + xs[i]];
   dst[(size_t)y * w + x] = (uint8_t)((acc + 8) >> 4);
 }
-int k_blur3(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int w, int h) {
-  dim3 block(32, 8), grid(cdiv(w, 32), cdiv(h, 8));
+int k_blur3(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int w, int h, int n) {
+  dim3 block(32, 8), grid(cdiv(w, 32), cdiv(h, 8), n);
   UWIP_LAUNCH(ctx, "blur3", blur3_kernel, grid, block, 0, d_src, d_dst, w, h);
   return UWIP_OK;
 }

@@ -1,8 +1,8 @@
 """Mirror of modules/aclahe/python/{functions,ACLAHE,main}.py (reference function names kept).
 
-Pixel work (GaussianBlur 3x3, CLAHE, entropy, the clip-limit sweep) runs in libuwip.so.  The knee
-search on the 49 entropy samples per block size (curve_fit + spline derivatives + curvature,
-functions.py:49-93) is host-side in the reference and stays host-side here, with the same scipy calls.
+Pixel work (GaussianBlur 3x3, CLAHE, entropy, the clip-limit sweep) runs in libuwip.so.  ParametrosACLAHE keeps the
+reference's host-side knee search on the 49 entropy samples per block size (curve_fit + spline derivatives + curvature,
+functions.py:49-93) with the same scipy calls; parametros_aclahe_batch runs the whole search for a batch on the device.
 """
 import warnings
 
@@ -91,6 +91,22 @@ def ParametrosACLAHE(imagen, loop="repaired"):
         res[1, m] = Entropia(CLAHE(imgfilt, k, d))
     w = int(np.flatnonzero(res[1] == res[1].max())[-1])  # last arg-max wins, ACLAHE.py:117-121
     return int(round(float(res[0, w]))), d
+
+
+def parametros_aclahe_batch(planes, loop="repaired"):
+    """ParametrosACLAHE of every plane of a batch, on the device: planes uint8 (N, H, W) host array or device tensor ->
+    (BS int32[N], CL int32[N]); -1 where the reference's curve fit raises."""
+    import torch
+
+    ctx = default_context()
+    t = planes if isinstance(planes, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(planes, dtype=np.uint8))
+    if t.dtype != torch.uint8 or t.dim() != 3:
+        raise ValueError("expected uint8 (N, H, W)")
+    t = t.to("cuda:%d" % ctx.device).contiguous()
+    torch.cuda.synchronize(ctx.device)
+    bs, cl = ctx.aclahe_params_dev(t, t.shape[0], t.shape[2], t.shape[1], loop)
+    ctx.synchronize()
+    return bs.cpu().numpy(), cl.cpu().numpy()
 
 
 def main(img):
