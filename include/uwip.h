@@ -179,8 +179,10 @@ int uwip_aclahe_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_ds
 typedef struct uwip_dehaze_params {
   int window;  /* dark-channel window of Background_light; default 15 (main.py:28).  The transmission
                   window is ALWAYS 15 because dehazed_BG calls refined_t without w (BGDehaze.py:52) */
-  int radius;  /* guided filter radius, 40 (BGDehaze.py:41,72)  */
-  double eps;  /* guided filter eps, 1e-3 (BGDehaze.py:42,73)   */
+  int radius;  /* guided filter radius, 40 (BGDehaze.py:41,72); 1..128: the window sums of the guide
+                  moments are 32-bit, exact while (2r+1)^2 255^2 < 2^32 */
+  double eps;  /* guided filter eps, 1e-3 (BGDehaze.py:42,73); >= 1e-3: the coefficients are stored in
+                  fixed point whose step grows as eps shrinks */
   double tmin; /* transmission floor, 0.2 (BGDehaze.py:40)      */
 } uwip_dehaze_params;
 void uwip_dehaze_defaults(uwip_dehaze_params* p);
@@ -190,7 +192,7 @@ void uwip_dehaze_defaults(uwip_dehaze_params* p);
 int uwip_boxfilter_f64(uwip_ctx* ctx, const double* src, int width, int height, int r, double* dst);
 /* guided_filter(I, p, r, eps)  guidedfilter.py:54-103 for a guide of the form I = guide8 / range, guide8 an 8-bit
  * three-channel image (every guide on the path is one: normI of main.py:17, normYiCrCb of BGDehaze.py:77-80);
- * p float64 in [0, 1.6] (held on a 2^-28 grid), q float64.  Runs the same two marches as the chain's filters. */
+ * p float64 in [0, 1.6] (held on a 2^-28 grid), q float64, r 1..128, eps >= 1e-3.  Runs the same two marches as the chain's filters. */
 int uwip_guided_filter_u8(uwip_ctx* ctx, const uint8_t* guide, size_t pitch, int width, int height,
                           int range, const double* p, int r, double eps, double* q);
 /* Background_light(normI, w)  BGDehaze.py:14-26 on the frame normalised as main.py:17.

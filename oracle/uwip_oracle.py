@@ -807,11 +807,11 @@ def _minmax_norm(x):
         return (x - x.min()) / (x.max() - x.min())
 
 
-def dehazed_bg(normI, w=15, stages=None):
-    """BGDehaze.py:50-57."""
+def dehazed_bg(normI, w=15, stages=None, r=40, eps=1e-3, tmin=0.2):
+    """BGDehaze.py:50-57; r, eps and tmin are the reference's fixed values (BGDehaze.py:41) unless given."""
     B = background_light(normI, w)
     B15 = B if w == 15 else background_light(normI, 15)
-    rb, rg = refined_t(normI, 15, B=B15)
+    rb, rg = refined_t(normI, 15, tmin, r, eps, B=B15)
     with np.errstate(divide="ignore", invalid="ignore"):
         Jb = (normI[..., 0] - B[0]) / rb + B[0]
         Jg = (normI[..., 1] - B[1]) / rg + B[1]
@@ -820,9 +820,9 @@ def dehazed_bg(normI, w=15, stages=None):
     return _minmax_norm(Jb), _minmax_norm(Jg)
 
 
-def rc_correction(normI, w=15, stages=None):
+def rc_correction(normI, w=15, stages=None, r=40, eps=1e-3, tmin=0.2):
     """BGDehaze.py:59-69."""
-    nb, ng = dehazed_bg(normI, w, stages)
+    nb, ng = dehazed_bg(normI, w, stages, r, eps, tmin)
     avgRr = 1.5 - np.average(nb.ravel()) - np.average(ng.ravel())
     with np.errstate(divide="ignore", invalid="ignore"):
         coef = avgRr / np.average(normI[..., 2].ravel())
@@ -836,10 +836,9 @@ def rc_correction(normI, w=15, stages=None):
     return restored
 
 
-def adaptive_exp_map(normI, w=15, stages=None):
-    """BGDehaze.py:71-89."""
-    r, eps = 40, 1e-3
-    restored = rc_correction(normI, w, stages)
+def adaptive_exp_map(normI, w=15, stages=None, r=40, eps=1e-3, tmin=0.2):
+    """BGDehaze.py:71-89; r and eps (fixed at 40 and 1e-3 at BGDehaze.py:72) serve all three guided filters."""
+    restored = rc_correction(normI, w, stages, r, eps, tmin)
     with np.errstate(invalid="ignore"):
         R = (restored * 255).astype(np.uint8)
         I = (normI * 255).astype(np.uint8)
@@ -857,11 +856,12 @@ def adaptive_exp_map(normI, w=15, stages=None):
     return _minmax_norm(out)
 
 
-def bgdehaze_frame(bgr8: np.ndarray, w: int = 15, stages=None):
+def bgdehaze_frame(bgr8: np.ndarray, w: int = 15, stages=None, r=40, eps=1e-3, tmin=0.2):
     """bgdehaze/main.py:16-19 minus file I/O: returns (float64 HxWx3 in [0,1], uint8 HxWx3 =
-    what imwrite hands to the encoder: sat(rint(restored * 255)), NaN -> 0)."""
+    what imwrite hands to the encoder: sat(rint(restored * 255)), NaN -> 0).  r, eps, tmin: the guided filters'
+    radius and regulariser and the floor of the raw transmission (uwip_dehaze_params)."""
     normI = normalize_frame(bgr8)
-    out = adaptive_exp_map(normI, w, stages)
+    out = adaptive_exp_map(normI, w, stages, r, eps, tmin)
     return out, _sat_u8_from_rint(out * 255)
 
 

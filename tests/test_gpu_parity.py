@@ -470,12 +470,12 @@ def test_cpp_shims_on_device():
     assert r.returncode == 0, r.stdout + r.stderr
 
 
-@pytest.mark.parametrize("radius", [3, 4, 7, 10, 16, 40, 63, 64, 65, 100, 160])
+@pytest.mark.parametrize("radius", [3, 4, 7, 10, 16, 40, 63, 64, 65, 100, 128])
 def test_refined_transmission_other_radii(ctx, radius):
     """The guided-filter radius is a parameter of the ABI (the reference fixes r=40, BGDehaze.py:41): radii that
     are multiples of 4 take the quad path, the others the scalar window path; windows wider than 127 pixels (r >= 64)
     recompute the per-column pixel counts per row instead of unpacking them; all against the oracle."""
-    fr = O.synth_frame(0x5EED0003, 2, 212, 118)   # width not a multiple of 4: pad columns are exercised too
+    fr = O.synth_frame(0x5EED0003, 2, 213, 118)   # width not a multiple of 4: pad columns are exercised too
     normI = O.normalize_frame(fr)
     for eps, tmin in [(1e-3, 0.2), (1e-2, 0.35)]:
         rb, rg = ctx.refined_transmission(fr, ctx.dehaze_params(radius=radius, eps=eps, tmin=tmin))
@@ -543,9 +543,14 @@ def test_abi_error_statuses(ctx):
         assert lib.uwip_channel_stretch_u8(ctx.h, plane.ctypes.data, 16, out.ctypes.data, 16, 16, 16, lo, hi, None, None) == -1
     # dehaze parameter ranges
     fr = np.zeros((32, 32, 3), np.uint8) + np.arange(32, dtype=np.uint8)[None, :, None] * 7
-    for kw in (dict(window=0), dict(window=35), dict(radius=0), dict(radius=161)):
+    for kw in (dict(window=0), dict(window=35), dict(radius=0), dict(radius=129), dict(radius=161)):
         with pytest.raises(u.UwipError) as e:
             ctx.bgdehaze(fr, ctx.dehaze_params(**kw))
+        assert e.value.status == -1
+    # radius 129: a full window's sum of k_i k_j can pass 2^32 (guided_filter_u8_dev's 32-bit moment sums)
+    for r in (0, 129):
+        with pytest.raises(u.UwipError) as e:
+            ctx.guided_filter_u8(fr, 255, np.full(fr.shape[:2], 0.5), r, 1e-3)
         assert e.value.status == -1
     # a call after an error works (the context stays usable)
     assert (ctx.histogram(plane) == O.get_histogram(plane)).all()

@@ -718,8 +718,9 @@ int dehaze_frames_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n
                       bool minmax_done, FrameState* fs, DehazeDebug* dbg, int32_t* d_flags) {
   UWIP_REQUIRE(ctx, n >= 1 && W >= 1 && H >= 1, "bad size");
   UWIP_REQUIRE(ctx, p.window >= 1 && p.window <= WK_MAXWIN, "window must be 1..33");
-  UWIP_REQUIRE(ctx, p.radius >= 1 && p.radius <= 160, "radius must be 1..160");
-  UWIP_REQUIRE(ctx, p.eps > 0.0 && p.tmin <= 1.0, "eps must be positive and tmin <= 1");
+  // (2r+1)^2 255^2 < 2^32: the 32-bit window sums of the guide moments stay exact (GP_MAX_RADIUS)
+  UWIP_REQUIRE(ctx, p.radius >= 1 && p.radius <= GP_MAX_RADIUS, "radius must be 1..128");
+  UWIP_REQUIRE(ctx, p.eps >= GP_MIN_EPS && p.tmin <= 1.0, "eps must be >= 1e-3 and tmin <= 1");
   UWIP_REQUIRE(ctx, (size_t)W * H < (1ull << 31), "frame too large");
   UWIP_REQUIRE(ctx, !dbg || n == 1, "stage outputs are single-frame");
   size_t n_px = (size_t)W * H;
@@ -843,7 +844,8 @@ __global__ void gfq_state_kernel(FrameState* fs, int range) {
 }
 int guided_filter_u8_dev(uwip_ctx* ctx, const uint8_t* d_guide, const double* d_p, double* d_q, int W, int H, int range, int r, double eps,
                          FrameState* fs) {
-  UWIP_REQUIRE(ctx, W >= 1 && H >= 1 && r >= 1 && r <= 160 && range >= 1 && range <= 255 && eps > 0.0, "bad argument");
+  // (2r+1)^2 255^2 < 2^32 for r <= GP_MAX_RADIUS, as in dehaze_frames_dev
+  UWIP_REQUIRE(ctx, W >= 1 && H >= 1 && r >= 1 && r <= GP_MAX_RADIUS && range >= 1 && range <= 255 && eps >= GP_MIN_EPS, "bad argument");
   const int Wp = (W + 3) & ~3;
   const size_t n_pp = (size_t)Wp * H;
   uint32_t* d_ycc = (uint32_t*)uwip_slot(ctx, SLOT_YCC, n_pp * 4);

@@ -128,6 +128,15 @@ struct GfCommon {
   double* dbg_tref;       // optional [2][H*W] (frame 0 only)
 };
 
+// Largest guided-filter radius: SOLVE forms the window sums of the guide moments k_i k_j (k <= 255) as uint32
+// (gp_window_pair), exact while a full window's (2r+1)^2 255^2 < 2^32 - up to r = 128 (4,294,836,225; r = 129 can reach
+// 4,361,942,025).  The entry points refuse larger radii.
+constexpr int GP_MAX_RADIUS = 128;
+// Smallest eps: the stored b of a coefficient chunk is int32 fixed point with the exponent of coef_scale's proven bound
+// 1.6 + 1.4 / sqrt(eps), so its step grows as eps shrinks (2^-24 at 1e-3, 2^-22 at 1e-4, 2^-19 at 1e-6).  Below 1e-3 the
+// rounding of b alone puts outputs near zero (a step edge of p, t near 0 with tmin = 0) past 1e-5 of max(|q|, 1e-3).
+constexpr double GP_MIN_EPS = 1e-3;
+
 // strip geometry of one launch (see the file header)
 struct GfGeom {
   int W, H, Wp;   // image size; pitch of the internal planes (multiple of 4)
