@@ -282,6 +282,20 @@ int uwip_jpeg_encode_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int width, in
 /* JPEG in -> histretch -> aclahe -> bgdehaze on the device -> JPEG out */
 int uwip_chain_jpeg(uwip_ctx* ctx, const uint8_t* jpeg_in, size_t len_in, const uwip_chain_params* p,
                     int quality, uint8_t* jpeg_out, size_t cap, size_t* len_out);
+/* Batched encoder whose files are byte-identical to cv2.imwrite / cv2.imencode(".jpg", frame, [IMWRITE_JPEG_QUALITY, quality])
+ * with libjpeg-turbo: baseline JFIF, 4:2:0, the standard quantisation tables scaled by quality and the standard Huffman tables;
+ * no restart markers, no optimised Huffman tables, not progressive (csrc/jpegenc.h restates the arithmetic).  This is the
+ * writer of the reference's command lines (histretch.cpp:268, bgdehaze/main.py:19), so device output can be compared with
+ * reference files byte for byte; the nvJPEG entry points above write other bytes.
+ * uwip_jpeg_encode_bound: the largest file a width x height frame can produce (every coefficient coded with the longest code,
+ * every scan byte stuffed), 0 for sizes outside 1..65535.  libjpeg itself refuses sizes above 65500. */
+size_t uwip_jpeg_encode_bound(int width, int height);
+/* n_frames contiguous bgr8 device frames -> frame f's file at d_out + f * out_stride (device memory, out_stride >=
+ * uwip_jpeg_encode_bound(width, height); the slot is also the encoder's scratch) and its length in d_len[f] (device
+ * uint64).  Refuses out_stride below the bound, quality outside 1..100 and sizes outside 1..65535 (UWIP_ERR_INVALID).
+ * A frame's bytes do not depend on the batch it is in.  Stream ordered, does not synchronise. */
+int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_frames, int width, int height, int quality,
+                                    uint8_t* d_out, size_t out_stride, uint64_t* d_len);
 
 /* ---- synthetic input + checksums (SURVEY 8d) ------------------------------------------------- */
 /* frames first_frame .. first_frame+n_frames-1 of the integer-only generator (twin of

@@ -316,6 +316,47 @@ class Context:
         self._ck(self.lib.uwip_chain_jpeg(self.h, _ptr(buf), buf.size, C.byref(p), int(quality), _ptr(out), cap, C.byref(n)))
         return out[: n.value].tobytes()
 
+    # ---- JPEG files byte-identical to cv2.imwrite (csrc/jpegenc.cu) ---------------------------------------------
+    def jpeg_encode_bound(self, width, height):
+        """Largest file uwip_jpeg_encode_bgr8_batch_dev can write for one width x height frame (0 outside 1..65535)."""
+        return int(self.lib.uwip_jpeg_encode_bound(int(width), int(height)))
+
+    def jpeg_encode_batch_dev(self, d_frames, quality=95):
+        """Device bgr8 frames (torch uint8 tensor (N, H, W, 3) or (H, W, 3)) -> list of N files, each the bytes of
+        cv2.imencode(".jpg", frame, [cv2.IMWRITE_JPEG_QUALITY, quality]).  The batch is encoded in one device call; then the
+        lengths are read and only each file's bytes are copied to the host."""
+        import torch
+
+        d = d_frames.unsqueeze(0) if d_frames.dim() == 3 else d_frames
+        if d.dtype != torch.uint8 or d.dim() != 4 or d.shape[3] != 3 or not d.is_cuda:
+            raise ValueError("expected a uint8 CUDA tensor (N, H, W, 3)")
+        n, h, w = d.shape[:3]
+        stride = self.jpeg_encode_bound(w, h)
+        with torch.cuda.device(d.device):
+            d = d.contiguous()
+            d_out = torch.empty((n, max(stride, 1)), dtype=torch.uint8, device=d.device)
+            d_len = torch.empty(n, dtype=torch.int64, device=d.device)
+            torch.cuda.current_stream().synchronize()   # the frames are complete before the context's stream reads them
+            self._ck(self.lib.uwip_jpeg_encode_bgr8_batch_dev(self.h, _ptr(d), n, w, h, int(quality), _ptr(d_out), stride, _ptr(d_len)))
+            self.synchronize()
+            lens = d_len.cpu().tolist()
+            return [d_out[f, :lens[f]].cpu().numpy().tobytes() for f in range(n)]
+
+    def jpeg_encode(self, frames, quality=95):
+        """Host bgr8 frames (N, H, W, 3) -> list of N files; one frame (H, W, 3) -> its file.  The bytes are those of
+        cv2.imencode(".jpg", frame, [cv2.IMWRITE_JPEG_QUALITY, quality]), encoded on the device."""
+        import torch
+
+        a = np.asarray(frames)
+        single = a.ndim == 3
+        if single:
+            a = a[None]
+        if a.dtype != np.uint8 or a.ndim != 4 or a.shape[3] != 3:
+            raise ValueError("expected uint8 (N, H, W, 3)")
+        with torch.cuda.device(self.device):
+            out = self.jpeg_encode_batch_dev(torch.from_numpy(np.ascontiguousarray(a)).to("cuda"), quality)
+        return out[0] if single else out
+
     def last_frame_flags(self, n):
         """Per-frame status bits of the last batched chain / bgdehaze / automatic-aclahe call: 1 = the reference output is NaN
         (D9), 2 = the automatic CLAHE fit failed (BS = CL = -1, fixed parameters used)."""

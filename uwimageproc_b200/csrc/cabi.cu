@@ -848,6 +848,20 @@ int uwip_chain_jpeg(uwip_ctx* ctx, const uint8_t* jpeg_in, size_t len_in, const 
   return jpeg_encode_dev(ctx, d_out, w, h, quality, jpeg_out, cap, len_out);
 }
 
+size_t uwip_jpeg_encode_bound(int width, int height) {
+  if (width < 1 || width > 65535 || height < 1 || height > 65535) return 0;
+  return jpeg_encode_bound(width, height);
+}
+int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_frames, int width, int height, int quality, uint8_t* d_out,
+                                    size_t out_stride, uint64_t* d_len) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, d_bgr && d_out && d_len && n_frames > 0, "bad argument");
+  UWIP_REQUIRE(ctx, width >= 1 && width <= 65535 && height >= 1 && height <= 65535, "width and height must lie in 1..65535");
+  UWIP_REQUIRE(ctx, quality >= 1 && quality <= 100, "quality must lie in 1..100");
+  UWIP_REQUIRE(ctx, out_stride >= jpeg_encode_bound(width, height), "out_stride is below uwip_jpeg_encode_bound(width, height)");
+  return jpeg_encode_batch_dev(ctx, d_bgr, n_frames, width, height, quality, d_out, out_stride, d_len);
+}
+
 int uwip_last_frame_flags(uwip_ctx* ctx, int n, int32_t* flags_host) {
   CTX_GUARD(ctx);
   UWIP_REQUIRE(ctx, flags_host && n > 0, "bad argument");

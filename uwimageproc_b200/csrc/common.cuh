@@ -87,6 +87,7 @@ enum Slot {
   SLOT_ABLUR,         // automatic CLAHE: blurred planes (u8)
   SLOT_AUTO,          // automatic CLAHE: clip-curve derivatives, per-frame parameters, pick histograms and entropies
   SLOT_AUTO_BSCL,     // automatic CLAHE: BS, CL of the frames when the caller does not ask for them (int32 x2)
+  SLOT_JPEGENC,       // batched JPEG encoder: tables, MCU bit offsets, block infos, int16 coefficients
 };
 
 const char* uwip_set_err(uwip_ctx* ctx, const char* fmt, ...);
@@ -404,6 +405,11 @@ int jpeg_info(uwip_ctx* ctx, const uint8_t* data, size_t len, int* w, int* h);
 int jpeg_decode_dev(uwip_ctx* ctx, const uint8_t* data, size_t len, uint8_t* d_bgr, int w, int h);
 int jpeg_encode_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int w, int h, int quality, uint8_t* out, size_t cap, size_t* out_len);
 void jpeg_io_destroy(uwip_ctx* ctx);
+
+// jpegenc.cu
+size_t jpeg_encode_bound(int w, int h);
+int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
+                          uint64_t* d_len);
 
 // synth.cu
 int synth_frames_dev(uwip_ctx* ctx, uint8_t* d_dst, uint32_t seed, int first, int n, int w, int h);
