@@ -104,11 +104,10 @@ def load():
     global _lib
     if _lib is not None:
         return _lib
-    path = os.environ.get("UWIP_LIB") or LIB_PATH   # UWIP_LIB: a build variant under test (scratch/variants.py)
-    if not os.path.exists(path):
+    if not os.path.exists(LIB_PATH):
         raise UwipError(-2, "libuwip.so is not built: run `python -c 'import __graft_entry__ as g; g.build()'` "
                             "(nvcc, sm_100a).  There is no CPU fallback.")
-    lib = C.CDLL(path)
+    lib = C.CDLL(LIB_PATH)
     for name, (res, args) in SIGNATURES.items():
         fn = getattr(lib, name)  # AttributeError if the symbol is missing
         fn.restype = res

@@ -44,7 +44,7 @@ struct uwip_ctx {
   size_t func_smem[kFuncs] = {};
 };
 
-enum FuncId { FUNC_GF1A = 0, FUNC_GF1B, FUNC_GF2A, FUNC_GF2B, FUNC_WINDOW, FUNC_WINDOW15, FUNC_SWEEP, FUNC_SWEEP_BATCH, FUNC_GFQ };
+enum FuncId { FUNC_GF1A = 0, FUNC_GF1B, FUNC_GF2A, FUNC_GF2B, FUNC_WINDOW, FUNC_WINDOW15, FUNC_SWEEP, FUNC_GFQ };
 
 // grant `bytes` of dynamic shared memory to `kern` on the context's device (once per context and size)
 template <class K>
@@ -66,7 +66,7 @@ enum Slot {
   SLOT_TMP_FRAME,     // intermediate bgr8 frames
   SLOT_MPLANES,       // dehaze: window-min plane of green (u8)
   SLOT_PARTIALS,      // dehaze: per-block arg-min partials
-  SLOT_AB,            // dehaze: guided-filter coefficient planes (f32 x8)
+  SLOT_AB,            // dehaze: guided-filter coefficient planes (int32 fixed point x8)
   SLOT_J,             // dehaze: J_blue, J_green (f32 x2)
   SLOT_REFS,          // dehaze: refined exposure map (f32)
   SLOT_F64OUT,        // float64 outputs for the stage-wise host API
@@ -79,8 +79,8 @@ enum Slot {
   SLOT_FLAGS,         // per-frame status words of the last chain / dehaze call (int32)
   SLOT_KQ,            // dehaze: packed k'_b k'_g k'_r m'_b (u32)
   SLOT_YCC,           // dehaze: packed Yi Cri Cbi Yj (u32)
-  SLOT_STAB,          // dehaze: exposure-ratio table (f64 x 65536 per frame)
-  SLOT_SPLANE,        // dehaze: exposure ratio per pixel (f32)
+  SLOT_STAB,          // dehaze: exposure-ratio table (u32 rint(S 2^28) x 65536 per frame)
+  SLOT_SPLANE,        // dehaze: exposure ratio per pixel (u32 rint(S 2^28))
   SLOT_BLURSUMS,      // calcBlur: per-frame sum and sum of squares of the 8-bit Laplacian (u64 x2)
   SLOT_BLUROUT,       // calcBlur: per-frame mean, stdev (f64 x2)
   SLOT_APLANE,        // automatic CLAHE: V planes of the frames (u8)
@@ -350,13 +350,6 @@ __device__ __forceinline__ unsigned int warp_reduce_max_u32(unsigned int v) {
 // ------------------------------------------------------------------------------------------------
 // stage entry points implemented in the other translation units (device pointers, stream ordered)
 // ------------------------------------------------------------------------------------------------
-struct ChainCfg {
-  int lo, hi, order, hsv_round;
-  double clip;
-  int tiles_x, tiles_y;
-  uwip_dehaze_params dz;
-};
-
 // histretch.cu
 int k_histogram_plane(uwip_ctx* ctx, const uint8_t* d_plane, int n_planes, size_t n_px, uint32_t* d_hist);
 int calc_blur_frames_dev(uwip_ctx* ctx, const uint8_t* d_src, int n, int w, int h, int aperture, double* d_mean_std, uint8_t* d_lap);

@@ -6,23 +6,17 @@
 // Data flow per frame (all frame-global reductions land in FrameState, no host round trips):
 //   minmax (D0)  ->  window: 15x15 window max / arg-min partials (D1), window min (D2), and the packed
 //                    plane kq = (k'_b, k'_g, k'_r, m'_b) + plane m'_g that every later pass reads
-//   -> GF1a: box sums of 17 moments + per-pixel 3x3 solve -> a,b planes (f32 x8)
+//   -> GF1a: box sums of 17 moments + per-pixel 3x3 solve -> a,b planes (int32 fixed point x8)
 //   -> GF1b: box(a,b) -> refined t (D3,D5) -> J (D6) + min/max/sum reductions -> J planes (f32 x2)
 //   -> E: restored -> R8/I8 -> YCrCb joint min/max (D7,D8 first half); packed plane ycc = (Yi,Cri,Cbi,Yj)
-//   -> S table (256x256 u32 per frame: the exposure ratio is a function of two bytes; rint(S 2^28))
-//   -> GF2a: S + 13 moments + solve -> a,b (f32 x4)   -> GF2b: box(a,b) -> refined S, exposure min/max
+//   -> S table (256x256 u32 per frame: the exposure ratio is a function of two bytes; rint(S 2^28)) -> S plane (u32)
+//   -> GF2a: S + 13 moments + solve -> a,b (int32 fixed point x4)   -> GF2b: box(a,b) -> refined S, exposure min/max
 //   -> final: normalise, x255, rint, saturate -> bgr8 (D8 second half, D10)
 //
-// Box sums ("quad march").  A CTA owns a strip of image columns (halo of r columns on both sides) and
-// walks down the rows.  Every thread owns FOUR adjacent columns: the vertical running sums of all
-// moments stay in registers (add the entering row, subtract the leaving row).  For every output row a
-// thread publishes the inclusive prefix over its own quad (one 16-byte shared store per moment) and
-// the quad total; a few threads turn the quad totals into a prefix over the strip; the window sum of
-// column 4t+c is then  G[t+r/4-1] - G[t-r/4-1] - quad[t-r/4][c-1] + quad[t+r/4][c]  (two 16-byte and
-// two 4-byte shared loads per moment for four pixels).  Guide moments are exact 32-bit integers (the
-// guide is k/range with k uint8); everything involving the filtered signal accumulates in fp64.  The
-// per-pixel solve works in "k units" (guide not divided by range) with eps_k = eps*range^2 on the
-// exact integer numerators N*S_ij - S_i*S_j.
+// The four GF passes are the guided-filter marches of gfpipe.cuh: per strip of columns, ACC threads keep the vertical
+// running sums of a quad of columns, AUX warps form the prefixes over the strip, SOLVE threads take the window sums of two
+// pixels and do the per-pixel work.  The solve works in "k units" (guide not divided by range) with eps_k = eps*range^2 on
+// the exact integer numerators N*S_ij - S_i*S_j.  Details and measurements: DESIGN.md section 3.
 #include <algorithm>
 
 #include "common.cuh"
@@ -531,10 +525,8 @@ __global__ void traw_kernel(const uint32_t* __restrict__ kq, const uint8_t* __re
 // -------------------------------------------------------------------------------------------------
 // E: restored -> R8, I8 -> YCrCb joint min / max (BGDehaze.py:75-80); stores (Yi, Cri, Cbi, Yj)
 // -------------------------------------------------------------------------------------------------
-#ifndef DZ_EW_CTAS
-#define DZ_EW_CTAS 4   // resident CTAs per SM of the two element-wise fp64 kernels
-#endif
-__global__ void __launch_bounds__(256, DZ_EW_CTAS) exposure_minmax_kernel(GfCommon g, int W, int H, int Wp, double* dbg_restored) {
+constexpr int DZ_ELEMENTWISE_CTAS = 4;   // resident CTAs per SM of the two element-wise fp64 kernels
+__global__ void __launch_bounds__(256, DZ_ELEMENTWISE_CTAS) exposure_minmax_kernel(GfCommon g, int W, int H, int Wp, double* dbg_restored) {
   __shared__ ExpShared sh;
   int f = blockIdx.y;
   size_t n_pp = (size_t)Wp * H;
@@ -595,8 +587,8 @@ __global__ void __launch_bounds__(256) stab_kernel(const FrameState* __restrict_
   stab[(size_t)f * 65536 + gy * 256 + j] = (S == S) ? __double2uint_rn(fmin(S, GP_S_PMAX) * GP_PSCALE) : GP_S_NAN;
 }
 
-// S per pixel as an f32 plane: GF2a then reads it through the same staged row copies as the guide instead
-// of gathering from the table inside the march (f32 keeps 2^-24 relative: far inside the 1e-5 budget).
+// S per pixel as a plane of the table's entries, rint(min(S, 1.6) 2^28) (0 where S is 0/0): GF2a then reads it through the
+// same staged row copies as the guide instead of gathering from the table inside the march.
 __global__ void __launch_bounds__(256) splane_kernel(GfCommon g, int H, int Wp) {
   int f = blockIdx.y;
   size_t n_pp = (size_t)Wp * H;
@@ -605,7 +597,7 @@ __global__ void __launch_bounds__(256) splane_kernel(GfCommon g, int H, int Wp) 
   const uint32_t ysub = a | (a << 8) | (a << 16) | (b << 24);
   const uint32_t* ycc = g.ycc + (size_t)f * n_pp;
   const uint32_t* stab = g.stab + (size_t)f * 65536;
-  uint32_t* sp = reinterpret_cast<uint32_t*>(g.splane) + (size_t)f * n_pp;
+  uint32_t* sp = g.splane + (size_t)f * n_pp;
   const size_t n_q = n_pp / 4;
   bool nan_seen = false;
   for (size_t qi = (size_t)blockIdx.x * 256 + threadIdx.x; qi < n_q; qi += (size_t)gridDim.x * 256) {
@@ -628,7 +620,7 @@ __global__ void __launch_bounds__(256) splane_kernel(GfCommon g, int H, int Wp) 
 }
 
 // final: (OutputExp - min)/(max - min) * 255 -> rint -> saturate (BGDehaze.py:88-89, main.py:19)
-__global__ void __launch_bounds__(256, DZ_EW_CTAS) final_kernel(GfCommon g, int W, int H, int Wp, uint8_t* __restrict__ dst, double* dbg_out, int32_t* __restrict__ flags) {
+__global__ void __launch_bounds__(256, DZ_ELEMENTWISE_CTAS) final_kernel(GfCommon g, int W, int H, int Wp, uint8_t* __restrict__ dst, double* dbg_out, int32_t* __restrict__ flags) {
   __shared__ ExpShared sh;
   int f = blockIdx.y;
   size_t n_pp = (size_t)Wp * H;
@@ -736,12 +728,12 @@ int dehaze_frames_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n
   uint8_t* d_mg = (uint8_t*)uwip_slot(ctx, SLOT_MPLANES, (size_t)n * n_pp);
   uint32_t* d_ycc = (uint32_t*)uwip_slot(ctx, SLOT_YCC, (size_t)n * n_pp * 4);
   uint32_t* d_stab = (uint32_t*)uwip_slot(ctx, SLOT_STAB, (size_t)n * 65536 * 4);
-  float* d_sp = (float*)uwip_slot(ctx, SLOT_SPLANE, (size_t)n * n_pp * sizeof(float));
+  uint32_t* d_sp = (uint32_t*)uwip_slot(ctx, SLOT_SPLANE, (size_t)n * n_pp * sizeof(uint32_t));
   dim3 gridw(cdiv(Wp, WK_TX), cdiv(H, WK_TY), n);    // generic-window kernel
   dim3 gridf(cdiv(Wp, WF_TX), cdiv(H, WF_TY), n);    // 15x15 kernel
   int n_part = gridw.x * gridw.y, n_partf = gridf.x * gridf.y;
   ArgPartial* d_part = (ArgPartial*)uwip_slot(ctx, SLOT_PARTIALS, (size_t)n * std::max(n_part, n_partf) * sizeof(ArgPartial));
-  float* d_ab = (float*)uwip_slot(ctx, SLOT_AB, (size_t)n * 8 * n_pp * sizeof(float));
+  int32_t* d_ab = (int32_t*)uwip_slot(ctx, SLOT_AB, (size_t)n * 8 * n_pp * sizeof(int32_t));
   float* d_J = (float*)uwip_slot(ctx, SLOT_J, (size_t)n * 2 * n_pp * sizeof(float));
   float* d_refS = (float*)uwip_slot(ctx, SLOT_REFS, (size_t)n * n_pp * sizeof(float));
   if (!d_kq || !d_mg || !d_ycc || !d_stab || !d_sp || !d_part || !d_ab || !d_J || !d_refS) return UWIP_ERR_NOMEM;
@@ -849,13 +841,13 @@ int guided_filter_u8_dev(uwip_ctx* ctx, const uint8_t* d_guide, const double* d_
   const int Wp = (W + 3) & ~3;
   const size_t n_pp = (size_t)Wp * H;
   uint32_t* d_ycc = (uint32_t*)uwip_slot(ctx, SLOT_YCC, n_pp * 4);
-  float* d_sp = (float*)uwip_slot(ctx, SLOT_SPLANE, n_pp * 4);
-  float* d_ab = (float*)uwip_slot(ctx, SLOT_AB, 8 * n_pp * 4);
+  uint32_t* d_sp = (uint32_t*)uwip_slot(ctx, SLOT_SPLANE, n_pp * 4);
+  int32_t* d_ab = (int32_t*)uwip_slot(ctx, SLOT_AB, 8 * n_pp * 4);
   if (!d_ycc || !d_sp || !d_ab) return UWIP_ERR_NOMEM;
   UWIP_CHECK(frame_state_reset(ctx, fs, 1));
   UWIP_LAUNCH(ctx, "gfq_state", gfq_state_kernel, 1, 1, 0, fs, range);
   dim3 grid(cdiv(Wp, 256), H);
-  UWIP_LAUNCH(ctx, "gfq_pack", gfq_pack_kernel, grid, 256, 0, d_guide, d_p, W, H, Wp, d_ycc, reinterpret_cast<uint32_t*>(d_sp), fs);
+  UWIP_LAUNCH(ctx, "gfq_pack", gfq_pack_kernel, grid, 256, 0, d_guide, d_p, W, H, Wp, d_ycc, d_sp, fs);
   GfCommon gc;
   memset(&gc, 0, sizeof(gc));
   gc.ycc = d_ycc; gc.splane = d_sp; gc.ab = d_ab; gc.fs = fs; gc.eps = eps; gc.tmin = 0.0; gc.dbg_tref = d_q;
@@ -863,9 +855,3 @@ int guided_filter_u8_dev(uwip_ctx* ctx, const uint8_t* d_guide, const double* d_
   UWIP_CHECK(gp_launch<PipGFq>(ctx, "gfq_out", FUNC_GFQ, gc, 1, W, H, r));
   return UWIP_OK;
 }
-
-#if GP_TRACE
-extern "C" int uwip_exp_trace(long long* out) {   // timing-experiment builds only (scratch/variants.py)
-  return (int)cudaMemcpyFromSymbol(out, gp_trace_buf, sizeof(gp_trace_buf));
-}
-#endif

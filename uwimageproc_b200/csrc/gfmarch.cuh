@@ -23,16 +23,6 @@ __device__ __forceinline__ double rcp_fast(double x) {
   return r;
 }
 
-// Round to a multiple of 2^-G (round-half-even) by the add/subtract of 1.5*2^(52-G); valid for |x| < 2^(51-G).
-// Every value that enters a running sum is put on such a grid: the vertical running sums (add the entering
-// row, subtract the leaving row) are then EXACT in fp64, so the result of a frame does not depend on where a
-// CTA's vertical segment starts - i.e. not on the batch size, the sub-batch split or the GPU count.
-template <int G>
-__device__ __forceinline__ double grid_round(double x) {
-  const double M = 6755399441055744.0 / (double)(1ull << G);  // 1.5 * 2^(52-G)
-  return (x + M) - M;
-}
-
 // cp.async (LDGSTS): global -> shared without a register in between
 __device__ __forceinline__ void cp_async16(void* smem, const void* g) {
   unsigned a = (unsigned)__cvta_generic_to_shared(smem);
@@ -48,7 +38,7 @@ __device__ __forceinline__ void cp_async4(void* smem, const void* g) {
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-// TMA 1-D bulk copy global -> shared, completion counted in bytes on an mbarrier (SASS: UBLKCP)
+// mbarriers (the TMA bulk copies of gfpipe.cuh count their completion in bytes on them)
 __device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) {
   unsigned a = (unsigned)__cvta_generic_to_shared(bar);
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(a), "r"(count) : "memory");
@@ -57,27 +47,12 @@ __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, unsigned by
   unsigned a = (unsigned)__cvta_generic_to_shared(bar);
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(a), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-  unsigned a = (unsigned)__cvta_generic_to_shared(bar);
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "WAIT_%=:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra DONE_%=;\n\t"
-      "bra WAIT_%=;\n\t"
-      "DONE_%=:\n\t}" ::"r"(a), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_bulk_g2s(void* smem, const void* g, unsigned bytes, uint64_t* bar) {
-  unsigned d = (unsigned)__cvta_generic_to_shared(smem), b = (unsigned)__cvta_generic_to_shared(bar);
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(d), "l"(g), "r"(bytes), "r"(b) : "memory");
-}
 
 // ------------------------------------------------------------------------------------------------
 // guided-filter helpers
 // ------------------------------------------------------------------------------------------------
-// 3x3 symmetric solve shared by GF1a / GF2a.  Inputs are window sums in k units:
-//   S[3] (sum k_i), SS[6] (sum k_i k_j: 00 01 02 11 12 22), N (window pixel count),
-//   Sp (sum p), Sip[3] (sum k_i p).  Output a[3] (k units) and b.
+// 3x3 symmetric system shared by GF1a / GF2a (gfpipe.cuh: gp_solve_rhs solves it for each signal).  Inputs are window sums
+// in k units: si[0..2] (sum k_i), si[3..8] (sum k_i k_j: 00 01 02 11 12 22), N (window pixel count).
 __device__ __forceinline__ void gf_build_M(const uint32_t* si, double N, double epsN2, double* M, double* Sd) {
   Sd[0] = u2d(si[0]); Sd[1] = u2d(si[1]); Sd[2] = u2d(si[2]);
   // exact: N*S_ij and S_i*S_j are integers < 2^53
@@ -99,28 +74,14 @@ __device__ __forceinline__ void gf_adjugate(const double* M, double* A, double& 
   double det = M[0] * A[0] + M[1] * A[1] + M[2] * A[2];
   rdet = rcp_fast(det);
 }
-__device__ __forceinline__ void gf_solve(const double* A, double rdet, const double* Sd, double N, double invN, double Sp,
-                                         const double* Sip, double* a, double& b) {
-  // C_i = N*S_ip - S_i*S_p  (= N^2 cov_k);  a_k = C * adj(M) / det(M)
-  double C0 = fma(N, Sip[0], -Sd[0] * Sp), C1 = fma(N, Sip[1], -Sd[1] * Sp), C2 = fma(N, Sip[2], -Sd[2] * Sp);
-  a[0] = (C0 * A[0] + C1 * A[1] + C2 * A[2]) * rdet;
-  a[1] = (C0 * A[1] + C1 * A[3] + C2 * A[4]) * rdet;
-  a[2] = (C0 * A[2] + C1 * A[4] + C2 * A[5]) * rdet;
-  b = (Sp - a[0] * Sd[0] - a[1] * Sd[1] - a[2] * Sd[2]) * invN;
-}
-
-// one coefficient chunk (a0, a1, a2, b) as stored: on the 2^-34 grid (absolute step 6e-11), then f32
-__device__ __forceinline__ float4 coef_pack(const double* a, double b) {
-  return make_float4((float)grid_round<34>(a[0]), (float)grid_round<34>(a[1]), (float)grid_round<34>(a[2]), (float)grid_round<34>(b));
-}
 
 struct GfCommon {
   const uint32_t* kq;     // [n][H][Wp] packed k'_b k'_g k'_r m'_b
   const uint8_t* mg;      // [n][H][Wp] m'_g
   uint32_t* ycc;          // [n][H][Wp] packed Yi Cri Cbi Yj
   const uint32_t* stab;   // [n][256][256] exposure ratio S(yi', yj') as rint(S 2^28), 0xffffffff where S is 0/0
-  float* splane;          // [n][H][Wp] S per pixel (f32)
-  float* ab;              // [n][8][H][Wp]
+  uint32_t* splane;       // [n][H][Wp] S per pixel as rint(S 2^28)
+  int32_t* ab;            // [n][8][H][Wp] coefficient rows, int32 fixed point (gfpipe.cuh: coef_scale)
   float* J;               // [n][2][H][Wp]
   float* refS;            // [n][H][Wp]
   FrameState* fs;
@@ -225,16 +186,6 @@ __device__ __forceinline__ int restored_byte(float j, const FrameConst& fc, int 
   return trunc_u8(v);
 }
 
-__device__ __forceinline__ unsigned long long warp_min_u64(unsigned long long v) {
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) { unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d); v = o < v ? o : v; }
-  return v;
-}
-__device__ __forceinline__ unsigned long long warp_max_u64(unsigned long long v) {
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) { unsigned long long o = __shfl_xor_sync(0xffffffffu, v, d); v = o > v ? o : v; }
-  return v;
-}
 __device__ __forceinline__ long long warp_sum_i64(long long v) {
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
@@ -248,11 +199,6 @@ __device__ __forceinline__ float warp_min_f32(float v) {
 __device__ __forceinline__ float warp_max_f32(float v) {
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, d));
-  return v;
-}
-__device__ __forceinline__ double warp_sum_f64(double v) {
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
   return v;
 }
 __device__ __forceinline__ double warp_min_f64(double v) {
@@ -284,10 +230,6 @@ __device__ __forceinline__ int coef_chunk(int gq, int c, int j) {  // physical c
 // -------------------------------------------------------------------------------------------------
 // the guided-filter marches: warp-specialised pipeline (gfpipe.cuh)
 // -------------------------------------------------------------------------------------------------
-// coefficient rows: int32 fixed point (gfpipe.cuh: coef_scale)
-#define GP_COEF_T int
-#define GP_COEF_V4 int4
-#define GP_COEF_PACK(a, b, cs) coef_pack_fix(a, b, (cs).sa, (cs).sb)
 #include "gfpipe.cuh"
 
 // geometry + launch -------------------------------------------------------------------------------------

@@ -1,110 +1,51 @@
-// gfpipe.cuh - the guided-filter box sums of bgdehaze as a warp-specialised pipeline (included by dehaze.cu).
+// gfpipe.cuh - the guided-filter box sums of bgdehaze as a warp-specialised pipeline (included by gfmarch.cuh).
 //   reference: modules/bgdehaze/guidedfilter.py:23-103 (boxfilter, guided_filter), BGDehaze.py:39-48,84.
 //
-// One CTA (512 threads, one per SM) owns a strip of up to 512 image columns (plus a halo of r columns on both sides)
-// and walks down the rows.  Three roles run concurrently and hand rows to each other through mbarriers over a ring of
-// published rows in shared memory (P::NSTAGE stages); there is no CTA-wide barrier in the march:
-//
-//   ACC   (warps 8-12, 160 threads): thread t owns the FOUR adjacent columns of quad t.  The vertical running sums of
-//         every moment stay in registers as INTEGERS (add the entering row, subtract the leaving row): the guide
-//         moments are 32-bit (guide = k/range, k uint8), everything that involves the filtered signal is a 64-bit sum
-//         of 32 x 32 bit products (the signal sits on a 2^-28 grid, the stored coefficients are int32 fixed point), so
-//         the sums are exact and a frame's bytes do not depend on where a vertical segment starts.  Per output row the
-//         thread publishes the inclusive prefix over its quad and the quad total (64-bit moments as exact doubles).
-//   AUX   (warps 13-15): turn the quad totals of a published row into prefixes over the strip (serial in-register
-//         scan of 20-quad segments, shuffle exchange of the segment totals; the moments are dealt out over the three
-//         warps); lane 0 of the first one is the TMA producer of the coefficient rows of the plane readers (one bulk
-//         copy per row into a two-slot ring).
-//   SOLVE (warps 0-7, 256 threads): thread v owns TWO adjacent output pixels.  Window sum of column 4t+c =
-//         G[t+r/4-1] - G[t-r/4-1] - quad[t-r/4][c-1] + quad[t+r/4][c]; the stage is released as soon as the sums are in
-//         registers; then the per-pixel work of the policy (3x3 solve in fp64 / the filter output and its reductions).
-//
-// Register budgets differ per role (setmaxnreg): the kernel starts with 128 registers for every thread, the two
-// warpgroups of a role grow / shrink to P::ACC_REGS and P::SOLVE_REGS (sum 256).  Warp order = issue priority (the
-// scheduler prefers the highest warp id): consumers first, producers after them, the auxiliary warps last.
+// One CTA (one per SM) owns a strip of image columns plus a halo of r columns on both sides and walks down the rows.  Three
+// roles hand rows to each other through mbarriers over a ring of published rows in shared memory (P::NSTAGE stages):
+//   ACC   one thread per quad of four columns keeps the vertical running sums of every moment in registers (32-bit integers
+//         for the guide moments, integer-valued doubles for the signal moments: exact) and publishes per output row the
+//         inclusive prefix over its quad and the quad total.
+//   AUX   turns the quad totals of a published row into prefixes over the strip; lane 0 of the first auxiliary warp is the
+//         TMA producer of the coefficient rows of the plane readers.
+//   SOLVE one thread per two adjacent output pixels forms their window sums from the published row, then does the per-pixel
+//         work of the policy (3x3 solve / the filter output and its reductions).
+// Warp order is issue priority (the scheduler prefers the highest warp id): SOLVE first, then ACC, the auxiliary warps last.
+// The two strip layouts, the register budgets per role and the measurements behind them: DESIGN.md section 3.
 #pragma once
 
-// tuning switches (scratch/variants.py builds and times the alternatives on the GPU)
-#ifndef GP_PARK
-#define GP_PARK 1          // mbarrier waits carry a suspend-time hint
-#endif
-#ifndef GP_EXP_SKIP_SOLVE
-#define GP_EXP_SKIP_SOLVE 0   // timing experiment: SOLVE loads its window sums but skips the per-pixel work
-#endif
-#ifndef GP_EXP_SKIP_ACC
-#define GP_EXP_SKIP_ACC 0     // timing experiment: ACC skips the accumulate (publishes stale sums)
-#endif
-#ifndef GP_L2_HINT
-#define GP_L2_HINT 1            // plane readers: entering coefficient rows evict_last (fraction GP_L2_FRAC), leaving rows evict_first
-#endif
-#ifndef GP_L2_FRAC_GF1B
-#define GP_L2_FRAC_GF1B 0.5f    // 81 rows x 148 strips of GF1b are 216 MB: keep half of it resident in the 126 MB L2
-#endif
-#ifndef GP_L2_FRAC_GF2B
-#define GP_L2_FRAC_GF2B 1.0f    // GF2b: 108 MB
-#endif
-#ifndef GP_EXP_SKIP_SCAN
-#define GP_EXP_SKIP_SCAN 0      // timing experiments on the skeleton (wrong results): AUX does not scan
-#endif
-#ifndef GP_EXP_SKIP_WINDOW
-#define GP_EXP_SKIP_WINDOW 0    // SOLVE does not read its window sums
-#endif
-#ifndef GP_EXP_SKIP_PUBLISH
-#define GP_EXP_SKIP_PUBLISH 0   // ACC does not store the published row
-#endif
-#ifndef GP_EXP_SKIP_TMA
-#define GP_EXP_SKIP_TMA 0       // plane readers: no TMA copies (the ring barriers are still cycled)
-#endif
-#ifndef GP_TRACE
-#define GP_TRACE 0              // timing experiment: clock stamps of the three roles for 64 rows of CTA (0,0,0)
-#endif
 #ifndef GP_NARROW
 #define GP_NARROW 0             // 1: strips of 128 quads - four ACC warps in one warpgroup, four auxiliary warps in another with their own (small) register count
 #endif
-#ifndef GP_AUX_REGS
-#define GP_AUX_REGS 88          // GP_NARROW: registers of an auxiliary thread
-#endif
-#ifndef GP_GF1A_ACC_REGS
-#define GP_GF1A_ACC_REGS (GP_NARROW ? 176 : GP_NGRP_SEL == 1 ? 152 : 96)
-#endif
-#ifndef GP_GF2A_ACC_REGS
-#define GP_GF2A_ACC_REGS (GP_NARROW ? 168 : GP_NGRP_SEL == 1 ? 144 : 96)
-#endif
-#ifndef GP_B_ACC_REGS
-#define GP_B_ACC_REGS (GP_NARROW ? 128 : GP_NGRP_SEL == 1 ? 136 : 80)
-#endif
+constexpr int GP_AUX_REGS = 88;   // GP_NARROW: registers of an auxiliary thread
+constexpr int GP_GF1A_ACC_REGS = GP_NARROW ? 176 : 152;
+constexpr int GP_GF2A_ACC_REGS = GP_NARROW ? 168 : 144;
+constexpr int GP_B_ACC_REGS = GP_NARROW ? 128 : 136;
 
-#ifndef GP_NGRP_SEL
-#define GP_NGRP_SEL 1                 // 2: two ACC threads per quad, each with half of the running sums (measured slower: r2_summary.md)
-#endif
-constexpr int GP_NT = GP_NARROW ? 128 : 160;   // quads of a strip (quad 0 is the zero guard) = ACC worker threads per moment group
+constexpr int GP_NT = GP_NARROW ? 128 : 160;   // quads of a strip (quad 0 is the zero guard) = ACC worker threads
 constexpr int GP_NTR = GP_NT < 152 ? GP_NT : 152;   // quads of a strip that can hold data (gf_geometry keeps NQ within it): the pitch of the TMA ring rows
-constexpr int GP_NGRP = GP_NGRP_SEL;  // ACC moment groups
-constexpr int GP_NAUX = GP_NARROW ? 4 : GP_NGRP == 1 ? 3 : 2;   // auxiliary warps
+constexpr int GP_NAUX = GP_NARROW ? 4 : 3;      // auxiliary warps
 constexpr int GP_SOLVE_THREADS = 256; // two warpgroups (threads 0..255)
-constexpr int GP_ACC_THREADS = GP_NGRP * GP_NT + 32 * GP_NAUX;   // 256 (two warpgroups) or 384 (three)
+constexpr int GP_ACC_THREADS = GP_NT + 32 * GP_NAUX;   // two warpgroups
 constexpr int GP_THREADS = GP_ACC_THREADS + GP_SOLVE_THREADS;
 constexpr int GP_MAXSW = 2 * GP_SOLVE_THREADS;   // output columns per strip
 constexpr int GP_NSEG = 8, GP_SEGQ = 20;         // scan: 8 lanes per moment, 20 quads per lane (5 x 16 bytes of u32: odd -> conflict-free)
 constexpr int GP_GP = GP_NSEG * GP_SEGQ;         // pitch of a quad-total row
 // fp64 quad-total rows: a scan segment of 20 doubles is ten 16-byte chunks - an even number, so the eight lanes of a moment
-// would start 2-way bank conflicted (segment stride 160 B = 8 banks x 5: lanes s and s + 4 share banks).  GP_DPAD doubles of
+// would start 2-way bank conflicted (segment stride 160 B = 8 banks x 5: lanes s and s + 4 share banks).  GP_SEG_PAD doubles of
 // padding after every segment make the stride an odd number of chunks: every 16-byte access of the scan is conflict-free.
-#ifndef GP_DPAD
-#define GP_DPAD 2
-#endif
-constexpr int GP_SEGD = GP_SEGQ + GP_DPAD;       // segment stride of an fp64 quad-total row
+constexpr int GP_SEG_PAD = 2;
+constexpr int GP_SEGD = GP_SEGQ + GP_SEG_PAD;    // segment stride of an fp64 quad-total row
 constexpr int GP_GPD = GP_NSEG * GP_SEGD;        // pitch of an fp64 quad-total row
-__device__ __forceinline__ int gp_dpos(int t) { return t + GP_DPAD * (t / GP_SEGQ); }   // position of quad t in such a row
-static_assert(GP_GP >= GP_NT && GP_NGRP * GP_NT + 32 * GP_NAUX == GP_ACC_THREADS, "thread layout");
+__device__ __forceinline__ int gp_dpos(int t) { return t + GP_SEG_PAD * (t / GP_SEGQ); }   // position of quad t in such a row
+static_assert(GP_GP >= GP_NT, "thread layout");
 
 // The filtered signal p (transmission, exposure ratio) is held as rint(p * 2^28): the guided filter amplifies a
 // perturbation of p by up to ~10^3 (a = cov / (var + eps) with eps = 10^-3): a 2^-25 grid already costs 1.7e-5.
 constexpr double GP_PSCALE = 268435456.0, GP_PINV = 1.0 / 268435456.0;
 constexpr double GP_T_PMAX = 1.0, GP_S_PMAX = 1.6;
 // registers left for a SOLVE thread when an ACC / AUX thread takes `acc` (pool = threads x launch registers), in units of 8
-#define GP_SOLVE_REGS_FOR(acc) \
-  (GP_NARROW ? ((((65536 - 128 * (acc) - 128 * GP_AUX_REGS) / 256) / 8) * 8) : GP_NGRP_SEL == 1 ? 256 - (acc) : ((((96 * 640 - 384 * (acc)) / 256) / 8) * 8))
+#define GP_SOLVE_REGS_FOR(acc) (GP_NARROW ? ((((65536 - 128 * (acc) - 128 * GP_AUX_REGS) / 256) / 8) * 8) : 256 - (acc))
 
 // wait for the phase with the given parity; the suspend-time hint lets the hardware park the warp until the phase
 // completes (or the time runs out) instead of re-issuing the test every few cycles
@@ -113,11 +54,7 @@ __device__ __forceinline__ void mbar_wait_park(uint64_t* bar, unsigned parity) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "WAIT_%=:\n\t"
-#if GP_PARK
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t"
-#else
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-#endif
       "@p bra DONE_%=;\n\t"
       "bra WAIT_%=;\n\t"
       "DONE_%=:\n\t}" ::"r"(a), "r"(parity), "r"(20000u) : "memory");
@@ -133,40 +70,15 @@ __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
   return p;
 }
+// TMA 1-D bulk copy global -> shared with an L2 cache policy, completion counted in bytes on an mbarrier (SASS: UBLKCP)
 __device__ __forceinline__ void tma_bulk_g2s_hint(void* smem, const void* g, unsigned bytes, uint64_t* bar, uint64_t policy) {
   unsigned d = (unsigned)__cvta_generic_to_shared(smem), b = (unsigned)__cvta_generic_to_shared(bar);
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(d), "l"(g),
                "r"(bytes), "r"(b), "l"(policy) : "memory");
 }
-#if GP_TRACE
-__device__ long long gp_trace_buf[4][64][12];  // [kernel][row][event]: ACC 0..2 + 8..10 (inside the accumulate), AUX 3..4, SOLVE 5..7
-#define GP_STAMP(P, row, ev)                                                                                 \
-  do {                                                                                                       \
-    if (blockIdx.x == 1 && blockIdx.y == 0 && blockIdx.z == 0 && (threadIdx.x & 31) == 0 && (row) >= 600 && (row) < 664) \
-      gp_trace_buf[P::TRACE_ID][(row) - 600][ev] = clock64();                                                \
-  } while (0)
-#else
-#define GP_STAMP(P, row, ev) do {} while (0)
-#endif
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   unsigned a = (unsigned)__cvta_generic_to_shared(bar);
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(a) : "memory");
-}
-
-// c + a * b with a signed 32 x 32 -> 64 bit product: ONE instruction (IMAD.WIDE) that accumulates in place.  Written in
-// PTX because the compiler turns `c += (long long)a * b` into an unsigned wide multiply plus sign fix-ups and moves.
-__device__ __forceinline__ long long mad_wide(int a, int b, long long c) {
-  long long d;
-  asm("mad.wide.s32 %0, %1, %2, %3;" : "=l"(d) : "r"(a), "r"(b), "l"(c));
-  return d;
-}
-
-// exact conversions of the 64-bit running sums (one integer add + one DADD)
-__device__ __forceinline__ double u64_to_double(unsigned long long v) {  // 0 <= v < 2^52
-  return __hiloint2double((int)((unsigned)(v >> 32) + 0x43300000u), (int)(unsigned)v) - 4503599627370496.0;
-}
-__device__ __forceinline__ double s64_to_double(long long v) {           // |v| < 2^51
-  return __hiloint2double((int)((unsigned)((unsigned long long)v >> 32) + 0x43380000u), (int)(unsigned)v) - 6755399441055744.0;
 }
 
 // coefficient planes: int32 fixed point (a0, a1, a2, b) per pixel and filter.  |a_k| <= std(p)/sqrt(eps_k)
@@ -298,19 +210,16 @@ __device__ __forceinline__ GpGeo gp_geo(const GfGeom& gg) {
 // ------------------------------------------------------------------------------------------------
 // ACC role
 // ------------------------------------------------------------------------------------------------
-// G = moment group of this thread: group 0 keeps the guide moments and the first P::NDA signal moments of its quad, group 1
-// the other signal moments (two threads per quad: half the running sums, half the work, twice the warps per row)
-template <class P, int G>
+template <class P>
 __device__ __forceinline__ void gp_acc_worker(const GfCommon& gc, const GfGeom& gg, unsigned char* smem) {
   constexpr int NI = P::NI, ND = P::ND, NT = GP_NT, GP = GP_GP, NSTAGE = P::NSTAGE;
   constexpr int NIa = NI > 0 ? NI : 1;
   typedef GpSmem<P> L;
   typedef typename P::Acc Acc;
-  typedef typename Acc::Sum Sum;   // unsigned long long (products of non-negative values) or long long
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::off_bar);
   unsigned char* stage_in = smem + L::off_in;
   const GpGeo g = gp_geo(gg);
-  const int t = threadIdx.x - GP_SOLVE_THREADS - (G == 1 ? GP_NT : 0);
+  const int t = threadIdx.x - GP_SOLVE_THREADS;
   const int gx = g.xs - g.HL - 4 + 4 * t;     // image column of this thread's quad (multiple of 4)
   const int tdp = gp_dpos(t);                 // position of its quad total in an fp64 quad-total row
   const bool qact = t < g.NQ;
@@ -324,7 +233,7 @@ __device__ __forceinline__ void gp_acc_worker(const GfCommon& gc, const GfGeom& 
   acc.init(gc, blockIdx.z, reinterpret_cast<typename P::Shared*>(smem + L::off_sh), gg);
 
   uint32_t Vi[4][NIa];
-  Sum Vl[4][ND];
+  double Vl[4][ND];
 #pragma unroll
   for (int c = 0; c < 4; c++) {
 #pragma unroll
@@ -335,19 +244,13 @@ __device__ __forceinline__ void gp_acc_worker(const GfCommon& gc, const GfGeom& 
   // first quad of this strip that lies inside the padded image (the TMA rows start there)
   const int tA = max(1, (g.HL + 4 - g.xs) >> 2);
 
-  // a-kernels, one thread per quad (G == 2): the raw quads of the next march row land in this thread's own shared-memory slots
-  // (cp.async, no register held meanwhile); two threads per quad: they are held in registers (no shared memory to spare)
-  typename Acc::Raw nxtE, nxtL;
+  // a-kernels: the raw quads of the next march row land in this thread's own shared-memory slots (cp.async, no register
+  // held meanwhile)
   if constexpr (!P::PLANE_READER) {
     const int yl = g.y_begin - 2 * g.r - 1;
-    if constexpr (G == 2) {
-      if (qload && g.y_begin >= 0 && g.y_begin < g.H) acc.stage_issue(stage_in, 0, g.y_begin, gx, t);
-      if (qload && yl >= g.y_first) acc.stage_issue(stage_in, 1, yl, gx, t);
-      cp_async_commit();
-    } else {
-      if (qload && g.y_begin >= 0 && g.y_begin < g.H) acc.raw_load(nxtE, g.y_begin, gx);
-      if (qload && yl >= g.y_first) acc.raw_load(nxtL, yl, gx);
-    }
+    if (qload && g.y_begin >= 0 && g.y_begin < g.H) acc.stage_issue(stage_in, 0, g.y_begin, gx, t);
+    if (qload && yl >= g.y_first) acc.stage_issue(stage_in, 1, yl, gx, t);
+    cp_async_commit();
   }
   GpRing ring, tring;
   int rows_out = 0;
@@ -355,69 +258,49 @@ __device__ __forceinline__ void gp_acc_worker(const GfCommon& gc, const GfGeom& 
     const int yli = yin - 2 * g.r - 1;
     const bool enter = (yin >= 0 && yin < g.H), leave = (yli >= g.y_first);
     if constexpr (!P::PLANE_READER) {
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 8);
       const int yn = yin + 1, yln = yli + 1;
-      if constexpr (G == 2) {
-        const int par = (yin - g.y_begin) & 1;
-        cp_async_wait_all();
-        if (qload && yn < g.y_end) {
-          if (yn >= 0 && yn < g.H) acc.stage_issue(stage_in, 2 * (par ^ 1), yn, gx, t);
-          if (yln >= g.y_first) acc.stage_issue(stage_in, 2 * (par ^ 1) + 1, yln, gx, t);
-        }
-        cp_async_commit();
-        if (qload && enter) acc.stage_read(stage_in, 2 * par, nxtE, t);
+      const int par = (yin - g.y_begin) & 1;
+      cp_async_wait_all();
+      if (qload && yn < g.y_end) {
+        if (yn >= 0 && yn < g.H) acc.stage_issue(stage_in, 2 * (par ^ 1), yn, gx, t);
+        if (yln >= g.y_first) acc.stage_issue(stage_in, 2 * (par ^ 1) + 1, yln, gx, t);
       }
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 9);
-      if (qload && enter && !(GP_EXP_SKIP_ACC && yin > g.y_begin + 4)) {
-        if (cmask == 0xfu) acc.template accum<+1, true, G>(nxtE, cmask, Vi, Vl);  // whole quad inside the image: straight-line code
-        else acc.template accum<+1, false, G>(nxtE, cmask, Vi, Vl);
+      cp_async_commit();
+      typename Acc::Raw rw;
+      if (qload && enter) {
+        acc.stage_read(stage_in, 2 * par, rw, t);
+        if (cmask == 0xfu) acc.template accum<+1, true>(rw, cmask, Vi, Vl);  // whole quad inside the image: straight-line code
+        else acc.template accum<+1, false>(rw, cmask, Vi, Vl);
       }
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 10);
-      if constexpr (G == 2) {
-        if (qload && leave) acc.stage_read(stage_in, 2 * ((yin - g.y_begin) & 1) + 1, nxtL, t);
-      }
-      if (qload && leave && !(GP_EXP_SKIP_ACC && yin > g.y_begin + 4)) {
-        if (cmask == 0xfu) acc.template accum<-1, true, G>(nxtL, cmask, Vi, Vl);
-        else acc.template accum<-1, false, G>(nxtL, cmask, Vi, Vl);
-      }
-      if constexpr (G != 2) {
-        // the quads of the next march row are requested now, into the same registers: they have the publish phase to arrive
-        if (qload && yn < g.y_end) {
-          if (yn >= 0 && yn < g.H) acc.raw_load(nxtE, yn, gx);
-          if (yln >= g.y_first) acc.raw_load(nxtL, yln, gx);
-        }
+      if (qload && leave) {
+        acc.stage_read(stage_in, 2 * par + 1, rw, t);
+        if (cmask == 0xfu) acc.template accum<-1, true>(rw, cmask, Vi, Vl);
+        else acc.template accum<-1, false>(rw, cmask, Vi, Vl);
       }
     } else {
       // the entering and the leaving coefficient row of this march row sit in slot `tring.s` of the TMA ring (auxiliary warp 0)
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 8);
       mbar_wait_park(bars + GPB_TFULL + tring.s, tring.ph);
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 9);
-      if (qload && (enter || leave) && !(GP_EXP_SKIP_ACC && yin > g.y_begin + 4)) {
+      if (qload && (enter || leave)) {
         const int4* slot = reinterpret_cast<const int4*>(stage_in) + ((size_t)tring.s * 2 * GP_NTR + (t - tA)) * P::NP;
-        acc.template accum_staged<G>(slot, slot + (size_t)GP_NTR * P::NP, gx >> 2, enter, leave, cmask, Vl);
+        acc.accum_staged(slot, slot + (size_t)GP_NTR * P::NP, gx >> 2, enter, leave, cmask, Vl);
       }
       mbar_arrive(bars + GPB_TEMPTY + tring.s);
       tring.template next<P::NRING>();
     }
     if (yin - g.r >= g.ys) {
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 0);
       if (rows_out >= NSTAGE) mbar_wait_park(bars + GPB_EMPTY + ring.s, ring.ph ^ 1u);  // SOLVE has left the row that used this stage
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out, 1);
       rows_out++;
       const GpStage st = gp_stage<P>(smem, ring.s);
-      if (qact && !(GP_EXP_SKIP_PUBLISH && rows_out > 3)) {
-        if constexpr (G != 1) {
+      if (qact) {
 #pragma unroll
-          for (int k = 0; k < NI; k++) {
-            uint32_t p0 = Vi[0][k], p1 = p0 + Vi[1][k], p2 = p1 + Vi[2][k], p3 = p2 + Vi[3][k];
-            st.Pi[k * NT + t] = make_uint4(p0, p1, p2, p3);
-            st.Gi[k * GP + t] = p3;
-          }
+        for (int k = 0; k < NI; k++) {
+          uint32_t p0 = Vi[0][k], p1 = p0 + Vi[1][k], p2 = p1 + Vi[2][k], p3 = p2 + Vi[3][k];
+          st.Pi[k * NT + t] = make_uint4(p0, p1, p2, p3);
+          st.Gi[k * GP + t] = p3;
         }
 #pragma unroll
-        for (int k = (G == 1 ? P::NDA : 0); k < (G == 0 ? P::NDA : ND); k++) {
-          const double p0 = Acc::to_double(Vl[0][k]), p1 = p0 + Acc::to_double(Vl[1][k]), p2 = p1 + Acc::to_double(Vl[2][k]),
-                       p3 = p2 + Acc::to_double(Vl[3][k]);
+        for (int k = 0; k < ND; k++) {
+          const double p0 = Vl[0][k], p1 = p0 + Vl[1][k], p2 = p1 + Vl[2][k], p3 = p2 + Vl[3][k];
           if constexpr (GP_EVEN_ODD(ND)) {
             st.Pa[k * NT + t] = make_double2(p0, p2);   // even elements
             st.Pb[k * NT + t] = make_double2(p1, p3);   // odd elements
@@ -429,7 +312,6 @@ __device__ __forceinline__ void gp_acc_worker(const GfCommon& gc, const GfGeom& 
         }
       }
       mbar_arrive(bars + GPB_FULL + ring.s);
-      if (t == 0 && G != 1) GP_STAMP(P, rows_out - 1, 2);
       ring.template next<NSTAGE>();
     }
   }
@@ -446,7 +328,7 @@ __device__ __forceinline__ void gp_aux(const GfCommon& gc, const GfGeom& gg, uns
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + L::off_bar);
   const GpGeo g = gp_geo(gg);
   const int lane = threadIdx.x & 31;
-  const int aw = (threadIdx.x - GP_SOLVE_THREADS - GP_NGRP * GP_NT) >> 5;   // 0..GP_NAUX-1
+  const int aw = (threadIdx.x - GP_SOLVE_THREADS - GP_NT) >> 5;   // 0..GP_NAUX-1
   const int tA = max(1, (g.HL + 4 - g.xs) >> 2), tB = min(g.NQ, (g.Wp - g.xs + g.HL + 4) >> 2);
   uint64_t pol_enter = 0, pol_leave = 0;
   if constexpr (P::PLANE_READER) { pol_enter = l2_policy_evict_last(P::L2_FRAC); pol_leave = l2_policy_evict_first(); }
@@ -458,19 +340,13 @@ __device__ __forceinline__ void gp_aux(const GfCommon& gc, const GfGeom& gg, uns
       const bool en = (yi >= 0 && yi < g.H), le = (yli >= g.y_first);
       const unsigned row_bytes = (unsigned)(tB - tA) * 16u * P::NP;
       uint64_t* bar = bars + GPB_TFULL + j;
-      if (GP_EXP_SKIP_TMA && yi > g.y_begin + 4) { mbar_arrive_expect_tx(bar, 0u); return; }
       mbar_arrive_expect_tx(bar, ((en ? 1u : 0u) + (le ? 1u : 0u)) * row_bytes);
       int4* slot = reinterpret_cast<int4*>(smem + L::off_in) + (size_t)j * 2 * GP_NTR * P::NP;
       const int gqa = (g.xs - g.HL - 4 + 4 * tA) >> 2;   // global quad index of strip quad tA
       const int4* rows = reinterpret_cast<const int4*>(P::coef_rows(gc, blockIdx.z, gg));
       const size_t qpr = (size_t)(g.Wp >> 2);
-#if GP_L2_HINT
       if (en) tma_bulk_g2s_hint(slot, rows + ((size_t)yi * qpr + gqa) * P::NP, row_bytes, bar, pol_enter);
       if (le) tma_bulk_g2s_hint(slot + (size_t)GP_NTR * P::NP, rows + ((size_t)yli * qpr + gqa) * P::NP, row_bytes, bar, pol_leave);
-#else
-      if (en) tma_bulk_g2s(slot, rows + ((size_t)yi * qpr + gqa) * P::NP, row_bytes, bar);
-      if (le) tma_bulk_g2s(slot + (size_t)GP_NTR * P::NP, rows + ((size_t)yli * qpr + gqa) * P::NP, row_bytes, bar);
-#endif
     }
   };
   GpRing ring, tring;
@@ -492,19 +368,17 @@ __device__ __forceinline__ void gp_aux(const GfCommon& gc, const GfGeom& gg, uns
     }
     if (yin - g.r < g.ys) continue;
     mbar_wait_park(bars + GPB_FULL + ring.s, ring.ph);
-    if (aw == 0) GP_STAMP(P, yin - g.r - g.ys, 3);
     const GpStage st = gp_stage<P>(smem, ring.s);
     // four moments per round (8 lanes each, GP_SEGQ quads per lane); the rounds are dealt out over the auxiliary warps
     const int seg = lane & 7, mq = lane >> 3;
     constexpr int RI = (NI + 3) / 4, RD = (ND + 3) / 4;
 #pragma unroll
     for (int rd = 0; rd < RI + RD; rd++) {
-      if (rd % GP_NAUX != aw || (GP_EXP_SKIP_SCAN && yin > g.y_begin + g.r + 3)) continue;
+      if (rd % GP_NAUX != aw) continue;
       if (rd < RI) { const int k0 = 4 * rd; gp_scan_task<uint32_t, uint4>(st.Gi + min(k0 + mq, NIa - 1) * GP, seg, k0 + mq < NI); }
       else { const int k0 = 4 * (rd - RI); gp_scan_task<double, double2>(st.Gd + min(k0 + mq, ND - 1) * GP_GPD, seg, k0 + mq < ND); }
     }
     mbar_arrive(bars + GPB_READY + ring.s);
-    if (aw == 0) GP_STAMP(P, yin - g.r - g.ys, 4);
     ring.template next<NSTAGE>();
   }
 }
@@ -629,14 +503,12 @@ __device__ __forceinline__ void gp_solve(const GfCommon& gc, const GfGeom& gg, u
   // groups of four warps on alternate rows with two pixel pairs per thread.
   for (int yo = g.ys; yo < g.ye; ++yo) {
     mbar_wait_park(bars + GPB_READY + ring.s, ring.ph);
-    if (v == 0) GP_STAMP(P, yo - g.ys, 5);
     uint32_t si[2][NIa];
     double sd[2][ND];
-    if (act && !(GP_EXP_SKIP_WINDOW && yo > g.ys + 1)) gp_window_pair<P>(gp_stage<P>(smem, ring.s), g, tq, h, si, sd);
+    if (act) gp_window_pair<P>(gp_stage<P>(smem, ring.s), g, tq, h, si, sd);
     mbar_arrive(bars + GPB_EMPTY + ring.s);   // everything this thread needs of the stage is in registers
-    if (v == 0) GP_STAMP(P, yo - g.ys, 6);
     ring.template next<NSTAGE>();
-    if (act && !(GP_EXP_SKIP_SOLVE && yo > g.ys)) {
+    if (act) {
       if constexpr (P::SOLVE_FIELDS > 0) {
         const int s2 = slot >= 1 ? slot - 1 : 2;   // (slot + 2) % 3
         if (yo + 2 < g.ye) sol.row_prefetch(yo + 2, gx, sin + s2 * SLOT);
@@ -655,7 +527,6 @@ __device__ __forceinline__ void gp_solve(const GfCommon& gc, const GfGeom& gg, u
       sol.column(1, yo, gx + 1, ny * nx1, si[1], sd[1], second);
       sol.store_pair(yo, gx, second);
     }
-    if (v == 0) GP_STAMP(P, yo - g.ys, 7);
   }
   sol.finish();
 }
@@ -664,7 +535,7 @@ __device__ __forceinline__ void gp_solve(const GfCommon& gc, const GfGeom& gg, u
 // the kernel
 // ------------------------------------------------------------------------------------------------
 // register budget of the calling warpgroup; the kernel starts with GP_LAUNCH_REGS for every thread
-constexpr int GP_LAUNCH_REGS = GP_NGRP == 1 ? 128 : 96;   // 65536 / GP_THREADS, in units of 8
+constexpr int GP_LAUNCH_REGS = 128;   // 65536 / GP_THREADS
 template <int R>
 __device__ __forceinline__ void gp_set_regs() {
   if constexpr (R > GP_LAUNCH_REGS) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(R));
@@ -677,7 +548,7 @@ __global__ void __launch_bounds__(GP_THREADS, 1) gp_kernel(GfCommon gc, GfGeom g
   static_assert((GP_NARROW ? GP_NT * P::ACC_REGS + 32 * GP_NAUX * GP_AUX_REGS : GP_ACC_THREADS * P::ACC_REGS) + GP_SOLVE_THREADS * P::SOLVE_REGS <=
                         GP_THREADS * GP_LAUNCH_REGS && P::SOLVE_REGS <= 255 && P::ACC_REGS <= 255 && P::NSTAGE >= 2 && P::NSTAGE <= 4,
                 "register pool / ring");
-  static_assert(!GP_NARROW || (GP_NGRP == 1 && GP_NT == 128 && GP_NAUX == 4), "narrow layout: one warpgroup of ACC workers, one of auxiliary warps");
+  static_assert(!GP_NARROW || (GP_NT == 128 && GP_NAUX == 4), "narrow layout: one warpgroup of ACC workers, one of auxiliary warps");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + L::off_bar);
   const int t = threadIdx.x;
@@ -697,13 +568,13 @@ __global__ void __launch_bounds__(GP_THREADS, 1) gp_kernel(GfCommon gc, GfGeom g
   }
   if (t == 0) {
     for (int s = 0; s < P::NSTAGE; s++) {
-      mbar_init(bars + GPB_FULL + s, GP_NGRP * GP_NT);
+      mbar_init(bars + GPB_FULL + s, GP_NT);
       mbar_init(bars + GPB_READY + s, 32 * GP_NAUX);
       mbar_init(bars + GPB_EMPTY + s, GP_SOLVE_THREADS);
     }
     for (int s = 0; s < 4; s++) {
       mbar_init(bars + GPB_TFULL + s, 1);
-      mbar_init(bars + GPB_TEMPTY + s, GP_NGRP * GP_NT);
+      mbar_init(bars + GPB_TEMPTY + s, GP_NT);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -714,21 +585,15 @@ __global__ void __launch_bounds__(GP_THREADS, 1) gp_kernel(GfCommon gc, GfGeom g
   } else if constexpr (GP_NARROW) {
     if (t < GP_SOLVE_THREADS + GP_NT) {
       gp_set_regs<P::ACC_REGS>();
-      gp_acc_worker<P, 2>(gc, gg, smem_raw);
+      gp_acc_worker<P>(gc, gg, smem_raw);
     } else {
       gp_set_regs<GP_AUX_REGS>();
       gp_aux<P>(gc, gg, smem_raw);
     }
   } else {
     gp_set_regs<P::ACC_REGS>();
-    if constexpr (GP_NGRP == 1) {
-      if (t < GP_SOLVE_THREADS + GP_NT) gp_acc_worker<P, 2>(gc, gg, smem_raw);
-      else gp_aux<P>(gc, gg, smem_raw);
-    } else {
-      if (t < GP_SOLVE_THREADS + GP_NT) gp_acc_worker<P, 0>(gc, gg, smem_raw);
-      else if (t < GP_SOLVE_THREADS + 2 * GP_NT) gp_acc_worker<P, 1>(gc, gg, smem_raw);
-      else gp_aux<P>(gc, gg, smem_raw);
-    }
+    if (t < GP_SOLVE_THREADS + GP_NT) gp_acc_worker<P>(gc, gg, smem_raw);
+    else gp_aux<P>(gc, gg, smem_raw);
   }
 }
 
@@ -763,11 +628,9 @@ __device__ __forceinline__ int4 coef_pack_fix(const double* a, double b, double 
 
 // GF1a: guide = normI (k units), p = max(t_blue, tmin) and max(t_green, tmin) (BGDehaze.py:39-48, guidedfilter.py:62-93)
 struct PipGF1a {
-  static constexpr int TRACE_ID = 0;
   static constexpr int NI = 9, ND = 8, NSTAGE = 3, ACC_REGS = GP_GF1A_ACC_REGS, SOLVE_REGS = GP_SOLVE_REGS_FOR(GP_GF1A_ACC_REGS);
   static constexpr bool PLANE_READER = false;
-  static constexpr int NDA = 2;
-  static constexpr int IN_BYTES = GP_NGRP == 1 ? 4 * GP_NT * 20 : 0;   // per worker: 4 cp.async slots (2 buffers x enter / leave) of one uint4 + one u32
+  static constexpr int IN_BYTES = 4 * GP_NT * 20;   // per worker: 4 cp.async slots (2 buffers x enter / leave) of one uint4 + one u32
   static constexpr int SOLVE_FIELDS = 0;   // 8-byte words of per-pixel-pair input SOLVE reads per row (staged by cp.async)
   struct Shared {
     double pT[2][256];    // rint(p_c * 2^28) as a function of the window-min k' (an exact integer-valued double)
@@ -796,8 +659,6 @@ struct PipGF1a {
     __syncthreads();
   }
   struct Acc {
-    typedef double Sum;   // exact: every term is an integer below 2^38, the sums stay below 2^53
-    static __device__ __forceinline__ double to_double(Sum v) { return v; }
     struct Raw { uint4 k; uint32_t m; };
     const Shared* sh; int Wp;
     const uint32_t* kq; const uint8_t* mg;
@@ -806,11 +667,6 @@ struct PipGF1a {
       const size_t n_pp = (size_t)gg.Wp * gg.H;
       kq = g.kq + (size_t)f * n_pp;
       mg = g.mg + (size_t)f * n_pp;
-    }
-    __device__ __forceinline__ void raw_load(Raw& r, int y, int gx) const {
-      const size_t o = (size_t)y * Wp + gx;
-      r.k = __ldg(reinterpret_cast<const uint4*>(kq + o));
-      r.m = __ldg(reinterpret_cast<const uint32_t*>(mg + o));
     }
     // staging slot s (0..3 = 2 buffers x enter / leave) of worker t: one uint4 + one u32, filled by cp.async
     __device__ __forceinline__ void stage_issue(unsigned char* st, int s, int y, int gx, int t) const {
@@ -825,40 +681,34 @@ struct PipGF1a {
     // The leaving row is the entering row with negated k: every update is one multiply-add in place - IMAD for the 32-bit
     // guide moments, DFMA for the signal moments (k and rint(p 2^28) are integers: products and sums are exact in fp64).
     // A 64-bit integer multiply-add costs three instructions on this machine (IMAD.WIDE + IADD3 + IADD3.X) against one DFMA.
-    // group 0: the nine guide moments and the two sums of p; group 1: the six sums of k p
-    template <int SIGN, bool FULL, int G>
-    __device__ __forceinline__ void accum(const Raw& r, unsigned cmask, uint32_t (&Vi)[4][NI], Sum (&Vl)[4][ND]) const {
+    // Every signal term is an integer below 2^38 and the sums stay below 2^53: exact.
+    template <int SIGN, bool FULL>
+    __device__ __forceinline__ void accum(const Raw& r, unsigned cmask, uint32_t (&Vi)[4][NI], double (&Vl)[4][ND]) const {
 #pragma unroll
       for (int c = 0; c < 4; c++) {
         const uint32_t w = quad_get(r.k, c);
         const int kb = (int)(w & 255u), kg = (int)((w >> 8) & 255u), kr = (int)((w >> 16) & 255u);
         const uint32_t mb = w >> 24, mgv = (r.m >> (8 * c)) & 255u;
         const int sb = SIGN > 0 ? kb : -kb, sg = SIGN > 0 ? kg : -kg, sr = SIGN > 0 ? kr : -kr;
-        if constexpr (G != 1) {
-          Vi[c][0] += (uint32_t)sb; Vi[c][1] += (uint32_t)sg; Vi[c][2] += (uint32_t)sr;
-          Vi[c][3] += (uint32_t)(sb * kb); Vi[c][4] += (uint32_t)(sb * kg); Vi[c][5] += (uint32_t)(sb * kr);
-          Vi[c][6] += (uint32_t)(sg * kg); Vi[c][7] += (uint32_t)(sg * kr); Vi[c][8] += (uint32_t)(sr * kr);
-        }
+        Vi[c][0] += (uint32_t)sb; Vi[c][1] += (uint32_t)sg; Vi[c][2] += (uint32_t)sr;
+        Vi[c][3] += (uint32_t)(sb * kb); Vi[c][4] += (uint32_t)(sb * kg); Vi[c][5] += (uint32_t)(sb * kr);
+        Vi[c][6] += (uint32_t)(sg * kg); Vi[c][7] += (uint32_t)(sg * kr); Vi[c][8] += (uint32_t)(sr * kr);
         if (FULL || (cmask & (1u << c))) {
           const double pb = sh->pT[0][mb], pg = sh->pT[1][mgv];
-          if constexpr (G != 1) {
-            Vl[c][0] += SIGN > 0 ? pb : -pb; Vl[c][1] += SIGN > 0 ? pg : -pg;
-          }
-          if constexpr (G != 0) {
-            const double db = (double)sb, dg = (double)sg, dr = (double)sr;
-            Vl[c][2] = fma(db, pb, Vl[c][2]); Vl[c][3] = fma(dg, pb, Vl[c][3]); Vl[c][4] = fma(dr, pb, Vl[c][4]);
-            Vl[c][5] = fma(db, pg, Vl[c][5]); Vl[c][6] = fma(dg, pg, Vl[c][6]); Vl[c][7] = fma(dr, pg, Vl[c][7]);
-          }
+          Vl[c][0] += SIGN > 0 ? pb : -pb; Vl[c][1] += SIGN > 0 ? pg : -pg;
+          const double db = (double)sb, dg = (double)sg, dr = (double)sr;
+          Vl[c][2] = fma(db, pb, Vl[c][2]); Vl[c][3] = fma(dg, pb, Vl[c][3]); Vl[c][4] = fma(dr, pb, Vl[c][4]);
+          Vl[c][5] = fma(db, pg, Vl[c][5]); Vl[c][6] = fma(dg, pg, Vl[c][6]); Vl[c][7] = fma(dr, pg, Vl[c][7]);
         }
       }
     }
   };
   struct Solve {
-    const Shared* sh; int Wp; GP_COEF_T* ab;
+    const Shared* sh; int Wp; int32_t* ab;
     GpInvN cinv;
     __device__ __forceinline__ void init(const GfCommon& g, int f, Shared* s, const GfGeom& gg) {
       sh = s; Wp = gg.Wp;
-      ab = reinterpret_cast<GP_COEF_T*>(g.ab) + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
+      ab = g.ab + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
     }
     __device__ __forceinline__ void row_prefetch(int, int, unsigned char*) {}
     __device__ __forceinline__ void row_pickup(const unsigned char*) {}
@@ -872,12 +722,12 @@ struct PipGF1a {
       rdet *= pinv;
       double a0[3], b0, a1[3], b1;
       const int gq = x >> 2, c = x & 3;
-      GP_COEF_V4* blk = reinterpret_cast<GP_COEF_V4*>(ab) + ((size_t)y * (Wp >> 2) + gq) * 8;
+      int4* blk = reinterpret_cast<int4*>(ab) + ((size_t)y * (Wp >> 2) + gq) * 8;
       gp_solve_rhs(A, rdet, Sd, N, invN, pinv, sd[0], sd + 2, a0, b0);
       gp_solve_rhs(A, rdet, Sd, N, invN, pinv, sd[1], sd + 5, a1, b1);
       if (valid) {
-        blk[coef_chunk<8>(gq, c, 0)] = GP_COEF_PACK(a0, b0, sh->cs);
-        blk[coef_chunk<8>(gq, c, 1)] = GP_COEF_PACK(a1, b1, sh->cs);
+        blk[coef_chunk<8>(gq, c, 0)] = coef_pack_fix(a0, b0, sh->cs.sa, sh->cs.sb);
+        blk[coef_chunk<8>(gq, c, 1)] = coef_pack_fix(a1, b1, sh->cs.sa, sh->cs.sb);
       }
     }
     __device__ __forceinline__ void store_pair(int, int, bool) {}
@@ -887,11 +737,9 @@ struct PipGF1a {
 
 // GF2a: guide = normYiCrCb (k units), p = S (BGDehaze.py:83-84)
 struct PipGF2a {
-  static constexpr int TRACE_ID = 2;
   static constexpr int NI = 9, ND = 4, NSTAGE = 3, ACC_REGS = GP_GF2A_ACC_REGS, SOLVE_REGS = GP_SOLVE_REGS_FOR(GP_GF2A_ACC_REGS);
   static constexpr bool PLANE_READER = false;
-  static constexpr int NDA = 1;
-  static constexpr int IN_BYTES = GP_NGRP == 1 ? 4 * GP_NT * 32 : 0;
+  static constexpr int IN_BYTES = 4 * GP_NT * 32;
   static constexpr int SOLVE_FIELDS = 0;   // 8-byte words of per-pixel-pair input SOLVE reads per row (staged by cp.async)
   struct Shared { FrameConst fc; double epsN_k, pinv; CoefScale cs; };
   static __device__ void init_shared(const GfCommon& g, int f, Shared* sh, const GfGeom& gg) {
@@ -905,8 +753,6 @@ struct PipGF2a {
     __syncthreads();
   }
   struct Acc {
-    typedef double Sum;
-    static __device__ __forceinline__ double to_double(Sum v) { return v; }
     struct Raw { uint4 y; uint4 s; };
     int Wp; const uint32_t* ycc; const uint32_t* sp;
     uint32_t ysub;   // (yi_min, yi_min, yi_min, yj_min): no byte can borrow
@@ -914,14 +760,9 @@ struct PipGF2a {
       Wp = gg.Wp;
       const size_t n_pp = (size_t)gg.Wp * gg.H;
       ycc = g.ycc + (size_t)f * n_pp;
-      sp = reinterpret_cast<const uint32_t*>(g.splane) + (size_t)f * n_pp;
+      sp = g.splane + (size_t)f * n_pp;
       const uint32_t a = (uint32_t)s->fc.yi_min, b = (uint32_t)s->fc.yj_min;
       ysub = a | (a << 8) | (a << 16) | (b << 24);
-    }
-    __device__ __forceinline__ void raw_load(Raw& r, int y, int gx) const {
-      const size_t o = (size_t)y * Wp + gx;
-      r.y = __ldg(reinterpret_cast<const uint4*>(ycc + o));
-      r.s = __ldg(reinterpret_cast<const uint4*>(sp + o));
     }
     __device__ __forceinline__ void stage_issue(unsigned char* st, int s, int y, int gx, int t) const {
       const size_t o = (size_t)y * Wp + gx;
@@ -933,9 +774,8 @@ struct PipGF2a {
       r.y = *reinterpret_cast<const uint4*>(st + ((size_t)s * GP_NT + t) * 32);
       r.s = *reinterpret_cast<const uint4*>(st + ((size_t)s * GP_NT + t) * 32 + 16);
     }
-    // group 0: the nine guide moments and the sum of S; group 1: the three sums of g S
-    template <int SIGN, bool FULL, int G>
-    __device__ __forceinline__ void accum(const Raw& r, unsigned cmask, uint32_t (&Vi)[4][NI], Sum (&Vl)[4][ND]) const {
+    template <int SIGN, bool FULL>
+    __device__ __forceinline__ void accum(const Raw& r, unsigned cmask, uint32_t (&Vi)[4][NI], double (&Vl)[4][ND]) const {
 #pragma unroll
       for (int c = 0; c < 4; c++) {
         if (FULL || (cmask & (1u << c))) {
@@ -943,25 +783,21 @@ struct PipGF2a {
           const int g0 = (int)(w & 255u), g1 = (int)((w >> 8) & 255u), g2 = (int)((w >> 16) & 255u);
           const double S = u2d(quad_get(r.s, c));   // rint(S 2^28) < 2^29
           const int s0 = SIGN > 0 ? g0 : -g0, s1 = SIGN > 0 ? g1 : -g1, s2 = SIGN > 0 ? g2 : -g2;
-          if constexpr (G != 1) {
-            Vi[c][0] += (uint32_t)s0; Vi[c][1] += (uint32_t)s1; Vi[c][2] += (uint32_t)s2;
-            Vi[c][3] += (uint32_t)(s0 * g0); Vi[c][4] += (uint32_t)(s0 * g1); Vi[c][5] += (uint32_t)(s0 * g2);
-            Vi[c][6] += (uint32_t)(s1 * g1); Vi[c][7] += (uint32_t)(s1 * g2); Vi[c][8] += (uint32_t)(s2 * g2);
-            Vl[c][0] += SIGN > 0 ? S : -S;
-          }
-          if constexpr (G != 0) {
-            Vl[c][1] = fma((double)s0, S, Vl[c][1]); Vl[c][2] = fma((double)s1, S, Vl[c][2]); Vl[c][3] = fma((double)s2, S, Vl[c][3]);
-          }
+          Vi[c][0] += (uint32_t)s0; Vi[c][1] += (uint32_t)s1; Vi[c][2] += (uint32_t)s2;
+          Vi[c][3] += (uint32_t)(s0 * g0); Vi[c][4] += (uint32_t)(s0 * g1); Vi[c][5] += (uint32_t)(s0 * g2);
+          Vi[c][6] += (uint32_t)(s1 * g1); Vi[c][7] += (uint32_t)(s1 * g2); Vi[c][8] += (uint32_t)(s2 * g2);
+          Vl[c][0] += SIGN > 0 ? S : -S;
+          Vl[c][1] = fma((double)s0, S, Vl[c][1]); Vl[c][2] = fma((double)s1, S, Vl[c][2]); Vl[c][3] = fma((double)s2, S, Vl[c][3]);
         }
       }
     }
   };
   struct Solve {
-    const Shared* sh; int Wp; GP_COEF_T* ab;
+    const Shared* sh; int Wp; int32_t* ab;
     GpInvN cinv;
     __device__ __forceinline__ void init(const GfCommon& g, int f, Shared* s, const GfGeom& gg) {
       sh = s; Wp = gg.Wp;
-      ab = reinterpret_cast<GP_COEF_T*>(g.ab) + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
+      ab = g.ab + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
     }
     __device__ __forceinline__ void row_prefetch(int, int, unsigned char*) {}
     __device__ __forceinline__ void row_pickup(const unsigned char*) {}
@@ -974,8 +810,8 @@ struct PipGF2a {
       rdet *= pinv;
       gp_solve_rhs(A, rdet, Sd, N, invN, pinv, sd[0], sd + 1, a, b);
       const int gq = x >> 2;
-      GP_COEF_V4* blk = reinterpret_cast<GP_COEF_V4*>(ab) + ((size_t)y * (Wp >> 2) + gq) * 4;
-      if (valid) blk[coef_chunk<4>(gq, x & 3, 0)] = GP_COEF_PACK(a, b, sh->cs);
+      int4* blk = reinterpret_cast<int4*>(ab) + ((size_t)y * (Wp >> 2) + gq) * 4;
+      if (valid) blk[coef_chunk<4>(gq, x & 3, 0)] = coef_pack_fix(a, b, sh->cs.sa, sh->cs.sb);
     }
     __device__ __forceinline__ void store_pair(int, int, bool) {}
     __device__ __forceinline__ void finish() {}
@@ -989,9 +825,7 @@ __device__ __forceinline__ int4 lds128i(unsigned addr) {
   return v;
 }
 // add the entering coefficient row to the running sums and drop the leaving one (int32 fixed point summed as doubles: exact)
-// G: GF1 rows (NP = 8, two filters) - group G takes the chunk of filter G; GF2 rows (NP = 4) - both groups read the pixel's one
-// chunk, group 0 sums (a0, a1), group 1 (a2, b)
-template <int NP, bool ENTER, bool LEAVE, bool FULL, int G>
+template <int NP, bool ENTER, bool LEAVE, bool FULL>
 __device__ __forceinline__ void gp_accum_coef_case(const int4* be_p, const int4* bl_p, int gq, unsigned cmask, double (&Vl)[4][NP]) {
   // quad blocks are NP*16 bytes and block-aligned, so (logical chunk ^ swizzle) * 16 is the block address with the
   // swizzle folded in, XOR a compile-time constant: one LOP3 per load
@@ -1002,37 +836,36 @@ __device__ __forceinline__ void gp_accum_coef_case(const int4* be_p, const int4*
   for (int c = 0; c < 4; c++) {
 #pragma unroll
     for (int j = 0; j < NP / 4; j++) {
-      if (NP == 8 && G != 2 && j != G) continue;   // two filters: group G takes the chunk of filter G
       const unsigned q16 = (unsigned)(NP == 8 ? 2 * c + j : c) << 4;
       int4 e = make_int4(0, 0, 0, 0), l = make_int4(0, 0, 0, 0);
       if (ENTER) e = lds128i(be ^ q16);
       if (LEAVE) l = lds128i(bl ^ q16);
       if (FULL || (cmask & (1u << c))) {   // |coefficient| < 2^30: the difference cannot wrap; integer-valued doubles: exact
-        if (NP == 8 || G != 1) { Vl[c][4 * j + 0] += (double)(e.x - l.x); Vl[c][4 * j + 1] += (double)(e.y - l.y); }
-        if (NP == 8 || G != 0) { Vl[c][4 * j + 2] += (double)(e.z - l.z); Vl[c][4 * j + 3] += (double)(e.w - l.w); }
+        Vl[c][4 * j + 0] += (double)(e.x - l.x); Vl[c][4 * j + 1] += (double)(e.y - l.y);
+        Vl[c][4 * j + 2] += (double)(e.z - l.z); Vl[c][4 * j + 3] += (double)(e.w - l.w);
       }
     }
   }
 }
-template <int NP, int G>
+template <int NP>
 __device__ __forceinline__ void gp_accum_coef(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, double (&Vl)[4][NP]) {
   if (enter && leave) {   // steady state (both rows, all four columns inside the image) is the straight-line case
-    if (cmask == 0xfu) gp_accum_coef_case<NP, true, true, true, G>(be, bl, gq, cmask, Vl);
-    else gp_accum_coef_case<NP, true, true, false, G>(be, bl, gq, cmask, Vl);
+    if (cmask == 0xfu) gp_accum_coef_case<NP, true, true, true>(be, bl, gq, cmask, Vl);
+    else gp_accum_coef_case<NP, true, true, false>(be, bl, gq, cmask, Vl);
   } else if (enter) {
-    gp_accum_coef_case<NP, true, false, false, G>(be, bl, gq, cmask, Vl);
+    gp_accum_coef_case<NP, true, false, false>(be, bl, gq, cmask, Vl);
   } else if (leave) {
-    gp_accum_coef_case<NP, false, true, false, G>(be, bl, gq, cmask, Vl);
+    gp_accum_coef_case<NP, false, true, false>(be, bl, gq, cmask, Vl);
   }
 }
 
 // GF1b: q = (box(a).k + box(b))/N for blue and green (guidedfilter.py:99-101) -> J (dehazed_BG, BGDehaze.py:53-56) + reductions
 struct PipGF1b {
-  static constexpr int TRACE_ID = 1;
-  static constexpr float L2_FRAC = GP_L2_FRAC_GF1B;
+  // fraction of the entering coefficient rows kept in L2 (evict_last) until they leave the window: 81 rows x 148 strips
+  // are 216 MB, keep half of it resident in the 126 MB L2
+  static constexpr float L2_FRAC = 0.5f;
   static constexpr int NI = 0, ND = 8, NP = 8, NSTAGE = 2, NRING = 3, ACC_REGS = GP_B_ACC_REGS, SOLVE_REGS = GP_SOLVE_REGS_FOR(GP_B_ACC_REGS);
   static constexpr bool PLANE_READER = true;
-  static constexpr int NDA = 4;   // group 0: the blue filter's sums, group 1: the green filter's
   static constexpr int IN_BYTES = NRING * 2 * GP_NTR * NP * 16;   // ring slots x (entering, leaving) row
   static constexpr int SOLVE_FIELDS = 0;   // the one word per row stays a register prefetch (the staged copy measured 5 % slower here)
   struct Shared {
@@ -1049,16 +882,12 @@ struct PipGF1b {
     __syncthreads();
   }
   static __device__ __forceinline__ const void* coef_rows(const GfCommon& g, int f, const GfGeom& gg) {
-    return reinterpret_cast<const int*>(g.ab) + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
+    return g.ab + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
   }
   struct Acc {
-    typedef double Sum;
-    struct Raw {};
-    static __device__ __forceinline__ double to_double(Sum v) { return v; }
     __device__ __forceinline__ void init(const GfCommon&, int, Shared*, const GfGeom&) {}
-    template <int G>
-    __device__ __forceinline__ void accum_staged(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, Sum (&Vl)[4][ND]) const {
-      gp_accum_coef<NP, G>(be, bl, gq, enter, leave, cmask, Vl);
+    __device__ __forceinline__ void accum_staged(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, double (&Vl)[4][ND]) const {
+      gp_accum_coef<NP>(be, bl, gq, enter, leave, cmask, Vl);
     }
   };
   struct Solve {
@@ -1144,11 +973,9 @@ struct PipGF1b {
 
 // GF2b: refined S -> exposure product -> min / max (BGDehaze.py:84-89)
 struct PipGF2b {
-  static constexpr int TRACE_ID = 3;
-  static constexpr float L2_FRAC = GP_L2_FRAC_GF2B;
+  static constexpr float L2_FRAC = 1.0f;   // as PipGF1b: 108 MB, all of it
   static constexpr int NI = 0, ND = 4, NP = 4, NSTAGE = 3, NRING = 4, ACC_REGS = GP_B_ACC_REGS, SOLVE_REGS = GP_SOLVE_REGS_FOR(GP_B_ACC_REGS);
   static constexpr bool PLANE_READER = true;
-  static constexpr int NDA = 2;
   static constexpr int IN_BYTES = NRING * 2 * GP_NTR * NP * 16;
   static constexpr int SOLVE_FIELDS = 4;   // 8-byte words of per-pixel-pair input SOLVE reads per row (staged by cp.async)
   struct Shared { ExpShared e; CoefScale cs; };
@@ -1158,16 +985,12 @@ struct PipGF2b {
     __syncthreads();
   }
   static __device__ __forceinline__ const void* coef_rows(const GfCommon& g, int f, const GfGeom& gg) {
-    return reinterpret_cast<const int*>(g.ab) + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
+    return g.ab + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
   }
   struct Acc {
-    typedef double Sum;
-    struct Raw {};
-    static __device__ __forceinline__ double to_double(Sum v) { return v; }
     __device__ __forceinline__ void init(const GfCommon&, int, Shared*, const GfGeom&) {}
-    template <int G>
-    __device__ __forceinline__ void accum_staged(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, Sum (&Vl)[4][ND]) const {
-      gp_accum_coef<NP, G>(be, bl, gq, enter, leave, cmask, Vl);
+    __device__ __forceinline__ void accum_staged(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, double (&Vl)[4][ND]) const {
+      gp_accum_coef<NP>(be, bl, gq, enter, leave, cmask, Vl);
     }
   };
   struct Solve {
@@ -1242,11 +1065,9 @@ struct PipGF2b {
 // GFq: the filter output itself, q = (box(a).I + box(b))/N (guidedfilter.py:99-101), as a float64 plane: the second half
 // of the stand-alone guided_filter stage entry (first half = PipGF2a on a packed 8-bit guide and a fixed-point p)
 struct PipGFq {
-  static constexpr int TRACE_ID = 3;
-  static constexpr float L2_FRAC = GP_L2_FRAC_GF2B;
+  static constexpr float L2_FRAC = 1.0f;
   static constexpr int NI = 0, ND = 4, NP = 4, NSTAGE = 3, NRING = 4, ACC_REGS = GP_B_ACC_REGS, SOLVE_REGS = GP_SOLVE_REGS_FOR(GP_B_ACC_REGS);
   static constexpr bool PLANE_READER = true;
-  static constexpr int NDA = 2;
   static constexpr int IN_BYTES = NRING * 2 * GP_NTR * NP * 16;
   static constexpr int SOLVE_FIELDS = 1;   // 8-byte words of per-pixel-pair input SOLVE reads per row (staged by cp.async)
   struct Shared { FrameConst fc; CoefScale cs; };
@@ -1255,16 +1076,12 @@ struct PipGFq {
     __syncthreads();
   }
   static __device__ __forceinline__ const void* coef_rows(const GfCommon& g, int f, const GfGeom& gg) {
-    return reinterpret_cast<const int*>(g.ab) + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
+    return g.ab + (size_t)f * 8 * (size_t)gg.Wp * gg.H;
   }
   struct Acc {
-    typedef double Sum;
-    struct Raw {};
-    static __device__ __forceinline__ double to_double(Sum v) { return v; }
     __device__ __forceinline__ void init(const GfCommon&, int, Shared*, const GfGeom&) {}
-    template <int G>
-    __device__ __forceinline__ void accum_staged(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, Sum (&Vl)[4][ND]) const {
-      gp_accum_coef<NP, G>(be, bl, gq, enter, leave, cmask, Vl);
+    __device__ __forceinline__ void accum_staged(const int4* be, const int4* bl, int gq, bool enter, bool leave, unsigned cmask, double (&Vl)[4][ND]) const {
+      gp_accum_coef<NP>(be, bl, gq, enter, leave, cmask, Vl);
     }
   };
   struct Solve {
