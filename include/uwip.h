@@ -37,7 +37,7 @@ typedef enum uwip_status {
   UWIP_OK = 0,
   UWIP_ERR_INVALID = -1,     /* bad pointer / size / parameter (reference: UB or silent skip)   */
   UWIP_ERR_CUDA = -2,        /* CUDA runtime error, text in uwip_last_error                     */
-  UWIP_ERR_UNSUPPORTED = -3, /* reserved: valid in the reference but not built (no such case now) */
+  UWIP_ERR_UNSUPPORTED = -3, /* valid input this build does not handle: JPEG codings uwip_jpeg_decode_bgr8_batch refuses */
   UWIP_ERR_NOMEM = -4
 } uwip_status;
 
@@ -251,9 +251,13 @@ int uwip_chain_bgr8(uwip_ctx* ctx, const uint8_t* src, uint8_t* dst, int n_frame
  * adaptiveExp_map is NaN for the whole frame (S = 0/0 where Yi = Yj = 0, BGDehaze.py:83, spreads through the box filters
  * and the final min-max; SURVEY 8a-D9) - the 8-bit output is then all zeros, exactly what imwrite would store.
  * UWIP_FRAME_ACLAHE_NOFIT: an automatic-CLAHE call could not fit an entropy curve of the frame (the reference's curve_fit
- * raises RuntimeError); the frame's BS = CL = -1 and it was processed with the fixed clip limit and grid. */
+ * raises RuntimeError); the frame's BS = CL = -1 and it was processed with the fixed clip limit and grid.
+ * UWIP_FRAME_JPEG_BAD (set by uwip_jpeg_decode_bgr8_batch): the file's entropy-coded data is bad - an invalid Huffman code, a
+ * coefficient past 63, the data ending before the last block or the wrong number of restart markers; the frame is all zeros
+ * (libjpeg's recovery from corrupt data is not restated). */
 #define UWIP_FRAME_NAN 1
 #define UWIP_FRAME_ACLAHE_NOFIT 2
+#define UWIP_FRAME_JPEG_BAD 4
 int uwip_last_frame_flags(uwip_ctx* ctx, int n_frames, int32_t* flags_host);
 
 /* ---- modules/videostrip: calcBlur (SURVEY 8f row N4, the frame-quality gate in front of the chain) */
@@ -296,6 +300,24 @@ size_t uwip_jpeg_encode_bound(int width, int height);
  * A frame's bytes do not depend on the batch it is in.  Stream ordered, does not synchronise. */
 int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_frames, int width, int height, int quality,
                                     uint8_t* d_out, size_t out_stride, uint64_t* d_len);
+
+/* Batched decoder whose pixels equal cv2.imread / cv2.imdecode(file, IMREAD_COLOR) with libjpeg-turbo (islow IDCT, fancy
+ * upsampling, csrc/jpegdec.h restates the arithmetic), the reader of the reference's command lines (histretch.cpp:158,
+ * bgdehaze/main.py:16), so that a .jpg input gives the device chain the reference's pixels; uwip_jpeg_decode_bgr8_dev above
+ * gives nvJPEG's.  Accepted: baseline and extended sequential Huffman, 8-bit, one scan, grey or YCbCr 4:4:4, 4:2:2, 4:4:0,
+ * 4:2:0, any restart interval, any tables.  The pixels are the stored orientation (IMREAD_IGNORE_ORIENTATION semantics; Exif
+ * is not read), which is what cv2.imdecode returns for every file without an Exif orientation.
+ * n host JPEG files (jpegs[f], lens[f]) of one size -> the bgr8 frames cv2.imdecode(file, IMREAD_COLOR) returns, contiguous
+ * at d_bgr.  Tables, sampling and restart interval may differ per file; width x height may not (UWIP_ERR_INVALID).
+ * Unsupported coding: UWIP_ERR_UNSUPPORTED.  Bad entropy-coded data: the frame is zeros and UWIP_FRAME_JPEG_BAD is set
+ * (uwip_last_frame_flags).  The headers are parsed and the files copied to pinned staging before the call returns, so the
+ * caller's memory is free again then.  A frame's pixels do not depend on the batch it is in.  Stream ordered, does not
+ * synchronise.  n_frames <= 65535. */
+int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
+                                uint8_t* d_bgr, int width, int height);
+/* per-frame statistics of the last uwip_jpeg_decode_bgr8_batch call (synchronises): stats[2f] = subsequence decodes the
+ * in-CTA synchronisation repeated, stats[2f + 1] = subsequences the cross-CTA fix-up re-decoded. */
+int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n_frames, int32_t* stats);
 
 /* ---- synthetic input + checksums (SURVEY 8d) ------------------------------------------------- */
 /* frames first_frame .. first_frame+n_frames-1 of the integer-only generator (twin of

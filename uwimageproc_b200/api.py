@@ -357,9 +357,48 @@ class Context:
             out = self.jpeg_encode_batch_dev(torch.from_numpy(np.ascontiguousarray(a)).to("cuda"), quality)
         return out[0] if single else out
 
+    # ---- JPEG files decoded as cv2.imdecode does (csrc/jpegdec.cu) ---------------------------------------------------
+    def jpeg_decode_batch_dev(self, files, d_out=None):
+        """JPEG files of one size (a list of bytes, or one bytes object) -> torch uint8 CUDA tensor (N, H, W, 3) holding
+        cv2.imdecode(file, cv2.IMREAD_COLOR) of each, decoded in one device call.  A file with bad entropy-coded data decodes
+        to zeros and sets bit 4 of last_frame_flags(N)."""
+        import torch
+
+        if isinstance(files, (bytes, bytearray, memoryview)):
+            files = [files]
+        bufs = [np.frombuffer(bytes(f), np.uint8) for f in files]
+        n = len(bufs)
+        if n == 0:
+            raise ValueError("no files")
+        w, h = self.jpeg_info(bufs[0])
+        if d_out is None:
+            d_out = torch.empty((n, h, w, 3), dtype=torch.uint8, device="cuda:%d" % self.device)
+        elif d_out.dtype != torch.uint8 or not d_out.is_cuda or not d_out.is_contiguous() or d_out.numel() != n * h * w * 3:
+            raise ValueError("d_out must be a contiguous uint8 CUDA tensor of N x H x W x 3 elements")
+        ptrs = (C.c_void_p * n)(*[b.ctypes.data for b in bufs])
+        lens = (C.c_size_t * n)(*[b.size for b in bufs])
+        self._ck(self.lib.uwip_jpeg_decode_bgr8_batch(self.h, ptrs, lens, n, _ptr(d_out), w, h))
+        self.synchronize()
+        return d_out
+
+    def jpeg_decode(self, files):
+        """JPEG files of one size -> numpy uint8 (N, H, W, 3) equal to cv2.imdecode(file, cv2.IMREAD_COLOR); one bytes object
+        -> (H, W, 3).  Decoded on the device."""
+        single = isinstance(files, (bytes, bytearray, memoryview))
+        out = self.jpeg_decode_batch_dev(files).cpu().numpy()
+        return out[0] if single else out
+
+    def jpeg_decode_stats(self, n):
+        """(N, 2) int32 of the last jpeg_decode_batch_dev call: subsequence decodes repeated by the in-CTA synchronisation,
+        subsequences re-decoded by the cross-CTA fix-up."""
+        out = np.empty((n, 2), np.int32)
+        self._ck(self.lib.uwip_jpeg_decode_stats(self.h, int(n), _ptr(out)))
+        return out
+
     def last_frame_flags(self, n):
-        """Per-frame status bits of the last batched chain / bgdehaze / automatic-aclahe call: 1 = the reference output is NaN
-        (D9), 2 = the automatic CLAHE fit failed (BS = CL = -1, fixed parameters used)."""
+        """Per-frame status bits of the last batched chain / bgdehaze / automatic-aclahe / exact JPEG decode call: 1 = the
+        reference output is NaN (D9), 2 = the automatic CLAHE fit failed (BS = CL = -1, fixed parameters used), 4 = the JPEG
+        file's entropy-coded data is bad (the frame is zeros)."""
         out = np.empty(n, np.int32)
         self._ck(self.lib.uwip_last_frame_flags(self.h, int(n), _ptr(out)))
         return out

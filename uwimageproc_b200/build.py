@@ -14,7 +14,7 @@ CSRC = os.path.join(HERE, "csrc")
 ROOT = os.path.dirname(HERE)
 LIB = os.path.join(HERE, "libuwip.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["cabi.cu", "histretch.cu", "clahe.cu", "dehaze.cu", "dehaze_gf1a.cu", "synth.cu", "blurmetric.cu", "jpegio.cu", "aclahe_knee.cu", "jpegenc.cu"]
+SOURCES = ["cabi.cu", "histretch.cu", "clahe.cu", "dehaze.cu", "dehaze_gf1a.cu", "synth.cu", "blurmetric.cu", "jpegio.cu", "aclahe_knee.cu", "jpegenc.cu", "jpegdec.cu"]
 # the knee search restates scipy's double-precision fit: no contraction into FMA
 SOURCE_FLAGS = {"aclahe_knee.cu": ["--fmad=false"]}
 NVCC_FLAGS = [

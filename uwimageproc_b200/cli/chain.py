@@ -1,4 +1,5 @@
-"""chain <input.jpg> <output.jpg> [-q=95] [-aclahe=auto [-loop=repaired|as_committed]] [-encoder=nvjpeg|exact]
+"""chain <input.jpg> <output.jpg> [-q=95] [-aclahe=auto [-loop=repaired|as_committed]] [-encoder=nvjpeg|exact] [-decoder=nvjpeg|exact]
+chain <input dir> <output dir> [options above] [-batch=64]
       the whole path on one file: histretch(V, 1/99) -> aclahe(8x8, clip 2) -> bgdehaze
 
 -aclahe=auto: the CLAHE clip limit and block size of the frame are chosen on the device (ParametrosACLAHE, ACLAHE.py:9-129) on
@@ -11,8 +12,77 @@ per-module CLIs (imread -> uwip_chain_bgr8 -> imwrite).
 -encoder=exact: the output JPEG is written by the project's own encoder (uwip_jpeg_encode_bgr8_batch_dev), whose file is byte
 for byte what cv2.imwrite(output, <chain output>) writes at -q, as the reference's command lines do.  The default, nvjpeg,
 writes nvJPEG's bytes (its own DCT, quantisation and entropy coding).
+
+-decoder=exact: the input JPEG is read by the project's own batched decoder (uwip_jpeg_decode_bgr8_batch), whose pixels are
+those cv2.imread(input) returns, as the reference's command lines read them.  The default, nvjpeg, gives nvJPEG's pixels (a
+few levels away, mostly in the 4:2:0 chroma upsampling), so the two decoders give different outputs, not the same output at
+different speeds.  With -decoder=exact -encoder=exact the file written is cv2.imwrite(output, chain(cv2.imread(input))), with
+-aclahe=auto too, and the pixels never exist on the host.
+
+When both arguments are directories, every *.jpg / *.jpeg of the input directory is enhanced into the output directory under
+the same name (what bgdehaze/main.py does over img/*.jpg -> result/): the files are grouped by size and run in batches of
+-batch frames through the same decoder, chain and encoder; BS, CL and the notes are printed per file.
 """
+import os
 import sys
+
+NOTES = (
+    (4, "note: the file's entropy-coded data is bad; the frame was decoded as zeros"),
+    (2, "note: the entropy curve fit failed for this frame (the reference raises); the fixed 8x8 grid and clip 2 were used"),
+    (1, "note: the reference's exposure map is NaN for this frame (S = 0/0); the output is all zeros, as imwrite would store it"),
+)
+
+
+def _notes(flags):
+    for bit, text in NOTES:
+        if flags & bit:
+            print(text)
+
+
+def _run_dir(ctx, src, dst, opt):
+    """Every *.jpg / *.jpeg of src -> dst/<same name>, grouped by size, in batches of opt['batch'] frames."""
+    import torch
+
+    names = sorted(f for f in os.listdir(src) if f.lower().endswith((".jpg", ".jpeg")) and os.path.isfile(os.path.join(src, f)))
+    groups = {}
+    for name in names:
+        with open(os.path.join(src, name), "rb") as f:
+            data = f.read()
+        groups.setdefault(ctx.jpeg_info(data), []).append((name, data))
+    auto, q = opt["aclahe"] == "auto", opt["q"]
+    for (w, h), files in groups.items():
+        for b0 in range(0, len(files), opt["batch"]):
+            part = files[b0:b0 + opt["batch"]]
+            n = len(part)
+            if opt["decoder"] == "exact":
+                d_in = ctx.jpeg_decode_batch_dev([d for _, d in part])
+                dflags = ctx.last_frame_flags(n)
+            else:
+                d_in = torch.empty((n, h, w, 3), dtype=torch.uint8, device="cuda:%d" % ctx.device)
+                for i, (_, data) in enumerate(part):
+                    ctx.jpeg_decode_dev(data, d_in[i])
+                dflags = [0] * n
+            d_out = torch.empty_like(d_in)
+            if auto:
+                d_bs = torch.empty(n, dtype=torch.int32, device=d_in.device)
+                d_cl = torch.empty(n, dtype=torch.int32, device=d_in.device)
+                ctx.chain_auto_dev(d_in, d_out, n, w, h, loop=opt["loop"], d_bs=d_bs, d_cl=d_cl)
+                bs, cl = d_bs.cpu().tolist(), d_cl.cpu().tolist()
+            else:
+                ctx.chain_dev(d_in, d_out, n, w, h)
+            flags = ctx.last_frame_flags(n)
+            if opt["encoder"] == "exact":
+                outs = ctx.jpeg_encode_batch_dev(d_out, q)
+            else:
+                outs = [ctx.jpeg_encode_dev(d_out[i], w, h, q) for i in range(n)]
+            for i, (name, _) in enumerate(part):
+                path = os.path.join(dst, name)
+                with open(path, "wb") as f:
+                    f.write(outs[i])
+                print(name + ":", *(("BS =", bs[i], "CL =", cl[i]) if auto else ()))
+                _notes(int(dflags[i]) | int(flags[i]))
+                print("saved", path)
+    return 0
 
 
 def main(argv=None):
@@ -20,11 +90,15 @@ def main(argv=None):
     from ._args import parse
 
     pos, opt, err = parse(argv, {"q": (95, int), "aclahe": ("fixed", str), "loop": ("repaired", str), "encoder": ("nvjpeg", str),
-                                "help": (False, bool)})
+                                "decoder": ("nvjpeg", str), "batch": (64, int), "help": (False, bool)})
     if opt["aclahe"] not in ("fixed", "auto") or opt["loop"] not in ("repaired", "as_committed"):
         err.append("-aclahe must be fixed or auto, -loop repaired or as_committed")
     if opt["encoder"] not in ("nvjpeg", "exact"):
         err.append("-encoder must be nvjpeg or exact")
+    if opt["decoder"] not in ("nvjpeg", "exact"):
+        err.append("-decoder must be nvjpeg or exact")
+    if opt["batch"] < 1:
+        err.append("-batch must be at least 1")
     if len(pos) < 2 or opt.get("help") or err:
         print(__doc__)
         return 0 if not err else -1
@@ -34,8 +108,31 @@ def main(argv=None):
     src, dst = pos[0], pos[1]
     auto = opt["aclahe"] == "auto"
     exact = opt["encoder"] == "exact"
+    if os.path.isdir(src) and os.path.isdir(dst):
+        return _run_dir(ctx, src, dst, opt)
     jpeg = src.lower().endswith((".jpg", ".jpeg")) and dst.lower().endswith((".jpg", ".jpeg"))
-    if auto and jpeg:
+    dflags = 0
+    if jpeg and opt["decoder"] == "exact":
+        import torch
+
+        with open(src, "rb") as f:
+            data = f.read()
+        d_in = ctx.jpeg_decode_batch_dev(data)[0]
+        dflags = int(ctx.last_frame_flags(1)[0])   # read now: the chain's call resets the flags
+        h, w = d_in.shape[:2]
+        d_out = torch.empty_like(d_in)
+        if auto:
+            d_bs = torch.empty(1, dtype=torch.int32, device=d_in.device)
+            d_cl = torch.empty(1, dtype=torch.int32, device=d_in.device)
+            ctx.chain_auto_dev(d_in, d_out, 1, w, h, loop=opt["loop"], d_bs=d_bs, d_cl=d_cl)
+        else:
+            ctx.chain_dev(d_in, d_out, 1, w, h)
+        out = ctx.jpeg_encode_batch_dev(d_out, opt["q"])[0] if exact else ctx.jpeg_encode_dev(d_out, w, h, opt["q"])
+        with open(dst, "wb") as f:
+            f.write(out)
+        if auto:
+            print("BS =", int(d_bs.cpu()[0]), "CL =", int(d_cl.cpu()[0]))
+    elif auto and jpeg:
         import torch
 
         with open(src, "rb") as f:
@@ -81,11 +178,7 @@ def main(argv=None):
         else:
             out = ctx.chain(img)
         cv2.imwrite(dst, out)
-    flags = ctx.last_frame_flags(1)
-    if flags[0] & 2:
-        print("note: the entropy curve fit failed for this frame (the reference raises); the fixed 8x8 grid and clip 2 were used")
-    if flags[0] & 1:
-        print("note: the reference's exposure map is NaN for this frame (S = 0/0); the output is all zeros, as imwrite would store it")
+    _notes(dflags | int(ctx.last_frame_flags(1)[0]))
     print("saved", dst)
     return 0
 

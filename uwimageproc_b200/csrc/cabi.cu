@@ -129,6 +129,7 @@ void uwip_destroy(uwip_ctx* ctx) {
   for (int i = 0; i < uwip_ctx::kSlots; i++)
     if (ctx->slot_ptr[i]) cudaFree(ctx->slot_ptr[i]);
   jpeg_io_destroy(ctx);
+  jpeg_dec_destroy(ctx);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   for (cudaEvent_t e : ctx->ev_pool) cudaEventDestroy(e);
   if (ctx->s_in) cudaStreamDestroy(ctx->s_in);
@@ -860,6 +861,25 @@ int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_f
   UWIP_REQUIRE(ctx, quality >= 1 && quality <= 100, "quality must lie in 1..100");
   UWIP_REQUIRE(ctx, out_stride >= jpeg_encode_bound(width, height), "out_stride is below uwip_jpeg_encode_bound(width, height)");
   return jpeg_encode_batch_dev(ctx, d_bgr, n_frames, width, height, quality, d_out, out_stride, d_len);
+}
+
+int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_bgr, int width,
+                                int height) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, jpegs && lens && d_bgr && n_frames > 0 && n_frames <= 65535, "bad argument (n_frames must lie in 1..65535)");
+  UWIP_REQUIRE(ctx, width >= 1 && width <= 65500 && height >= 1 && height <= 65500, "width and height must lie in 1..65500");
+  for (int f = 0; f < n_frames; f++) UWIP_REQUIRE(ctx, jpegs[f] && lens[f] > 0, "a file pointer is NULL or a length is 0");
+  int32_t* flags = flags_get(ctx, n_frames);
+  if (!flags) return UWIP_ERR_NOMEM;
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags);
+}
+int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n, int32_t* stats_host) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, stats_host && n > 0, "bad argument");
+  UWIP_REQUIRE(ctx, ctx->jdec_stats && n <= ctx->jdec_n, "more frames requested than the last batched JPEG decode processed");
+  UWIP_CUDA(ctx, cudaMemcpyAsync(stats_host, ctx->jdec_stats, sizeof(int32_t) * 2 * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+  UWIP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return UWIP_OK;
 }
 
 int uwip_last_frame_flags(uwip_ctx* ctx, int n, int32_t* flags_host) {

@@ -31,7 +31,7 @@ struct uwip_ctx {
   cudaStream_t s_in = nullptr, s_out = nullptr;   // copy streams of the host-buffer pipeline (created on first use)
   std::string err;
   // named, grow-only device buffers
-  static const int kSlots = 32;
+  static const int kSlots = 33;
   void* slot_ptr[kSlots] = {};
   size_t slot_bytes[kSlots] = {};
   void* pinned = nullptr;  // small pinned scratch for scalar results
@@ -40,6 +40,13 @@ struct uwip_ctx {
   // opt-in dynamic shared memory already granted on THIS context's device, per kernel (cudaFuncSetAttribute is
   // per device: a process-global flag would leave the second device of a process without the opt-in)
   void* jpeg = nullptr;    // nvJPEG handles of the file entry points (jpegio.cu), created on first use
+  // batched exact JPEG decoder (jpegdec.cu): pinned staging of the entropy-coded segments and tables, the event after the
+  // copies that read it, and the per-frame statistics of the last call (device, 2 x int32 per frame)
+  void* jdec_pinned = nullptr;
+  size_t jdec_pinned_bytes = 0;
+  cudaEvent_t jdec_ev = nullptr;
+  int32_t* jdec_stats = nullptr;
+  int jdec_n = 0;
   static const int kFuncs = 16;
   size_t func_smem[kFuncs] = {};
 };
@@ -88,6 +95,7 @@ enum Slot {
   SLOT_AUTO,          // automatic CLAHE: clip-curve derivatives, per-frame parameters, pick histograms and entropies
   SLOT_AUTO_BSCL,     // automatic CLAHE: BS, CL of the frames when the caller does not ask for them (int32 x2)
   SLOT_JPEGENC,       // batched JPEG encoder: tables, MCU bit offsets, block infos, int16 coefficients
+  SLOT_JPEGDEC,       // batched JPEG decoder: tables, segments, compact streams, subsequence states, coefficients, sample planes
 };
 
 const char* uwip_set_err(uwip_ctx* ctx, const char* fmt, ...);
@@ -403,6 +411,11 @@ void jpeg_io_destroy(uwip_ctx* ctx);
 size_t jpeg_encode_bound(int w, int h);
 int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
                           uint64_t* d_len);
+
+// jpegdec.cu
+int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_bgr, int w, int h,
+                      int32_t* d_flags);
+void jpeg_dec_destroy(uwip_ctx* ctx);
 
 // synth.cu
 int synth_frames_dev(uwip_ctx* ctx, uint8_t* d_dst, uint32_t seed, int first, int n, int w, int h);
