@@ -37,6 +37,17 @@ def _frame(a):
     return a
 
 
+def _frames(a):
+    """uint8 (N, H, W, 3) or (H, W, 3) host frames -> (contiguous (N, H, W, 3) array, whether one frame was given)."""
+    a = np.asarray(a)
+    single = a.ndim == 3
+    if single:
+        a = a[None]
+    if a.dtype != np.uint8 or a.ndim != 4 or a.shape[3] != 3:
+        raise ValueError("expected uint8 (N, H, W, 3)")
+    return np.ascontiguousarray(a), single
+
+
 class Context:
     """One context per (host thread, device); all work is ordered on its stream."""
 
@@ -227,13 +238,7 @@ class Context:
 
     def chain(self, frames, params=None):
         """frames: uint8 (N, H, W, 3) or (H, W, 3) host array -> same shape."""
-        a = np.asarray(frames)
-        single = a.ndim == 3
-        if single:
-            a = a[None]
-        if a.dtype != np.uint8 or a.ndim != 4 or a.shape[3] != 3:
-            raise ValueError("expected uint8 (N, H, W, 3)")
-        a = np.ascontiguousarray(a)
+        a, single = _frames(frames)
         out = np.empty_like(a)
         p = params or self.chain_params()
         self._ck(self.lib.uwip_chain_bgr8(self.h, _ptr(a), _ptr(out), a.shape[0], a.shape[2], a.shape[1], C.byref(p)))
@@ -245,15 +250,10 @@ class Context:
         params' fixed clip and tiles)."""
         import torch
 
-        a = np.asarray(frames)
-        single = a.ndim == 3
-        if single:
-            a = a[None]
-        if a.dtype != np.uint8 or a.ndim != 4 or a.shape[3] != 3:
-            raise ValueError("expected uint8 (N, H, W, 3)")
+        a, single = _frames(frames)
         n, h, w = a.shape[:3]
         with torch.cuda.device(self.device):
-            d_src = torch.from_numpy(np.ascontiguousarray(a)).to("cuda")
+            d_src = torch.from_numpy(a).to("cuda")
             d_dst = torch.empty_like(d_src)
             d_bs = torch.empty(n, dtype=torch.int32, device="cuda")
             d_cl = torch.empty(n, dtype=torch.int32, device="cuda")
@@ -347,14 +347,9 @@ class Context:
         cv2.imencode(".jpg", frame, [cv2.IMWRITE_JPEG_QUALITY, quality]), encoded on the device."""
         import torch
 
-        a = np.asarray(frames)
-        single = a.ndim == 3
-        if single:
-            a = a[None]
-        if a.dtype != np.uint8 or a.ndim != 4 or a.shape[3] != 3:
-            raise ValueError("expected uint8 (N, H, W, 3)")
+        a, single = _frames(frames)
         with torch.cuda.device(self.device):
-            out = self.jpeg_encode_batch_dev(torch.from_numpy(np.ascontiguousarray(a)).to("cuda"), quality)
+            out = self.jpeg_encode_batch_dev(torch.from_numpy(a).to("cuda"), quality)
         return out[0] if single else out
 
     # ---- JPEG files decoded as cv2.imdecode does (csrc/jpegdec.cu) ---------------------------------------------------

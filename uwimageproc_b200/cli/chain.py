@@ -5,9 +5,9 @@ chain <input dir> <output dir> [options above] [-batch=64]
 -aclahe=auto: the CLAHE clip limit and block size of the frame are chosen on the device (ParametrosACLAHE, ACLAHE.py:9-129) on
 the V plane of the histretch output and printed as BS and CL; when the curve fit fails the fixed 8x8 / clip 2 are used.
 
-JPEG files go through nvJPEG on the device (uwip_chain_jpeg): the file is read as bytes, decoded, enhanced and encoded on the
-GPU, and written as bytes - the pixels never exist on the host (SURVEY 8f row N3).  Other formats take the cv2 route of the
-per-module CLIs (imread -> uwip_chain_bgr8 -> imwrite).
+JPEG files are read as bytes, decoded (nvJPEG by default), enhanced and encoded (nvJPEG by default) on the GPU, and written as
+bytes - the pixels never exist on the host (SURVEY 8f row N3).  Other formats take the cv2 route of the per-module CLIs
+(imread -> uwip_chain_bgr8 -> imwrite).
 
 -encoder=exact: the output JPEG is written by the project's own encoder (uwip_jpeg_encode_bgr8_batch_dev), whose file is byte
 for byte what cv2.imwrite(output, <chain output>) writes at -q, as the reference's command lines do.  The default, nvjpeg,
@@ -21,7 +21,8 @@ different speeds.  With -decoder=exact -encoder=exact the file written is cv2.im
 
 When both arguments are directories, every *.jpg / *.jpeg of the input directory is enhanced into the output directory under
 the same name (what bgdehaze/main.py does over img/*.jpg -> result/): the files are grouped by size and run in batches of
--batch frames through the same decoder, chain and encoder; BS, CL and the notes are printed per file.
+-batch frames through the same decoder, chain and encoder; BS, CL and the notes are printed per file.  One JPEG file takes
+the same route as a batch of one.
 """
 import os
 import sys
@@ -39,16 +40,19 @@ def _notes(flags):
             print(text)
 
 
-def _run_dir(ctx, src, dst, opt):
-    """Every *.jpg / *.jpeg of src -> dst/<same name>, grouped by size, in batches of opt['batch'] frames."""
+def _read(path):
+    with open(path, "rb") as f:
+        return f.read()
+
+
+def _run_jpegs(ctx, jobs, opt, named):
+    """jobs: (output path, JPEG file bytes) pairs, grouped by size and run in batches of opt['batch'] frames through the
+    decoder, chain and encoder that opt names.  named: each file's report starts with its name (directory mode)."""
     import torch
 
-    names = sorted(f for f in os.listdir(src) if f.lower().endswith((".jpg", ".jpeg")) and os.path.isfile(os.path.join(src, f)))
     groups = {}
-    for name in names:
-        with open(os.path.join(src, name), "rb") as f:
-            data = f.read()
-        groups.setdefault(ctx.jpeg_info(data), []).append((name, data))
+    for path, data in jobs:
+        groups.setdefault(ctx.jpeg_info(data), []).append((path, data))
     auto, q = opt["aclahe"] == "auto", opt["q"]
     for (w, h), files in groups.items():
         for b0 in range(0, len(files), opt["batch"]):
@@ -56,7 +60,7 @@ def _run_dir(ctx, src, dst, opt):
             n = len(part)
             if opt["decoder"] == "exact":
                 d_in = ctx.jpeg_decode_batch_dev([d for _, d in part])
-                dflags = ctx.last_frame_flags(n)
+                dflags = ctx.last_frame_flags(n)   # read now: the chain's call resets the flags
             else:
                 d_in = torch.empty((n, h, w, 3), dtype=torch.uint8, device="cuda:%d" % ctx.device)
                 for i, (_, data) in enumerate(part):
@@ -67,19 +71,21 @@ def _run_dir(ctx, src, dst, opt):
                 d_bs = torch.empty(n, dtype=torch.int32, device=d_in.device)
                 d_cl = torch.empty(n, dtype=torch.int32, device=d_in.device)
                 ctx.chain_auto_dev(d_in, d_out, n, w, h, loop=opt["loop"], d_bs=d_bs, d_cl=d_cl)
-                bs, cl = d_bs.cpu().tolist(), d_cl.cpu().tolist()
             else:
                 ctx.chain_dev(d_in, d_out, n, w, h)
-            flags = ctx.last_frame_flags(n)
+            flags = ctx.last_frame_flags(n)   # waits for the context's stream, which writes BS and CL: read them after it
+            if auto:
+                bs, cl = d_bs.cpu().tolist(), d_cl.cpu().tolist()
             if opt["encoder"] == "exact":
                 outs = ctx.jpeg_encode_batch_dev(d_out, q)
             else:
                 outs = [ctx.jpeg_encode_dev(d_out[i], w, h, q) for i in range(n)]
-            for i, (name, _) in enumerate(part):
-                path = os.path.join(dst, name)
+            for i, (path, _) in enumerate(part):
                 with open(path, "wb") as f:
                     f.write(outs[i])
-                print(name + ":", *(("BS =", bs[i], "CL =", cl[i]) if auto else ()))
+                head = [os.path.basename(path) + ":"] if named else []
+                if named or auto:
+                    print(*head, *(("BS =", bs[i], "CL =", cl[i]) if auto else ()))
                 _notes(int(dflags[i]) | int(flags[i]))
                 print("saved", path)
     return 0
@@ -106,79 +112,24 @@ def main(argv=None):
 
     ctx = default_context()
     src, dst = pos[0], pos[1]
-    auto = opt["aclahe"] == "auto"
-    exact = opt["encoder"] == "exact"
     if os.path.isdir(src) and os.path.isdir(dst):
-        return _run_dir(ctx, src, dst, opt)
-    jpeg = src.lower().endswith((".jpg", ".jpeg")) and dst.lower().endswith((".jpg", ".jpeg"))
-    dflags = 0
-    if jpeg and opt["decoder"] == "exact":
-        import torch
+        names = sorted(f for f in os.listdir(src) if f.lower().endswith((".jpg", ".jpeg")) and os.path.isfile(os.path.join(src, f)))
+        return _run_jpegs(ctx, [(os.path.join(dst, name), _read(os.path.join(src, name))) for name in names], opt, True)
+    if src.lower().endswith((".jpg", ".jpeg")) and dst.lower().endswith((".jpg", ".jpeg")):
+        return _run_jpegs(ctx, [(dst, _read(src))], opt, False)
+    import cv2
 
-        with open(src, "rb") as f:
-            data = f.read()
-        d_in = ctx.jpeg_decode_batch_dev(data)[0]
-        dflags = int(ctx.last_frame_flags(1)[0])   # read now: the chain's call resets the flags
-        h, w = d_in.shape[:2]
-        d_out = torch.empty_like(d_in)
-        if auto:
-            d_bs = torch.empty(1, dtype=torch.int32, device=d_in.device)
-            d_cl = torch.empty(1, dtype=torch.int32, device=d_in.device)
-            ctx.chain_auto_dev(d_in, d_out, 1, w, h, loop=opt["loop"], d_bs=d_bs, d_cl=d_cl)
-        else:
-            ctx.chain_dev(d_in, d_out, 1, w, h)
-        out = ctx.jpeg_encode_batch_dev(d_out, opt["q"])[0] if exact else ctx.jpeg_encode_dev(d_out, w, h, opt["q"])
-        with open(dst, "wb") as f:
-            f.write(out)
-        if auto:
-            print("BS =", int(d_bs.cpu()[0]), "CL =", int(d_cl.cpu()[0]))
-    elif auto and jpeg:
-        import torch
-
-        with open(src, "rb") as f:
-            data = f.read()
-        d_in = ctx.jpeg_decode_dev(data)
-        h, w = d_in.shape[:2]
-        d_out = torch.empty_like(d_in)
-        d_bs = torch.empty(1, dtype=torch.int32, device=d_in.device)
-        d_cl = torch.empty(1, dtype=torch.int32, device=d_in.device)
-        ctx.chain_auto_dev(d_in, d_out, 1, w, h, loop=opt["loop"], d_bs=d_bs, d_cl=d_cl)
-        out = ctx.jpeg_encode_batch_dev(d_out, opt["q"])[0] if exact else ctx.jpeg_encode_dev(d_out, w, h, opt["q"])
-        with open(dst, "wb") as f:
-            f.write(out)
-        print("BS =", int(d_bs.cpu()[0]), "CL =", int(d_cl.cpu()[0]))
-    elif jpeg and exact:
-        import torch
-
-        with open(src, "rb") as f:
-            data = f.read()
-        d_in = ctx.jpeg_decode_dev(data)
-        h, w = d_in.shape[:2]
-        d_out = torch.empty_like(d_in)
-        ctx.chain_dev(d_in, d_out, 1, w, h)
-        out = ctx.jpeg_encode_batch_dev(d_out, opt["q"])[0]
-        with open(dst, "wb") as f:
-            f.write(out)
-    elif jpeg:
-        with open(src, "rb") as f:
-            data = f.read()
-        out = ctx.chain_jpeg(data, quality=opt["q"])
-        with open(dst, "wb") as f:
-            f.write(out)
+    img = cv2.imread(src, cv2.IMREAD_COLOR)
+    if img is None:
+        print("Failed to read input image, exiting...")
+        return -1
+    if opt["aclahe"] == "auto":
+        out, bs, cl = ctx.chain_auto(img, loop=opt["loop"])
+        print("BS =", int(bs[0]), "CL =", int(cl[0]))
     else:
-        import cv2
-
-        img = cv2.imread(src, cv2.IMREAD_COLOR)
-        if img is None:
-            print("Failed to read input image, exiting...")
-            return -1
-        if auto:
-            out, bs, cl = ctx.chain_auto(img, loop=opt["loop"])
-            print("BS =", int(bs[0]), "CL =", int(cl[0]))
-        else:
-            out = ctx.chain(img)
-        cv2.imwrite(dst, out)
-    _notes(dflags | int(ctx.last_frame_flags(1)[0]))
+        out = ctx.chain(img)
+    cv2.imwrite(dst, out)
+    _notes(int(ctx.last_frame_flags(1)[0]))
     print("saved", dst)
     return 0
 

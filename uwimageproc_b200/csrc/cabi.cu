@@ -260,6 +260,44 @@ static int check_percentiles(uwip_ctx* ctx, int lo, int hi) {
   return UWIP_OK;
 }
 
+static int32_t* flags_get(uwip_ctx* ctx, int n) {
+  int32_t* f = (int32_t*)uwip_slot(ctx, SLOT_FLAGS, sizeof(int32_t) * (size_t)n);
+  ctx->flags_n = f ? n : 0;
+  return f;
+}
+
+// sub-batch size: the dehaze workspace is 60 B/px/frame (+ a 256 KB table; budgeted as 512 KB); keep it below 80 GB of the 180 GB
+// (UWIP_WORKSPACE_GB overrides) and below 70 % of what the device has free plus what this context already holds, and among
+// the sizes that fit take the one that wastes the fewest CTA waves of the marches (dehaze_sub_batch)
+static int sub_batch(const uwip_ctx* ctx, int n, int w, int h) {
+  size_t per_frame = (size_t)w * h * 60 + (512u << 10);
+  double gb = 80.0;
+  if (const char* e = getenv("UWIP_WORKSPACE_GB")) { double v = atof(e); if (v >= 1.0) gb = v; }
+  size_t cap_bytes = (size_t)(gb * 1e9);
+  size_t free_b = 0, total_b = 0;
+  if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
+    size_t held = 0;
+    for (int i = 0; i < uwip_ctx::kSlots; i++) held += ctx->slot_bytes[i];
+    cap_bytes = std::min(cap_bytes, (size_t)(0.7 * (double)(free_b + held)));
+  } else {
+    cudaGetLastError();
+  }
+  size_t cap = std::max<size_t>(1, cap_bytes / per_frame);
+  return dehaze_sub_batch(ctx, n, w, (int)std::min<size_t>(cap, (size_t)n));
+}
+
+// n device frames in sub-batches of sub_batch's size: fn(first, m, fs, flags + first) for each, stopping at the first error.
+// One FrameState block of the largest sub-batch serves them all; the flags of the call are indexed by frame.
+template <class Fn>
+static int each_sub_batch(uwip_ctx* ctx, int n, int w, int h, Fn&& fn) {
+  int nb = sub_batch(ctx, n, w, h);
+  FrameState* fs = frame_state_get(ctx, nb);
+  int32_t* flags = flags_get(ctx, n);
+  if (!fs || !flags) return UWIP_ERR_NOMEM;
+  for (int i = 0; i < n; i += nb) UWIP_CHECK(fn(i, std::min(nb, n - i), fs, flags + i));
+  return UWIP_OK;
+}
+
 extern "C" {
 
 int uwip_histogram_u8_dev(uwip_ctx* ctx, const uint8_t* d_plane, int w, int h, float* d_hist) {
@@ -413,8 +451,6 @@ int uwip_aclahe_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t sp, uint8_t* dst,
   UWIP_CHECK(uwip_aclahe_bgr8_dev(ctx, d, d, 1, w, h, clip, tx, ty, hsv_round));
   return stage_out(ctx, d, dst, dp, w, h, 3);
 }
-
-static int32_t* flags_get(uwip_ctx* ctx, int n);
 
 // BS / CL outputs of the automatic calls: the caller's device arrays or the context's
 static int auto_outputs(uwip_ctx* ctx, int n, int32_t*& d_bs, int32_t*& d_cl) {
@@ -596,52 +632,20 @@ int uwip_guided_filter_u8(uwip_ctx* ctx, const uint8_t* guide, size_t pitch, int
   return UWIP_OK;
 }
 
-static int32_t* flags_get(uwip_ctx* ctx, int n) {
-  int32_t* f = (int32_t*)uwip_slot(ctx, SLOT_FLAGS, sizeof(int32_t) * (size_t)n);
-  ctx->flags_n = f ? n : 0;
-  return f;
-}
-
-// sub-batch size: the dehaze workspace is 60 B/px/frame (+ a 256 KB table; budgeted as 512 KB); keep it below 80 GB of the 180 GB
-// (UWIP_WORKSPACE_GB overrides) and below 70 % of what the device has free plus what this context already holds, and among
-// the sizes that fit take the one that wastes the fewest CTA waves of the marches (dehaze_sub_batch)
-static int sub_batch(const uwip_ctx* ctx, int n, int w, int h) {
-  size_t per_frame = (size_t)w * h * 60 + (512u << 10);
-  double gb = 80.0;
-  if (const char* e = getenv("UWIP_WORKSPACE_GB")) { double v = atof(e); if (v >= 1.0) gb = v; }
-  size_t cap_bytes = (size_t)(gb * 1e9);
-  size_t free_b = 0, total_b = 0;
-  if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
-    size_t held = 0;
-    for (int i = 0; i < uwip_ctx::kSlots; i++) held += ctx->slot_bytes[i];
-    cap_bytes = std::min(cap_bytes, (size_t)(0.7 * (double)(free_b + held)));
-  } else {
-    cudaGetLastError();
-  }
-  size_t cap = std::max<size_t>(1, cap_bytes / per_frame);
-  return dehaze_sub_batch(ctx, n, w, (int)std::min<size_t>(cap, (size_t)n));
-}
-
 int uwip_bgdehaze_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, const uwip_dehaze_params* pp) {
   CTX_GUARD(ctx);
   UWIP_REQUIRE(ctx, d_src && d_dst && n > 0, "bad argument");
   uwip_dehaze_params p;
   if (pp) p = *pp; else uwip_dehaze_defaults(&p);
-  int nb = sub_batch(ctx, n, w, h);
-  FrameState* fs = frame_state_get(ctx, nb);
-  int32_t* flags = flags_get(ctx, n);
-  if (!fs || !flags) return UWIP_ERR_NOMEM;
-  size_t fbytes = (size_t)w * h * 3;
-  for (int i = 0; i < n; i += nb) {
-    int m = std::min(nb, n - i);
+  const size_t fbytes = (size_t)w * h * 3;
+  return each_sub_batch(ctx, n, w, h, [&](int i, int m, FrameState* fs, int32_t* flags) {
     UWIP_CHECK(frame_state_reset(ctx, fs, m));
-    UWIP_CHECK(dehaze_frames_dev(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, p, false, fs, nullptr, flags + i));
-  }
-  return UWIP_OK;
+    return dehaze_frames_dev(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, p, false, fs, nullptr, flags);
+  });
 }
 
 // ---- the chain ------------------------------------------------------------------------------------------
-// automatic CLAHE parameters of a chain call (uwip_chain_bgr8_auto_dev): per-frame outputs of the sub-batch
+// automatic CLAHE parameters of a chain call (uwip_chain_bgr8_auto_dev): per-frame outputs of the frames it covers
 struct ChainAuto {
   int loop;
   int32_t* d_bs;
@@ -704,20 +708,25 @@ static int chain_check(uwip_ctx* ctx, const uwip_chain_params* p, int n, int w, 
   return check_percentiles(ctx, p->lo, p->hi);
 }
 
+// the device-buffer chain on checked arguments; au: the automatic CLAHE outputs of the n frames, null for the fixed parameters
+static int chain_batch_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, const uwip_chain_params& p,
+                           const ChainAuto* au) {
+  ChainAuto a = au ? *au : ChainAuto{0, nullptr, nullptr};
+  // before sub_batch: the BS / CL slot auto_outputs may grow counts toward what the context already holds
+  if (au) UWIP_CHECK(auto_outputs(ctx, n, a.d_bs, a.d_cl));
+  const size_t fbytes = (size_t)w * h * 3;
+  return each_sub_batch(ctx, n, w, h, [&](int i, int m, FrameState* fs, int32_t* flags) {
+    ChainAuto sub = a;
+    if (au) { sub.d_bs += i; sub.d_cl += i; }
+    return chain_sub(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, p, fs, flags, au ? &sub : nullptr);
+  });
+}
+
 int uwip_chain_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, const uwip_chain_params* p) {
   CTX_GUARD(ctx);
   UWIP_REQUIRE(ctx, d_src && d_dst, "null pointer");
   UWIP_CHECK(chain_check(ctx, p, n, w, h));
-  int nb = sub_batch(ctx, n, w, h);
-  FrameState* fs = frame_state_get(ctx, nb);
-  int32_t* flags = flags_get(ctx, n);
-  if (!fs || !flags) return UWIP_ERR_NOMEM;
-  size_t fbytes = (size_t)w * h * 3;
-  for (int i = 0; i < n; i += nb) {
-    int m = std::min(nb, n - i);
-    UWIP_CHECK(chain_sub(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, *p, fs, flags + i));
-  }
-  return UWIP_OK;
+  return chain_batch_dev(ctx, d_src, d_dst, n, w, h, *p, nullptr);
 }
 
 int uwip_chain_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, const uwip_chain_params* p, int loop,
@@ -727,18 +736,8 @@ int uwip_chain_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst
   UWIP_CHECK(chain_check(ctx, p, n, w, h));
   UWIP_REQUIRE(ctx, loop == UWIP_ACLAHE_LOOP_REPAIRED || loop == UWIP_ACLAHE_LOOP_AS_COMMITTED, "bad loop");
   UWIP_CHECK(aclahe_check_auto_size(ctx, w, h));
-  UWIP_CHECK(auto_outputs(ctx, n, d_bs, d_cl));
-  int nb = sub_batch(ctx, n, w, h);
-  FrameState* fs = frame_state_get(ctx, nb);
-  int32_t* flags = flags_get(ctx, n);
-  if (!fs || !flags) return UWIP_ERR_NOMEM;
-  size_t fbytes = (size_t)w * h * 3;
-  for (int i = 0; i < n; i += nb) {
-    int m = std::min(nb, n - i);
-    ChainAuto au = {loop, d_bs + i, d_cl + i};
-    UWIP_CHECK(chain_sub(ctx, d_src + (size_t)i * fbytes, d_dst + (size_t)i * fbytes, m, w, h, *p, fs, flags + i, &au));
-  }
-  return UWIP_OK;
+  const ChainAuto au = {loop, d_bs, d_cl};
+  return chain_batch_dev(ctx, d_src, d_dst, n, w, h, *p, &au);
 }
 
 // host buffers: H2D / compute / D2H pipelined over sub-batches with two staging buffers per direction
@@ -841,11 +840,11 @@ int uwip_chain_jpeg(uwip_ctx* ctx, const uint8_t* jpeg_in, size_t len_in, const 
   const size_t fbytes = (size_t)w * h * 3;
   uint8_t* d_in = (uint8_t*)uwip_slot(ctx, SLOT_CHAIN_IN0, fbytes);
   uint8_t* d_out = (uint8_t*)uwip_slot(ctx, SLOT_CHAIN_OUT0, fbytes);
-  FrameState* fs = frame_state_get(ctx, 1);
-  int32_t* flags = flags_get(ctx, 1);
-  if (!d_in || !d_out || !fs || !flags) return UWIP_ERR_NOMEM;
-  UWIP_CHECK(jpeg_decode_dev(ctx, jpeg_in, len_in, d_in, w, h));
-  UWIP_CHECK(chain_sub(ctx, d_in, d_out, 1, w, h, *p, fs, flags));
+  if (!d_in || !d_out) return UWIP_ERR_NOMEM;
+  UWIP_CHECK(each_sub_batch(ctx, 1, w, h, [&](int, int, FrameState* fs, int32_t* flags) {
+    UWIP_CHECK(jpeg_decode_dev(ctx, jpeg_in, len_in, d_in, w, h));
+    return chain_sub(ctx, d_in, d_out, 1, w, h, *p, fs, flags);
+  }));
   return jpeg_encode_dev(ctx, d_out, w, h, quality, jpeg_out, cap, len_out);
 }
 
