@@ -174,6 +174,14 @@ int uwip_aclahe_params_u8_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_plan
 int uwip_aclahe_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_frames, int width, int height,
                               int loop, int hsv_round, double clip, int tiles_x, int tiles_y, int32_t* d_bs,
                               int32_t* d_cl);
+/* automatic CLAHE on n device u8 planes, the grey prototype (modules/aclahe/python/main.py:18-20) for a batch: the plane's
+ * (BS, CL) from uwip_aclahe_params_u8_dev (which blurs internally, ACLAHE.py:15), then createCLAHE(CL, (BS, BS)).apply of the
+ * unblurred plane.  A plane whose fit failed gets BS = CL = -1, UWIP_FRAME_ACLAHE_NOFIT, and CLAHE with clip and
+ * tiles_x x tiles_y.  d_src may equal d_dst.  d_bs, d_cl: optional device int32[n] outputs (NULL: not returned).  The size
+ * refusals are those of uwip_aclahe_params_u8_dev.  A plane's bytes do not depend on the batch it is in.  Stream ordered,
+ * does not synchronise. */
+int uwip_aclahe_u8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n_planes, int width, int height,
+                            int loop, double clip, int tiles_x, int tiles_y, int32_t* d_bs, int32_t* d_cl);
 
 /* ---- modules/bgdehaze ---------------------------------------------------------------------- */
 typedef struct uwip_dehaze_params {
@@ -247,12 +255,13 @@ int uwip_chain_bgr8(uwip_ctx* ctx, const uint8_t* src, uint8_t* dst, int n_frame
                     int height, const uwip_chain_params* p);
 
 /* per-frame status bits of the LAST uwip_chain_bgr8[_auto][_dev] / uwip_bgdehaze_bgr8_dev / uwip_aclahe_params_u8_dev /
- * uwip_aclahe_bgr8_auto_dev call on this context (synchronises the stream).  UWIP_FRAME_NAN: the reference's
+ * uwip_aclahe_bgr8_auto_dev / uwip_aclahe_u8_auto_dev / uwip_jpeg_decode_bgr8_batch / uwip_jpeg_decode_u8_batch call on
+ * this context (synchronises the stream).  UWIP_FRAME_NAN: the reference's
  * adaptiveExp_map is NaN for the whole frame (S = 0/0 where Yi = Yj = 0, BGDehaze.py:83, spreads through the box filters
  * and the final min-max; SURVEY 8a-D9) - the 8-bit output is then all zeros, exactly what imwrite would store.
  * UWIP_FRAME_ACLAHE_NOFIT: an automatic-CLAHE call could not fit an entropy curve of the frame (the reference's curve_fit
  * raises RuntimeError); the frame's BS = CL = -1 and it was processed with the fixed clip limit and grid.
- * UWIP_FRAME_JPEG_BAD (set by uwip_jpeg_decode_bgr8_batch): the file's entropy-coded data is bad - an invalid Huffman code, a
+ * UWIP_FRAME_JPEG_BAD (set by the two batched JPEG readers): the file's entropy-coded data is bad - an invalid Huffman code, a
  * coefficient past 63, the data ending before the last block or the wrong number of restart markers; the frame is all zeros
  * (libjpeg's recovery from corrupt data is not restated). */
 #define UWIP_FRAME_NAN 1
@@ -300,6 +309,13 @@ size_t uwip_jpeg_encode_bound(int width, int height);
  * A frame's bytes do not depend on the batch it is in.  Stream ordered, does not synchronise. */
 int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_frames, int width, int height, int quality,
                                     uint8_t* d_out, size_t out_stride, uint64_t* d_len);
+/* The grey twin: the bytes of cv2.imwrite / cv2.imencode(".jpg", plane, [IMWRITE_JPEG_QUALITY, quality]) for a 2-D u8 plane -
+ * one component (h = v = 1, quantisation table 0, Huffman tables 0), an MCU of one block, the right and bottom edges
+ * replicated into the last blocks, JFIF APP0.  Same slot layout, refusals and guarantees as the bgr8 call, with
+ * uwip_jpeg_encode_u8_bound in place of uwip_jpeg_encode_bound. */
+size_t uwip_jpeg_encode_u8_bound(int width, int height);
+int uwip_jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_frames, int width, int height, int quality,
+                                  uint8_t* d_out, size_t out_stride, uint64_t* d_len);
 
 /* Batched decoder whose pixels equal cv2.imread / cv2.imdecode(file, IMREAD_COLOR) with libjpeg-turbo (islow IDCT, fancy
  * upsampling, csrc/jpegdec.h restates the arithmetic), the reader of the reference's command lines (histretch.cpp:158,
@@ -315,7 +331,13 @@ int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_f
  * synchronise.  n_frames <= 65535. */
 int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
                                 uint8_t* d_bgr, int width, int height);
-/* per-frame statistics of the last uwip_jpeg_decode_bgr8_batch call (synchronises): stats[2f] = subsequence decodes the
+/* The grey twin: the u8 planes cv2.imdecode(file, IMREAD_GRAYSCALE) returns, contiguous at d_planes.  For a grey file these
+ * are its samples; for a YCbCr file its Y component (islow and range limit, cropped; the chroma is entropy-decoded but not
+ * transformed), which is not cvtColor(BGR2GRAY) of the colour pixels.  Accepts, refuses and flags exactly as
+ * uwip_jpeg_decode_bgr8_batch. */
+int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
+                              uint8_t* d_planes, int width, int height);
+/* per-frame statistics of the last batched JPEG decode (either reader; synchronises): stats[2f] = subsequence decodes the
  * in-CTA synchronisation repeated, stats[2f + 1] = subsequences the cross-CTA fix-up re-decoded. */
 int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n_frames, int32_t* stats);
 

@@ -70,6 +70,7 @@ SIGNATURES = {
     "uwip_aclahe_bgr8_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, _d, _i, _i, _i]),
     "uwip_aclahe_params_u8_dev": (_i, [_P, _u8p, _i, _i, _i, _i, _P, _P]),
     "uwip_aclahe_bgr8_auto_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, _i, _i, _d, _i, _i, _P, _P]),
+    "uwip_aclahe_u8_auto_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, _i, _d, _i, _i, _P, _P]),
     "uwip_dehaze_defaults": (None, [C.POINTER(DehazeParams)]),
     "uwip_chain_defaults": (None, [C.POINTER(ChainParams)]),
     "uwip_boxfilter_f64": (_i, [_P, _P, _i, _i, _i, _P]),
@@ -90,7 +91,10 @@ SIGNATURES = {
     "uwip_chain_jpeg": (_i, [_P, _u8p, _sz, C.POINTER(ChainParams), _i, _u8p, _sz, C.POINTER(_sz)]),
     "uwip_jpeg_encode_bound": (_sz, [_i, _i]),
     "uwip_jpeg_encode_bgr8_batch_dev": (_i, [_P, _u8p, _i, _i, _i, _i, _u8p, _sz, _P]),
+    "uwip_jpeg_encode_u8_bound": (_sz, [_i, _i]),
+    "uwip_jpeg_encode_u8_batch_dev": (_i, [_P, _u8p, _i, _i, _i, _i, _u8p, _sz, _P]),
     "uwip_jpeg_decode_bgr8_batch": (_i, [_P, _P, _P, _i, _u8p, _i, _i]),
+    "uwip_jpeg_decode_u8_batch": (_i, [_P, _P, _P, _i, _u8p, _i, _i]),
     "uwip_jpeg_decode_stats": (_i, [_P, _i, _P]),
     "uwip_calc_blur_bgr8": (_i, [_P, _u8p, _sz, _i, _i, _i, C.POINTER(C.c_float), C.POINTER(_d), _u8p, _sz]),
     "uwip_calc_blur_bgr8_dev": (_i, [_P, _u8p, _i, _i, _i, _i, _P]),

@@ -330,14 +330,18 @@ class Context:
         d = d_frames.unsqueeze(0) if d_frames.dim() == 3 else d_frames
         if d.dtype != torch.uint8 or d.dim() != 4 or d.shape[3] != 3 or not d.is_cuda:
             raise ValueError("expected a uint8 CUDA tensor (N, H, W, 3)")
+        return self._jpeg_encode_batch(d, quality, self.jpeg_encode_bound(d.shape[2], d.shape[1]), self.lib.uwip_jpeg_encode_bgr8_batch_dev)
+
+    def _jpeg_encode_batch(self, d, quality, stride, encode):
+        import torch
+
         n, h, w = d.shape[:3]
-        stride = self.jpeg_encode_bound(w, h)
         with torch.cuda.device(d.device):
             d = d.contiguous()
             d_out = torch.empty((n, max(stride, 1)), dtype=torch.uint8, device=d.device)
             d_len = torch.empty(n, dtype=torch.int64, device=d.device)
             torch.cuda.current_stream().synchronize()   # the frames are complete before the context's stream reads them
-            self._ck(self.lib.uwip_jpeg_encode_bgr8_batch_dev(self.h, _ptr(d), n, w, h, int(quality), _ptr(d_out), stride, _ptr(d_len)))
+            self._ck(encode(self.h, _ptr(d), n, w, h, int(quality), _ptr(d_out), stride, _ptr(d_len)))
             self.synchronize()
             lens = d_len.cpu().tolist()
             return [d_out[f, :lens[f]].cpu().numpy().tobytes() for f in range(n)]
@@ -352,11 +356,47 @@ class Context:
             out = self.jpeg_encode_batch_dev(torch.from_numpy(a).to("cuda"), quality)
         return out[0] if single else out
 
+    def jpeg_encode_grey_bound(self, width, height):
+        """Largest file uwip_jpeg_encode_u8_batch_dev can write for one width x height plane (0 outside 1..65535)."""
+        return int(self.lib.uwip_jpeg_encode_u8_bound(int(width), int(height)))
+
+    def jpeg_encode_grey_batch_dev(self, d_planes, quality=95):
+        """Device grey planes (torch uint8 tensor (N, H, W) or (H, W)) -> list of N files, each the bytes of
+        cv2.imencode(".jpg", plane, [cv2.IMWRITE_JPEG_QUALITY, quality]) (one-component JPEG), encoded in one device call."""
+        import torch
+
+        d = d_planes.unsqueeze(0) if d_planes.dim() == 2 else d_planes
+        if d.dtype != torch.uint8 or d.dim() != 3 or not d.is_cuda:
+            raise ValueError("expected a uint8 CUDA tensor (N, H, W)")
+        return self._jpeg_encode_batch(d, quality, self.jpeg_encode_grey_bound(d.shape[2], d.shape[1]), self.lib.uwip_jpeg_encode_u8_batch_dev)
+
+    def jpeg_encode_grey(self, planes, quality=95):
+        """Host grey planes (N, H, W) -> list of N files; one plane (H, W) -> its file: cv2.imencode's bytes, encoded on the
+        device."""
+        import torch
+
+        a = np.asarray(planes)
+        single = a.ndim == 2
+        if a.dtype != np.uint8 or a.ndim not in (2, 3):
+            raise ValueError("expected uint8 (N, H, W) or (H, W)")
+        with torch.cuda.device(self.device):
+            out = self.jpeg_encode_grey_batch_dev(torch.from_numpy(np.ascontiguousarray(a)).to("cuda"), quality)
+        return out[0] if single else out
+
     # ---- JPEG files decoded as cv2.imdecode does (csrc/jpegdec.cu) ---------------------------------------------------
     def jpeg_decode_batch_dev(self, files, d_out=None):
         """JPEG files of one size (a list of bytes, or one bytes object) -> torch uint8 CUDA tensor (N, H, W, 3) holding
         cv2.imdecode(file, cv2.IMREAD_COLOR) of each, decoded in one device call.  A file with bad entropy-coded data decodes
         to zeros and sets bit 4 of last_frame_flags(N)."""
+        return self._jpeg_decode_batch(files, d_out, 3, self.lib.uwip_jpeg_decode_bgr8_batch)
+
+    def jpeg_decode_grey_batch_dev(self, files, d_out=None):
+        """JPEG files of one size -> torch uint8 CUDA tensor (N, H, W) holding cv2.imdecode(file, cv2.IMREAD_GRAYSCALE) of
+        each (for a colour file its Y component), decoded in one device call.  Bad entropy-coded data: zeros and bit 4 of
+        last_frame_flags(N)."""
+        return self._jpeg_decode_batch(files, d_out, 1, self.lib.uwip_jpeg_decode_u8_batch)
+
+    def _jpeg_decode_batch(self, files, d_out, channels, decode):
         import torch
 
         if isinstance(files, (bytes, bytearray, memoryview)):
@@ -366,15 +406,23 @@ class Context:
         if n == 0:
             raise ValueError("no files")
         w, h = self.jpeg_info(bufs[0])
+        shape = (n, h, w, 3) if channels == 3 else (n, h, w)
         if d_out is None:
-            d_out = torch.empty((n, h, w, 3), dtype=torch.uint8, device="cuda:%d" % self.device)
-        elif d_out.dtype != torch.uint8 or not d_out.is_cuda or not d_out.is_contiguous() or d_out.numel() != n * h * w * 3:
-            raise ValueError("d_out must be a contiguous uint8 CUDA tensor of N x H x W x 3 elements")
+            d_out = torch.empty(shape, dtype=torch.uint8, device="cuda:%d" % self.device)
+        elif d_out.dtype != torch.uint8 or not d_out.is_cuda or not d_out.is_contiguous() or d_out.numel() != n * h * w * channels:
+            raise ValueError("d_out must be a contiguous uint8 CUDA tensor of %s elements" % " x ".join(("N", "H", "W", "3")[:len(shape)]))
         ptrs = (C.c_void_p * n)(*[b.ctypes.data for b in bufs])
         lens = (C.c_size_t * n)(*[b.size for b in bufs])
-        self._ck(self.lib.uwip_jpeg_decode_bgr8_batch(self.h, ptrs, lens, n, _ptr(d_out), w, h))
+        self._ck(decode(self.h, ptrs, lens, n, _ptr(d_out), w, h))
         self.synchronize()
         return d_out
+
+    def jpeg_decode_grey(self, files):
+        """JPEG files of one size -> numpy uint8 (N, H, W) equal to cv2.imdecode(file, cv2.IMREAD_GRAYSCALE); one bytes object
+        -> (H, W).  Decoded on the device."""
+        single = isinstance(files, (bytes, bytearray, memoryview))
+        out = self.jpeg_decode_grey_batch_dev(files).cpu().numpy()
+        return out[0] if single else out
 
     def jpeg_decode(self, files):
         """JPEG files of one size -> numpy uint8 (N, H, W, 3) equal to cv2.imdecode(file, cv2.IMREAD_COLOR); one bytes object
@@ -391,7 +439,7 @@ class Context:
         return out
 
     def last_frame_flags(self, n):
-        """Per-frame status bits of the last batched chain / bgdehaze / automatic-aclahe / exact JPEG decode call: 1 = the
+        """Per-frame status bits of the last batched chain / bgdehaze / automatic-aclahe / exact JPEG decode (bgr8 or grey) call: 1 = the
         reference output is NaN (D9), 2 = the automatic CLAHE fit failed (BS = CL = -1, fixed parameters used), 4 = the JPEG
         file's entropy-coded data is bad (the frame is zeros)."""
         out = np.empty(n, np.int32)
@@ -424,6 +472,13 @@ class Context:
                                                     HSV_ROUND[hsv_round], float(clip), int(tiles[0]), int(tiles[1]),
                                                     _ptr(d_bs) if d_bs is not None else None,
                                                     _ptr(d_cl) if d_cl is not None else None))
+
+    def aclahe_grey_auto_dev(self, d_src, d_dst, n, width, height, loop="repaired", clip=2.0, tiles=(8, 8), d_bs=None, d_cl=None):
+        """main.py:18-20 on n device grey planes: each plane's automatic (BS, CL), then CLAHE of the plane with them; clip and
+        tiles apply to planes whose fit failed (BS = CL = -1, bit 2 of last_frame_flags).  Stream ordered."""
+        self._ck(self.lib.uwip_aclahe_u8_auto_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, ACLAHE_LOOP[loop], float(clip),
+                                                  int(tiles[0]), int(tiles[1]), _ptr(d_bs) if d_bs is not None else None,
+                                                  _ptr(d_cl) if d_cl is not None else None))
 
     def clahe_dev(self, d_src, d_dst, n, width, height, clip=40.0, tiles=(8, 8)):
         self._ck(self.lib.uwip_clahe_u8_dev(self.h, _ptr(d_src), _ptr(d_dst), n, width, height, float(clip), int(tiles[0]), int(tiles[1])))

@@ -5,7 +5,17 @@ entropy table and stops at its TODO list (find the knee, pick the block size, ap
 aclahe.cpp:209-218).  This shim prints the same table (one pixel pass per grid on the GPU) and then carries the TODO list
 out with the procedure of the Python prototype (ACLAHE.py:69-129): knee of the entropy curve -> clip limit, float16
 arg-max -> block size, CLAHE on V, HSV -> BGR, imwrite.  `-grey=1` is the Python main.py: grey image in, CLAHE image out.
+
+aclahe <input> <output> -grey=1 -device=1 [-q=95] [-loop=repaired|as_committed]
+aclahe <input dir> <output dir> -grey=1 -device=1 [-q=95] [-loop=..] [-batch=64]
+      main.py with the whole procedure on the device (uwip_aclahe_u8_auto_dev): a JPEG input is read by the project's grey
+      reader (the pixels of cv2.imread(input, 0)), any other format by cv2.imread(input, 0); a .jpg output is written by the
+      project's grey writer (the bytes of cv2.imwrite), any other format by cv2.imwrite.  When the curve fit fails (the
+      reference raises), the fixed 8x8 grid and clip 2 are used and a note is printed.  When both arguments are directories,
+      every *.jpg / *.jpeg of the input directory is processed into the output directory under the same name, grouped by
+      size and in batches of -batch planes; each file's name, BS, CL and notes are printed.
 """
+import os
 import sys
 
 
@@ -13,7 +23,14 @@ def main(argv=None):
     argv = sys.argv[1:] if argv is None else argv
     from ._args import parse
 
-    pos, opt, err = parse(argv, {"grey": (0, int), "loop": ("repaired", str), "help": (False, bool)})
+    pos, opt, err = parse(argv, {"grey": (0, int), "loop": ("repaired", str), "device": (0, int), "q": (95, int), "batch": (64, int),
+                                 "help": (False, bool)})
+    if opt["device"] and not opt["grey"]:
+        err.append("-device=1 needs -grey=1")
+    if opt["device"] and opt["loop"] not in ("repaired", "as_committed"):
+        err.append("-loop must be repaired or as_committed")
+    if opt["batch"] < 1:
+        err.append("-batch must be at least 1")
     print("ACLAHE: Automatic Contrast Limited Adaptive Histogram Equalization (B200 build)")
     if len(pos) < 2 or opt.get("help"):
         print("\n\tExample:\n\t$ aclahe input.jpg output.jpg")
@@ -33,6 +50,12 @@ def main(argv=None):
     print("Input:", pos[0])
     print("Output:", pos[1])
     ctx = default_context()
+    if opt["device"]:
+        src, dst = pos[0], pos[1]
+        if os.path.isdir(src) and os.path.isdir(dst):
+            names = sorted(f for f in os.listdir(src) if f.lower().endswith((".jpg", ".jpeg")) and os.path.isfile(os.path.join(src, f)))
+            return _grey_device(ctx, [(os.path.join(src, f), os.path.join(dst, f)) for f in names], opt, True)
+        return _grey_device(ctx, [(src, dst)], opt, False)
     if opt["grey"]:
         img = cv2.imread(pos[0], 0)
         if img is None:
@@ -55,6 +78,62 @@ def main(argv=None):
     BS, CL = A.ParametrosACLAHE(v, loop=opt["loop"])
     print("BS = %d, CL = %g" % (BS, CL))
     cv2.imwrite(pos[1], ctx.aclahe(src, float(CL), (BS, BS)))
+    return 0
+
+
+def _grey_device(ctx, jobs, opt, named):
+    """jobs: (input path, output path) pairs, grouped by size and run in batches of opt['batch'] planes through the grey
+    reader (JPEG) or cv2.imread(.., 0), uwip_aclahe_u8_auto_dev, and the grey writer (.jpg) or cv2.imwrite.  named: each
+    file's report starts with its name (directory mode)."""
+    import cv2
+    import torch
+
+    from .chain import _notes
+
+    groups = {}
+    for src, dst in jobs:
+        if src.lower().endswith((".jpg", ".jpeg")):
+            with open(src, "rb") as f:
+                data = f.read()
+            item = (dst, data, None)
+            size = ctx.jpeg_info(data)
+        else:
+            img = cv2.imread(src, 0)
+            if img is None:
+                print("Failed to read input image, exiting...")
+                return -1
+            item = (dst, None, img)
+            size = (img.shape[1], img.shape[0])
+        groups.setdefault(size, []).append(item)
+    dev = "cuda:%d" % ctx.device
+    for (w, h), items in groups.items():
+        for b0 in range(0, len(items), opt["batch"]):
+            part = items[b0:b0 + opt["batch"]]
+            n = len(part)
+            if part[0][1] is not None:   # one JPEG job per batch unless in directory mode, which reads only JPEG files
+                d_in = ctx.jpeg_decode_grey_batch_dev([data for _, data, _ in part])
+                dflags = ctx.last_frame_flags(n)   # read now: the CLAHE call resets the flags
+            else:
+                d_in = torch.from_numpy(part[0][2]).to(dev)[None]
+                dflags = [0]
+            d_out = torch.empty_like(d_in)
+            d_bs = torch.empty(n, dtype=torch.int32, device=dev)
+            d_cl = torch.empty(n, dtype=torch.int32, device=dev)
+            ctx.aclahe_grey_auto_dev(d_in, d_out, n, w, h, loop=opt["loop"], d_bs=d_bs, d_cl=d_cl)
+            flags = ctx.last_frame_flags(n)   # waits for the context's stream, which writes BS and CL
+            bs, cl = d_bs.cpu().tolist(), d_cl.cpu().tolist()
+            jpeg_out = [i for i, (dst, _, _) in enumerate(part) if dst.lower().endswith((".jpg", ".jpeg"))]
+            files = dict(zip(jpeg_out, ctx.jpeg_encode_grey_batch_dev(d_out[jpeg_out], opt["q"]))) if jpeg_out else {}
+            for i, (dst, _, _) in enumerate(part):
+                if i in files:
+                    with open(dst, "wb") as f:
+                        f.write(files[i])
+                else:
+                    cv2.imwrite(dst, d_out[i].cpu().numpy(), [cv2.IMWRITE_JPEG_QUALITY, opt["q"]])
+                print(*([os.path.basename(dst) + ":"] if named else []), "BS = %d, CL = %g" % (bs[i], cl[i]))
+                _notes(int(dflags[i]) | int(flags[i]))
+                if named:
+                    print("saved", dst)
     return 0
 
 

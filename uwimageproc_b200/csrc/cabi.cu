@@ -480,6 +480,16 @@ int uwip_aclahe_bgr8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_ds
   UWIP_CHECK(aclahe_frames_auto_dev(ctx, d_src, d_dst, n, w, h, loop, clip, tx, ty, hsv_round, nullptr, nullptr, d_bs, d_cl));
   return aclahe_nofit_flags(ctx, d_cl, n, flags, false);
 }
+int uwip_aclahe_u8_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty,
+                            int32_t* d_bs, int32_t* d_cl) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, d_src && d_dst && n > 0 && w > 0 && h > 0, "bad argument");
+  UWIP_CHECK(auto_outputs(ctx, n, d_bs, d_cl));
+  int32_t* flags = flags_get(ctx, n);
+  if (!flags) return UWIP_ERR_NOMEM;
+  UWIP_CHECK(aclahe_planes_auto_dev(ctx, d_src, d_dst, n, w, h, loop, clip, tx, ty, d_bs, d_cl));
+  return aclahe_nofit_flags(ctx, d_cl, n, flags, false);
+}
 
 // ---- videostrip calcBlur ------------------------------------------------------------------------------
 int uwip_calc_blur_bgr8_dev(uwip_ctx* ctx, const uint8_t* d_src, int n, int w, int h, int aperture, double* d_mean_std) {
@@ -861,16 +871,40 @@ int uwip_jpeg_encode_bgr8_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n_f
   UWIP_REQUIRE(ctx, out_stride >= jpeg_encode_bound(width, height), "out_stride is below uwip_jpeg_encode_bound(width, height)");
   return jpeg_encode_batch_dev(ctx, d_bgr, n_frames, width, height, quality, d_out, out_stride, d_len);
 }
+size_t uwip_jpeg_encode_u8_bound(int width, int height) {
+  if (width < 1 || width > 65535 || height < 1 || height > 65535) return 0;
+  return jpeg_encode_u8_bound(width, height);
+}
+int uwip_jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_frames, int width, int height, int quality, uint8_t* d_out,
+                                  size_t out_stride, uint64_t* d_len) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, d_planes && d_out && d_len && n_frames > 0, "bad argument");
+  UWIP_REQUIRE(ctx, width >= 1 && width <= 65535 && height >= 1 && height <= 65535, "width and height must lie in 1..65535");
+  UWIP_REQUIRE(ctx, quality >= 1 && quality <= 100, "quality must lie in 1..100");
+  UWIP_REQUIRE(ctx, out_stride >= jpeg_encode_u8_bound(width, height), "out_stride is below uwip_jpeg_encode_u8_bound(width, height)");
+  return jpeg_encode_u8_batch_dev(ctx, d_planes, n_frames, width, height, quality, d_out, out_stride, d_len);
+}
 
+// the argument checks of the two batched readers (in the caller, whose name the messages carry)
+#define DECODE_BATCH_REQUIRE(ctx, d_out)                                                                                         \
+  UWIP_REQUIRE(ctx, jpegs && lens && d_out && n_frames > 0 && n_frames <= 65535, "bad argument (n_frames must lie in 1..65535)"); \
+  UWIP_REQUIRE(ctx, width >= 1 && width <= 65500 && height >= 1 && height <= 65500, "width and height must lie in 1..65500");    \
+  for (int f = 0; f < n_frames; f++) UWIP_REQUIRE(ctx, jpegs[f] && lens[f] > 0, "a file pointer is NULL or a length is 0")
 int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_bgr, int width,
                                 int height) {
   CTX_GUARD(ctx);
-  UWIP_REQUIRE(ctx, jpegs && lens && d_bgr && n_frames > 0 && n_frames <= 65535, "bad argument (n_frames must lie in 1..65535)");
-  UWIP_REQUIRE(ctx, width >= 1 && width <= 65500 && height >= 1 && height <= 65500, "width and height must lie in 1..65500");
-  for (int f = 0; f < n_frames; f++) UWIP_REQUIRE(ctx, jpegs[f] && lens[f] > 0, "a file pointer is NULL or a length is 0");
+  DECODE_BATCH_REQUIRE(ctx, d_bgr);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false);
+}
+int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_planes, int width,
+                              int height) {
+  CTX_GUARD(ctx);
+  DECODE_BATCH_REQUIRE(ctx, d_planes);
+  int32_t* flags = flags_get(ctx, n_frames);
+  if (!flags) return UWIP_ERR_NOMEM;
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true);
 }
 int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n, int32_t* stats_host) {
   CTX_GUARD(ctx);

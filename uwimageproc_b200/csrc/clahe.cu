@@ -801,31 +801,26 @@ int aclahe_params_planes_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int 
   return UWIP_OK;
 }
 
-// BGR->HSV, CLAHE on V with each frame's own (BS, CL), HSV->BGR on n frames (optionally behind the fused histretch head and
-// with the dehaze min / max, like aclahe_frames_dev).  The parameters are found on the V plane of the frame that enters CLAHE;
-// frames whose fit fails (CL = -1) get the fixed clip / tx x ty.
-int aclahe_frames_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty,
-                           int hsv_round, const uint8_t* d_prelut, FrameState* fs, int* d_bs, int* d_cl) {
+// the refusals of the automatic calls: the fallback grid must suit the image and the image the five automatic grids
+static int aclahe_auto_check(uwip_ctx* ctx, int n, int w, int h, int tx, int ty) {
   UWIP_REQUIRE(ctx, tx >= 1 && ty >= 1 && tx <= 256 && ty <= 256, "tile grid out of range");
   UWIP_REQUIRE(ctx, w >= 1 && h >= 1 && n >= 1, "bad size");
   const TileGeom gf = make_geom(w, h, tx, ty);
   UWIP_REQUIRE(ctx, (gf.EW == w || 2 * w - 2 >= gf.EW - 1 || w == 1) && (gf.EH == h || 2 * h - 2 >= gf.EH - 1 || h == 1),
                "image too small for this tile grid (reflect-101 padding undefined)");
-  UWIP_CHECK(aclahe_check_auto_size(ctx, w, h));
-  const size_t n_px = (size_t)w * h;
-  const int bw = body_width(w, hsv_round);
-  uint8_t* d_v = (uint8_t*)uwip_slot(ctx, SLOT_APLANE, (size_t)n * n_px);
-  if (!d_v) return UWIP_ERR_NOMEM;
-  uint8_t* d_pre2 = nullptr;
-  if (d_prelut) {
-    d_pre2 = (uint8_t*)uwip_slot(ctx, SLOT_LUT, (size_t)n * 256 * 4) + (size_t)n * 256;  // second half of the LUT slot
-    if (!d_pre2) return UWIP_ERR_NOMEM;
-    UWIP_LAUNCH(ctx, "prelut2", prelut2_kernel, n, 256, 0, d_prelut, d_pre2);
-  }
-  UWIP_LAUNCH(ctx, "aclahe_vplane", vplane_kernel, dim3(std::max(1, std::min(cdiv((int)std::min<size_t>(n_px, 1 << 30), 256), 1024)), n), 256, 0,
-              d_src, w, h, (const uint8_t*)d_pre2, bw, d_v);
-  UWIP_CHECK(aclahe_params_planes_dev(ctx, d_v, n, w, h, loop, d_bs, d_cl));
+  return aclahe_check_auto_size(ctx, w, h);
+}
+
+// The parameter search on the n planes d_search, then CLAHE of d_src into d_dst with each frame's own (BS, CL); frames
+// whose fit fails (CL = -1) get the fixed clip / tx x ty.  FRAME: bgr8 frames, CLAHE on the V of HSV (optionally behind
+// the fused histretch head: d_pre2, d_prelut, bw) with the dehaze min / max into fs; otherwise u8 planes.
+template <bool FRAME>
+static int aclahe_auto_core(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, const uint8_t* d_search, int n, int w, int h, int loop,
+                            double clip, int tx, int ty, const uint8_t* d_pre2, const uint8_t* d_prelut, int bw, FrameState* fs,
+                            int* d_bs, int* d_cl) {
+  UWIP_CHECK(aclahe_params_planes_dev(ctx, d_search, n, w, h, loop, d_bs, d_cl));
   // per-frame geometry in the PF workspace: tpf tiles per frame
+  const TileGeom gf = make_geom(w, h, tx, ty);
   const int tpf = std::max(AUTO_TPF, tx * ty);
   char* d_ws = (char*)uwip_slot(ctx, SLOT_AUTO, 0);   // the params call sized it: [2][49] doubles, then FrameClahe[5][n]
   FrameClahe* d_pf = (FrameClahe*)(d_ws + 256 * 8);   // reuses the pick's [0][n] block, consumed by then in stream order
@@ -840,19 +835,51 @@ int aclahe_frames_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, 
   UWIP_CUDA(ctx, cudaMemsetAsync(d_th, 0, (size_t)n * tpf * 256 * 4, ctx->stream));
   // row splits sized for the coarsest grid (2 x 2: the tallest tiles); finer grids leave the upper splits idle
   const int splits = pick_splits(ctx, make_geom(w, h, 2, 2), n);
-  UWIP_LAUNCH(ctx, "clahe_tilehist", (tilehist_kernel<true, true>), dim3(tpf, splits, n), TH_THREADS, 0, d_src, gf, splits,
-              (const uint8_t*)d_pre2, bw, d_th, (const FrameClahe*)d_pf, tpf);
+  UWIP_LAUNCH(ctx, "clahe_tilehist", (tilehist_kernel<FRAME, true>), dim3(tpf, splits, n), TH_THREADS, 0, d_src, gf, splits,
+              d_pre2, bw, d_th, (const FrameClahe*)d_pf, tpf);
   UWIP_LAUNCH(ctx, "clahe_lut", clahe_lut_kernel<true>, (unsigned)((size_t)tpf * n), 256, 0, d_th, (const int*)nullptr, 1, 0.f, d_tl,
               (const FrameClahe*)d_pf, tpf);
   int rows_per = 8;
   while (rows_per > 1 && (long long)cdiv(h, rows_per) * n < (long long)ctx->sm_count * 4) rows_per /= 2;
   dim3 grid3(cdiv(h, rows_per), n);
   const size_t smem = (size_t)3 * 32 * 256;   // staged LUT rows of grids up to 32 tiles wide
-  if (d_prelut)
+  if (!FRAME)
+    UWIP_LAUNCH(ctx, "clahe_apply", (clahe_apply_kernel<0, false, true>), grid3, AP_THREADS, smem, d_src, d_dst, gf, rows_per, d_tl,
+                d_prelut, bw, fs, (const FrameClahe*)d_pf, tpf);
+  else if (d_prelut)
     UWIP_LAUNCH(ctx, "clahe_apply", (clahe_apply_kernel<1, true, true>), grid3, AP_THREADS, smem, d_src, d_dst, gf, rows_per, d_tl, d_prelut,
                 bw, fs, (const FrameClahe*)d_pf, tpf);
   else
     UWIP_LAUNCH(ctx, "clahe_apply", (clahe_apply_kernel<1, false, true>), grid3, AP_THREADS, smem, d_src, d_dst, gf, rows_per, d_tl,
                 d_prelut, bw, fs, (const FrameClahe*)d_pf, tpf);
   return UWIP_OK;
+}
+
+// BGR->HSV, CLAHE on V with each frame's own (BS, CL), HSV->BGR on n frames (optionally behind the fused histretch head and
+// with the dehaze min / max, like aclahe_frames_dev).  The parameters are found on the V plane of the frame that enters CLAHE;
+// frames whose fit fails (CL = -1) get the fixed clip / tx x ty.
+int aclahe_frames_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty,
+                           int hsv_round, const uint8_t* d_prelut, FrameState* fs, int* d_bs, int* d_cl) {
+  UWIP_CHECK(aclahe_auto_check(ctx, n, w, h, tx, ty));
+  const size_t n_px = (size_t)w * h;
+  const int bw = body_width(w, hsv_round);
+  uint8_t* d_v = (uint8_t*)uwip_slot(ctx, SLOT_APLANE, (size_t)n * n_px);
+  if (!d_v) return UWIP_ERR_NOMEM;
+  uint8_t* d_pre2 = nullptr;
+  if (d_prelut) {
+    d_pre2 = (uint8_t*)uwip_slot(ctx, SLOT_LUT, (size_t)n * 256 * 4) + (size_t)n * 256;  // second half of the LUT slot
+    if (!d_pre2) return UWIP_ERR_NOMEM;
+    UWIP_LAUNCH(ctx, "prelut2", prelut2_kernel, n, 256, 0, d_prelut, d_pre2);
+  }
+  UWIP_LAUNCH(ctx, "aclahe_vplane", vplane_kernel, dim3(std::max(1, std::min(cdiv((int)std::min<size_t>(n_px, 1 << 30), 256), 1024)), n), 256, 0,
+              d_src, w, h, (const uint8_t*)d_pre2, bw, d_v);
+  return aclahe_auto_core<true>(ctx, d_src, d_dst, d_v, n, w, h, loop, clip, tx, ty, d_pre2, d_prelut, bw, fs, d_bs, d_cl);
+}
+
+// main.py:18-20 on n u8 planes: the parameters of each plane (found on its blurred copy, ACLAHE.py:15), then CLAHE of the
+// unblurred plane with them; planes whose fit fails get the fixed clip / tx x ty.
+int aclahe_planes_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty,
+                           int* d_bs, int* d_cl) {
+  UWIP_CHECK(aclahe_auto_check(ctx, n, w, h, tx, ty));
+  return aclahe_auto_core<false>(ctx, d_src, d_dst, d_src, n, w, h, loop, clip, tx, ty, nullptr, nullptr, 0, nullptr, d_bs, d_cl);
 }

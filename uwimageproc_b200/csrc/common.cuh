@@ -379,6 +379,7 @@ int clahe_entropy_sweep_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n,
 int aclahe_check_auto_size(uwip_ctx* ctx, int w, int h);   // UWIP_ERR_INVALID when a plane is too small for a grid of 2..32
 int aclahe_params_planes_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int loop, int* d_bs, int* d_cl);
 int aclahe_frames_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty, int hsv_round, const uint8_t* d_prelut, FrameState* fs_minmax, int* d_bs, int* d_cl);
+int aclahe_planes_auto_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n, int w, int h, int loop, double clip, int tx, int ty, int* d_bs, int* d_cl);
 int aclahe_nofit_flags(uwip_ctx* ctx, const int* d_cl, int n, int32_t* d_flags, bool keep);   // flags |= NOFIT where CL < 0
 
 // aclahe_knee.cu
@@ -409,12 +410,15 @@ void jpeg_io_destroy(uwip_ctx* ctx);
 
 // jpegenc.cu
 size_t jpeg_encode_bound(int w, int h);
+size_t jpeg_encode_u8_bound(int w, int h);
 int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
                           uint64_t* d_len);
+int jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
+                             uint64_t* d_len);
 
-// jpegdec.cu
-int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_bgr, int w, int h,
-                      int32_t* d_flags);
+// jpegdec.cu: d_out receives bgr8 frames, or grey planes (IMREAD_GRAYSCALE) when grey is set
+int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_out, int w, int h,
+                      int32_t* d_flags, bool grey);
 void jpeg_dec_destroy(uwip_ctx* ctx);
 
 // synth.cu

@@ -1,5 +1,5 @@
-// jpegdec.cu - batched sequential JPEG decoder whose pixels equal cv2.imdecode(file, IMREAD_COLOR) / libjpeg-turbo (SURVEY 8f
-// row N3, the read half of the device path).  The arithmetic is csrc/jpegdec.h; this file spreads it over the GPU.  The
+// jpegdec.cu - batched sequential JPEG decoder whose pixels equal cv2.imdecode(file, IMREAD_COLOR) or
+// cv2.imdecode(file, IMREAD_GRAYSCALE) / libjpeg-turbo (SURVEY 8f row N3, the read half of the device path).  The arithmetic is csrc/jpegdec.h; this file spreads it over the GPU.  The
 // headers are parsed on the host (the files come from there): per-frame tables and geometry go to the device in one copy, the
 // entropy-coded segments, concatenated in a pinned staging buffer, in another.  Then every launch covers all n frames:
 //   destuff  a CTA per frame: the segment without the 0x00 after each 0xFF, fill bytes and RST markers, and the byte offset
@@ -18,6 +18,8 @@
 //            blocks in natural order, DC as values
 //   idct     a thread per block: jpeg_idct_islow into the padded sample planes
 //   color    a thread per output pixel: upsampling with its one-row / one-column context and YCbCr -> B,G,R, cropped to W x H
+// Grey output (IMREAD_GRAYSCALE) runs the same passes up to huff; then the idct of the component-0 blocks only and a grey
+// pass that crops the Y plane (jdcolor.c grayscale_convert: no chroma IDCT, upsampling or colour conversion).
 // Bad entropy-coded data (an invalid code, a coefficient past 63, the data ending before the last block, the wrong number of
 // RST markers) leaves the frame all zeros and sets UWIP_FRAME_JPEG_BAD.  A frame's pixels do not depend on the batch it is in.
 #include <algorithm>
@@ -380,6 +382,8 @@ __global__ void __launch_bounds__(SYNC_T) jpeg_dec_huff_kernel(const FrameTab* _
   if (bad) atomicOr(flags + f, UWIP_FRAME_JPEG_BAD);
 }
 
+// Y_ONLY: the blocks of component 0 (grey output); the chroma blocks' threads exit
+template <bool Y_ONLY>
 __global__ void __launch_bounds__(IDCT_T) jpeg_dec_idct_kernel(const FrameTab* __restrict__ tabs, const int16_t* __restrict__ coef,
                                                                 uint8_t* __restrict__ smp) {
   __shared__ uint16_t s_q[3][64];
@@ -393,6 +397,7 @@ __global__ void __launch_bounds__(IDCT_T) jpeg_dec_idct_kernel(const FrameTab* _
   const int m = (int)(blk / g.bpm), bi = (int)(blk % g.bpm);
   int c, bx, by;
   jpegdec::block_pos(g, m, bi, c, bx, by);
+  if (Y_ONLY && c != 0) return;
   int16_t cb[64];
   const uint4* src = reinterpret_cast<const uint4*>(coef + (t.blk_off + blk) * 64);
 #pragma unroll
@@ -416,6 +421,21 @@ __global__ void __launch_bounds__(COLOR_T) jpeg_dec_color_kernel(const FrameTab*
   jpegdec::pixel(g, smp + t.smp_off, (int)(i % w), (int)(i / w), o);
 }
 
+__global__ void __launch_bounds__(COLOR_T) jpeg_dec_grey_kernel(const FrameTab* __restrict__ tabs, const uint8_t* __restrict__ smp,
+                                                                 const int32_t* __restrict__ flags, uint8_t* __restrict__ out, int w,
+                                                                 int h) {
+  const int f = blockIdx.y;
+  const size_t i = (size_t)blockIdx.x * COLOR_T + threadIdx.x;
+  if (i >= (size_t)w * h) return;
+  uint8_t* o = out + (size_t)f * w * h + i;
+  if (flags[f] & UWIP_FRAME_JPEG_BAD) {
+    *o = 0;
+    return;
+  }
+  const FrameTab& t = tabs[f];
+  *o = smp[t.smp_off + (i / w) * t.g.pw[0] + i % w];
+}
+
 size_t a16(size_t x) { return (x + 15) / 16 * 16; }
 
 }  // namespace
@@ -428,8 +448,9 @@ void jpeg_dec_destroy(uwip_ctx* ctx) {
   ctx->jdec_pinned_bytes = 0;
 }
 
-int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_bgr, int w, int h,
-                      int32_t* d_flags) {
+int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_out, int w, int h,
+                      int32_t* d_flags, bool grey) {
+  const char* fn = grey ? "uwip_jpeg_decode_u8_batch" : "uwip_jpeg_decode_bgr8_batch";
   // ---- parse every header on the host
   std::vector<FrameTab> tabs((size_t)n);
   jpegdec::Header hd;
@@ -439,14 +460,14 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
   for (int f = 0; f < n; f++) {
     const int rc = jpegdec::parse_header(jpegs[f], lens[f], hd);
     if (rc != jpegdec::OK) {
-      uwip_set_err(ctx, "uwip_jpeg_decode_bgr8_batch: file %d: %s", f,
+      uwip_set_err(ctx, "%s: file %d: %s", fn, f,
                    rc == jpegdec::UNSUPPORTED ? "coding not supported (progressive, arithmetic, lossless, 12-bit, multi-scan, CMYK, RGB "
                                                 "or sampling other than 4:4:4 / 4:2:2 / 4:4:0 / 4:2:0 / grey)"
                                               : "malformed or truncated header");
       return rc;
     }
     if (hd.width != w || hd.height != h) {
-      uwip_set_err(ctx, "uwip_jpeg_decode_bgr8_batch: file %d is %d x %d, not %d x %d", f, hd.width, hd.height, w, h);
+      uwip_set_err(ctx, "%s: file %d is %d x %d, not %d x %d", fn, f, hd.width, hd.height, w, h);
       return UWIP_ERR_INVALID;
     }
     FrameTab& t = tabs[f];
@@ -454,13 +475,13 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
     for (int c = 0; c < hd.ncomp; c++) {
       memcpy(t.q[c], hd.q[hd.comp[c].tq], sizeof(t.q[c]));
       if (!jpegdec::make_derived(hd.dc[hd.comp[c].td], true, t.dc[c]) || !jpegdec::make_derived(hd.ac[hd.comp[c].ta], false, t.ac[c])) {
-        uwip_set_err(ctx, "uwip_jpeg_decode_bgr8_batch: file %d: bad Huffman table", f);
+        uwip_set_err(ctx, "%s: file %d: bad Huffman table", fn, f);
         return UWIP_ERR_INVALID;
       }
     }
     t.seg_len = lens[f] - hd.scan_off;
     if (t.seg_len > (size_t)0x1FFFFFF0) {
-      uwip_set_err(ctx, "uwip_jpeg_decode_bgr8_batch: file %d: entropy-coded segment above 512 MB", f);
+      uwip_set_err(ctx, "%s: file %d: entropy-coded segment above 512 MB", fn, f);
       return UWIP_ERR_INVALID;
     }
     t.seg_off = seg_total;
@@ -543,9 +564,15 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
               (const uint32_t*)d_ibase, d_cd, d_px);
   UWIP_LAUNCH(ctx, "jpeg_dec_huff", jpeg_dec_huff_kernel, gsub, SYNC_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
               (const Sub*)d_sub, (const int*)d_nsub, (const uint64_t*)d_entry, (const int4*)d_cd, d_coef, d_flags);
-  UWIP_LAUNCH(ctx, "jpeg_dec_idct", jpeg_dec_idct_kernel, dim3((unsigned)((max_blocks + IDCT_T - 1) / IDCT_T), ny), IDCT_T, 0,
-              (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
-  UWIP_LAUNCH(ctx, "jpeg_dec_color", jpeg_dec_color_kernel, dim3((unsigned)(((size_t)w * h + COLOR_T - 1) / COLOR_T), ny), COLOR_T, 0,
-              (const FrameTab*)d_tab, (const uint8_t*)d_smp, (const int32_t*)d_flags, d_bgr, w, h);
+  const dim3 gblk((unsigned)((max_blocks + IDCT_T - 1) / IDCT_T), ny), gpix((unsigned)(((size_t)w * h + COLOR_T - 1) / COLOR_T), ny);
+  if (grey) {
+    UWIP_LAUNCH(ctx, "jpeg_dec_idct_y", jpeg_dec_idct_kernel<true>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
+    UWIP_LAUNCH(ctx, "jpeg_dec_grey", jpeg_dec_grey_kernel, gpix, COLOR_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_smp,
+                (const int32_t*)d_flags, d_out, w, h);
+  } else {
+    UWIP_LAUNCH(ctx, "jpeg_dec_idct", jpeg_dec_idct_kernel<false>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
+    UWIP_LAUNCH(ctx, "jpeg_dec_color", jpeg_dec_color_kernel, gpix, COLOR_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_smp,
+                (const int32_t*)d_flags, d_out, w, h);
+  }
   return UWIP_OK;
 }

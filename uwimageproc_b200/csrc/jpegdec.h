@@ -1,8 +1,12 @@
 // jpegdec.h - the sequential Huffman JPEG decoder of libjpeg-turbo 3.1.2 (the codec behind cv2.imread / cv2.imdecode of
-// cv2 4.13.0) as OpenCV drives it - JDCT_ISLOW, do_fancy_upsampling = TRUE, output JCS_EXT_BGR - restated in plain C++ that
-// compiles for the host and the device.  csrc/jpegdec.cu runs this arithmetic batched on the GPU; decode_frame() below is
-// the scalar reference for one frame, which only the host test compiles.  Every function names the libjpeg-turbo function
-// it restates.
+// cv2 4.13.0) as OpenCV drives it - JDCT_ISLOW, do_fancy_upsampling = TRUE, output JCS_EXT_BGR (IMREAD_COLOR) or
+// JCS_GRAYSCALE (IMREAD_GRAYSCALE) - restated in plain C++ that compiles for the host and the device.  csrc/jpegdec.cu runs
+// this arithmetic batched on the GPU; decode_frame() below is the scalar reference for one frame, which only the host test
+// compiles.  Every function names the libjpeg-turbo function it restates.
+//
+// Grey output of a YCbCr file is its Y component and nothing else: jdcolor.c's grayscale_convert copies component 0 and
+// marks Cb and Cr as not needed, so their blocks are entropy-decoded (the scan interleaves them) but never transformed,
+// upsampled or converted.  A different thing from cvtColor(BGR2GRAY) of the colour pixels.
 //
 // Accepted: baseline or extended sequential Huffman (SOF0, SOF1), 8-bit samples, one interleaved scan, one component (grey)
 // or three YCbCr components with Cb = Cr = 1x1 and Y 1x1, 2x1, 1x2 or 2x2 (4:4:4, 4:2:2, 4:4:0, 4:2:0), any restart
@@ -559,9 +563,10 @@ JPEG_HD inline int byte_kind(int prev, int b, int next) {   // prev / next: -1 o
 
 #ifndef __CUDA_ARCH__
 // The scalar reference of one frame: decode_mcu over the whole scan with process_restart, decompress_onepass's IDCTs, then
-// upsampling and colour conversion.  out: w * h * 3 bytes.  Returns OK, INVALID, UNSUPPORTED, or 1 for bad entropy-coded
-// data (the frame is then all zeros, as the batched decoder leaves it).
-inline int decode_frame(const uint8_t* data, size_t len, uint8_t* out) {
+// upsampling and colour conversion.  out: w * h * 3 bytes, or w * h for grey (IMREAD_GRAYSCALE: the IDCTs of component 0
+// only, cropped).  Returns OK, INVALID, UNSUPPORTED, or 1 for bad entropy-coded data (the frame is then all zeros, as the
+// batched decoder leaves it).
+inline int decode_frame(const uint8_t* data, size_t len, uint8_t* out, bool grey = false) {
   Header hd;
   int rc = parse_header(data, len, hd);
   if (rc != OK) return rc;
@@ -608,11 +613,13 @@ inline int decode_frame(const uint8_t* data, size_t len, uint8_t* out) {
           if (st.kind == 0) { pred[c] += st.v; blk[0] = (int16_t)pred[c]; }
           if (st.kind == 1) blk[natural_order(st.zz)] = (int16_t)st.v;
         } while (!st.done);
-        if (!bad) idct_islow(blk, hd.q[hd.comp[c].tq], smp + g.poff[c] + (size_t)8 * by * g.pw[c] + 8 * bx, g.pw[c]);
+        if (!bad && (!grey || c == 0)) idct_islow(blk, hd.q[hd.comp[c].tq], smp + g.poff[c] + (size_t)8 * by * g.pw[c] + 8 * bx, g.pw[c]);
       }
   }
   if (bad) {
-    memset(out, 0, (size_t)g.w * g.h * 3);
+    memset(out, 0, (size_t)g.w * g.h * (grey ? 1 : 3));
+  } else if (grey) {
+    for (int y = 0; y < g.h; y++) memcpy(out + (size_t)y * g.w, smp + (size_t)y * g.pw[0], g.w);
   } else {
     for (int y = 0; y < g.h; y++)
       for (int x = 0; x < g.w; x++) pixel(g, smp, x, y, out + ((size_t)y * g.w + x) * 3);

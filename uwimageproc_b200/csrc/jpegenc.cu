@@ -4,13 +4,17 @@
 // the work splits into five launches, each covering all n frames:
 //   setup   one thread: quantiser reciprocals, Huffman code tables and the header (they depend only on W, H and quality)
 //   blocks  a CTA per 32 MCUs: colour conversion, edge expansion and h2v2 in shared memory, one thread per block runs islow,
-//           quantises and stores the zig-zag int16 coefficients, their non-zero mask, the quantised DC and the AC code bits
+//           quantises and stores the zig-zag int16 coefficients, their non-zero mask, the quantised DC and the AC code bits.
+//           A grey plane (one component, an MCU of one block) has its own load: a thread per block reads its 8 x 8 samples
+//           with the edges replicated, then codes the block the same way.
 //   scan    a CTA per frame: MCU code lengths (DC differences taken across MCUs here) -> exclusive prefix sum = bit offsets
 //   emit    a thread per MCU writes its bits at its offset into the frame's bit buffer; only the words two MCUs share are
 //           combined with atomicOr (the scan zeroed them)
 //   stuff   a CTA per frame: header, the scan bytes with 0x00 after every 0xFF, EOI, and the file length
 // The unstuffed bit buffer of frame f lives in the tail of its own output slot (jpegenc::raw_capacity), so the only workspace
-// is the coefficient store of the blocks pass (about 3 B/px).  A frame's bytes do not depend on the batch it is in.
+// is the coefficient store of the blocks pass (about 3 B/px, 2 B/px grey).  A frame's bytes do not depend on the batch it is
+// in.  The scan, emit and stuff passes and the host sequence take the component count NC (3: 4:2:0, 1: grey) as a template
+// parameter: blocks per MCU, their tables and the header length follow from it (jpegenc.h).
 #include <algorithm>
 
 #include "common.cuh"
@@ -26,11 +30,12 @@ constexpr int MCUS_PER_CTA = 32;         // blocks pass: 32 MCUs x 6 blocks = 19
 constexpr int SCAN_THREADS = 1024;
 constexpr int EMIT_THREADS = 128;
 constexpr int STUFF_BYTES = 16;          // per thread and tile of the stuffing pass
+constexpr int GREY_BLOCKS_T = 128;       // blocks pass of a grey plane: a thread per block
 
 struct Tables {
   Recip q[2][64];   // natural order; 0 luma, 1 chroma
   Huff hf[4];       // DC0, AC0, DC1, AC1
-  uint8_t header[jpegenc::HEADER_BYTES];
+  uint8_t header[jpegenc::HEADER_BYTES];   // the longer of the two headers
 };
 
 struct BlockInfo {
@@ -40,17 +45,19 @@ struct BlockInfo {
 };
 
 // the frame's unstuffed bit buffer: 16-byte aligned, after room for the header and the stuffed copy of everything before it
+template <int NC>
 __host__ __device__ inline uint8_t* raw_buffer(uint8_t* out_f, size_t raw_cap) {
-  return (uint8_t*)(((uintptr_t)out_f + jpegenc::HEADER_BYTES + raw_cap + 2 + 15) & ~(uintptr_t)15);
+  return (uint8_t*)(((uintptr_t)out_f + jpegenc::header_bytes(NC) + raw_cap + 2 + 15) & ~(uintptr_t)15);
 }
 
 __device__ __forceinline__ uint32_t bswap32(uint32_t v) { return __byte_perm(v, 0, 0x0123); }
 
+template <int NC>
 __global__ void jpe_setup_kernel(Tables* __restrict__ t, int w, int h, int quality) {
   const int i = threadIdx.x;
   if (i < 128) t->q[i >> 6][i & 63] = jpegenc::compute_reciprocal((unsigned)jpegenc::quant_value(i >> 6, i & 63, quality) << 3);
   if (i < 4) jpegenc::make_derived(i, t->hf[i]);
-  if (i == 4) jpegenc::write_header(t->header, w, h, quality);
+  if (i == 4) jpegenc::write_header(t->header, w, h, quality, NC);
 }
 
 // 16 pixels of row y from column x0 (clamped at the right edge), as 48 bytes
@@ -68,6 +75,46 @@ __device__ __forceinline__ void load_row16(const uint8_t* __restrict__ frame, co
       px[3 * j] = row[3 * x]; px[3 * j + 1] = row[3 * x + 1]; px[3 * j + 2] = row[3 * x + 2];
     }
   }
+}
+
+// islow, quantisation and the zig-zag store (to cb) of one block whose samples minus 128 are d; its quantised DC goes to dc,
+// its non-zero mask, DC and AC code bits (acs: AC code lengths of its table) to bi
+__device__ __forceinline__ void code_block(int (&d)[64], const Recip* q, const uint8_t* acs, short* cb, int& dc, BlockInfo* bi) {
+#pragma unroll
+  for (int r = 0; r < 8; r++) jpegenc::fdct_1d(d + 8 * r, 1, true);
+#pragma unroll
+  for (int c = 0; c < 8; c++) jpegenc::fdct_1d(d + c, 8, false);
+  int zz[64];
+#pragma unroll
+  for (int k = 0; k < 64; k++) zz[k] = jpegenc::quantize(d[jpegenc::natural_order(k)], q[jpegenc::natural_order(k)]);
+  unsigned long long mask = 0;
+  unsigned bits = 0;
+  int run = 0;
+#pragma unroll
+  for (int k = 1; k < 64; k++) {
+    if (zz[k] == 0) {
+      run++;
+    } else {
+      mask |= 1ull << k;
+      while (run > 15) { bits += acs[0xF0]; run -= 16; }
+      const int nb = jpegenc::nbits(zz[k]);
+      bits += acs[(run << 4) | nb] + nb;
+      run = 0;
+    }
+  }
+  if (run) bits += acs[0];
+  uint4* cw = reinterpret_cast<uint4*>(cb);
+#pragma unroll
+  for (int k = 0; k < 8; k++) {
+    uint32_t v[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) v[j] = (uint32_t)(uint16_t)zz[8 * k + 2 * j] | ((uint32_t)(uint16_t)zz[8 * k + 2 * j + 1] << 16);
+    cw[k] = make_uint4(v[0], v[1], v[2], v[3]);
+  }
+  dc = zz[0];
+  bi->mask = mask;
+  bi->dc = zz[0];
+  bi->acbits = bits;
 }
 
 __global__ void __launch_bounds__(MCUS_PER_CTA * 6) jpe_blocks_kernel(const uint8_t* __restrict__ src, int n, Geometry g,
@@ -133,43 +180,7 @@ __global__ void __launch_bounds__(MCUS_PER_CTA * 6) jpe_blocks_kernel(const uint
           d[i] = jpegenc::h2v2(s[o], s[o + 1], s[o + 16], s[o + 17], i) - 128;
         }
       }
-#pragma unroll
-      for (int r = 0; r < 8; r++) jpegenc::fdct_1d(d + 8 * r, 1, true);
-#pragma unroll
-      for (int c = 0; c < 8; c++) jpegenc::fdct_1d(d + c, 8, false);
-      const Recip* q = s_q[luma ? 0 : 1];
-      const uint8_t* acs = s_acsize[luma ? 0 : 1];
-      int zz[64];
-#pragma unroll
-      for (int k = 0; k < 64; k++) zz[k] = jpegenc::quantize(d[jpegenc::natural_order(k)], q[jpegenc::natural_order(k)]);
-      unsigned long long mask = 0;
-      unsigned bits = 0;
-      int run = 0;
-#pragma unroll
-      for (int k = 1; k < 64; k++) {
-        if (zz[k] == 0) {
-          run++;
-        } else {
-          mask |= 1ull << k;
-          while (run > 15) { bits += acs[0xF0]; run -= 16; }
-          const int nb = jpegenc::nbits(zz[k]);
-          bits += acs[(run << 4) | nb] + nb;
-          run = 0;
-        }
-      }
-      if (run) bits += acs[0];
-      uint4* cw = reinterpret_cast<uint4*>(coef + (((size_t)f * nmcu + m) * 6 + b) * 64);
-#pragma unroll
-      for (int k = 0; k < 8; k++) {
-        uint32_t v[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) v[j] = (uint32_t)(uint16_t)zz[8 * k + 2 * j] | ((uint32_t)(uint16_t)zz[8 * k + 2 * j + 1] << 16);
-        cw[k] = make_uint4(v[0], v[1], v[2], v[3]);
-      }
-      s_dc[lm][b] = zz[0];
-      bi->mask = mask;
-      bi->dc = zz[0];
-      bi->acbits = bits;
+      code_block(d, s_q[luma ? 0 : 1], s_acsize[luma ? 0 : 1], coef + (((size_t)f * nmcu + m) * 6 + b) * 64, s_dc[lm][b], bi);
     }
     __syncthreads();
     if (m < nmcu && !real) {   // compress_data: right of the edge the DC on the left, below it the DC of the MCU's block 1
@@ -180,6 +191,43 @@ __global__ void __launch_bounds__(MCUS_PER_CTA * 6) jpe_blocks_kernel(const uint
       bi->dc = bottom ? dc1 : s_dc[lm][b - 1];
       bi->acbits = s_acsize[0][0];
     }
+  }
+}
+
+// a grey plane: a thread per block (= MCU) loads its 8 x 8 samples, the column and row past the edge replicated (jcsample.c
+// expand_right_edge, jcprepct.c expand_bottom_edge), and codes it with table 0
+__global__ void __launch_bounds__(GREY_BLOCKS_T) jpe_blocks_u8_kernel(const uint8_t* __restrict__ src, int n, Geometry g,
+                                                                      const Tables* __restrict__ tab, short* __restrict__ coef,
+                                                                      BlockInfo* __restrict__ info) {
+  __shared__ Recip s_q[64];
+  __shared__ uint8_t s_acsize[256];
+  for (int i = threadIdx.x; i < 64; i += blockDim.x) s_q[i] = tab->q[0][i];
+  for (int i = threadIdx.x; i < 256; i += blockDim.x) s_acsize[i] = tab->hf[1].size[i];
+  __syncthreads();
+  const int nblk = g.mcux * g.mcuy;
+  const int m = blockIdx.x * GREY_BLOCKS_T + threadIdx.x;
+  if (m >= nblk) return;
+  const int x0 = 8 * (m % g.mcux), y0 = 8 * (m / g.mcux);
+  for (int f = blockIdx.y; f < n; f += gridDim.y) {
+    const uint8_t* plane = src + (size_t)f * g.w * g.h;
+    int d[64];
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+      const uint8_t* row = plane + (size_t)min(y0 + r, g.h - 1) * g.w;
+      if (x0 + 8 <= g.w && ((uintptr_t)(row + x0) & 7) == 0) {
+        const uint2 v = __ldg(reinterpret_cast<const uint2*>(row + x0));
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+          d[8 * r + j] = (int)((v.x >> (8 * j)) & 255u) - 128;
+          d[8 * r + 4 + j] = (int)((v.y >> (8 * j)) & 255u) - 128;
+        }
+      } else {
+#pragma unroll
+        for (int j = 0; j < 8; j++) d[8 * r + j] = (int)row[min(x0 + j, g.w - 1)] - 128;
+      }
+    }
+    int dc;
+    code_block(d, s_q, s_acsize, coef + ((size_t)f * nblk + m) * 64, dc, info + (size_t)f * nblk + m);
   }
 }
 
@@ -211,33 +259,35 @@ __device__ __forceinline__ T cta_exclusive_scan(T v, T& excl, T* s_warp) {
   return total;
 }
 
+template <int NC>
 __global__ void __launch_bounds__(SCAN_THREADS) jpe_scan_kernel(const BlockInfo* __restrict__ info, int nmcu, const Tables* __restrict__ tab,
                                                                  unsigned long long* __restrict__ offs, unsigned long long* __restrict__ total,
                                                                  uint8_t* __restrict__ out, size_t stride, size_t raw_cap) {
+  constexpr int NB = jpegenc::blocks_per_mcu(NC);
   __shared__ unsigned long long s_warp[32];
   __shared__ uint8_t s_dcsize[2][12];
   const int f = blockIdx.x;
   if (threadIdx.x < 24) s_dcsize[threadIdx.x / 12][threadIdx.x % 12] = tab->hf[2 * (threadIdx.x / 12)].size[threadIdx.x % 12];
   __syncthreads();
-  const BlockInfo* fi = info + (size_t)f * nmcu * 6;
-  uint32_t* raw = reinterpret_cast<uint32_t*>(raw_buffer(out + (size_t)f * stride, raw_cap));
+  const BlockInfo* fi = info + (size_t)f * nmcu * NB;
+  uint32_t* raw = reinterpret_cast<uint32_t*>(raw_buffer<NC>(out + (size_t)f * stride, raw_cap));
   unsigned long long carry = 0;
   for (int base = 0; base < nmcu; base += SCAN_THREADS) {
     const int m = base + threadIdx.x;
     unsigned long long bits = 0;
     if (m < nmcu) {
-      const BlockInfo* b = fi + (size_t)m * 6;
-      int py = 0, pcb = 0, pcr = 0;
-      if (m > 0) { py = b[-3].dc; pcb = b[-2].dc; pcr = b[-1].dc; }
+      const BlockInfo* b = fi + (size_t)m * NB;
+      int pred[NC];   // DC predictors: the last block of each component in the MCU before
+#pragma unroll
+      for (int c = 0; c < NC; c++) pred[c] = m > 0 ? b[c - NC].dc : 0;
       unsigned s = 0;
 #pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const int nb = jpegenc::nbits(b[k].dc - py);
-        s += b[k].acbits + s_dcsize[0][nb] + nb;
-        py = b[k].dc;
+      for (int k = 0; k < NB; k++) {
+        const int c = jpegenc::block_comp(k);
+        const int nb = jpegenc::nbits(b[k].dc - pred[c]);
+        s += b[k].acbits + s_dcsize[jpegenc::block_table(k)][nb] + nb;
+        pred[c] = b[k].dc;
       }
-      const int nb4 = jpegenc::nbits(b[4].dc - pcb), nb5 = jpegenc::nbits(b[5].dc - pcr);
-      s += b[4].acbits + s_dcsize[1][nb4] + nb4 + b[5].acbits + s_dcsize[1][nb5] + nb5;
       bits = s;
     }
     unsigned long long excl;
@@ -278,6 +328,7 @@ struct BitOut {
   }
 };
 
+template <int NC>
 __global__ void __launch_bounds__(EMIT_THREADS) jpe_emit_kernel(const BlockInfo* __restrict__ info, const short* __restrict__ coef, int n,
                                                                  int nmcu, const Tables* __restrict__ tab,
                                                                  const unsigned long long* __restrict__ offs,
@@ -290,23 +341,25 @@ __global__ void __launch_bounds__(EMIT_THREADS) jpe_emit_kernel(const BlockInfo*
     s_size[i >> 8][i & 255] = tab->hf[i >> 8].size[i & 255];
   }
   __syncthreads();
+  constexpr int NB = jpegenc::blocks_per_mcu(NC);
   const int m = blockIdx.x * EMIT_THREADS + threadIdx.x;
   if (m >= nmcu) return;
   for (int f = blockIdx.y; f < n; f += gridDim.y) {
     const size_t mi = (size_t)f * nmcu + m;
-    const BlockInfo* b = info + mi * 6;
-    const short* c = coef + mi * 6 * 64;
+    const BlockInfo* b = info + mi * NB;
+    const short* c = coef + mi * NB * 64;
     const unsigned long long off = offs[mi];
     BitOut o;
-    o.raw = reinterpret_cast<uint32_t*>(raw_buffer(out + (size_t)f * stride, raw_cap));
+    o.raw = reinterpret_cast<uint32_t*>(raw_buffer<NC>(out + (size_t)f * stride, raw_cap));
     o.word = o.first = off >> 5;
     o.first_shared = (off & 31) != 0;
     o.acc = 0;
     o.nacc = (int)(off & 31);   // leading bits of the first word belong to the MCU before: zeros here
-    int pred[3] = {0, 0, 0};
-    if (m > 0) { pred[0] = b[-3].dc; pred[1] = b[-2].dc; pred[2] = b[-1].dc; }
-    for (int k = 0; k < 6; k++) {
-      const int comp = k < 4 ? 0 : k - 3, t = k < 4 ? 0 : 2;
+    int pred[NC];
+#pragma unroll
+    for (int k = 0; k < NC; k++) pred[k] = m > 0 ? b[k - NC].dc : 0;
+    for (int k = 0; k < NB; k++) {
+      const int comp = jpegenc::block_comp(k), t = 2 * jpegenc::block_table(k);
       const BlockInfo bk = b[k];
       const int diff = bk.dc - pred[comp];
       pred[comp] = bk.dc;
@@ -336,16 +389,18 @@ __global__ void __launch_bounds__(EMIT_THREADS) jpe_emit_kernel(const BlockInfo*
   }
 }
 
+template <int NC>
 __global__ void __launch_bounds__(SCAN_THREADS) jpe_stuff_kernel(const Tables* __restrict__ tab, const unsigned long long* __restrict__ total,
                                                                   uint8_t* __restrict__ out, size_t stride, size_t raw_cap,
                                                                   unsigned long long* __restrict__ len) {
+  constexpr int HEADER = jpegenc::header_bytes(NC);
   __shared__ unsigned long long s_warp[32];
   const int f = blockIdx.x;
   uint8_t* o = out + (size_t)f * stride;
-  const uint8_t* raw = raw_buffer(o, raw_cap);
-  for (int i = threadIdx.x; i < jpegenc::HEADER_BYTES; i += blockDim.x) o[i] = tab->header[i];
+  const uint8_t* raw = raw_buffer<NC>(o, raw_cap);
+  for (int i = threadIdx.x; i < HEADER; i += blockDim.x) o[i] = tab->header[i];
   const unsigned long long nraw = (total[f] + 7) >> 3;
-  uint8_t* dst = o + jpegenc::HEADER_BYTES;
+  uint8_t* dst = o + HEADER;
   unsigned long long carry = 0;   // 0x00 bytes inserted so far
   // Tile by tile: every thread reads its 16 bytes before any thread writes (the scan below synchronises), and a tile's
   // output ends below the raw bytes of the next tile (raw_buffer leaves room for the stuffed copy of everything before it).
@@ -372,24 +427,22 @@ __global__ void __launch_bounds__(SCAN_THREADS) jpe_stuff_kernel(const Tables* _
   if (threadIdx.x == 0) {
     dst[nraw + carry] = 0xFF;
     dst[nraw + carry + 1] = 0xD9;
-    len[f] = jpegenc::HEADER_BYTES + nraw + carry + 2;
+    len[f] = HEADER + nraw + carry + 2;
   }
 }
 
-}  // namespace
-
-size_t jpeg_encode_bound(int w, int h) { return jpegenc::encode_bound(w, h); }
-
-int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
-                          uint64_t* d_len) {
-  const Geometry g = jpegenc::geometry(w, h);
+// the five passes over n frames (NC = 3: bgr8 frames as 4:2:0, NC = 1: grey planes)
+template <int NC>
+int encode_batch(uwip_ctx* ctx, const uint8_t* d_src, int n, int w, int h, int quality, uint8_t* d_out, size_t stride, uint64_t* d_len) {
+  constexpr int NB = jpegenc::blocks_per_mcu(NC);
+  const Geometry g = jpegenc::geometry(w, h, NC);
   const size_t nmcu = (size_t)g.mcux * g.mcuy;
-  const size_t raw_cap = jpegenc::raw_capacity(w, h);
+  const size_t raw_cap = jpegenc::raw_capacity(w, h, NC);
   // workspace: tables | MCU bit offsets | per-frame totals | block infos | coefficients
   const size_t b_tab = align_up(sizeof(Tables), 256);
   const size_t b_off = align_up((size_t)n * nmcu * 8, 256), b_tot = align_up((size_t)n * 8, 256);
-  const size_t b_info = align_up((size_t)n * nmcu * 6 * sizeof(BlockInfo), 256);
-  const size_t b_coef = (size_t)n * nmcu * 6 * 64 * sizeof(short);
+  const size_t b_info = align_up((size_t)n * nmcu * NB * sizeof(BlockInfo), 256);
+  const size_t b_coef = (size_t)n * nmcu * NB * 64 * sizeof(short);
   uint8_t* ws = (uint8_t*)uwip_slot(ctx, SLOT_JPEGENC, b_tab + b_off + b_tot + b_info + b_coef);
   if (!ws) return UWIP_ERR_NOMEM;
   Tables* tab = (Tables*)ws;
@@ -398,15 +451,33 @@ int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int
   BlockInfo* info = (BlockInfo*)(ws + b_tab + b_off + b_tot);
   short* coef = (short*)(ws + b_tab + b_off + b_tot + b_info);
   const int ny = std::min(n, 65535);
-  UWIP_LAUNCH(ctx, "jpeg_enc_setup", jpe_setup_kernel, 1, 128, 0, tab, w, h, quality);
-  UWIP_LAUNCH(ctx, "jpeg_enc_blocks", jpe_blocks_kernel, dim3((unsigned)((nmcu + MCUS_PER_CTA - 1) / MCUS_PER_CTA), ny),
-              MCUS_PER_CTA * 6, 0, d_bgr, n, g, (const Tables*)tab, coef, info);
-  UWIP_LAUNCH(ctx, "jpeg_enc_scan", jpe_scan_kernel, n, SCAN_THREADS, 0, (const BlockInfo*)info, (int)nmcu, (const Tables*)tab, offs,
+  UWIP_LAUNCH(ctx, "jpeg_enc_setup", jpe_setup_kernel<NC>, 1, 128, 0, tab, w, h, quality);
+  if (NC == 3)
+    UWIP_LAUNCH(ctx, "jpeg_enc_blocks", jpe_blocks_kernel, dim3((unsigned)((nmcu + MCUS_PER_CTA - 1) / MCUS_PER_CTA), ny),
+                MCUS_PER_CTA * 6, 0, d_src, n, g, (const Tables*)tab, coef, info);
+  else
+    UWIP_LAUNCH(ctx, "jpeg_enc_blocks_u8", jpe_blocks_u8_kernel, dim3((unsigned)((nmcu + GREY_BLOCKS_T - 1) / GREY_BLOCKS_T), ny),
+                GREY_BLOCKS_T, 0, d_src, n, g, (const Tables*)tab, coef, info);
+  UWIP_LAUNCH(ctx, "jpeg_enc_scan", jpe_scan_kernel<NC>, n, SCAN_THREADS, 0, (const BlockInfo*)info, (int)nmcu, (const Tables*)tab, offs,
               tot, d_out, stride, raw_cap);
-  UWIP_LAUNCH(ctx, "jpeg_enc_emit", jpe_emit_kernel, dim3((unsigned)((nmcu + EMIT_THREADS - 1) / EMIT_THREADS), ny), EMIT_THREADS, 0,
+  UWIP_LAUNCH(ctx, "jpeg_enc_emit", jpe_emit_kernel<NC>, dim3((unsigned)((nmcu + EMIT_THREADS - 1) / EMIT_THREADS), ny), EMIT_THREADS, 0,
               (const BlockInfo*)info, (const short*)coef, n, (int)nmcu, (const Tables*)tab, (const unsigned long long*)offs,
               (const unsigned long long*)tot, d_out, stride, raw_cap);
-  UWIP_LAUNCH(ctx, "jpeg_enc_stuff", jpe_stuff_kernel, n, SCAN_THREADS, 0, (const Tables*)tab, (const unsigned long long*)tot, d_out,
+  UWIP_LAUNCH(ctx, "jpeg_enc_stuff", jpe_stuff_kernel<NC>, n, SCAN_THREADS, 0, (const Tables*)tab, (const unsigned long long*)tot, d_out,
               stride, raw_cap, (unsigned long long*)d_len);
   return UWIP_OK;
+}
+
+}  // namespace
+
+size_t jpeg_encode_bound(int w, int h) { return jpegenc::encode_bound(w, h); }
+size_t jpeg_encode_u8_bound(int w, int h) { return jpegenc::encode_bound(w, h, 1); }
+
+int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
+                          uint64_t* d_len) {
+  return encode_batch<3>(ctx, d_bgr, n, w, h, quality, d_out, stride, d_len);
+}
+int jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
+                             uint64_t* d_len) {
+  return encode_batch<1>(ctx, d_planes, n, w, h, quality, d_out, stride, d_len);
 }

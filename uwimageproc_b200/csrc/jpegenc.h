@@ -1,11 +1,14 @@
 // jpegenc.h - the baseline JPEG encoder of libjpeg-turbo 3.1.2 (the codec behind cv2.imwrite / cv2.imencode of cv2 4.13.0)
-// restated in plain C++ that compiles for the host and the device: 4:2:0 (Y 2x2, Cb and Cr 1x1), the standard Annex K
-// quantisation tables scaled by quality, the standard Annex K Huffman tables, no restart markers, no optimised Huffman
-// tables, not progressive.  csrc/jpegenc.cu runs this arithmetic batched on the GPU; encode_frame() below is the scalar
-// reference for one frame, which only the host test compiles.
+// restated in plain C++ that compiles for the host and the device: the standard Annex K quantisation tables scaled by
+// quality, the standard Annex K Huffman tables, no restart markers, no optimised Huffman tables, not progressive.  Two
+// component layouts, `nc` below: a bgr8 frame is written as YCbCr 4:2:0 (nc = 3: Y 2x2, Cb and Cr 1x1, an MCU of six blocks),
+// a grey plane as one component (nc = 1, jpeg_set_colorspace(JCS_GRAYSCALE): an MCU of one block).  csrc/jpegenc.cu runs
+// this arithmetic batched on the GPU; encode_frame() and encode_grey_frame() below are the scalar references for one frame,
+// which only the host test compiles.
 //
-// The bytes of a file are: SOI, APP0 (JFIF 1.01, density 1x1, no thumbnail), DQT 0, DQT 1, SOF0, DHT DC0, AC0, DC1, AC1, SOS,
-// the entropy-coded segment, EOI.  Every function names the libjpeg-turbo function it restates.
+// The bytes of a file are: SOI, APP0 (JFIF 1.01, density 1x1, no thumbnail), DQT 0 [, DQT 1], SOF0, DHT DC0, AC0 [, DC1, AC1],
+// SOS, the entropy-coded segment, EOI; the bracketed tables only for nc = 3.  Every function names the libjpeg-turbo
+// function it restates.
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
@@ -18,7 +21,14 @@
 
 namespace jpegenc {
 
-constexpr int HEADER_BYTES = 623;   // SOI .. SOS of the layout above (write_file_header, write_frame_header, write_scan_header)
+// SOI .. SOS of the layout above (write_file_header, write_frame_header, write_scan_header)
+JPEG_HD constexpr int header_bytes(int nc) { return nc == 3 ? 623 : 328; }
+constexpr int HEADER_BYTES = header_bytes(3);
+constexpr int GREY_HEADER_BYTES = header_bytes(1);
+// blocks of an MCU, and the component and table pair (0 luma, 1 chroma) of block b: Y Y Y Y Cb Cr, or one grey block
+JPEG_HD constexpr int blocks_per_mcu(int nc) { return nc == 3 ? 6 : 1; }
+JPEG_HD constexpr int block_comp(int b) { return b < 4 ? 0 : b - 3; }
+JPEG_HD constexpr int block_table(int b) { return b < 4 ? 0 : 1; }
 
 // jpeg_natural_order (jutils.c): natural index of zig-zag position k
 JPEG_HD constexpr int natural_order(int k) {
@@ -190,15 +200,17 @@ JPEG_HD inline int nbits(int v) {
   return n;
 }
 
-// geometry of a 4:2:0 frame: MCUs of 16 x 16 pixels, luma blocks of the padded plane, chroma rows after h2v2
+// geometry of a frame: MCUs of 16 x 16 pixels (4:2:0) or 8 x 8 (grey), luma blocks of the padded plane, chroma rows after
+// h2v2.  A grey scan has no dummy blocks: its MCUs are the blocks.
 struct Geometry {
   int w, h, mcux, mcuy, ybw, ybh, ch;
 };
-JPEG_HD inline Geometry geometry(int w, int h) {
+JPEG_HD inline Geometry geometry(int w, int h, int nc = 3) {
   Geometry g;
   g.w = w; g.h = h;
-  g.mcux = (w + 15) / 16; g.mcuy = (h + 15) / 16;
   g.ybw = (w + 7) / 8; g.ybh = (h + 7) / 8;
+  g.mcux = nc == 3 ? (w + 15) / 16 : g.ybw;
+  g.mcuy = nc == 3 ? (h + 15) / 16 : g.ybh;
   g.ch = (h + 1) / 2;
   return g;
 }
@@ -206,41 +218,50 @@ JPEG_HD inline Geometry geometry(int w, int h) {
 // Largest entropy-coded bits of one MCU: per block the longest DC code plus category 11 (luma 9 + 11, chroma 11 + 11)
 // and 63 AC codes of the longest length (16) plus category 10; an AC magnitude stays below 2^10 because quantiser << 3
 // >= 8 divides an islow output below 2^13.  Every byte may be 0xFF and then be followed by a stuffed 0x00.
-constexpr long MCU_MAX_BITS = 4L * (9 + 11 + 63 * (16 + 10)) + 2L * (11 + 11 + 63 * (16 + 10));
+JPEG_HD constexpr long mcu_max_bits(int nc) {
+  return nc == 3 ? 4L * (9 + 11 + 63 * (16 + 10)) + 2L * (11 + 11 + 63 * (16 + 10)) : 9 + 11 + 63 * (16 + 10);
+}
+constexpr long MCU_MAX_BITS = mcu_max_bits(3);
 
 // bytes of the unstuffed entropy-coded segment reserved at the end of an output slot (whole 16-byte lines, one spare)
-JPEG_HD inline size_t raw_capacity(int w, int h) {
-  const Geometry g = geometry(w, h);
-  const size_t bits = (size_t)g.mcux * g.mcuy * (size_t)MCU_MAX_BITS;
+JPEG_HD inline size_t raw_capacity(int w, int h, int nc = 3) {
+  const Geometry g = geometry(w, h, nc);
+  const size_t bits = (size_t)g.mcux * g.mcuy * (size_t)mcu_max_bits(nc);
   return ((bits + 7) / 8 + 16 + 15) / 16 * 16;
 }
 
 // worst-case file size: header, every scan byte doubled by stuffing, EOI.  The batched encoder keeps the unstuffed scan in
 // the last raw_capacity() bytes of the slot (16-byte aligned, hence the 16 spare bytes) while it stuffs it into the front.
-JPEG_HD inline size_t encode_bound(int w, int h) { return (size_t)HEADER_BYTES + 2 * raw_capacity(w, h) + 2 + 16; }
+JPEG_HD inline size_t encode_bound(int w, int h, int nc = 3) {
+  return (size_t)header_bytes(nc) + 2 * raw_capacity(w, h, nc) + 2 + 16;
+}
 
-// write_file_header, write_frame_header, write_scan_header (jcmarker.c): SOI .. SOS, HEADER_BYTES bytes
-JPEG_HD inline int write_header(uint8_t* o, int w, int h, int quality) {
+// write_file_header, write_frame_header, write_scan_header (jcmarker.c): SOI .. SOS, header_bytes(nc) bytes.  Only the
+// tables the components use are written (emit_dqt per component's table, emit_dht per table the scan names).
+JPEG_HD inline int write_header(uint8_t* o, int w, int h, int quality, int nc = 3) {
   int n = 0;
   auto b = [&](int v) { o[n++] = (uint8_t)v; };
   auto w16 = [&](int v) { b(v >> 8); b(v & 255); };
+  const int ntab = nc == 3 ? 2 : 1;
   b(0xFF); b(0xD8);                                                 // SOI
   b(0xFF); b(0xE0); w16(16);                                        // APP0: JFIF 1.01, density unit 0, 1 x 1, no thumbnail
   b('J'); b('F'); b('I'); b('F'); b(0); b(1); b(1); b(0); w16(1); w16(1); b(0); b(0);
-  for (int t = 0; t < 2; t++) {                                     // emit_dqt: 8-bit precision, zig-zag order
+  for (int t = 0; t < ntab; t++) {                                  // emit_dqt: 8-bit precision, zig-zag order
     b(0xFF); b(0xDB); w16(67); b(t);
     for (int k = 0; k < 64; k++) b(quant_value(t, natural_order(k), quality));
   }
-  b(0xFF); b(0xC0); w16(17); b(8); w16(h); w16(w); b(3);             // emit_sof(M_SOF0)
-  b(1); b(0x22); b(0); b(2); b(0x11); b(1); b(3); b(0x11); b(1);
-  for (int t = 0; t < 4; t++) {                                     // emit_dht in the order the scan header sends them
+  b(0xFF); b(0xC0); w16(8 + 3 * nc); b(8); w16(h); w16(w); b(nc);   // emit_sof(M_SOF0): id, h << 4 | v, quantisation table
+  for (int c = 0; c < nc; c++) { b(c + 1); b(nc == 3 && c == 0 ? 0x22 : 0x11); b(c ? 1 : 0); }
+  for (int t = 0; t < 2 * ntab; t++) {                              // emit_dht in the order the scan header sends them
     int count = 0;
     for (int l = 1; l <= 16; l++) count += std_huff_bits(t, l);
     b(0xFF); b(0xC4); w16(2 + 1 + 16 + count); b(((t & 1) << 4) | (t >> 1));
     for (int l = 1; l <= 16; l++) b(std_huff_bits(t, l));
     for (int i = 0; i < count; i++) b(std_huff_val(t, i));
   }
-  b(0xFF); b(0xDA); w16(12); b(3); b(1); b(0x00); b(2); b(0x11); b(3); b(0x11); b(0); b(63); b(0);   // emit_sos
+  b(0xFF); b(0xDA); w16(6 + 2 * nc); b(nc);                         // emit_sos: id, DC << 4 | AC table; Ss 0, Se 63, Ah Al 0
+  for (int c = 0; c < nc; c++) { b(c + 1); b(c ? 0x11 : 0x00); }
+  b(0); b(63); b(0);
   return n;
 }
 
@@ -356,6 +377,32 @@ inline size_t encode_frame(const uint8_t* bgr, int w, int h, int quality, uint8_
       for (int b = 0; b < 4; b++) encode_block(s, zz[b], pred[0], hf[0], hf[1]);
       encode_block(s, zz[4], pred[1], hf[2], hf[3]);
       encode_block(s, zz[5], pred[2], hf[2], hf[3]);
+    }
+  s.flush();
+  out[s.n++] = 0xFF;
+  out[s.n++] = 0xD9;
+  return s.n;
+}
+
+// The grey twin (nc = 1): grayscale_convert copies the plane, expand_right_edge / expand_bottom_edge replicate the last column
+// and row into the padded blocks, and every block is an MCU.  plane: w * h bytes; `out` must hold encode_bound(w, h, 1).
+inline size_t encode_grey_frame(const uint8_t* plane, int w, int h, int quality, uint8_t* out) {
+  const Geometry g = geometry(w, h, 1);
+  Recip q[64];
+  for (int i = 0; i < 64; i++) q[i] = compute_reciprocal((unsigned)quant_value(0, i, quality) << 3);
+  static Huff hf[2];
+  for (int t = 0; t < 2; t++) make_derived(t, hf[t]);
+  BitSink s{out, (size_t)write_header(out, w, h, quality, 1), 0, 0};
+  int pred = 0;
+  for (int by = 0; by < g.ybh; by++)
+    for (int bx = 0; bx < g.ybw; bx++) {
+      int zz[64], smp[64];
+      for (int i = 0; i < 64; i++) {
+        const int x = 8 * bx + (i & 7), y = 8 * by + (i >> 3);
+        smp[i] = plane[(size_t)(y < h ? y : h - 1) * w + (x < w ? x : w - 1)];
+      }
+      block_coefs(smp, q, zz);
+      encode_block(s, zz, pred, hf[0], hf[1]);
     }
   s.flush();
   out[s.n++] = 0xFF;

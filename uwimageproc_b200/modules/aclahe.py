@@ -2,7 +2,8 @@
 
 Pixel work (GaussianBlur 3x3, CLAHE, entropy, the clip-limit sweep) runs in libuwip.so.  ParametrosACLAHE keeps the
 reference's host-side knee search on the 49 entropy samples per block size (curve_fit + spline derivatives + curvature,
-functions.py:49-93) with the same scipy calls; parametros_aclahe_batch runs the whole search for a batch on the device.
+functions.py:49-93) with the same scipy calls; parametros_aclahe_batch runs the whole search for a batch on the device, and
+main_batch the whole grey prototype (search and CLAHE).
 """
 import warnings
 
@@ -113,3 +114,24 @@ def main(img):
     """aclahe/python/main.py:17-20 without the file I/O."""
     BS, CL = ParametrosACLAHE(img)
     return CLAHE(img, BS, CL)
+
+
+def main_batch(planes, loop="repaired"):
+    """main.py:18-20 for a batch, on the device: planes uint8 (N, H, W) host array or device tensor -> (out uint8 (N, H, W),
+    BS int32[N], CL int32[N]) as host arrays; out[i] = createCLAHE(CL[i], (BS[i], BS[i])).apply(planes[i]).  Where the
+    reference's curve fit raises, BS = CL = -1 and the plane gets the fixed 8 x 8 grid and clip 2 of the chain."""
+    import torch
+
+    ctx = default_context()
+    t = planes if isinstance(planes, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(planes, dtype=np.uint8))
+    if t.dtype != torch.uint8 or t.dim() != 3:
+        raise ValueError("expected uint8 (N, H, W)")
+    t = t.to("cuda:%d" % ctx.device).contiguous()
+    torch.cuda.synchronize(ctx.device)
+    n, h, w = t.shape
+    out = torch.empty_like(t)
+    bs = torch.empty(n, dtype=torch.int32, device=t.device)
+    cl = torch.empty(n, dtype=torch.int32, device=t.device)
+    ctx.aclahe_grey_auto_dev(t, out, n, w, h, loop, d_bs=bs, d_cl=cl)
+    ctx.synchronize()
+    return out.cpu().numpy(), bs.cpu().numpy(), cl.cpu().numpy()
