@@ -255,13 +255,13 @@ int uwip_chain_bgr8(uwip_ctx* ctx, const uint8_t* src, uint8_t* dst, int n_frame
                     int height, const uwip_chain_params* p);
 
 /* per-frame status bits of the LAST uwip_chain_bgr8[_auto][_dev] / uwip_bgdehaze_bgr8_dev / uwip_aclahe_params_u8_dev /
- * uwip_aclahe_bgr8_auto_dev / uwip_aclahe_u8_auto_dev / uwip_jpeg_decode_bgr8_batch / uwip_jpeg_decode_u8_batch call on
+ * uwip_aclahe_bgr8_auto_dev / uwip_aclahe_u8_auto_dev / uwip_jpeg_decode_{bgr8,u8}_batch[_oriented] call on
  * this context (synchronises the stream).  UWIP_FRAME_NAN: the reference's
  * adaptiveExp_map is NaN for the whole frame (S = 0/0 where Yi = Yj = 0, BGDehaze.py:83, spreads through the box filters
  * and the final min-max; SURVEY 8a-D9) - the 8-bit output is then all zeros, exactly what imwrite would store.
  * UWIP_FRAME_ACLAHE_NOFIT: an automatic-CLAHE call could not fit an entropy curve of the frame (the reference's curve_fit
  * raises RuntimeError); the frame's BS = CL = -1 and it was processed with the fixed clip limit and grid.
- * UWIP_FRAME_JPEG_BAD (set by the two batched JPEG readers): the file's entropy-coded data is bad - an invalid Huffman code, a
+ * UWIP_FRAME_JPEG_BAD (set by the batched JPEG readers): the file's entropy-coded data is bad - an invalid Huffman code, a
  * coefficient past 63, the data ending before the last block or the wrong number of restart markers; the frame is all zeros
  * (libjpeg's recovery from corrupt data is not restated). */
 #define UWIP_FRAME_NAN 1
@@ -321,8 +321,9 @@ int uwip_jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_
  * upsampling, csrc/jpegdec.h restates the arithmetic), the reader of the reference's command lines (histretch.cpp:158,
  * bgdehaze/main.py:16), so that a .jpg input gives the device chain the reference's pixels; uwip_jpeg_decode_bgr8_dev above
  * gives nvJPEG's.  Accepted: baseline and extended sequential Huffman, 8-bit, one scan, grey or YCbCr 4:4:4, 4:2:2, 4:4:0,
- * 4:2:0, any restart interval, any tables.  The pixels are the stored orientation (IMREAD_IGNORE_ORIENTATION semantics; Exif
- * is not read), which is what cv2.imdecode returns for every file without an Exif orientation.
+ * 4:2:0, any restart interval, any tables.  The pixels are the stored orientation (cv2.IMREAD_COLOR |
+ * IMREAD_IGNORE_ORIENTATION), which is what cv2.imdecode(file, IMREAD_COLOR) returns for every file without an Exif
+ * orientation; uwip_jpeg_decode_bgr8_batch_oriented below applies it.
  * n host JPEG files (jpegs[f], lens[f]) of one size -> the bgr8 frames cv2.imdecode(file, IMREAD_COLOR) returns, contiguous
  * at d_bgr.  Tables, sampling and restart interval may differ per file; width x height may not (UWIP_ERR_INVALID).
  * Unsupported coding: UWIP_ERR_UNSUPPORTED.  Bad entropy-coded data: the frame is zeros and UWIP_FRAME_JPEG_BAD is set
@@ -337,6 +338,19 @@ int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, cons
  * uwip_jpeg_decode_bgr8_batch. */
 int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
                               uint8_t* d_planes, int width, int height);
+/* The readers above with each file's Exif orientation applied as cv2.imdecode(file, IMREAD_COLOR) and
+ * cv2.imdecode(file, IMREAD_GRAYSCALE) apply it with their default flags: flipped for orientations 2, 3, 4, transposed for
+ * 5 to 8 (uwip_jpeg_orientation gives the value).  width x height is the size after orientation: a file's stored size must
+ * be width x height for orientations 1 to 4 and height x width for 5 to 8 (UWIP_ERR_INVALID otherwise), so a batch may mix
+ * orientations.  They accept, refuse and flag exactly as the readers above; a flagged frame is zeros of width x height. */
+int uwip_jpeg_decode_bgr8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
+                                         uint8_t* d_bgr, int width, int height);
+int uwip_jpeg_decode_u8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
+                                       uint8_t* d_planes, int width, int height);
+/* The Exif orientation, 1 to 8, that cv2.imdecode (cv2 4.13.0) applies to a file: the first Exif APP1 before the scan whose
+ * IFD0 holds an orientation tag decides, and 1 stands for no tag or a value outside 1..8.  Runs the host marker reader of
+ * the readers above: UWIP_ERR_INVALID / UWIP_ERR_UNSUPPORTED for a header they refuse.  No context, no device. */
+int uwip_jpeg_orientation(const uint8_t* jpeg, size_t len, int* orientation);
 /* per-frame statistics of the last batched JPEG decode (either reader; synchronises): stats[2f] = subsequence decodes the
  * in-CTA synchronisation repeated, stats[2f + 1] = subsequences the cross-CTA fix-up re-decoded. */
 int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n_frames, int32_t* stats);

@@ -384,19 +384,39 @@ class Context:
         return out[0] if single else out
 
     # ---- JPEG files decoded as cv2.imdecode does (csrc/jpegdec.cu) ---------------------------------------------------
-    def jpeg_decode_batch_dev(self, files, d_out=None):
+    def jpeg_decode_batch_dev(self, files, d_out=None, orientation=False):
         """JPEG files of one size (a list of bytes, or one bytes object) -> torch uint8 CUDA tensor (N, H, W, 3) holding
-        cv2.imdecode(file, cv2.IMREAD_COLOR) of each, decoded in one device call.  A file with bad entropy-coded data decodes
-        to zeros and sets bit 4 of last_frame_flags(N)."""
-        return self._jpeg_decode_batch(files, d_out, 3, self.lib.uwip_jpeg_decode_bgr8_batch)
-
-    def jpeg_decode_grey_batch_dev(self, files, d_out=None):
-        """JPEG files of one size -> torch uint8 CUDA tensor (N, H, W) holding cv2.imdecode(file, cv2.IMREAD_GRAYSCALE) of
-        each (for a colour file its Y component), decoded in one device call.  Bad entropy-coded data: zeros and bit 4 of
+        cv2.imdecode(file, cv2.IMREAD_COLOR | cv2.IMREAD_IGNORE_ORIENTATION) of each, decoded in one device call; with
+        orientation=True, cv2.imdecode(file, cv2.IMREAD_COLOR): each file's Exif orientation applied, and "one size" is the
+        size after it (jpeg_size).  A file with bad entropy-coded data decodes to zeros and sets bit 4 of
         last_frame_flags(N)."""
-        return self._jpeg_decode_batch(files, d_out, 1, self.lib.uwip_jpeg_decode_u8_batch)
+        decode = self.lib.uwip_jpeg_decode_bgr8_batch_oriented if orientation else self.lib.uwip_jpeg_decode_bgr8_batch
+        return self._jpeg_decode_batch(files, d_out, 3, decode, orientation)
 
-    def _jpeg_decode_batch(self, files, d_out, channels, decode):
+    def jpeg_decode_grey_batch_dev(self, files, d_out=None, orientation=False):
+        """JPEG files of one size -> torch uint8 CUDA tensor (N, H, W) holding cv2.imdecode(file, cv2.IMREAD_GRAYSCALE |
+        cv2.IMREAD_IGNORE_ORIENTATION) of each (for a colour file its Y component), decoded in one device call; with
+        orientation=True, cv2.imdecode(file, cv2.IMREAD_GRAYSCALE), the Exif orientation applied.  Bad entropy-coded data:
+        zeros and bit 4 of last_frame_flags(N)."""
+        decode = self.lib.uwip_jpeg_decode_u8_batch_oriented if orientation else self.lib.uwip_jpeg_decode_u8_batch
+        return self._jpeg_decode_batch(files, d_out, 1, decode, orientation)
+
+    def jpeg_orientation(self, data):
+        """The Exif orientation (1..8) cv2.imdecode applies to JPEG file `data`; 1 when it has none (host marker reader)."""
+        buf = np.frombuffer(bytes(data), np.uint8)
+        o = C.c_int()
+        rc = self.lib.uwip_jpeg_orientation(_ptr(buf), buf.size, C.byref(o))
+        if rc != 0:
+            raise UwipError(rc, "uwip_jpeg_orientation: the JPEG header is malformed or its coding is not supported")
+        return o.value
+
+    def jpeg_size(self, data, orientation=True):
+        """(width, height) of the image cv2.imdecode returns for JPEG file `data`: the stored size, transposed for Exif
+        orientations 5 to 8 unless orientation=False."""
+        w, h = self.jpeg_info(data)
+        return (h, w) if orientation and self.jpeg_orientation(data) >= 5 else (w, h)
+
+    def _jpeg_decode_batch(self, files, d_out, channels, decode, orientation):
         import torch
 
         if isinstance(files, (bytes, bytearray, memoryview)):
@@ -405,7 +425,7 @@ class Context:
         n = len(bufs)
         if n == 0:
             raise ValueError("no files")
-        w, h = self.jpeg_info(bufs[0])
+        w, h = self.jpeg_size(bufs[0], orientation)
         shape = (n, h, w, 3) if channels == 3 else (n, h, w)
         if d_out is None:
             d_out = torch.empty(shape, dtype=torch.uint8, device="cuda:%d" % self.device)
@@ -417,18 +437,18 @@ class Context:
         self.synchronize()
         return d_out
 
-    def jpeg_decode_grey(self, files):
-        """JPEG files of one size -> numpy uint8 (N, H, W) equal to cv2.imdecode(file, cv2.IMREAD_GRAYSCALE); one bytes object
-        -> (H, W).  Decoded on the device."""
+    def jpeg_decode_grey(self, files, orientation=False):
+        """JPEG files of one size -> numpy uint8 (N, H, W) equal to cv2.imdecode(file, cv2.IMREAD_GRAYSCALE) of files without
+        an Exif orientation, and of every file with orientation=True; one bytes object -> (H, W).  Decoded on the device."""
         single = isinstance(files, (bytes, bytearray, memoryview))
-        out = self.jpeg_decode_grey_batch_dev(files).cpu().numpy()
+        out = self.jpeg_decode_grey_batch_dev(files, orientation=orientation).cpu().numpy()
         return out[0] if single else out
 
-    def jpeg_decode(self, files):
-        """JPEG files of one size -> numpy uint8 (N, H, W, 3) equal to cv2.imdecode(file, cv2.IMREAD_COLOR); one bytes object
-        -> (H, W, 3).  Decoded on the device."""
+    def jpeg_decode(self, files, orientation=False):
+        """JPEG files of one size -> numpy uint8 (N, H, W, 3) equal to cv2.imdecode(file, cv2.IMREAD_COLOR) of files without
+        an Exif orientation, and of every file with orientation=True; one bytes object -> (H, W, 3).  Decoded on the device."""
         single = isinstance(files, (bytes, bytearray, memoryview))
-        out = self.jpeg_decode_batch_dev(files).cpu().numpy()
+        out = self.jpeg_decode_batch_dev(files, orientation=orientation).cpu().numpy()
         return out[0] if single else out
 
     def jpeg_decode_stats(self, n):

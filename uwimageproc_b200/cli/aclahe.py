@@ -6,14 +6,18 @@ aclahe.cpp:209-218).  This shim prints the same table (one pixel pass per grid o
 out with the procedure of the Python prototype (ACLAHE.py:69-129): knee of the entropy curve -> clip limit, float16
 arg-max -> block size, CLAHE on V, HSV -> BGR, imwrite.  `-grey=1` is the Python main.py: grey image in, CLAHE image out.
 
-aclahe <input> <output> -grey=1 -device=1 [-q=95] [-loop=repaired|as_committed]
-aclahe <input dir> <output dir> -grey=1 -device=1 [-q=95] [-loop=..] [-batch=64]
+aclahe <input> <output> -grey=1 -device=1 [-q=95] [-loop=repaired|as_committed] [-orientation=ignore|exif]
+aclahe <input dir> <output dir> -grey=1 -device=1 [-q=95] [-loop=..] [-batch=64] [-orientation=..]
       main.py with the whole procedure on the device (uwip_aclahe_u8_auto_dev): a JPEG input is read by the project's grey
       reader (the pixels of cv2.imread(input, 0)), any other format by cv2.imread(input, 0); a .jpg output is written by the
       project's grey writer (the bytes of cv2.imwrite), any other format by cv2.imwrite.  When the curve fit fails (the
       reference raises), the fixed 8x8 grid and clip 2 are used and a note is printed.  When both arguments are directories,
       every *.jpg / *.jpeg of the input directory is processed into the output directory under the same name, grouped by
       size and in batches of -batch planes; each file's name, BS, CL and notes are printed.
+      -orientation=exif: a JPEG input is turned by its Exif orientation as cv2.imread(input, 0) does (the project's oriented
+      grey reader), so the output is that of the host route for every file, and directory mode groups files by their size
+      after orientation.  The default, ignore, keeps a JPEG file's stored orientation; the two agree on files without an
+      Exif orientation tag.
 """
 import os
 import sys
@@ -24,9 +28,13 @@ def main(argv=None):
     from ._args import parse
 
     pos, opt, err = parse(argv, {"grey": (0, int), "loop": ("repaired", str), "device": (0, int), "q": (95, int), "batch": (64, int),
-                                 "help": (False, bool)})
+                                 "orientation": ("ignore", str), "help": (False, bool)})
     if opt["device"] and not opt["grey"]:
         err.append("-device=1 needs -grey=1")
+    if opt["orientation"] not in ("ignore", "exif"):
+        err.append("-orientation must be ignore or exif")
+    elif opt["orientation"] == "exif" and not opt["device"]:
+        err.append("-orientation=exif needs -grey=1 -device=1")
     if opt["device"] and opt["loop"] not in ("repaired", "as_committed"):
         err.append("-loop must be repaired or as_committed")
     if opt["batch"] < 1:
@@ -90,13 +98,14 @@ def _grey_device(ctx, jobs, opt, named):
 
     from .chain import _notes
 
+    exif = opt["orientation"] == "exif"
     groups = {}
     for src, dst in jobs:
         if src.lower().endswith((".jpg", ".jpeg")):
             with open(src, "rb") as f:
                 data = f.read()
             item = (dst, data, None)
-            size = ctx.jpeg_info(data)
+            size = ctx.jpeg_size(data) if exif else ctx.jpeg_info(data)
         else:
             img = cv2.imread(src, 0)
             if img is None:
@@ -111,7 +120,7 @@ def _grey_device(ctx, jobs, opt, named):
             part = items[b0:b0 + opt["batch"]]
             n = len(part)
             if part[0][1] is not None:   # one JPEG job per batch unless in directory mode, which reads only JPEG files
-                d_in = ctx.jpeg_decode_grey_batch_dev([data for _, data, _ in part])
+                d_in = ctx.jpeg_decode_grey_batch_dev([data for _, data, _ in part], orientation=exif)
                 dflags = ctx.last_frame_flags(n)   # read now: the CLAHE call resets the flags
             else:
                 d_in = torch.from_numpy(part[0][2]).to(dev)[None]

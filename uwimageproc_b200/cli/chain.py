@@ -1,4 +1,5 @@
 """chain <input.jpg> <output.jpg> [-q=95] [-aclahe=auto [-loop=repaired|as_committed]] [-encoder=nvjpeg|exact] [-decoder=nvjpeg|exact]
+      [-orientation=ignore|exif]
 chain <input dir> <output dir> [options above] [-batch=64]
       the whole path on one file: histretch(V, 1/99) -> aclahe(8x8, clip 2) -> bgdehaze
 
@@ -17,11 +18,17 @@ writes nvJPEG's bytes (its own DCT, quantisation and entropy coding).
 those cv2.imread(input) returns, as the reference's command lines read them.  The default, nvjpeg, gives nvJPEG's pixels (a
 few levels away, mostly in the 4:2:0 chroma upsampling), so the two decoders give different outputs, not the same output at
 different speeds.  With -decoder=exact -encoder=exact the file written is cv2.imwrite(output, chain(cv2.imread(input))), with
--aclahe=auto too, and the pixels never exist on the host.
+-aclahe=auto too, and the pixels never exist on the host: for every file with -orientation=exif, and for files without an
+Exif orientation tag with the default.
+
+-orientation=exif (needs -decoder=exact; nvJPEG does not read Exif): each file is turned by its Exif orientation as
+cv2.imread does (uwip_jpeg_decode_bgr8_batch_oriented), so a photograph taken with the camera on its side comes out upright,
+with width and height swapped for orientations 5 to 8.  The default, ignore, keeps the stored orientation
+(cv2.IMREAD_IGNORE_ORIENTATION).
 
 When both arguments are directories, every *.jpg / *.jpeg of the input directory is enhanced into the output directory under
-the same name (what bgdehaze/main.py does over img/*.jpg -> result/): the files are grouped by size and run in batches of
--batch frames through the same decoder, chain and encoder; BS, CL and the notes are printed per file.  One JPEG file takes
+the same name (what bgdehaze/main.py does over img/*.jpg -> result/): the files are grouped by size (after orientation with
+-orientation=exif) and run in batches of -batch frames through the same decoder, chain and encoder; BS, CL and the notes are printed per file.  One JPEG file takes
 the same route as a batch of one.
 """
 import os
@@ -50,16 +57,17 @@ def _run_jpegs(ctx, jobs, opt, named):
     decoder, chain and encoder that opt names.  named: each file's report starts with its name (directory mode)."""
     import torch
 
+    exif = opt["orientation"] == "exif"
     groups = {}
     for path, data in jobs:
-        groups.setdefault(ctx.jpeg_info(data), []).append((path, data))
+        groups.setdefault(ctx.jpeg_size(data) if exif else ctx.jpeg_info(data), []).append((path, data))
     auto, q = opt["aclahe"] == "auto", opt["q"]
     for (w, h), files in groups.items():
         for b0 in range(0, len(files), opt["batch"]):
             part = files[b0:b0 + opt["batch"]]
             n = len(part)
             if opt["decoder"] == "exact":
-                d_in = ctx.jpeg_decode_batch_dev([d for _, d in part])
+                d_in = ctx.jpeg_decode_batch_dev([d for _, d in part], orientation=exif)
                 dflags = ctx.last_frame_flags(n)   # read now: the chain's call resets the flags
             else:
                 d_in = torch.empty((n, h, w, 3), dtype=torch.uint8, device="cuda:%d" % ctx.device)
@@ -96,13 +104,17 @@ def main(argv=None):
     from ._args import parse
 
     pos, opt, err = parse(argv, {"q": (95, int), "aclahe": ("fixed", str), "loop": ("repaired", str), "encoder": ("nvjpeg", str),
-                                "decoder": ("nvjpeg", str), "batch": (64, int), "help": (False, bool)})
+                                "decoder": ("nvjpeg", str), "orientation": ("ignore", str), "batch": (64, int), "help": (False, bool)})
     if opt["aclahe"] not in ("fixed", "auto") or opt["loop"] not in ("repaired", "as_committed"):
         err.append("-aclahe must be fixed or auto, -loop repaired or as_committed")
     if opt["encoder"] not in ("nvjpeg", "exact"):
         err.append("-encoder must be nvjpeg or exact")
     if opt["decoder"] not in ("nvjpeg", "exact"):
         err.append("-decoder must be nvjpeg or exact")
+    if opt["orientation"] not in ("ignore", "exif"):
+        err.append("-orientation must be ignore or exif")
+    elif opt["orientation"] == "exif" and opt["decoder"] != "exact":
+        err.append("-orientation=exif needs -decoder=exact (nvJPEG does not read Exif)")
     if opt["batch"] < 1:
         err.append("-batch must be at least 1")
     if len(pos) < 2 or opt.get("help") or err:

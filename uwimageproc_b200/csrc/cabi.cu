@@ -896,7 +896,7 @@ int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, cons
   DECODE_BATCH_REQUIRE(ctx, d_bgr);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false, false);
 }
 int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_planes, int width,
                               int height) {
@@ -904,7 +904,27 @@ int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const 
   DECODE_BATCH_REQUIRE(ctx, d_planes);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true, false);
+}
+int uwip_jpeg_decode_bgr8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_bgr,
+                                         int width, int height) {
+  CTX_GUARD(ctx);
+  DECODE_BATCH_REQUIRE(ctx, d_bgr);
+  int32_t* flags = flags_get(ctx, n_frames);
+  if (!flags) return UWIP_ERR_NOMEM;
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false, true);
+}
+int uwip_jpeg_decode_u8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_planes,
+                                       int width, int height) {
+  CTX_GUARD(ctx);
+  DECODE_BATCH_REQUIRE(ctx, d_planes);
+  int32_t* flags = flags_get(ctx, n_frames);
+  if (!flags) return UWIP_ERR_NOMEM;
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true, true);
+}
+int uwip_jpeg_orientation(const uint8_t* jpeg, size_t len, int* orientation) {
+  if (!jpeg || !len || !orientation) return UWIP_ERR_INVALID;
+  return jpeg_orientation(jpeg, len, orientation);
 }
 int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n, int32_t* stats_host) {
   CTX_GUARD(ctx);

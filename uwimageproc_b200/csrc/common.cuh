@@ -416,9 +416,12 @@ int jpeg_encode_batch_dev(uwip_ctx* ctx, const uint8_t* d_bgr, int n, int w, int
 int jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int w, int h, int quality, uint8_t* d_out, size_t stride,
                              uint64_t* d_len);
 
-// jpegdec.cu: d_out receives bgr8 frames, or grey planes (IMREAD_GRAYSCALE) when grey is set
+// jpegdec.cu: d_out receives bgr8 frames, or grey planes (IMREAD_GRAYSCALE) when grey is set; orient: each frame turned by
+// its Exif orientation (cv2.imdecode's default flags), w x h being the size after it
 int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_out, int w, int h,
-                      int32_t* d_flags, bool grey);
+                      int32_t* d_flags, bool grey, bool orient);
+// the Exif orientation cv2.imdecode applies (1..8) from the host marker reader; its status when the header is refused
+int jpeg_orientation(const uint8_t* data, size_t len, int* orientation);
 void jpeg_dec_destroy(uwip_ctx* ctx);
 
 // synth.cu

@@ -20,6 +20,9 @@
 //   color    a thread per output pixel: upsampling with its one-row / one-column context and YCbCr -> B,G,R, cropped to W x H
 // Grey output (IMREAD_GRAYSCALE) runs the same passes up to huff; then the idct of the component-0 blocks only and a grey
 // pass that crops the Y plane (jdcolor.c grayscale_convert: no chroma IDCT, upsampling or colour conversion).
+// The oriented readers apply each frame's Exif orientation (cv2.imdecode's default flags) in the output pass only: the
+// oriented pass replaces color / grey with a CTA per 32 x 32 output tile that forms the tile's stored pixels in shared memory
+// from rows of the sample planes and writes them out as rows of the output (a column of stored pixels for 5..8).
 // Bad entropy-coded data (an invalid code, a coefficient past 63, the data ending before the last block, the wrong number of
 // RST markers) leaves the frame all zeros and sets UWIP_FRAME_JPEG_BAD.  A frame's pixels do not depend on the batch it is in.
 #include <algorithm>
@@ -41,6 +44,7 @@ constexpr int CTA_T = 1024;        // destuff and scan passes
 constexpr int DESTUFF_BYTES = 16;  // per thread and tile
 constexpr int IDCT_T = 128;
 constexpr int COLOR_T = 256;
+constexpr int TILE = 32;           // output tile edge of the oriented pass
 
 struct FrameTab {
   Geo g;
@@ -51,6 +55,7 @@ struct FrameTab {
   uint64_t blk_off, smp_off;   // first block of the coefficient store, first byte of the sample planes
   uint64_t sub_off, int_off;   // first subsequence slot, first interval slot (nint + 1 of them)
   uint32_t sub_cap;            // subsequence slots (a multiple of SYNC_T)
+  int32_t orient;              // Exif orientation applied by the oriented pass, 1..8
 };
 
 struct Sub {
@@ -436,6 +441,62 @@ __global__ void __launch_bounds__(COLOR_T) jpeg_dec_grey_kernel(const FrameTab* 
   *o = smp[t.smp_off + (i / w) * t.g.pw[0] + i % w];
 }
 
+// The output pass of the oriented readers (GREY: the Y plane, else B,G,R), a CTA per TILE x TILE tile of the w x h output.
+// The stored pixels the tile shows (the tile, flipped and, for orientations 5..8, transposed) are formed along rows of the
+// sample planes into shared memory; then each warp writes a row of the output tile.  Loads and stores stay coalesced for
+// every orientation, and the column reads of the transposing orientations hit distinct banks (row pitch TILE + 1 words).
+template <bool GREY>
+__global__ void __launch_bounds__(COLOR_T) jpeg_dec_oriented_kernel(const FrameTab* __restrict__ tabs, const uint8_t* __restrict__ smp,
+                                                                     const int32_t* __restrict__ flags, uint8_t* __restrict__ out,
+                                                                     int w, int h, int tiles_x) {
+  constexpr int CH = GREY ? 1 : 3, ROWS = COLOR_T / TILE;
+  __shared__ uint32_t s_px[TILE][TILE + 1];
+  const int f = blockIdx.y;
+  const int x0 = (int)(blockIdx.x % tiles_x) * TILE, y0 = (int)(blockIdx.x / tiles_x) * TILE;
+  const int tw = min(TILE, w - x0), th = min(TILE, h - y0);
+  const int tx = threadIdx.x % TILE, ty = threadIdx.x / TILE;
+  const FrameTab& t = tabs[f];
+  const int o = t.orient;
+  const bool bad = (flags[f] & UWIP_FRAME_JPEG_BAD) != 0;
+  int ax, ay, bx, by;   // the stored pixels of two opposite corners: the stored rectangle starts at their minimum
+  jpegdec::oriented_src(o, w, h, x0, y0, ax, ay);
+  jpegdec::oriented_src(o, w, h, x0 + tw - 1, y0 + th - 1, bx, by);
+  const int sx0 = min(ax, bx), sy0 = min(ay, by);
+  if (!bad) {
+    const int sw = o >= 5 ? th : tw, sh = o >= 5 ? tw : th;
+    const Geo g = t.g;
+    const uint8_t* p = smp + t.smp_off;
+    for (int v = ty; v < sh; v += ROWS) {
+      if (tx >= sw) continue;
+      uint32_t px;
+      if (GREY) {
+        px = p[(size_t)(sy0 + v) * g.pw[0] + sx0 + tx];
+      } else {
+        uint8_t c[3];
+        jpegdec::pixel(g, p, sx0 + tx, sy0 + v, c);
+        px = c[0] | (uint32_t)c[1] << 8 | (uint32_t)c[2] << 16;
+      }
+      s_px[v][tx] = px;
+    }
+    __syncthreads();
+  }
+  for (int ly = ty; ly < th; ly += ROWS) {
+    if (tx >= tw) continue;
+    uint32_t px = 0;
+    if (!bad) {
+      int sx, sy;
+      jpegdec::oriented_src(o, w, h, x0 + tx, y0 + ly, sx, sy);
+      px = s_px[sy - sy0][sx - sx0];
+    }
+    uint8_t* q = out + ((size_t)f * w * h + (size_t)(y0 + ly) * w + x0 + tx) * CH;
+    q[0] = (uint8_t)px;
+    if (!GREY) {
+      q[1] = (uint8_t)(px >> 8);
+      q[2] = (uint8_t)(px >> 16);
+    }
+  }
+}
+
 size_t a16(size_t x) { return (x + 15) / 16 * 16; }
 
 }  // namespace
@@ -448,9 +509,17 @@ void jpeg_dec_destroy(uwip_ctx* ctx) {
   ctx->jdec_pinned_bytes = 0;
 }
 
+int jpeg_orientation(const uint8_t* data, size_t len, int* orientation) {
+  jpegdec::Header hd;
+  const int rc = jpegdec::parse_header(data, len, hd);
+  if (rc == jpegdec::OK) *orientation = hd.orientation;
+  return rc;
+}
+
 int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_out, int w, int h,
-                      int32_t* d_flags, bool grey) {
-  const char* fn = grey ? "uwip_jpeg_decode_u8_batch" : "uwip_jpeg_decode_bgr8_batch";
+                      int32_t* d_flags, bool grey, bool orient) {
+  const char* fn = grey ? orient ? "uwip_jpeg_decode_u8_batch_oriented" : "uwip_jpeg_decode_u8_batch"
+                        : orient ? "uwip_jpeg_decode_bgr8_batch_oriented" : "uwip_jpeg_decode_bgr8_batch";
   // ---- parse every header on the host
   std::vector<FrameTab> tabs((size_t)n);
   jpegdec::Header hd;
@@ -466,12 +535,15 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
                                               : "malformed or truncated header");
       return rc;
     }
-    if (hd.width != w || hd.height != h) {
-      uwip_set_err(ctx, "%s: file %d is %d x %d, not %d x %d", fn, f, hd.width, hd.height, w, h);
+    const int o = orient ? hd.orientation : 1;   // the stored size is the output size, transposed for 5..8
+    if (hd.width != (o >= 5 ? h : w) || hd.height != (o >= 5 ? w : h)) {
+      if (o == 1) uwip_set_err(ctx, "%s: file %d is %d x %d, not %d x %d", fn, f, hd.width, hd.height, w, h);
+      else uwip_set_err(ctx, "%s: file %d is %d x %d with Exif orientation %d, which does not turn it into %d x %d", fn, f, hd.width, hd.height, o, w, h);
       return UWIP_ERR_INVALID;
     }
     FrameTab& t = tabs[f];
     t.g = jpegdec::geometry(hd);
+    t.orient = o;
     for (int c = 0; c < hd.ncomp; c++) {
       memcpy(t.q[c], hd.q[hd.comp[c].tq], sizeof(t.q[c]));
       if (!jpegdec::make_derived(hd.dc[hd.comp[c].td], true, t.dc[c]) || !jpegdec::make_derived(hd.ac[hd.comp[c].ta], false, t.ac[c])) {
@@ -565,12 +637,21 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
   UWIP_LAUNCH(ctx, "jpeg_dec_huff", jpeg_dec_huff_kernel, gsub, SYNC_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
               (const Sub*)d_sub, (const int*)d_nsub, (const uint64_t*)d_entry, (const int4*)d_cd, d_coef, d_flags);
   const dim3 gblk((unsigned)((max_blocks + IDCT_T - 1) / IDCT_T), ny), gpix((unsigned)(((size_t)w * h + COLOR_T - 1) / COLOR_T), ny);
-  if (grey) {
-    UWIP_LAUNCH(ctx, "jpeg_dec_idct_y", jpeg_dec_idct_kernel<true>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
+  if (grey) UWIP_LAUNCH(ctx, "jpeg_dec_idct_y", jpeg_dec_idct_kernel<true>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
+  else UWIP_LAUNCH(ctx, "jpeg_dec_idct", jpeg_dec_idct_kernel<false>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
+  if (orient) {
+    const int tiles_x = (w + TILE - 1) / TILE;
+    const dim3 gtile((unsigned)((size_t)tiles_x * ((h + TILE - 1) / TILE)), ny);
+    if (grey)
+      UWIP_LAUNCH(ctx, "jpeg_dec_grey_oriented", jpeg_dec_oriented_kernel<true>, gtile, COLOR_T, 0, (const FrameTab*)d_tab,
+                  (const uint8_t*)d_smp, (const int32_t*)d_flags, d_out, w, h, tiles_x);
+    else
+      UWIP_LAUNCH(ctx, "jpeg_dec_color_oriented", jpeg_dec_oriented_kernel<false>, gtile, COLOR_T, 0, (const FrameTab*)d_tab,
+                  (const uint8_t*)d_smp, (const int32_t*)d_flags, d_out, w, h, tiles_x);
+  } else if (grey) {
     UWIP_LAUNCH(ctx, "jpeg_dec_grey", jpeg_dec_grey_kernel, gpix, COLOR_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_smp,
                 (const int32_t*)d_flags, d_out, w, h);
   } else {
-    UWIP_LAUNCH(ctx, "jpeg_dec_idct", jpeg_dec_idct_kernel<false>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
     UWIP_LAUNCH(ctx, "jpeg_dec_color", jpeg_dec_color_kernel, gpix, COLOR_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_smp,
                 (const int32_t*)d_flags, d_out, w, h);
   }

@@ -11,8 +11,12 @@
 // Accepted: baseline or extended sequential Huffman (SOF0, SOF1), 8-bit samples, one interleaved scan, one component (grey)
 // or three YCbCr components with Cb = Cr = 1x1 and Y 1x1, 2x1, 1x2 or 2x2 (4:4:4, 4:2:2, 4:4:0, 4:2:0), any restart
 // interval, any quantisation and Huffman tables.  Refused as unsupported: progressive, arithmetic, lossless, 12-bit,
-// other sampling factors, multi-scan, four components, RGB-coded three-component files.  The pixels are the stored
-// orientation (cv2.IMREAD_IGNORE_ORIENTATION semantics): Exif is not parsed.
+// other sampling factors, multi-scan, four components, RGB-coded three-component files.
+//
+// Exif orientation: parse_header records the value cv2 4.13.0's Exif reader reports (exif_orientation below), and
+// oriented_src() maps an output pixel to its stored pixel as cv2's ApplyExifOrientation flips and transposes.  A reader
+// that applies it equals cv2.imdecode with its default flags; one that does not gives the stored orientation
+// (cv2.IMREAD_IGNORE_ORIENTATION), which is also what cv2.imdecode returns for every file without an orientation tag.
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
@@ -57,6 +61,7 @@ struct Header {
   bool jfif, adobe;
   int adobe_transform;
   size_t scan_off;     // first byte of the entropy-coded segment (after the SOS header)
+  int orientation;     // the Exif orientation cv2 applies, 1..8 (1: none, or a value cv2 ignores)
 };
 
 struct Reader {
@@ -70,11 +75,41 @@ struct Reader {
   int u16() { const int a = u8(); return (a << 8) | u8(); }
 };
 
+// The orientation cv2 4.13.0 takes from the payload of one APP1 segment (OpenCV's ExifReader over the TIFF structure after
+// "Exif\0\0", as it behaves, not as TIFF specifies): -1 when the segment gives no orientation entry, so that the next Exif
+// APP1 is read; otherwise the entry's value, which cv2 applies only when it lies in 1..8.
+//  - The byte order is little-endian for "II" and big-endian for anything else, "MM" or not; the next u16 must be 42.
+//  - IFD0 is wherever the u32 at offset 4 points; IFD1 and later directories are not read.
+//  - Entries are read in order; the first orientation tag (0x0112) wins, whatever its type and count: its value is the u16 at
+//    the entry's value field, so a LONG value reads as 0 in a big-endian file.
+//  - Every read must lie inside the payload, or the segment gives nothing from that read on (an entry count running past the
+//    segment is harmless when the orientation tag comes first).
+inline int exif_orientation(const uint8_t* p, size_t n) {
+  if (n < 6 || memcmp(p, "Exif\0\0", 6) != 0) return -1;
+  p += 6;
+  n -= 6;
+  const bool le = n >= 2 && p[0] == 'I' && p[1] == 'I';
+  auto u16 = [&](uint64_t o) -> int { return o + 2 > n ? -1 : le ? p[o] | p[o + 1] << 8 : p[o] << 8 | p[o + 1]; };
+  if (u16(2) != 42 || n < 8) return -1;
+  const uint64_t ifd = le ? (uint32_t)p[4] | (uint32_t)p[5] << 8 | (uint32_t)p[6] << 16 | (uint32_t)p[7] << 24
+                          : (uint32_t)p[4] << 24 | (uint32_t)p[5] << 16 | (uint32_t)p[6] << 8 | (uint32_t)p[7];
+  const int count = u16(ifd);
+  for (int k = 0; k < count; k++) {
+    const uint64_t e = ifd + 2 + 12 * (uint64_t)k;
+    const int tag = u16(e);
+    if (tag < 0) return -1;
+    if (tag == 0x0112) return u16(e + 8);
+  }
+  return -1;
+}
+
 // read_markers / first_marker / next_marker / get_sof / get_sos / get_dht / get_dqt / get_dri / examine_app0 / examine_app14 /
 // skip_variable, then the colour-space decision of default_decompress_parms (jdapimin.c) and the checks of initial_setup
 // (jdinput.c) and jinit_upsampler (jdsample.c) that this decoder restricts further.  Stops after the first SOS.
 inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
   memset(&hd, 0, sizeof(hd));
+  hd.orientation = 1;
+  bool exif = false;   // an Exif APP1 gave an orientation entry: later ones are not read
   Reader r{data, len, 0, true};
   if (r.u8() != 0xFF || r.u8() != 0xD8 || !r.ok) return INVALID;   // first_marker: SOI
   bool sof = false;
@@ -201,6 +236,11 @@ inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
     } else if ((c >= 0xE1 && c <= 0xEF) || c == 0xFE || c == 0xCC || c == 0xDC) {   // APPn, COM, DAC, DNL: skip_variable
       const int length = r.u16() - 2;
       if (!r.ok || length < 0 || r.pos + (size_t)length > len) return INVALID;
+      if (c == 0xE1 && !exif) {
+        const int o = exif_orientation(data + r.pos, (size_t)length);
+        exif = o >= 0;
+        if (o >= 1 && o <= 8) hd.orientation = o;
+      }
       r.pos += length;
     } else if ((c >= 0xD0 && c <= 0xD7) || c == 0x01) {   // RSTn, TEM: no parameters
     } else {
@@ -545,6 +585,22 @@ JPEG_HD inline void pixel(const Geo& g, const uint8_t* smp, int x, int y, uint8_
   ycc_bgr(Y, cb, cr, o);
 }
 
+// ---- Exif orientation (OpenCV's ApplyExifOrientation) ---------------------------------------------------------------------
+// The stored pixel (sx, sy) that output pixel (x, y) of orientation o shows; w x h is the output size (the stored size is
+// w x h for o = 1..4 and h x w for 5..8).  2: flip(1), 3: flip(-1), 4: flip(0); 5: transpose, 6: transpose + flip(1),
+// 7: transpose + flip(-1), 8: transpose + flip(0).
+JPEG_HD inline void oriented_src(int o, int w, int h, int x, int y, int& sx, int& sy) {
+  const int fx = o == 2 || o == 3 || o == 6 || o == 7 ? w - 1 - x : x;
+  const int fy = o == 3 || o == 4 || o == 7 || o == 8 ? h - 1 - y : y;
+  if (o >= 5) {
+    sx = fy;
+    sy = fx;
+  } else {
+    sx = fx;
+    sy = fy;
+  }
+}
+
 // ---- destuffing: the bytes fill_bit_buffer hands to the decoder -----------------------------------------------------------
 // Kind of byte i of the entropy-coded segment s[0..len): 0 data, 1 dropped (stuffed 0x00, fill 0xFF, RSTn marker), 2 RSTn
 // code byte (dropped; a restart interval ends before it), 3 the 0xFF of any other marker: the segment ends there.
@@ -564,12 +620,26 @@ JPEG_HD inline int byte_kind(int prev, int b, int next) {   // prev / next: -1 o
 #ifndef __CUDA_ARCH__
 // The scalar reference of one frame: decode_mcu over the whole scan with process_restart, decompress_onepass's IDCTs, then
 // upsampling and colour conversion.  out: w * h * 3 bytes, or w * h for grey (IMREAD_GRAYSCALE: the IDCTs of component 0
-// only, cropped).  Returns OK, INVALID, UNSUPPORTED, or 1 for bad entropy-coded data (the frame is then all zeros, as the
-// batched decoder leaves it).
-inline int decode_frame(const uint8_t* data, size_t len, uint8_t* out, bool grey = false) {
+// only, cropped).  orient: the frame is then turned by the Exif orientation (h x w for 5..8), as cv2.imdecode's default
+// flags do.  Returns OK, INVALID, UNSUPPORTED, or 1 for bad entropy-coded data (the frame is then all zeros, as the batched
+// decoder leaves it).
+inline int decode_frame(const uint8_t* data, size_t len, uint8_t* out, bool grey = false, bool orient = false) {
   Header hd;
   int rc = parse_header(data, len, hd);
   if (rc != OK) return rc;
+  if (orient && hd.orientation != 1) {
+    const int ch = grey ? 1 : 3, o = hd.orientation, w = o >= 5 ? hd.height : hd.width, h = o >= 5 ? hd.width : hd.height;
+    uint8_t* st = new uint8_t[(size_t)hd.width * hd.height * ch];
+    rc = decode_frame(data, len, st, grey, false);
+    for (int y = 0; y < h; y++)
+      for (int x = 0; x < w; x++) {
+        int sx, sy;
+        oriented_src(o, w, h, x, y, sx, sy);
+        memcpy(out + ((size_t)y * w + x) * ch, st + ((size_t)sy * hd.width + sx) * ch, ch);
+      }
+    delete[] st;
+    return rc;
+  }
   static DTbl dct[3], act[3];
   for (int c = 0; c < hd.ncomp; c++)
     if (!make_derived(hd.dc[hd.comp[c].td], true, dct[c]) || !make_derived(hd.ac[hd.comp[c].ta], false, act[c])) return INVALID;
