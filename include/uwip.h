@@ -220,6 +220,16 @@ int uwip_rc_correction_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t pitch, int
 /* generate_results(src, dest, adaptiveExp_map)  bgdehaze/main.py:14-20 minus file I/O:
  * dst8 = sat(rint(out*255)) (what imwrite hands to the encoder); out_f64 (optional, may be NULL)
  * = adaptiveExp_map(normI, w)  BGDehaze.py:71-89, float64 H x W x 3. */
+/* adaptiveExp_map(normI, w)  BGDehaze.py:71-89, stage by stage (a test hook: one frame, not on the throughput path).  One
+ * full run of uwip_bgdehaze_bgr8, then its intermediates, width*height each, row-major:
+ * ycc = Yi | Cri << 8 | Cbi << 16 | Yj << 24 (YCrCb of (normI*255).astype(uint8) and luma of (restored*255).astype(uint8),
+ * BGDehaze.py:75-78); splane = rint(S 2^28) of the exposure ratio S (BGDehaze.py:83; 0 where S is 0/0); refined_s = the
+ * refined S (BGDehaze.py:85, float32); restored = RC_correction's output and out = adaptiveExp_map's (float64 H x W x 3,
+ * out NaN for a flagged frame); stats = yi_min, yi_max, yj_min, yj_max (joint three-channel extremes of the two YCrCb
+ * images) and the frame's NaN flag word (nonzero: UWIP_FRAME_NAN). */
+int uwip_exposure_stages_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t pitch, int width, int height,
+                              const uwip_dehaze_params* p, uint32_t* ycc, uint32_t* splane, float* refined_s,
+                              double* restored, double* out, uint32_t stats[5]);
 int uwip_bgdehaze_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t src_pitch, uint8_t* dst8,
                        size_t dst_pitch, int width, int height, const uwip_dehaze_params* p,
                        double* out_f64);

@@ -79,6 +79,7 @@ SIGNATURES = {
     "uwip_transmission_bgr8": (_i, [_P, _u8p, _sz, _i, _i, _i, _P, _P]),
     "uwip_refined_transmission_bgr8": (_i, [_P, _u8p, _sz, _i, _i, C.POINTER(DehazeParams), _P, _P]),
     "uwip_rc_correction_bgr8": (_i, [_P, _u8p, _sz, _i, _i, C.POINTER(DehazeParams), _P]),
+    "uwip_exposure_stages_bgr8": (_i, [_P, _u8p, _sz, _i, _i, C.POINTER(DehazeParams), _P, _P, _P, _P, _P, _P]),
     "uwip_bgdehaze_bgr8": (_i, [_P, _u8p, _sz, _u8p, _sz, _i, _i, C.POINTER(DehazeParams), _P]),
     "uwip_bgdehaze_bgr8_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, C.POINTER(DehazeParams)]),
     "uwip_chain_bgr8_dev": (_i, [_P, _u8p, _u8p, _i, _i, _i, C.POINTER(ChainParams)]),

@@ -216,6 +216,25 @@ class Context:
         self._ck(self.lib.uwip_rc_correction_bgr8(self.h, _ptr(f), f.strides[0], f.shape[1], f.shape[0], C.byref(p), _ptr(out)))
         return out
 
+    def exposure_stages(self, frame, params=None):
+        """adaptiveExp_map's intermediates from one full bgdehaze run of the frame (uwip_exposure_stages_bgr8): dict of
+        numpy arrays ycc (H, W, 4) uint8 (Yi, Cri, Cbi, Yj), splane (H, W) uint32 (rint(S 2^28)), refined_s (H, W)
+        float32, restored and out (H, W, 3) float64, and the scalars yi_min, yi_max, yj_min, yj_max, nan_flag."""
+        f = _frame(frame)
+        h, w = f.shape[:2]
+        ycc = np.empty((h, w), np.uint32)
+        splane = np.empty((h, w), np.uint32)
+        refs = np.empty((h, w), np.float32)
+        restored = np.empty(f.shape, np.float64)
+        out = np.empty(f.shape, np.float64)
+        stats = np.empty(5, np.uint32)
+        p = params or self.dehaze_params()
+        self._ck(self.lib.uwip_exposure_stages_bgr8(self.h, _ptr(f), f.strides[0], w, h, C.byref(p), _ptr(ycc), _ptr(splane),
+                                                    _ptr(refs), _ptr(restored), _ptr(out), _ptr(stats)))
+        d = dict(ycc=ycc.view(np.uint8).reshape(h, w, 4), splane=splane, refined_s=refs, restored=restored, out=out)
+        d.update(zip(("yi_min", "yi_max", "yj_min", "yj_max", "nan_flag"), (int(v) for v in stats)))
+        return d
+
     def bgdehaze(self, frame, params=None, return_float=False):
         f = _frame(frame)
         out8 = np.empty(f.shape, np.uint8)

@@ -531,23 +531,31 @@ void uwip_chain_defaults(uwip_chain_params* p) {
   uwip_dehaze_defaults(&p->dehaze);
 }
 
+// host outputs of uwip_exposure_stages_bgr8 (pad columns dropped)
+struct ExposureStagesOut {
+  uint32_t* ycc;
+  uint32_t* splane;
+  float* refS;
+  uint32_t* ystats;   // yi_min, yi_max, yj_min, yj_max, nan_flag
+};
+
 static int dehaze_host(uwip_ctx* ctx, const uint8_t* src, size_t pitch, int w, int h, const uwip_dehaze_params* pp, int stop_after,
                        uint8_t* dst8, size_t dst_pitch, double B[3], int64_t idx[2], double* t_raw, double* t_ref, double* restored,
-                       double* out) {
+                       double* out, const ExposureStagesOut* xs = nullptr) {
   uwip_dehaze_params p;
   if (pp) p = *pp; else uwip_dehaze_defaults(&p);
   uint8_t* d;
   UWIP_CHECK(stage_in(ctx, SLOT_STAGE_IN, src, pitch, w, h, 3, &d));
   size_t n_px = (size_t)w * h;
   uint8_t* o = (uint8_t*)uwip_slot(ctx, SLOT_STAGE_OUT, n_px * 3);
-  double* f64 = (double*)uwip_slot(ctx, SLOT_F64OUT, n_px * 8 * 8);  // t_raw[2] t_ref[2] (restored|out)[3] + slack
+  double* f64 = (double*)uwip_slot(ctx, SLOT_F64OUT, n_px * 8 * 10);  // t_raw[2] t_ref[2] restored[3] out[3]
   FrameState* fs = frame_state_get(ctx, 1);
   if (!o || !f64 || !fs) return UWIP_ERR_NOMEM;
   DehazeDebug dbg;
   dbg.t_raw = t_raw ? f64 : nullptr;
   dbg.t_ref = t_ref ? f64 + 2 * n_px : nullptr;
   dbg.restored = restored ? f64 + 4 * n_px : nullptr;
-  dbg.out = out ? f64 + 4 * n_px : nullptr;
+  dbg.out = out ? f64 + 7 * n_px : nullptr;
   dbg.stop_after = stop_after;
   UWIP_CHECK(frame_state_reset(ctx, fs, 1));
   UWIP_CHECK(dehaze_frames_dev(ctx, d, o, 1, w, h, p, false, fs, &dbg));
@@ -557,7 +565,21 @@ static int dehaze_host(uwip_ctx* ctx, const uint8_t* src, size_t pitch, int w, i
   if (t_ref) UWIP_CUDA(ctx, cudaMemcpyAsync(t_ref, dbg.t_ref, 2 * n_px * 8, cudaMemcpyDeviceToHost, ctx->stream));
   if (restored) UWIP_CUDA(ctx, cudaMemcpyAsync(restored, dbg.restored, 3 * n_px * 8, cudaMemcpyDeviceToHost, ctx->stream));
   if (out) UWIP_CUDA(ctx, cudaMemcpyAsync(out, dbg.out, 3 * n_px * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  if (xs) {
+    // the planes of the run just made (same sizes: the slots come back unchanged); pitch Wp, pad columns dropped
+    const size_t wp4 = (size_t)((w + 3) & ~3) * 4, n_pp4 = wp4 * h;
+    const void* d_ycc = uwip_slot(ctx, SLOT_YCC, n_pp4);
+    const void* d_sp = uwip_slot(ctx, SLOT_SPLANE, n_pp4);
+    const void* d_refS = uwip_slot(ctx, SLOT_REFS, n_pp4);
+    UWIP_CUDA(ctx, cudaMemcpy2DAsync(xs->ycc, (size_t)w * 4, d_ycc, wp4, (size_t)w * 4, h, cudaMemcpyDeviceToHost, ctx->stream));
+    UWIP_CUDA(ctx, cudaMemcpy2DAsync(xs->splane, (size_t)w * 4, d_sp, wp4, (size_t)w * 4, h, cudaMemcpyDeviceToHost, ctx->stream));
+    UWIP_CUDA(ctx, cudaMemcpy2DAsync(xs->refS, (size_t)w * 4, d_refS, wp4, (size_t)w * 4, h, cudaMemcpyDeviceToHost, ctx->stream));
+  }
   UWIP_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (xs) {
+    xs->ystats[0] = hs->yi_min; xs->ystats[1] = hs->yi_max; xs->ystats[2] = hs->yj_min; xs->ystats[3] = hs->yj_max;
+    xs->ystats[4] = hs->nan_flag;
+  }
   if (B) { B[0] = hs->B[0]; B[1] = hs->B[1]; B[2] = hs->B[2]; }
   if (idx) { idx[0] = hs->idx0; idx[1] = hs->idx1; }
   if (dst8) return stage_out(ctx, o, dst8, dst_pitch, w, h, 3);
@@ -599,6 +621,13 @@ int uwip_rc_correction_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t pitch, int
   CTX_GUARD(ctx);
   UWIP_REQUIRE(ctx, restored, "null output");
   return dehaze_host(ctx, src, pitch, w, h, p, 4, nullptr, 0, nullptr, nullptr, nullptr, nullptr, restored, nullptr);
+}
+int uwip_exposure_stages_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t pitch, int w, int h, const uwip_dehaze_params* p, uint32_t* ycc,
+                              uint32_t* splane, float* refined_s, double* restored, double* out, uint32_t stats[5]) {
+  CTX_GUARD(ctx);
+  UWIP_REQUIRE(ctx, ycc && splane && refined_s && restored && out && stats, "null output");
+  ExposureStagesOut xs{ycc, splane, refined_s, stats};
+  return dehaze_host(ctx, src, pitch, w, h, p, 0, nullptr, 0, nullptr, nullptr, nullptr, nullptr, restored, out, &xs);
 }
 int uwip_bgdehaze_bgr8(uwip_ctx* ctx, const uint8_t* src, size_t sp, uint8_t* dst8, size_t dp, int w, int h, const uwip_dehaze_params* p,
                        double* out_f64) {

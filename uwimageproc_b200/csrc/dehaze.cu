@@ -589,7 +589,7 @@ __global__ void __launch_bounds__(256) stab_kernel(const FrameState* __restrict_
 
 // S per pixel as a plane of the table's entries, rint(min(S, 1.6) 2^28) (0 where S is 0/0): GF2a then reads it through the
 // same staged row copies as the guide instead of gathering from the table inside the march.
-__global__ void __launch_bounds__(256) splane_kernel(GfCommon g, int H, int Wp) {
+__global__ void __launch_bounds__(256) splane_kernel(GfCommon g, int W, int H, int Wp) {
   int f = blockIdx.y;
   size_t n_pp = (size_t)Wp * H;
   const FrameState& s = g.fs[f];
@@ -599,15 +599,18 @@ __global__ void __launch_bounds__(256) splane_kernel(GfCommon g, int H, int Wp) 
   const uint32_t* stab = g.stab + (size_t)f * 65536;
   uint32_t* sp = g.splane + (size_t)f * n_pp;
   const size_t n_q = n_pp / 4;
+  const int qpr = Wp / 4;   // Wp is a multiple of 4: a quad never crosses a row
   bool nan_seen = false;
   for (size_t qi = (size_t)blockIdx.x * 256 + threadIdx.x; qi < n_q; qi += (size_t)gridDim.x * 256) {
     uint4 yw = __ldg(reinterpret_cast<const uint4*>(ycc) + qi);
+    const int x0 = (int)((unsigned)qi % (unsigned)qpr) * 4;   // qi < n_pp / 4 < 2^30
     uint32_t o[4];
 #pragma unroll
     for (int c = 0; c < 4; c++) {
       uint32_t w = quad_get(yw, c);
-      // pad columns hold zeros: keep them away from the table (their S is never used)
-      const bool pad = (w & 255u) < a || (w >> 24) < b;
+      // pad columns hold zeros: keep them away from the table and the flag (their S is never used).  Decided by the
+      // column: when both joint minima are 0 a pad entry is indistinguishable from a real (Yi', Yj') = (0, 0)
+      const bool pad = x0 + c >= W;
       w -= ysub;
       // S = 0/0 where Yi' = Yj' = 0 (SURVEY D9): the NaN reaches every output of the reference -> flag the frame
       const uint32_t S = pad ? 0u : __ldg(stab + (((w & 255u) << 8) | (w >> 24)));
@@ -774,7 +777,7 @@ int dehaze_frames_dev(uwip_ctx* ctx, const uint8_t* d_src, uint8_t* d_dst, int n
   if (dbg && dbg->stop_after == 4) return UWIP_OK;
   dim3 grid_s(256, n);
   UWIP_LAUNCH(ctx, "dz_stab", stab_kernel, grid_s, 256, 0, fs, d_stab);
-  UWIP_LAUNCH(ctx, "dz_splane", splane_kernel, grid_e, 256, 0, gc, H, Wp);
+  UWIP_LAUNCH(ctx, "dz_splane", splane_kernel, grid_e, 256, 0, gc, W, H, Wp);
   UWIP_CHECK(gp_launch<PipGF2a>(ctx, "dz_gf2a", FUNC_GF2A, gc, n, W, H, p.radius));
   UWIP_CHECK(gp_launch<PipGF2b>(ctx, "dz_gf2b", FUNC_GF2B, gc, n, W, H, p.radius));
   UWIP_LAUNCH(ctx, "dz_final", final_kernel, grid_e, 256, 0, gc, W, H, Wp, d_dst, dbg ? dbg->out : (double*)nullptr, d_flags);
