@@ -265,7 +265,7 @@ int uwip_chain_bgr8(uwip_ctx* ctx, const uint8_t* src, uint8_t* dst, int n_frame
                     int height, const uwip_chain_params* p);
 
 /* per-frame status bits of the LAST uwip_chain_bgr8[_auto][_dev] / uwip_bgdehaze_bgr8_dev / uwip_aclahe_params_u8_dev /
- * uwip_aclahe_bgr8_auto_dev / uwip_aclahe_u8_auto_dev / uwip_jpeg_decode_{bgr8,u8}_batch[_oriented] call on
+ * uwip_aclahe_bgr8_auto_dev / uwip_aclahe_u8_auto_dev / uwip_jpeg_decode_{bgr8,u8}_batch[_oriented] / uwip_jpeg_decode_batch_ex call on
  * this context (synchronises the stream).  UWIP_FRAME_NAN: the reference's
  * adaptiveExp_map is NaN for the whole frame (S = 0/0 where Yi = Yj = 0, BGDehaze.py:83, spreads through the box filters
  * and the final min-max; SURVEY 8a-D9) - the 8-bit output is then all zeros, exactly what imwrite would store.
@@ -361,6 +361,28 @@ int uwip_jpeg_decode_u8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpeg
  * IFD0 holds an orientation tag decides, and 1 stands for no tag or a value outside 1..8.  Runs the host marker reader of
  * the readers above: UWIP_ERR_INVALID / UWIP_ERR_UNSUPPORTED for a header they refuse.  No context, no device. */
 int uwip_jpeg_orientation(const uint8_t* jpeg, size_t len, int* orientation);
+/* The exact reader for sequential and progressive files alike, in one call: everything the four readers above accept,
+ * plus progressive Huffman files (SOF2) of the same samplings, such as cv2.imwrite(.., [IMWRITE_JPEG_PROGRESSIVE, 1]) and
+ * Pillow's save(.., progressive=True) write.  flags: UWIP_JPEG_GREY for the planes of cv2.imdecode(file, IMREAD_GRAYSCALE)
+ * in place of bgr8 frames, UWIP_JPEG_ORIENT for the Exif orientation applied (width x height then the size after it), as
+ * the readers above.  A batch may mix sequential and progressive files; a frame's pixels do not depend on the batch it is
+ * in.  Every scan is entropy-decoded, in grey output too.  Refused as the readers above (UWIP_ERR_INVALID,
+ * UWIP_ERR_UNSUPPORTED), and besides: bad Ss / Se / Ah / Al in a progressive scan (UWIP_ERR_INVALID); a scan whose Ah is
+ * not the Al of the previous scan of the same coefficients, an AC scan before the component's DC scan, more than 128 scans,
+ * and a progression that is incomplete at EOI - some coefficient of some component not refined down to Al = 0
+ * (UWIP_ERR_UNSUPPORTED: libjpeg-turbo decodes such files with block smoothing, which this reader does not restate).  Bad
+ * entropy-coded data zeroes the frame and sets UWIP_FRAME_JPEG_BAD as above, and so does a progressive file whose data ends
+ * inside a scan.  The headers are parsed and the files copied to pinned staging before the call returns.  Stream ordered,
+ * does not synchronise.  n_frames <= 65535. */
+#define UWIP_JPEG_GREY 1
+#define UWIP_JPEG_ORIENT 2
+int uwip_jpeg_decode_batch_ex(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames,
+                              uint8_t* d_out, int width, int height, int flags);
+/* The marker reader of uwip_jpeg_decode_batch_ex over a whole file, without a context or a device: the size of the image
+ * cv2.imdecode returns (after the Exif orientation: width and height swapped for orientations 5 to 8), the orientation
+ * (1 to 8) and whether the file is progressive.  Returns what uwip_jpeg_decode_batch_ex would refuse the file with, or
+ * UWIP_OK (also for a file whose entropy-coded data is bad: that is found by decoding). */
+int uwip_jpeg_probe(const uint8_t* jpeg, size_t len, int* width, int* height, int* orientation, int* progressive);
 /* per-frame statistics of the last batched JPEG decode (either reader; synchronises): stats[2f] = subsequence decodes the
  * in-CTA synchronisation repeated, stats[2f + 1] = subsequences the cross-CTA fix-up re-decoded. */
 int uwip_jpeg_decode_stats(uwip_ctx* ctx, int n_frames, int32_t* stats);

@@ -99,6 +99,8 @@ SIGNATURES = {
     "uwip_jpeg_decode_bgr8_batch_oriented": (_i, [_P, _P, _P, _i, _u8p, _i, _i]),
     "uwip_jpeg_decode_u8_batch_oriented": (_i, [_P, _P, _P, _i, _u8p, _i, _i]),
     "uwip_jpeg_orientation": (_i, [_u8p, _sz, C.POINTER(_i)]),
+    "uwip_jpeg_decode_batch_ex": (_i, [_P, _P, _P, _i, _u8p, _i, _i, _i]),
+    "uwip_jpeg_probe": (_i, [_u8p, _sz, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),
     "uwip_jpeg_decode_stats": (_i, [_P, _i, _P]),
     "uwip_calc_blur_bgr8": (_i, [_P, _u8p, _sz, _i, _i, _i, C.POINTER(C.c_float), C.POINTER(_d), _u8p, _sz]),
     "uwip_calc_blur_bgr8_dev": (_i, [_P, _u8p, _i, _i, _i, _i, _P]),

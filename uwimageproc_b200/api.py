@@ -8,6 +8,7 @@ from ._lib import ChainParams, DehazeParams, UwipError
 
 HSV_ROUND = {"cv2": 0, "trunc": 1, "rint": 2}
 ACLAHE_LOOP = {"repaired": 0, "as_committed": 1}
+JPEG_GREY, JPEG_ORIENT = 1, 2   # the flags of uwip_jpeg_decode_batch_ex
 ORDER = {"intended": 0, "literal": 1}
 
 
@@ -403,22 +404,43 @@ class Context:
         return out[0] if single else out
 
     # ---- JPEG files decoded as cv2.imdecode does (csrc/jpegdec.cu) ---------------------------------------------------
-    def jpeg_decode_batch_dev(self, files, d_out=None, orientation=False):
+    def jpeg_decode_batch_dev(self, files, d_out=None, orientation=False, progressive=False):
         """JPEG files of one size (a list of bytes, or one bytes object) -> torch uint8 CUDA tensor (N, H, W, 3) holding
         cv2.imdecode(file, cv2.IMREAD_COLOR | cv2.IMREAD_IGNORE_ORIENTATION) of each, decoded in one device call; with
         orientation=True, cv2.imdecode(file, cv2.IMREAD_COLOR): each file's Exif orientation applied, and "one size" is the
         size after it (jpeg_size).  A file with bad entropy-coded data decodes to zeros and sets bit 4 of
-        last_frame_flags(N)."""
+        last_frame_flags(N).  progressive=True: progressive files are read too, in the same batch as sequential ones
+        (uwip_jpeg_decode_batch_ex); a progression incomplete at EOI is refused."""
+        if progressive:
+            return self._jpeg_decode_batch(files, d_out, 3, self._decode_ex(orientation, False), orientation, True)
         decode = self.lib.uwip_jpeg_decode_bgr8_batch_oriented if orientation else self.lib.uwip_jpeg_decode_bgr8_batch
         return self._jpeg_decode_batch(files, d_out, 3, decode, orientation)
 
-    def jpeg_decode_grey_batch_dev(self, files, d_out=None, orientation=False):
+    def jpeg_decode_grey_batch_dev(self, files, d_out=None, orientation=False, progressive=False):
         """JPEG files of one size -> torch uint8 CUDA tensor (N, H, W) holding cv2.imdecode(file, cv2.IMREAD_GRAYSCALE |
         cv2.IMREAD_IGNORE_ORIENTATION) of each (for a colour file its Y component), decoded in one device call; with
         orientation=True, cv2.imdecode(file, cv2.IMREAD_GRAYSCALE), the Exif orientation applied.  Bad entropy-coded data:
-        zeros and bit 4 of last_frame_flags(N)."""
+        zeros and bit 4 of last_frame_flags(N).  progressive=True: progressive files are read too."""
+        if progressive:
+            return self._jpeg_decode_batch(files, d_out, 1, self._decode_ex(orientation, True), orientation, True)
         decode = self.lib.uwip_jpeg_decode_u8_batch_oriented if orientation else self.lib.uwip_jpeg_decode_u8_batch
         return self._jpeg_decode_batch(files, d_out, 1, decode, orientation)
+
+    def _decode_ex(self, orientation, grey):
+        """uwip_jpeg_decode_batch_ex with the flags of one reader, in the argument order of the other readers"""
+        flags = (JPEG_GREY if grey else 0) | (JPEG_ORIENT if orientation else 0)
+        return lambda h, ptrs, lens, n, out, w, hh: self.lib.uwip_jpeg_decode_batch_ex(h, ptrs, lens, n, out, w, hh, flags)
+
+    def jpeg_probe(self, data):
+        """(width, height, orientation, progressive) of JPEG file `data` from the host marker reader of the progressive-capable
+        reader, without the device: the size is that of the image cv2.imdecode returns (after the Exif orientation)."""
+        buf = np.frombuffer(bytes(data), np.uint8)
+        w, h, o, p = C.c_int(), C.c_int(), C.c_int(), C.c_int()
+        rc = self.lib.uwip_jpeg_probe(_ptr(buf), buf.size, C.byref(w), C.byref(h), C.byref(o), C.byref(p))
+        if rc != 0:
+            raise UwipError(rc, "uwip_jpeg_probe: the JPEG header is malformed, its coding is not supported or its progression is "
+                                "incomplete")
+        return w.value, h.value, o.value, bool(p.value)
 
     def jpeg_orientation(self, data):
         """The Exif orientation (1..8) cv2.imdecode applies to JPEG file `data`; 1 when it has none (host marker reader)."""
@@ -435,7 +457,7 @@ class Context:
         w, h = self.jpeg_info(data)
         return (h, w) if orientation and self.jpeg_orientation(data) >= 5 else (w, h)
 
-    def _jpeg_decode_batch(self, files, d_out, channels, decode, orientation):
+    def _jpeg_decode_batch(self, files, d_out, channels, decode, orientation, progressive=False):
         import torch
 
         if isinstance(files, (bytes, bytearray, memoryview)):
@@ -444,7 +466,12 @@ class Context:
         n = len(bufs)
         if n == 0:
             raise ValueError("no files")
-        w, h = self.jpeg_size(bufs[0], orientation)
+        if progressive:   # the progressive-capable reader: its own marker reader gives the size
+            w, h, o, _ = self.jpeg_probe(bufs[0])
+            if not orientation and o >= 5:
+                w, h = h, w
+        else:
+            w, h = self.jpeg_size(bufs[0], orientation)
         shape = (n, h, w, 3) if channels == 3 else (n, h, w)
         if d_out is None:
             d_out = torch.empty(shape, dtype=torch.uint8, device="cuda:%d" % self.device)
@@ -456,18 +483,20 @@ class Context:
         self.synchronize()
         return d_out
 
-    def jpeg_decode_grey(self, files, orientation=False):
+    def jpeg_decode_grey(self, files, orientation=False, progressive=False):
         """JPEG files of one size -> numpy uint8 (N, H, W) equal to cv2.imdecode(file, cv2.IMREAD_GRAYSCALE) of files without
-        an Exif orientation, and of every file with orientation=True; one bytes object -> (H, W).  Decoded on the device."""
+        an Exif orientation, and of every file with orientation=True; one bytes object -> (H, W).  Decoded on the device;
+        progressive=True reads progressive files too."""
         single = isinstance(files, (bytes, bytearray, memoryview))
-        out = self.jpeg_decode_grey_batch_dev(files, orientation=orientation).cpu().numpy()
+        out = self.jpeg_decode_grey_batch_dev(files, orientation=orientation, progressive=progressive).cpu().numpy()
         return out[0] if single else out
 
-    def jpeg_decode(self, files, orientation=False):
+    def jpeg_decode(self, files, orientation=False, progressive=False):
         """JPEG files of one size -> numpy uint8 (N, H, W, 3) equal to cv2.imdecode(file, cv2.IMREAD_COLOR) of files without
-        an Exif orientation, and of every file with orientation=True; one bytes object -> (H, W, 3).  Decoded on the device."""
+        an Exif orientation, and of every file with orientation=True; one bytes object -> (H, W, 3).  Decoded on the device;
+        progressive=True reads progressive files too."""
         single = isinstance(files, (bytes, bytearray, memoryview))
-        out = self.jpeg_decode_batch_dev(files, orientation=orientation).cpu().numpy()
+        out = self.jpeg_decode_batch_dev(files, orientation=orientation, progressive=progressive).cpu().numpy()
         return out[0] if single else out
 
     def jpeg_decode_stats(self, n):

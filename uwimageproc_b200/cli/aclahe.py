@@ -8,8 +8,9 @@ arg-max -> block size, CLAHE on V, HSV -> BGR, imwrite.  `-grey=1` is the Python
 
 aclahe <input> <output> -grey=1 -device=1 [-q=95] [-loop=repaired|as_committed] [-orientation=ignore|exif]
 aclahe <input dir> <output dir> -grey=1 -device=1 [-q=95] [-loop=..] [-batch=64] [-orientation=..]
-      main.py with the whole procedure on the device (uwip_aclahe_u8_auto_dev): a JPEG input is read by the project's grey
-      reader (the pixels of cv2.imread(input, 0)), any other format by cv2.imread(input, 0); a .jpg output is written by the
+      main.py with the whole procedure on the device (uwip_aclahe_u8_auto_dev): a JPEG input, baseline or progressive, is
+      read by the project's grey reader (the pixels of cv2.imread(input, 0); a progression incomplete at EOI is refused),
+      any other format by cv2.imread(input, 0); a .jpg output is written by the
       project's grey writer (the bytes of cv2.imwrite), any other format by cv2.imwrite.  When the curve fit fails (the
       reference raises), the fixed 8x8 grid and clip 2 are used and a note is printed.  When both arguments are directories,
       every *.jpg / *.jpeg of the input directory is processed into the output directory under the same name, grouped by
@@ -96,7 +97,7 @@ def _grey_device(ctx, jobs, opt, named):
     import cv2
     import torch
 
-    from .chain import _notes
+    from .chain import _exact_size, _notes
 
     exif = opt["orientation"] == "exif"
     groups = {}
@@ -105,7 +106,7 @@ def _grey_device(ctx, jobs, opt, named):
             with open(src, "rb") as f:
                 data = f.read()
             item = (dst, data, None)
-            size = ctx.jpeg_size(data) if exif else ctx.jpeg_info(data)
+            size = _exact_size(ctx, data, exif)
         else:
             img = cv2.imread(src, 0)
             if img is None:
@@ -120,7 +121,7 @@ def _grey_device(ctx, jobs, opt, named):
             part = items[b0:b0 + opt["batch"]]
             n = len(part)
             if part[0][1] is not None:   # one JPEG job per batch unless in directory mode, which reads only JPEG files
-                d_in = ctx.jpeg_decode_grey_batch_dev([data for _, data, _ in part], orientation=exif)
+                d_in = ctx.jpeg_decode_grey_batch_dev([data for _, data, _ in part], orientation=exif, progressive=True)
                 dflags = ctx.last_frame_flags(n)   # read now: the CLAHE call resets the flags
             else:
                 d_in = torch.from_numpy(part[0][2]).to(dev)[None]

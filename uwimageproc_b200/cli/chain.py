@@ -14,15 +14,16 @@ bytes - the pixels never exist on the host (SURVEY 8f row N3).  Other formats ta
 for byte what cv2.imwrite(output, <chain output>) writes at -q, as the reference's command lines do.  The default, nvjpeg,
 writes nvJPEG's bytes (its own DCT, quantisation and entropy coding).
 
--decoder=exact: the input JPEG is read by the project's own batched decoder (uwip_jpeg_decode_bgr8_batch), whose pixels are
-those cv2.imread(input) returns, as the reference's command lines read them.  The default, nvjpeg, gives nvJPEG's pixels (a
+-decoder=exact: the input JPEG is read by the project's own batched decoder (uwip_jpeg_decode_batch_ex), whose pixels are
+those cv2.imread(input) returns, as the reference's command lines read them; baseline and progressive files alike, in one
+batch.  A progressive file whose progression is incomplete at EOI is refused (cv2 reads it with block smoothing).  The default, nvjpeg, gives nvJPEG's pixels (a
 few levels away, mostly in the 4:2:0 chroma upsampling), so the two decoders give different outputs, not the same output at
 different speeds.  With -decoder=exact -encoder=exact the file written is cv2.imwrite(output, chain(cv2.imread(input))), with
 -aclahe=auto too, and the pixels never exist on the host: for every file with -orientation=exif, and for files without an
 Exif orientation tag with the default.
 
 -orientation=exif (needs -decoder=exact; nvJPEG does not read Exif): each file is turned by its Exif orientation as
-cv2.imread does (uwip_jpeg_decode_bgr8_batch_oriented), so a photograph taken with the camera on its side comes out upright,
+cv2.imread does (uwip_jpeg_decode_batch_ex with UWIP_JPEG_ORIENT), so a photograph taken with the camera on its side comes out upright,
 with width and height swapped for orientations 5 to 8.  The default, ignore, keeps the stored orientation
 (cv2.IMREAD_IGNORE_ORIENTATION).
 
@@ -52,22 +53,28 @@ def _read(path):
         return f.read()
 
 
+def _exact_size(ctx, data, exif):
+    """(width, height) of the image the exact reader gives: after the Exif orientation with exif, else the stored size"""
+    w, h, o, _ = ctx.jpeg_probe(data)
+    return (h, w) if not exif and o >= 5 else (w, h)
+
+
 def _run_jpegs(ctx, jobs, opt, named):
     """jobs: (output path, JPEG file bytes) pairs, grouped by size and run in batches of opt['batch'] frames through the
     decoder, chain and encoder that opt names.  named: each file's report starts with its name (directory mode)."""
     import torch
 
-    exif = opt["orientation"] == "exif"
+    exif, exact = opt["orientation"] == "exif", opt["decoder"] == "exact"
     groups = {}
     for path, data in jobs:
-        groups.setdefault(ctx.jpeg_size(data) if exif else ctx.jpeg_info(data), []).append((path, data))
+        groups.setdefault(_exact_size(ctx, data, exif) if exact else ctx.jpeg_info(data), []).append((path, data))
     auto, q = opt["aclahe"] == "auto", opt["q"]
     for (w, h), files in groups.items():
         for b0 in range(0, len(files), opt["batch"]):
             part = files[b0:b0 + opt["batch"]]
             n = len(part)
             if opt["decoder"] == "exact":
-                d_in = ctx.jpeg_decode_batch_dev([d for _, d in part], orientation=exif)
+                d_in = ctx.jpeg_decode_batch_dev([d for _, d in part], orientation=exif, progressive=True)
                 dflags = ctx.last_frame_flags(n)   # read now: the chain's call resets the flags
             else:
                 d_in = torch.empty((n, h, w, 3), dtype=torch.uint8, device="cuda:%d" % ctx.device)

@@ -914,7 +914,7 @@ int uwip_jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n_
   return jpeg_encode_u8_batch_dev(ctx, d_planes, n_frames, width, height, quality, d_out, out_stride, d_len);
 }
 
-// the argument checks of the two batched readers (in the caller, whose name the messages carry)
+// the argument checks of the batched readers (in the caller, whose name the messages carry)
 #define DECODE_BATCH_REQUIRE(ctx, d_out)                                                                                         \
   UWIP_REQUIRE(ctx, jpegs && lens && d_out && n_frames > 0 && n_frames <= 65535, "bad argument (n_frames must lie in 1..65535)"); \
   UWIP_REQUIRE(ctx, width >= 1 && width <= 65500 && height >= 1 && height <= 65500, "width and height must lie in 1..65500");    \
@@ -925,7 +925,7 @@ int uwip_jpeg_decode_bgr8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, cons
   DECODE_BATCH_REQUIRE(ctx, d_bgr);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false, false);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false, false, false);
 }
 int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_planes, int width,
                               int height) {
@@ -933,7 +933,7 @@ int uwip_jpeg_decode_u8_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const 
   DECODE_BATCH_REQUIRE(ctx, d_planes);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true, false);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true, false, false);
 }
 int uwip_jpeg_decode_bgr8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_bgr,
                                          int width, int height) {
@@ -941,7 +941,7 @@ int uwip_jpeg_decode_bgr8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jp
   DECODE_BATCH_REQUIRE(ctx, d_bgr);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false, true);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_bgr, width, height, flags, false, true, false);
 }
 int uwip_jpeg_decode_u8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_planes,
                                        int width, int height) {
@@ -949,7 +949,21 @@ int uwip_jpeg_decode_u8_batch_oriented(uwip_ctx* ctx, const uint8_t* const* jpeg
   DECODE_BATCH_REQUIRE(ctx, d_planes);
   int32_t* flags = flags_get(ctx, n_frames);
   if (!flags) return UWIP_ERR_NOMEM;
-  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true, true);
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_planes, width, height, flags, true, true, false);
+}
+int uwip_jpeg_decode_batch_ex(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n_frames, uint8_t* d_out, int width,
+                              int height, int flags) {
+  CTX_GUARD(ctx);
+  DECODE_BATCH_REQUIRE(ctx, d_out);
+  UWIP_REQUIRE(ctx, (flags & ~(UWIP_JPEG_GREY | UWIP_JPEG_ORIENT)) == 0, "flags must be a combination of UWIP_JPEG_GREY and UWIP_JPEG_ORIENT");
+  int32_t* fl = flags_get(ctx, n_frames);
+  if (!fl) return UWIP_ERR_NOMEM;
+  return jpeg_decode_batch(ctx, jpegs, lens, n_frames, d_out, width, height, fl, (flags & UWIP_JPEG_GREY) != 0,
+                           (flags & UWIP_JPEG_ORIENT) != 0, true);
+}
+int uwip_jpeg_probe(const uint8_t* jpeg, size_t len, int* width, int* height, int* orientation, int* progressive) {
+  if (!jpeg || !len || !width || !height || !orientation || !progressive) return UWIP_ERR_INVALID;
+  return jpeg_probe(jpeg, len, width, height, orientation, progressive);
 }
 int uwip_jpeg_orientation(const uint8_t* jpeg, size_t len, int* orientation) {
   if (!jpeg || !len || !orientation) return UWIP_ERR_INVALID;

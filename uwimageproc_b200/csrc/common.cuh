@@ -417,9 +417,11 @@ int jpeg_encode_u8_batch_dev(uwip_ctx* ctx, const uint8_t* d_planes, int n, int 
                              uint64_t* d_len);
 
 // jpegdec.cu: d_out receives bgr8 frames, or grey planes (IMREAD_GRAYSCALE) when grey is set; orient: each frame turned by
-// its Exif orientation (cv2.imdecode's default flags), w x h being the size after it
+// its Exif orientation (cv2.imdecode's default flags), w x h being the size after it; prog_ok: progressive files accepted
+// too (uwip_jpeg_decode_batch_ex)
 int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_out, int w, int h,
-                      int32_t* d_flags, bool grey, bool orient);
+                      int32_t* d_flags, bool grey, bool orient, bool prog_ok);
+int jpeg_probe(const uint8_t* data, size_t len, int* width, int* height, int* orientation, int* progressive);
 // the Exif orientation cv2.imdecode applies (1..8) from the host marker reader; its status when the header is refused
 int jpeg_orientation(const uint8_t* data, size_t len, int* orientation);
 void jpeg_dec_destroy(uwip_ctx* ctx);

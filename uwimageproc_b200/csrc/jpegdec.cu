@@ -23,9 +23,19 @@
 // The oriented readers apply each frame's Exif orientation (cv2.imdecode's default flags) in the output pass only: the
 // oriented pass replaces color / grey with a CTA per 32 x 32 output tile that forms the tile's stored pixels in shared memory
 // from rows of the sample planes and writes them out as rows of the output (a column of stored pixels for 5..8).
-// Bad entropy-coded data (an invalid code, a coefficient past 63, the data ending before the last block, the wrong number of
-// RST markers) leaves the frame all zeros and sets UWIP_FRAME_JPEG_BAD.  A frame's pixels do not depend on the batch it is in.
+// Progressive frames (uwip_jpeg_decode_batch_ex) skip destuff .. huff and take two passes of their own, which write the same
+// zeroed coefficient store, so one batch may mix them with sequential frames:
+//   pdestuff a CTA per (frame, scan): the scan's compact stream and restart offsets
+//   prog     one launch per dependency level (1 + the level of the latest earlier scan of the frame that touches an
+//            overlapping component and coefficient range), a warp per (frame, scan, restart interval) whose lane 0 runs
+//            the scan's jdphuff.c decoder.  A refinement scan's bit consumption depends on the coefficients already decoded,
+//            so a scan does not cut into self-synchronising pieces; frames, disjoint scans and restart intervals run in
+//            parallel.
+// Bad entropy-coded data (an invalid code, a coefficient past 63 or past Se, the data ending before the last block, the wrong
+// number of RST markers, a progressive file cut inside a scan) leaves the frame all zeros and sets UWIP_FRAME_JPEG_BAD.  A
+// frame's pixels do not depend on the batch it is in.
 #include <algorithm>
+#include <memory>
 #include <vector>
 
 #include "common.cuh"
@@ -45,6 +55,8 @@ constexpr int DESTUFF_BYTES = 16;  // per thread and tile
 constexpr int IDCT_T = 128;
 constexpr int COLOR_T = 256;
 constexpr int TILE = 32;           // output tile edge of the oriented pass
+constexpr int PROG_T = 128;        // progressive entropy decode: threads per CTA, a warp per (scan, restart interval)
+constexpr int PROG_PAD = 512;      // bytes after each scan's compact stream: a unit may look this far past short data
 
 struct FrameTab {
   Geo g;
@@ -56,6 +68,16 @@ struct FrameTab {
   uint64_t sub_off, int_off;   // first subsequence slot, first interval slot (nint + 1 of them)
   uint32_t sub_cap;            // subsequence slots (a multiple of SYNC_T)
   int32_t orient;              // Exif orientation applied by the oriented pass, 1..8
+  int32_t prog;                // 0: sequential; 1: progressive (the sequential passes skip it); 2: progressive, cut short
+};
+
+// A scan of a progressive frame.  Its segment is staged at seg_off and its compact stream written at the same offset of the
+// compact buffer; ist (nint + 1 entries at int_off) holds the compact byte offset of each restart interval.
+struct ScanTab {
+  jpegdec::PScan s;
+  int32_t frame;
+  int32_t tbl[3];              // the decoding table of each scan component (index into the scan tables), -1: none
+  uint64_t seg_off, seg_len, int_off;
 };
 
 struct Sub {
@@ -93,19 +115,11 @@ __device__ __forceinline__ T cta_exclusive_scan(T v, T& excl, T* s_warp) {
   return total;
 }
 
-__global__ void __launch_bounds__(CTA_T) jpeg_dec_destuff_kernel(const FrameTab* __restrict__ tabs, const uint8_t* __restrict__ stage,
-                                                                   uint8_t* __restrict__ comp, uint32_t* __restrict__ istart,
-                                                                   uint32_t* __restrict__ ibase, Sub* __restrict__ subs,
-                                                                   int* __restrict__ nsub, int32_t* __restrict__ flags) {
-  __shared__ unsigned long long s_warp[32];
-  __shared__ unsigned long long s_end;
-  const int f = blockIdx.x;
-  const FrameTab& t = tabs[f];
-  const uint64_t len = t.seg_len;
-  const int nint = t.g.nint;
-  const uint8_t* seg = stage + t.seg_off;
-  uint8_t* cs = comp + t.seg_off;
-  uint32_t* ist = istart + t.int_off;
+// One entropy-coded segment seg[0..len) -> its compact stream cs (without the 0x00 after each 0xFF, fill bytes and RST
+// markers) and the compact byte offset of each of its nint restart intervals, ist[0..nint].  The segment ends at the first
+// marker other than RSTn.  Returns true for the wrong number of RST markers.  The whole CTA calls it.
+__device__ __forceinline__ bool destuff_segment(const uint8_t* __restrict__ seg, uint64_t len, int nint, uint8_t* __restrict__ cs,
+                                                uint32_t* __restrict__ ist, unsigned long long* s_warp, unsigned long long& s_end) {
   if (threadIdx.x == 0) s_end = len;
   __syncthreads();
   unsigned long long carry = 0;   // kept bytes | RST markers << 40
@@ -151,12 +165,32 @@ __global__ void __launch_bounds__(CTA_T) jpeg_dec_destuff_kernel(const FrameTab*
     stop = e;
   }
   const uint32_t ncomp_bytes = (uint32_t)(carry & KEEP);
-  const bool bad = (carry >> 40) != (unsigned long long)(nint - 1);
   if (threadIdx.x == 0) {
     ist[0] = 0;
     ist[nint] = ncomp_bytes;
   }
   __syncthreads();
+  return (carry >> 40) != (unsigned long long)(nint - 1);
+}
+
+__global__ void __launch_bounds__(CTA_T) jpeg_dec_destuff_kernel(const FrameTab* __restrict__ tabs, const uint8_t* __restrict__ stage,
+                                                                   uint8_t* __restrict__ comp, uint32_t* __restrict__ istart,
+                                                                   uint32_t* __restrict__ ibase, Sub* __restrict__ subs,
+                                                                   int* __restrict__ nsub, int32_t* __restrict__ flags) {
+  __shared__ unsigned long long s_warp[32];
+  __shared__ unsigned long long s_end;
+  const int f = blockIdx.x;
+  const FrameTab& t = tabs[f];
+  if (t.prog) {   // a progressive frame: the progressive passes decode it
+    if (threadIdx.x == 0) {
+      nsub[f] = 0;
+      if (t.prog == 2) atomicOr(flags + f, UWIP_FRAME_JPEG_BAD);
+    }
+    return;
+  }
+  const int nint = t.g.nint;
+  uint32_t* ist = istart + t.int_off;
+  const bool bad = destuff_segment(stage + t.seg_off, t.seg_len, nint, comp + t.seg_off, ist, s_warp, s_end);
   if (bad) {   // the wrong number of restart markers
     if (threadIdx.x == 0) {
       nsub[f] = 0;
@@ -387,6 +421,50 @@ __global__ void __launch_bounds__(SYNC_T) jpeg_dec_huff_kernel(const FrameTab* _
   if (bad) atomicOr(flags + f, UWIP_FRAME_JPEG_BAD);
 }
 
+// ---- progressive frames ----------------------------------------------------------------------------------------------
+// a CTA per scan: its compact stream and restart offsets
+__global__ void __launch_bounds__(CTA_T) jpeg_dec_pdestuff_kernel(const ScanTab* __restrict__ scans, const uint8_t* __restrict__ stage,
+                                                                    uint8_t* __restrict__ comp, uint32_t* __restrict__ pist,
+                                                                    int32_t* __restrict__ flags) {
+  __shared__ unsigned long long s_warp[32];
+  __shared__ unsigned long long s_end;
+  const ScanTab& st = scans[blockIdx.x];
+  const bool bad = destuff_segment(stage + st.seg_off, st.seg_len, st.s.nint, comp + st.seg_off, pist + st.int_off, s_warp, s_end);
+  if (bad && threadIdx.x == 0) atomicOr(flags + st.frame, UWIP_FRAME_JPEG_BAD);
+}
+
+// A warp per (scan, restart interval) of one dependency level, decoded by its lane 0: list[0..nlist) are the level's scans
+// and first[i] the first item of scan list[i].  The decode is serial and its branches depend on the data, so items that
+// shared a warp would run one after another; a warp each keeps them concurrent.  The scans of a level touch disjoint
+// coefficients, so their items write the store concurrently.  A frame already flagged (bad data in an earlier pass, or the
+// wrong number of RST markers) is skipped: its restart offsets may be incomplete.
+__global__ void __maxnreg__(128) jpeg_dec_prog_kernel(const FrameTab* __restrict__ tabs, const ScanTab* __restrict__ scans,
+                                                                const DTbl* __restrict__ dtbl, const uint8_t* __restrict__ comp,
+                                                                const uint32_t* __restrict__ pist, const int32_t* __restrict__ list,
+                                                                const uint64_t* __restrict__ first, int nlist, uint64_t total,
+                                                                int16_t* __restrict__ coef, int32_t* __restrict__ flags) {
+  const uint64_t i = ((uint64_t)blockIdx.x * PROG_T + threadIdx.x) / 32;
+  if (i >= total || (threadIdx.x & 31)) return;
+  int lo = 0, hi = nlist - 1;   // the last scan whose first item is at or before i
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (first[mid] <= i) lo = mid;
+    else hi = mid - 1;
+  }
+  const ScanTab& st = scans[list[lo]];
+  const int f = st.frame;
+  if (*(volatile const int32_t*)(flags + f) & UWIP_FRAME_JPEG_BAD) return;
+  const FrameTab& t = tabs[f];
+  const jpegdec::PScan& s = st.s;
+  const int k = (int)(i - first[lo]);
+  const uint32_t* ist = pist + st.int_off;
+  Bits b;
+  b.init(comp + st.seg_off, ist[k] * 8u);
+  const int u0 = s.ri ? k * s.ri : 0, u1 = s.ri ? min(u0 + s.ri, s.nunits) : s.nunits;
+  const DTbl* tb[3] = {dtbl + max(st.tbl[0], 0), dtbl + max(st.tbl[1], 0), dtbl + max(st.tbl[2], 0)};
+  if (!jpegdec::decode_interval(t.g, s, tb, b, ist[k + 1] * 8u, coef + t.blk_off * 64, u0, u1)) atomicOr(flags + f, UWIP_FRAME_JPEG_BAD);
+}
+
 // Y_ONLY: the blocks of component 0 (grey output); the chroma blocks' threads exit
 template <bool Y_ONLY>
 __global__ void __launch_bounds__(IDCT_T) jpeg_dec_idct_kernel(const FrameTab* __restrict__ tabs, const int16_t* __restrict__ coef,
@@ -516,23 +594,51 @@ int jpeg_orientation(const uint8_t* data, size_t len, int* orientation) {
   return rc;
 }
 
+int jpeg_probe(const uint8_t* data, size_t len, int* width, int* height, int* orientation, int* progressive) {
+  jpegdec::Header hd;
+  std::unique_ptr<jpegdec::Prog> pg(new jpegdec::Prog);
+  const int rc = jpegdec::parse_file(data, len, hd, pg.get());
+  if (rc != jpegdec::OK) return rc;
+  const bool t = hd.orientation >= 5;
+  *width = t ? hd.height : hd.width;
+  *height = t ? hd.width : hd.height;
+  *orientation = hd.orientation;
+  *progressive = pg->nscans > 0;
+  return UWIP_OK;
+}
+
 int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* lens, int n, uint8_t* d_out, int w, int h,
-                      int32_t* d_flags, bool grey, bool orient) {
-  const char* fn = grey ? orient ? "uwip_jpeg_decode_u8_batch_oriented" : "uwip_jpeg_decode_u8_batch"
-                        : orient ? "uwip_jpeg_decode_bgr8_batch_oriented" : "uwip_jpeg_decode_bgr8_batch";
+                      int32_t* d_flags, bool grey, bool orient, bool prog_ok) {
+  const char* fn = prog_ok ? "uwip_jpeg_decode_batch_ex"
+                   : grey  ? orient ? "uwip_jpeg_decode_u8_batch_oriented" : "uwip_jpeg_decode_u8_batch"
+                           : orient ? "uwip_jpeg_decode_bgr8_batch_oriented" : "uwip_jpeg_decode_bgr8_batch";
   // ---- parse every header on the host
   std::vector<FrameTab> tabs((size_t)n);
+  std::vector<ScanTab> scans;   // the scans of the progressive frames, frame by frame
+  std::vector<int> level;       // each scan's dependency level, 1..
+  std::vector<DTbl> dtbl;       // their decoding tables
+  struct Copy {
+    const uint8_t* src;
+    size_t len;
+    uint64_t off;
+  };
+  std::vector<Copy> copies;     // the segments to stage
+  std::unique_ptr<jpegdec::Prog> pg(prog_ok ? new jpegdec::Prog : nullptr);
   jpegdec::Header hd;
-  size_t seg_total = 0, int_total = 0, sub_total = 0, blk_total = 0, smp_total = 0;
+  size_t seg_total = 0, int_total = 0, sub_total = 0, blk_total = 0, smp_total = 0, pint_total = 0;
   uint32_t max_cap = 0;
   size_t max_blocks = 0;
+  int max_level = 0;
   for (int f = 0; f < n; f++) {
-    const int rc = jpegdec::parse_header(jpegs[f], lens[f], hd);
+    const int rc = jpegdec::parse_file(jpegs[f], lens[f], hd, pg.get());
     if (rc != jpegdec::OK) {
       uwip_set_err(ctx, "%s: file %d: %s", fn, f,
-                   rc == jpegdec::UNSUPPORTED ? "coding not supported (progressive, arithmetic, lossless, 12-bit, multi-scan, CMYK, RGB "
-                                                "or sampling other than 4:4:4 / 4:2:2 / 4:4:0 / 4:2:0 / grey)"
-                                              : "malformed or truncated header");
+                   rc != jpegdec::UNSUPPORTED ? "malformed or truncated header"
+                   : prog_ok ? "coding not supported (arithmetic, lossless, 12-bit, multi-scan sequential, CMYK, RGB, sampling other than "
+                               "4:4:4 / 4:2:2 / 4:4:0 / 4:2:0 / grey, or a progression incomplete at EOI or with an Ah that is not "
+                               "the previous Al)"
+                             : "coding not supported (progressive, arithmetic, lossless, 12-bit, multi-scan, CMYK, RGB "
+                               "or sampling other than 4:4:4 / 4:2:2 / 4:4:0 / 4:2:0 / grey)");
       return rc;
     }
     const int o = orient ? hd.orientation : 1;   // the stored size is the output size, transposed for 5..8
@@ -541,27 +647,79 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
       else uwip_set_err(ctx, "%s: file %d is %d x %d with Exif orientation %d, which does not turn it into %d x %d", fn, f, hd.width, hd.height, o, w, h);
       return UWIP_ERR_INVALID;
     }
+    const bool prog = pg && pg->nscans > 0;
+    if (prog) hd.restart = 0;   // each scan has its own
     FrameTab& t = tabs[f];
     t.g = jpegdec::geometry(hd);
     t.orient = o;
-    for (int c = 0; c < hd.ncomp; c++) {
-      memcpy(t.q[c], hd.q[hd.comp[c].tq], sizeof(t.q[c]));
-      if (!jpegdec::make_derived(hd.dc[hd.comp[c].td], true, t.dc[c]) || !jpegdec::make_derived(hd.ac[hd.comp[c].ta], false, t.ac[c])) {
-        uwip_set_err(ctx, "%s: file %d: bad Huffman table", fn, f);
+    t.prog = prog ? (pg->truncated ? 2 : 1) : 0;
+    if (!prog) {
+      for (int c = 0; c < hd.ncomp; c++) {
+        memcpy(t.q[c], hd.q[hd.comp[c].tq], sizeof(t.q[c]));
+        if (!jpegdec::make_derived(hd.dc[hd.comp[c].td], true, t.dc[c]) || !jpegdec::make_derived(hd.ac[hd.comp[c].ta], false, t.ac[c])) {
+          uwip_set_err(ctx, "%s: file %d: bad Huffman table", fn, f);
+          return UWIP_ERR_INVALID;
+        }
+      }
+      t.seg_len = lens[f] - hd.scan_off;
+      if (t.seg_len > (size_t)0x1FFFFFF0) {
+        uwip_set_err(ctx, "%s: file %d: entropy-coded segment above 512 MB", fn, f);
         return UWIP_ERR_INVALID;
       }
+      t.seg_off = seg_total;
+      seg_total += a16(t.seg_len) + 16;
+      copies.push_back({jpegs[f] + (lens[f] - t.seg_len), t.seg_len, t.seg_off});
+      const uint64_t cap = (t.seg_len * 8 + SUB_BITS - 1) / SUB_BITS + (uint64_t)t.g.nint;
+      t.sub_cap = (uint32_t)((cap + SYNC_T - 1) / SYNC_T * SYNC_T);
+    } else {
+      for (int c = 0; c < hd.ncomp; c++) memcpy(t.q[c], pg->q[c], sizeof(t.q[c]));
+      t.seg_off = seg_total;
+      t.seg_len = 0;
+      t.sub_cap = 0;
+      const size_t s0 = scans.size();
+      for (int i = 0; i < pg->nscans && !pg->truncated; i++) {   // a frame cut short is only flagged
+        const jpegdec::ProgScan& p = pg->scan[i];
+        ScanTab sc;
+        memset(&sc, 0, sizeof(sc));
+        sc.s = p.s;
+        sc.frame = f;
+        for (int j = 0; j < 3; j++) {
+          sc.tbl[j] = -1;
+          if (j >= p.s.ns || (p.s.ss == 0 && p.s.ah != 0)) continue;   // DC refinement reads raw bits
+          DTbl d;
+          if (!jpegdec::make_derived(p.tab[j], p.s.ss == 0, d)) {
+            uwip_set_err(ctx, "%s: file %d: bad Huffman table in scan %d", fn, f, i);
+            return UWIP_ERR_INVALID;
+          }
+          sc.tbl[j] = (int32_t)dtbl.size();
+          dtbl.push_back(d);
+        }
+        if (p.len > (size_t)0x1FFFFFF0) {
+          uwip_set_err(ctx, "%s: file %d: entropy-coded segment above 512 MB", fn, f);
+          return UWIP_ERR_INVALID;
+        }
+        sc.seg_off = seg_total;
+        sc.seg_len = p.len;
+        seg_total += a16(p.len) + PROG_PAD;
+        copies.push_back({jpegs[f] + p.off, p.len, sc.seg_off});
+        sc.int_off = pint_total;
+        pint_total += (size_t)p.s.nint + 1;
+        // 1 + the level of the latest earlier scan of the frame that touches an overlapping (component, coefficient range)
+        int lv = 1;
+        for (size_t e = s0; e < scans.size(); e++) {
+          const jpegdec::PScan& q = scans[e].s;
+          bool overlap = false;
+          for (int a = 0; a < p.s.ns; a++)
+            for (int b = 0; b < q.ns; b++) overlap |= p.s.comp[a] == q.comp[b] && p.s.ss <= q.se && q.ss <= p.s.se;
+          if (overlap) lv = std::max(lv, level[e] + 1);
+        }
+        scans.push_back(sc);
+        level.push_back(lv);
+        max_level = std::max(max_level, lv);
+      }
     }
-    t.seg_len = lens[f] - hd.scan_off;
-    if (t.seg_len > (size_t)0x1FFFFFF0) {
-      uwip_set_err(ctx, "%s: file %d: entropy-coded segment above 512 MB", fn, f);
-      return UWIP_ERR_INVALID;
-    }
-    t.seg_off = seg_total;
-    seg_total += a16(t.seg_len) + 16;
     t.int_off = int_total;
     int_total += (size_t)t.g.nint + 1;
-    const uint64_t cap = (t.seg_len * 8 + SUB_BITS - 1) / SUB_BITS + (uint64_t)t.g.nint;
-    t.sub_cap = (uint32_t)((cap + SYNC_T - 1) / SYNC_T * SYNC_T);
     t.sub_off = sub_total;
     sub_total += t.sub_cap;
     t.blk_off = blk_total;
@@ -571,21 +729,47 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
     max_cap = std::max(max_cap, t.sub_cap);
     max_blocks = std::max(max_blocks, t.g.nblocks);
   }
-  // ---- device workspace: tables | staged segments | compact streams | interval starts, first subsequences | nsub | stats |
-  //      subsequences | entry states | exit states | counts / DC | prefixes | coefficients | sample planes
-  const size_t b_tab = a16((size_t)n * sizeof(FrameTab)), b_seg = a16(seg_total + 16), b_int = a16(int_total * 4);
+  // the scans by level, and the first thread (scan, restart interval) of each in its level's launch
+  const size_t ns = scans.size();
+  std::vector<int32_t> list;
+  std::vector<uint64_t> first;
+  std::vector<size_t> lv_start((size_t)max_level + 2, 0);
+  std::vector<uint64_t> lv_total((size_t)max_level + 1, 0);
+  for (int l = 1; l <= max_level; l++) {
+    lv_start[l] = list.size();
+    for (size_t i = 0; i < ns; i++)
+      if (level[i] == l) {
+        list.push_back((int32_t)i);
+        first.push_back(lv_total[l]);
+        lv_total[l] += (uint64_t)scans[i].s.nint;
+      }
+  }
+  lv_start[max_level + 1] = list.size();
+  // ---- device workspace: tables (frames | scans | scan decoding tables | level lists | first threads) | staged segments |
+  //      compact streams | interval starts, first subsequences | scan interval starts | nsub | stats | subsequences |
+  //      entry states | exit states | counts / DC | prefixes | coefficients | sample planes
+  const size_t b_tab = a16((size_t)n * sizeof(FrameTab)), b_scan = a16(ns * sizeof(ScanTab)), b_dt = a16(dtbl.size() * sizeof(DTbl)),
+               b_list = a16(ns * 4), b_first = a16(ns * 8);
+  const size_t b_tabs = b_tab + b_scan + b_dt + b_list + b_first;
+  const size_t tab_bytes = ns ? b_tabs : (size_t)n * sizeof(FrameTab);   // the bytes copied up
+  const size_t b_seg = a16(seg_total + 16), b_int = a16(int_total * 4), b_pint = a16(pint_total * 4);
   const size_t b_ns = a16((size_t)n * 4), b_st = a16((size_t)n * 8), b_sub = sub_total * sizeof(Sub), b_e = sub_total * 8,
                b_cd = sub_total * 16, b_coef = blk_total * 128;
-  const size_t total = b_tab + 2 * b_seg + 2 * b_int + b_ns + b_st + b_sub + 2 * b_e + 2 * b_cd + b_coef + smp_total;
+  const size_t total = b_tabs + 2 * b_seg + 2 * b_int + b_pint + b_ns + b_st + b_sub + 2 * b_e + 2 * b_cd + b_coef + smp_total;
   uint8_t* ws = (uint8_t*)uwip_slot(ctx, SLOT_JPEGDEC, total);
   if (!ws) return UWIP_ERR_NOMEM;
   uint8_t* p = ws;
   auto take = [&](size_t b) { uint8_t* r = p; p += b; return r; };
   FrameTab* d_tab = (FrameTab*)take(b_tab);
+  ScanTab* d_scan = (ScanTab*)take(b_scan);
+  DTbl* d_dt = (DTbl*)take(b_dt);
+  int32_t* d_list = (int32_t*)take(b_list);
+  uint64_t* d_first = (uint64_t*)take(b_first);
   uint8_t* d_seg = take(b_seg);
   uint8_t* d_comp = take(b_seg);
   uint32_t* d_ist = (uint32_t*)take(b_int);
   uint32_t* d_ibase = (uint32_t*)take(b_int);
+  uint32_t* d_pist = (uint32_t*)take(b_pint);
   int* d_nsub = (int*)take(b_ns);
   int32_t* d_stats = (int32_t*)take(b_st);
   int4* d_cd = (int4*)take(b_cd);
@@ -598,7 +782,7 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
   ctx->jdec_stats = d_stats;
   ctx->jdec_n = n;
   // ---- pinned staging: segments then tables; the copies of the previous call must have read it
-  const size_t pin_bytes = seg_total + 16 + b_tab;
+  const size_t pin_bytes = seg_total + 16 + b_tabs;
   if (ctx->jdec_ev) UWIP_CUDA(ctx, cudaEventSynchronize(ctx->jdec_ev));
   else UWIP_CUDA(ctx, cudaEventCreateWithFlags(&ctx->jdec_ev, cudaEventDisableTiming));
   if (ctx->jdec_pinned_bytes < pin_bytes) {
@@ -615,10 +799,17 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
     ctx->jdec_pinned_bytes = want;
   }
   uint8_t* pin = (uint8_t*)ctx->jdec_pinned;
-  for (int f = 0; f < n; f++) memcpy(pin + tabs[f].seg_off, jpegs[f] + (lens[f] - tabs[f].seg_len), tabs[f].seg_len);
-  memcpy(pin + seg_total + 16, tabs.data(), (size_t)n * sizeof(FrameTab));
+  for (const Copy& c : copies) memcpy(pin + c.off, c.src, c.len);
+  uint8_t* ptab = pin + seg_total + 16;
+  memcpy(ptab, tabs.data(), (size_t)n * sizeof(FrameTab));
+  if (ns) {
+    memcpy(ptab + b_tab, scans.data(), ns * sizeof(ScanTab));
+    memcpy(ptab + b_tab + b_scan, dtbl.data(), dtbl.size() * sizeof(DTbl));
+    memcpy(ptab + b_tab + b_scan + b_dt, list.data(), ns * 4);
+    memcpy(ptab + b_tab + b_scan + b_dt + b_list, first.data(), ns * 8);
+  }
   UWIP_CUDA(ctx, cudaMemcpyAsync(d_seg, pin, seg_total, cudaMemcpyHostToDevice, ctx->stream));
-  UWIP_CUDA(ctx, cudaMemcpyAsync(d_tab, pin + seg_total + 16, (size_t)n * sizeof(FrameTab), cudaMemcpyHostToDevice, ctx->stream));
+  UWIP_CUDA(ctx, cudaMemcpyAsync(d_tab, ptab, tab_bytes, cudaMemcpyHostToDevice, ctx->stream));
   UWIP_CUDA(ctx, cudaEventRecord(ctx->jdec_ev, ctx->stream));
   UWIP_CUDA(ctx, cudaMemsetAsync(d_flags, 0, (size_t)n * 4, ctx->stream));
   UWIP_CUDA(ctx, cudaMemsetAsync(d_stats, 0, (size_t)n * 8, ctx->stream));
@@ -627,15 +818,29 @@ int jpeg_decode_batch(uwip_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
   const unsigned ny = (unsigned)n;
   UWIP_LAUNCH(ctx, "jpeg_dec_destuff", jpeg_dec_destuff_kernel, n, CTA_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_seg, d_comp, d_ist,
               d_ibase, d_sub, d_nsub, d_flags);
-  const dim3 gsub(max_cap / SYNC_T, ny);
-  UWIP_LAUNCH(ctx, "jpeg_dec_sync", jpeg_dec_sync_kernel, gsub, SYNC_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
-              (const Sub*)d_sub, (const int*)d_nsub, d_entry, d_exit, d_cd, d_stats);
-  UWIP_LAUNCH(ctx, "jpeg_dec_fixup", jpeg_dec_fixup_kernel, (n + 31) / 32, 32, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
-              (const Sub*)d_sub, (const int*)d_nsub, d_entry, d_exit, d_cd, d_stats, n);
-  UWIP_LAUNCH(ctx, "jpeg_dec_scan", jpeg_dec_scan_kernel, n, CTA_T, 0, (const FrameTab*)d_tab, (const Sub*)d_sub, (const int*)d_nsub,
-              (const uint32_t*)d_ibase, d_cd, d_px);
-  UWIP_LAUNCH(ctx, "jpeg_dec_huff", jpeg_dec_huff_kernel, gsub, SYNC_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
-              (const Sub*)d_sub, (const int*)d_nsub, (const uint64_t*)d_entry, (const int4*)d_cd, d_coef, d_flags);
+  if (max_cap) {   // the sequential frames
+    const dim3 gsub(max_cap / SYNC_T, ny);
+    UWIP_LAUNCH(ctx, "jpeg_dec_sync", jpeg_dec_sync_kernel, gsub, SYNC_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
+                (const Sub*)d_sub, (const int*)d_nsub, d_entry, d_exit, d_cd, d_stats);
+    UWIP_LAUNCH(ctx, "jpeg_dec_fixup", jpeg_dec_fixup_kernel, (n + 31) / 32, 32, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
+                (const Sub*)d_sub, (const int*)d_nsub, d_entry, d_exit, d_cd, d_stats, n);
+    UWIP_LAUNCH(ctx, "jpeg_dec_scan", jpeg_dec_scan_kernel, n, CTA_T, 0, (const FrameTab*)d_tab, (const Sub*)d_sub, (const int*)d_nsub,
+                (const uint32_t*)d_ibase, d_cd, d_px);
+    UWIP_LAUNCH(ctx, "jpeg_dec_huff", jpeg_dec_huff_kernel, gsub, SYNC_T, 0, (const FrameTab*)d_tab, (const uint8_t*)d_comp,
+                (const Sub*)d_sub, (const int*)d_nsub, (const uint64_t*)d_entry, (const int4*)d_cd, d_coef, d_flags);
+  }
+  if (ns) {   // the progressive frames: every scan destuffed, then one launch per dependency level
+    UWIP_LAUNCH(ctx, "jpeg_dec_pdestuff", jpeg_dec_pdestuff_kernel, (unsigned)ns, CTA_T, 0, (const ScanTab*)d_scan, (const uint8_t*)d_seg,
+                d_comp, d_pist, d_flags);
+    for (int l = 1; l <= max_level; l++) {
+      const uint64_t tot = lv_total[l];
+      if (!tot) continue;
+      UWIP_LAUNCH(ctx, "jpeg_dec_prog", jpeg_dec_prog_kernel, (unsigned)((tot + PROG_T / 32 - 1) / (PROG_T / 32)), PROG_T, 0, (const FrameTab*)d_tab,
+                  (const ScanTab*)d_scan, (const DTbl*)d_dt, (const uint8_t*)d_comp, (const uint32_t*)d_pist,
+                  (const int32_t*)(d_list + lv_start[l]), (const uint64_t*)(d_first + lv_start[l]), (int)(lv_start[l + 1] - lv_start[l]), tot,
+                  d_coef, d_flags);
+    }
+  }
   const dim3 gblk((unsigned)((max_blocks + IDCT_T - 1) / IDCT_T), ny), gpix((unsigned)(((size_t)w * h + COLOR_T - 1) / COLOR_T), ny);
   if (grey) UWIP_LAUNCH(ctx, "jpeg_dec_idct_y", jpeg_dec_idct_kernel<true>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);
   else UWIP_LAUNCH(ctx, "jpeg_dec_idct", jpeg_dec_idct_kernel<false>, gblk, IDCT_T, 0, (const FrameTab*)d_tab, (const int16_t*)d_coef, d_smp);

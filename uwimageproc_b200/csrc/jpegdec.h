@@ -13,6 +13,12 @@
 // interval, any quantisation and Huffman tables.  Refused as unsupported: progressive, arithmetic, lossless, 12-bit,
 // other sampling factors, multi-scan, four components, RGB-coded three-component files.
 //
+// Progressive files (SOF2): parse_file reads the whole file and records every scan; dc_first / dc_refine / ac_first /
+// ac_refine restate the four decoders of jdphuff.c one block at a time on the same bit reader and tables; decode_frame_ex
+// is the scalar reference of sequential and progressive files alike.  A progression that is not complete at EOI (some
+// coefficient of some component not refined down to Al = 0) is refused: libjpeg-turbo smooths such files
+// (decompress_smooth_data, jdcoefct.c) and this decoder does not restate that.
+//
 // Exif orientation: parse_header records the value cv2 4.13.0's Exif reader reports (exif_orientation below), and
 // oriented_src() maps an output pixel to its stored pixel as cv2's ApplyExifOrientation flips and transposes.  A reader
 // that applies it equals cv2.imdecode with its default flags; one that does not gives the stored orientation
@@ -24,8 +30,10 @@
 
 #ifdef __CUDACC__
 #define JPEG_HD __host__ __device__
+#define JPEG_HDF __host__ __device__ __forceinline__
 #else
 #define JPEG_HD
+#define JPEG_HDF inline
 #endif
 
 namespace jpegdec {
@@ -103,12 +111,75 @@ inline int exif_orientation(const uint8_t* p, size_t n) {
   return -1;
 }
 
+// ---- progressive files (jdphuff.c): what the whole-file marker reader records of each scan ------------------------------
+constexpr int MAX_SCANS = 128;   // more scans than this are refused as unsupported (cv2 and Pillow write 6 to 10)
+
+// A scan's geometry and parameters.  A scan of one component is non-interleaved: its units are that component's own blocks,
+// bw x bh = ceil(dw_c / 8) x ceil(dh_c / 8), in raster order.  A scan of several components (a DC scan) is interleaved: its
+// units are the frame's MCUs made of only its components' blocks, bw x bh = the MCU grid.  ri counts units.
+struct PScan {
+  int ns, comp[3];   // frame component indices in scan order
+  int ss, se, ah, al;
+  int ri, bw, bh, nunits, nint;
+};
+struct ProgScan {
+  PScan s;
+  HuffSpec tab[3];   // per scan component, the table as it stood at this SOS: DC for a DC first scan, AC for an AC scan
+  size_t off, len;   // the entropy-coded segment, up to the marker that ends it
+};
+struct Prog {
+  int nscans;        // 0: a sequential file (the reader then stops at its first SOS, as parse_header does)
+  bool truncated;    // the data ended inside a scan, before the progression was complete: bad data
+  uint16_t q[3][64]; // quantisers latched at each component's first scan (latch_quant_tables), natural order
+  ProgScan scan[MAX_SCANS];
+};
+
+// the colour-space decision of default_decompress_parms (jdapimin.c) and the sampling this decoder accepts
+inline int frame_checks(const Header& hd) {
+  if (hd.ncomp == 3) {
+    bool rgb;
+    if (hd.jfif) rgb = false;
+    else if (hd.adobe) rgb = hd.adobe_transform == 0;
+    else rgb = hd.comp[0].id == 82 && hd.comp[1].id == 71 && hd.comp[2].id == 66;
+    if (rgb) return UNSUPPORTED;
+  } else if (hd.ncomp != 1) {
+    return UNSUPPORTED;   // CMYK / YCCK and other component counts
+  }
+  if (hd.ncomp == 3) {
+    const int hy = hd.comp[0].h, vy = hd.comp[0].v;
+    for (int i = 1; i < 3; i++)
+      if (hd.comp[i].h != 1 || hd.comp[i].v != 1) return UNSUPPORTED;
+    if (hy > 2 || vy > 2) return UNSUPPORTED;
+  }
+  return OK;
+}
+
 // read_markers / first_marker / next_marker / get_sof / get_sos / get_dht / get_dqt / get_dri / examine_app0 / examine_app14 /
 // skip_variable, then the colour-space decision of default_decompress_parms (jdapimin.c) and the checks of initial_setup
-// (jdinput.c) and jinit_upsampler (jdsample.c) that this decoder restricts further.  Stops after the first SOS.
-inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
+// (jdinput.c) and jinit_upsampler (jdsample.c) that this decoder restricts further.
+// pg == nullptr (parse_header): SOF2 is refused and the reader stops after the first SOS.  Otherwise (parse_file) SOF2 is
+// accepted too: a sequential file still ends the read at its first SOS (pg->nscans = 0); a progressive one is read to EOI,
+// recording every scan with the checks of start_pass_phuff_decoder (jdphuff.c) - bad Ss / Se / Ah / Al are INVALID; an Ah
+// other than the Al of the previous scan of that coefficient (libjpeg warns and decodes on) and an incomplete progression
+// at EOI (libjpeg-turbo smooths such files, decompress_smooth_data) are UNSUPPORTED.
+inline int parse_file(const uint8_t* data, size_t len, Header& hd, Prog* pg) {
   memset(&hd, 0, sizeof(hd));
   hd.orientation = 1;
+  if (pg) {
+    pg->nscans = 0;
+    pg->truncated = false;
+  }
+  bool progressive = false;
+  int coef_bits[3][64];   // Al of the last scan of each coefficient, -1: none yet
+  bool latched[3] = {false, false, false};
+  for (int c = 0; c < 3; c++)
+    for (int k = 0; k < 64; k++) coef_bits[c][k] = -1;
+  auto complete = [&]() {
+    for (int c = 0; c < hd.ncomp; c++)
+      for (int k = 0; k < 64; k++)
+        if (coef_bits[c][k] != 0) return false;
+    return true;
+  };
   bool exif = false;   // an Exif APP1 gave an orientation entry: later ones are not read
   Reader r{data, len, 0, true};
   if (r.u8() != 0xFF || r.u8() != 0xD8 || !r.ok) return INVALID;   // first_marker: SOI
@@ -117,10 +188,17 @@ inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
     int c = r.u8();
     while (r.ok && c != 0xFF) c = r.u8();   // next_marker: garbage before a marker is skipped
     do { c = r.u8(); } while (r.ok && c == 0xFF);
-    if (!r.ok) return INVALID;
-    if (c == 0xC0 || c == 0xC1) {   // get_sof: baseline / extended sequential Huffman
+    if (!r.ok) {
+      if (progressive && pg->nscans > 0) {   // the data ended right after a scan, before EOI
+        pg->truncated = !complete();
+        return OK;
+      }
+      return INVALID;
+    }
+    if (c == 0xC0 || c == 0xC1 || (pg && c == 0xC2)) {   // get_sof: baseline / extended sequential / progressive Huffman
       if (sof) return INVALID;
       sof = true;
+      progressive = c == 0xC2;
       const int length = r.u16() - 2;
       const int prec = r.u8();
       hd.height = r.u16();
@@ -142,7 +220,7 @@ inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
       }
       if (!r.ok) return INVALID;
     } else if (c == 0xC2 || c == 0xC3 || (c >= 0xC5 && c <= 0xC7) || (c >= 0xC9 && c <= 0xCB) || (c >= 0xCD && c <= 0xCF)) {
-      return UNSUPPORTED;   // progressive, lossless, differential, arithmetic
+      return UNSUPPORTED;   // progressive (parse_header), lossless, differential, arithmetic
     } else if (c == 0xC4) {   // get_dht
       int length = r.u16() - 2;
       while (length > 16) {
@@ -187,42 +265,103 @@ inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
       const int ns = r.u8();
       if (!r.ok || length != ns * 2 + 6 || ns < 1 || ns > 4) return INVALID;
       bool seen[4] = {false, false, false, false};
+      int sc[4];
       for (int i = 0; i < ns; i++) {
         const int id = r.u8(), t = r.u8();
         int ci = 0;
         while (ci < hd.ncomp && (hd.comp[ci].id != id || seen[ci])) ci++;
         if (ci == hd.ncomp) return INVALID;
         seen[ci] = true;
+        sc[i] = ci;
         hd.comp[ci].td = t >> 4;
         hd.comp[ci].ta = t & 15;
         if (hd.comp[ci].td > 3 || hd.comp[ci].ta > 3) return INVALID;
       }
-      r.u8(); r.u8(); r.u8();   // Ss, Se, Ah/Al: a sequential scan takes them as 0, 63, 0
+      const int ss = r.u8(), se = r.u8(), ahl = r.u8();   // a sequential scan takes them as 0, 63, 0
       if (!r.ok) return INVALID;
       hd.scan_off = r.pos;
-      // default_decompress_parms
-      if (hd.ncomp == 3) {
-        bool rgb;
-        if (hd.jfif) rgb = false;
-        else if (hd.adobe) rgb = hd.adobe_transform == 0;
-        else rgb = hd.comp[0].id == 82 && hd.comp[1].id == 71 && hd.comp[2].id == 66;
-        if (rgb) return UNSUPPORTED;
-      } else if (hd.ncomp != 1) {
-        return UNSUPPORTED;   // CMYK / YCCK and other component counts
+      const int fc = frame_checks(hd);
+      if (fc != OK) return fc;
+      if (!progressive) {
+        if (ns != hd.ncomp) return UNSUPPORTED;   // a multi-scan sequential file
+        for (int i = 0; i < hd.ncomp; i++) {   // latch_quant_tables, jpeg_make_d_derived_tbl's missing-table check
+          if (!hd.qdef[hd.comp[i].tq] || !hd.dc[hd.comp[i].td].defined || !hd.ac[hd.comp[i].ta].defined) return INVALID;
+        }
+        return OK;
       }
-      if (ns != hd.ncomp) return UNSUPPORTED;   // a multi-scan sequential file
-      if (hd.ncomp == 3) {
-        const int hy = hd.comp[0].h, vy = hd.comp[0].v;
-        for (int i = 1; i < 3; i++)
-          if (hd.comp[i].h != 1 || hd.comp[i].v != 1) return UNSUPPORTED;
-        if (hy > 2 || vy > 2) return UNSUPPORTED;
+      // start_pass_phuff_decoder's checks
+      const int ah = ahl >> 4, al = ahl & 15;
+      const bool dc = ss == 0;
+      if (dc ? se != 0 : (ss > se || se > 63 || ns != 1)) return INVALID;
+      if ((ah != 0 && al != ah - 1) || al > 13) return INVALID;
+      if (pg->nscans == MAX_SCANS) return UNSUPPORTED;
+      ProgScan& p = pg->scan[pg->nscans];
+      memset(&p, 0, sizeof(p));
+      p.s.ns = ns;
+      p.s.ss = ss;
+      p.s.se = se;
+      p.s.ah = ah;
+      p.s.al = al;
+      p.s.ri = hd.restart;
+      for (int i = 0; i < ns; i++) {
+        const int ci = sc[i];
+        p.s.comp[i] = ci;
+        if (!latched[ci]) {   // latch_quant_tables: a later DQT does not change a component already latched
+          if (!hd.qdef[hd.comp[ci].tq]) return INVALID;
+          memcpy(pg->q[ci], hd.q[hd.comp[ci].tq], sizeof(pg->q[ci]));
+          latched[ci] = true;
+        }
+        if (dc && ah == 0) {
+          if (!hd.dc[hd.comp[ci].td].defined) return INVALID;
+          p.tab[i] = hd.dc[hd.comp[ci].td];
+        } else if (!dc) {
+          if (!hd.ac[hd.comp[ci].ta].defined) return INVALID;
+          p.tab[i] = hd.ac[hd.comp[ci].ta];
+        }
+        if (!dc && coef_bits[ci][0] < 0) return UNSUPPORTED;   // an AC scan before the component's DC (libjpeg warns)
+        for (int k = ss; k <= se; k++) {
+          if (ah != (coef_bits[ci][k] < 0 ? 0 : coef_bits[ci][k])) return UNSUPPORTED;   // libjpeg warns and decodes on
+          coef_bits[ci][k] = al;
+        }
       }
-      for (int i = 0; i < hd.ncomp; i++) {   // latch_quant_tables, jpeg_make_d_derived_tbl's missing-table check
-        if (!hd.qdef[hd.comp[i].tq] || !hd.dc[hd.comp[i].td].defined || !hd.ac[hd.comp[i].ta].defined) return INVALID;
+      // the units of the scan (per_scan_setup)
+      int hmax = 1, vmax = 1;
+      for (int i = 0; i < hd.ncomp; i++) {
+        hmax = hd.comp[i].h > hmax ? hd.comp[i].h : hmax;
+        vmax = hd.comp[i].v > vmax ? hd.comp[i].v : vmax;
       }
-      return OK;
-    } else if (c == 0xD9) {   // EOI before any scan: no image
-      return INVALID;
+      if (ns == 1) {
+        const int ci = sc[0];
+        const int dw = (int)(((long)hd.width * hd.comp[ci].h + hmax - 1) / hmax), dh = (int)(((long)hd.height * hd.comp[ci].v + vmax - 1) / vmax);
+        p.s.bw = (dw + 7) / 8;
+        p.s.bh = (dh + 7) / 8;
+      } else {
+        p.s.bw = (hd.width + 8 * hmax - 1) / (8 * hmax);
+        p.s.bh = (hd.height + 8 * vmax - 1) / (8 * vmax);
+      }
+      p.s.nunits = p.s.bw * p.s.bh;
+      p.s.nint = p.s.ri ? (p.s.nunits + p.s.ri - 1) / p.s.ri : 1;
+      // the entropy-coded segment ends at the first marker other than RSTn
+      p.off = r.pos;
+      size_t e = r.pos;
+      for (;;) {
+        const uint8_t* q = e < len ? (const uint8_t*)memchr(data + e, 0xFF, len - e) : nullptr;
+        if (!q) { e = len; break; }
+        e = (size_t)(q - data);
+        const int next = e + 1 < len ? data[e + 1] : -1;
+        if (next == 0x00 || next == 0xFF || (next >= 0xD0 && next <= 0xD7)) { e++; continue; }
+        break;
+      }
+      p.len = e - p.off;
+      pg->nscans++;
+      if (e == len) {   // the data ended inside this scan
+        pg->truncated = !complete();
+        return OK;
+      }
+      r.pos = e;
+    } else if (c == 0xD9) {   // EOI
+      if (!progressive || pg->nscans == 0) return INVALID;   // before any scan: no image
+      return complete() ? OK : UNSUPPORTED;
     } else if (c == 0xE0 || c == 0xEE) {   // examine_app0 / examine_app14
       const int length = r.u16() - 2;
       if (!r.ok || length < 0 || r.pos + (size_t)length > len) return INVALID;
@@ -236,7 +375,7 @@ inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
     } else if ((c >= 0xE1 && c <= 0xEF) || c == 0xFE || c == 0xCC || c == 0xDC) {   // APPn, COM, DAC, DNL: skip_variable
       const int length = r.u16() - 2;
       if (!r.ok || length < 0 || r.pos + (size_t)length > len) return INVALID;
-      if (c == 0xE1 && !exif) {
+      if (c == 0xE1 && !exif && !(progressive && pg->nscans > 0)) {   // cv2 reads Exif before the first scan only
         const int o = exif_orientation(data + r.pos, (size_t)length);
         exif = o >= 0;
         if (o >= 1 && o <= 8) hd.orientation = o;
@@ -248,6 +387,7 @@ inline int parse_header(const uint8_t* data, size_t len, Header& hd) {
     }
   }
 }
+inline int parse_header(const uint8_t* data, size_t len, Header& hd) { return parse_file(data, len, hd, nullptr); }
 
 // ---- jpeg_make_d_derived_tbl (jdhuff.c) --------------------------------------------------------------------------------
 // look[c]: (length << 8) | symbol of the code that the LOOK-bit prefix c starts with, 0 when the code is longer.
@@ -617,7 +757,166 @@ JPEG_HD inline int byte_kind(int prev, int b, int next) {   // prev / next: -1 o
   return 0;
 }
 
+// ---- the progressive Huffman decoder (jdphuff.c), one block at a time ---------------------------------------------------
+// Position of block (bx, by) of component c in the coefficient store (the MCU order of Geo above)
+JPEG_HDF size_t comp_block(const Geo& g, int c, int bx, int by) {
+  if (c == 0) return ((size_t)(by / g.vy) * g.mcux + bx / g.hy) * g.bpm + (by % g.vy) * g.hy + bx % g.hy;
+  return ((size_t)by * g.mcux + bx) * g.bpm + g.hy * g.vy + c - 1;
+}
+JPEG_HDF int16_t left_shift(int v, int al) { return (int16_t)(int)((unsigned)v << al); }   // (JCOEF)LEFT_SHIFT
+// decode_mcu_DC_first for one block
+JPEG_HDF bool dc_first(const DTbl& t, Bits& b, int& pred, int al, int16_t* blk) {
+  const int s = huff_decode(t, b);
+  if (s < 0) return false;
+  if (s) {
+    pred += huff_extend((int)b.peek(s), s);
+    b.skip(s);
+  }
+  blk[0] = left_shift(pred, al);
+  return true;
+}
+// decode_mcu_DC_refine for one block
+JPEG_HDF void dc_refine(Bits& b, int al, int16_t* blk) {
+  if (b.peek(1)) blk[0] = (int16_t)(blk[0] | (1 << al));
+  b.skip(1);
+}
+// decode_mcu_AC_first for one block; a coefficient past Se is bad data
+JPEG_HDF bool ac_first(const DTbl& t, Bits& b, int ss, int se, int al, int& eobrun, int16_t* blk) {
+  if (eobrun > 0) {
+    eobrun--;
+    return true;
+  }
+  for (int k = ss; k <= se; k++) {
+    const int sym = huff_decode(t, b);
+    if (sym < 0) return false;
+    const int r = sym >> 4, s = sym & 15;
+    if (s) {
+      k += r;
+      if (k > se) return false;
+      blk[natural_order(k)] = left_shift(huff_extend((int)b.peek(s), s), al);
+      b.skip(s);
+    } else if (r == 15) {
+      k += 15;
+    } else {
+      eobrun = 1 << r;
+      if (r) {
+        eobrun += (int)b.peek(r);
+        b.skip(r);
+      }
+      eobrun--;
+      break;
+    }
+  }
+  return true;
+}
+// correction bit of a nonzero coefficient (decode_mcu_AC_refine)
+JPEG_HDF void refine_coef(Bits& b, int p1, int16_t& c) {
+  if (b.peek(1) && (c & p1) == 0) c = (int16_t)(c >= 0 ? c + p1 : c - p1);
+  b.skip(1);
+}
+// decode_mcu_AC_refine for one block; a new coefficient of a size other than 1, or past Se, is bad data
+JPEG_HDF bool ac_refine(const DTbl& t, Bits& b, int ss, int se, int al, int& eobrun, int16_t* blk) {
+  const int p1 = 1 << al;
+  int k = ss;
+  if (eobrun == 0) {
+    for (; k <= se; k++) {
+      const int sym = huff_decode(t, b);
+      if (sym < 0) return false;
+      int r = sym >> 4, s = sym & 15;
+      if (s) {
+        if (s != 1) return false;
+        s = b.peek(1) ? p1 : -p1;
+        b.skip(1);
+      } else if (r != 15) {
+        eobrun = 1 << r;
+        if (r) {
+          eobrun += (int)b.peek(r);
+          b.skip(r);
+        }
+        break;   // the rest of the block is handled by the EOB run
+      }
+      do {   // advance over nonzero coefficients (with their correction bits) and r zero ones
+        int16_t& c = blk[natural_order(k)];
+        if (c != 0) refine_coef(b, p1, c);
+        else if (--r < 0) break;
+        k++;
+      } while (k <= se);
+      if (s) {
+        if (k > se) return false;
+        blk[natural_order(k)] = (int16_t)s;
+      }
+    }
+  }
+  if (eobrun > 0) {
+    for (; k <= se; k++) {
+      int16_t& c = blk[natural_order(k)];
+      if (c != 0) refine_coef(b, p1, c);
+    }
+    eobrun--;
+  }
+  return true;
+}
+// Units [u0, u1) of restart interval of scan s from the bits at b (the interval's data ends at bit lim), with DC predictors
+// and EOBRUN reset at its start; tbl[i]: the table of scan component i.  Returns false for bad data.  coef: the frame's store.
+// KIND: the decoder, 0 DC first, 1 DC refine, 2 AC first, 3 AC refine (scan_kind).
+JPEG_HDF int scan_kind(const PScan& s) { return (s.ss == 0 ? 0 : 2) + (s.ah != 0 ? 1 : 0); }
+template <int KIND>
+JPEG_HDF bool decode_units(const Geo& g, const PScan& s, const DTbl* const* tbl, Bits& b, uint32_t lim, int16_t* coef, int u0, int u1) {
+  // the scan components' predictors, tables and indices in registers (no dynamically indexed arrays on the device)
+  int pred0 = 0, pred1 = 0, pred2 = 0, eobrun = 0;
+  const DTbl *t0 = tbl[0], *t1 = tbl[1], *t2 = tbl[2];
+  const int c0 = s.comp[0], c1 = s.comp[1], c2 = s.comp[2], al = s.al;
+  for (int u = u0; u < u1; u++) {
+    const int ux = u % s.bw, uy = u / s.bw;
+    if (KIND < 2 && s.ns > 1) {   // an interleaved DC scan: the MCU's blocks of each scan component in turn
+      for (int i = 0; i < s.ns; i++) {
+        const int c = i == 0 ? c0 : i == 1 ? c1 : c2, hc = c == 0 ? g.hy : 1, vc = c == 0 ? g.vy : 1;
+        int pred = i == 0 ? pred0 : i == 1 ? pred1 : pred2;
+        const DTbl& t = i == 0 ? *t0 : i == 1 ? *t1 : *t2;
+        for (int dy = 0; dy < vc; dy++)
+          for (int dx = 0; dx < hc; dx++) {
+            int16_t* blk = coef + 64 * comp_block(g, c, ux * hc + dx, uy * vc + dy);
+            if (KIND == 1) dc_refine(b, al, blk);
+            else if (!dc_first(t, b, pred, al, blk)) return false;
+          }
+        if (i == 0) pred0 = pred;
+        else if (i == 1) pred1 = pred;
+        else pred2 = pred;
+      }
+    } else {
+      int16_t* blk = coef + 64 * comp_block(g, c0, ux, uy);
+      if (KIND == 0 && !dc_first(*t0, b, pred0, al, blk)) return false;
+      if (KIND == 1) dc_refine(b, al, blk);
+      if (KIND == 2 && !ac_first(*t0, b, s.ss, s.se, al, eobrun, blk)) return false;
+      if (KIND == 3 && !ac_refine(*t0, b, s.ss, s.se, al, eobrun, blk)) return false;
+    }
+    if (b.p > lim) return false;   // the interval's data ended before this unit
+  }
+  return true;
+}
+JPEG_HDF bool decode_interval(const Geo& g, const PScan& s, const DTbl* const* tbl, Bits& b, uint32_t lim, int16_t* coef, int u0,
+                              int u1) {
+  switch (scan_kind(s)) {
+    case 0: return decode_units<0>(g, s, tbl, b, lim, coef, u0, u1);
+    case 1: return decode_units<1>(g, s, tbl, b, lim, coef, u0, u1);
+    case 2: return decode_units<2>(g, s, tbl, b, lim, coef, u0, u1);
+    default: return decode_units<3>(g, s, tbl, b, lim, coef, u0, u1);
+  }
+}
+
 #ifndef __CUDA_ARCH__
+// the cropped output of a decoded frame (sample planes smp), or zeros for bad data
+inline void emit_frame(const Geo& g, const uint8_t* smp, uint8_t* out, bool grey, bool bad) {
+  if (bad) {
+    memset(out, 0, (size_t)g.w * g.h * (grey ? 1 : 3));
+  } else if (grey) {
+    for (int y = 0; y < g.h; y++) memcpy(out + (size_t)y * g.w, smp + (size_t)y * g.pw[0], g.w);
+  } else {
+    for (int y = 0; y < g.h; y++)
+      for (int x = 0; x < g.w; x++) pixel(g, smp, x, y, out + ((size_t)y * g.w + x) * 3);
+  }
+}
+
 // The scalar reference of one frame: decode_mcu over the whole scan with process_restart, decompress_onepass's IDCTs, then
 // upsampling and colour conversion.  out: w * h * 3 bytes, or w * h for grey (IMREAD_GRAYSCALE: the IDCTs of component 0
 // only, cropped).  orient: the frame is then turned by the Exif orientation (h x w for 5..8), as cv2.imdecode's default
@@ -686,17 +985,92 @@ inline int decode_frame(const uint8_t* data, size_t len, uint8_t* out, bool grey
         if (!bad && (!grey || c == 0)) idct_islow(blk, hd.q[hd.comp[c].tq], smp + g.poff[c] + (size_t)8 * by * g.pw[c] + 8 * bx, g.pw[c]);
       }
   }
-  if (bad) {
-    memset(out, 0, (size_t)g.w * g.h * (grey ? 1 : 3));
-  } else if (grey) {
-    for (int y = 0; y < g.h; y++) memcpy(out + (size_t)y * g.w, smp + (size_t)y * g.pw[0], g.w);
-  } else {
-    for (int y = 0; y < g.h; y++)
-      for (int x = 0; x < g.w; x++) pixel(g, smp, x, y, out + ((size_t)y * g.w + x) * 3);
-  }
+  emit_frame(g, smp, out, grey, bad);
   delete[] cs;
   delete[] istart;
   delete[] smp;
+  return bad ? 1 : OK;
+}
+// The scalar reference of sequential and progressive files alike: decode_frame for a sequential file; for a progressive
+// one, every scan in file order (destuffed, its restart intervals decoded with decode_interval) into the zeroed coefficient
+// store, then the IDCTs of the blocks (component 0 only for grey) and the output of decode_frame.  Returns OK, INVALID,
+// UNSUPPORTED, or 1 for bad entropy-coded data (an invalid code, a coefficient past Se, the wrong number of RST markers in a
+// scan, a scan whose data ends before its last block, a file cut inside a scan): the frame is then all zeros.
+inline int decode_frame_ex(const uint8_t* data, size_t len, uint8_t* out, bool grey = false, bool orient = false) {
+  Header hd;
+  Prog* pg = new Prog;
+  int rc = parse_file(data, len, hd, pg);
+  if (rc != OK || pg->nscans == 0) {
+    delete pg;
+    return rc != OK ? rc : decode_frame(data, len, out, grey, orient);
+  }
+  if (orient && hd.orientation != 1) {
+    delete pg;
+    const int ch = grey ? 1 : 3, o = hd.orientation, w = o >= 5 ? hd.height : hd.width, h = o >= 5 ? hd.width : hd.height;
+    uint8_t* st = new uint8_t[(size_t)hd.width * hd.height * ch];
+    rc = decode_frame_ex(data, len, st, grey, false);
+    for (int y = 0; y < h; y++)
+      for (int x = 0; x < w; x++) {
+        int sx, sy;
+        oriented_src(o, w, h, x, y, sx, sy);
+        memcpy(out + ((size_t)y * w + x) * ch, st + ((size_t)sy * hd.width + sx) * ch, ch);
+      }
+    delete[] st;
+    return rc;
+  }
+  hd.restart = 0;
+  const Geo g = geometry(hd);
+  DTbl* tbl = new DTbl[(size_t)pg->nscans * 3];
+  for (int i = 0; i < pg->nscans && rc == OK; i++) {
+    const ProgScan& p = pg->scan[i];
+    if (p.s.ss == 0 && p.s.ah != 0) continue;   // DC refinement: no table
+    for (int j = 0; j < p.s.ns; j++)
+      if (!make_derived(p.tab[j], p.s.ss == 0, tbl[3 * i + j])) rc = INVALID;
+  }
+  if (rc != OK) {
+    delete[] tbl;
+    delete pg;
+    return rc;
+  }
+  bool bad = pg->truncated;
+  int16_t* coef = new int16_t[g.nblocks * 64]();
+  for (int i = 0; i < pg->nscans && !bad; i++) {
+    const ProgScan& p = pg->scan[i];
+    const uint8_t* seg = data + p.off;
+    uint8_t* cs = new uint8_t[p.len + 1024]();   // a unit may look up to 256 bytes past the data before it is found short
+    size_t* istart = new size_t[p.s.nint + 1];
+    size_t n = 0;
+    int nrst = 0;
+    istart[0] = 0;
+    for (size_t j = 0; j < p.len; j++) {
+      const int k = byte_kind(j ? seg[j - 1] : -1, seg[j], j + 1 < p.len ? seg[j + 1] : -1);
+      if (k == 0) cs[n++] = seg[j];
+      if (k == 2 && ++nrst < p.s.nint) istart[nrst] = n;
+    }
+    if (nrst != p.s.nint - 1) bad = true;
+    istart[p.s.nint] = n;
+    const DTbl* t[3] = {tbl + 3 * i, tbl + 3 * i + 1, tbl + 3 * i + 2};
+    for (int k = 0; k < p.s.nint && !bad; k++) {
+      Bits b;
+      b.init(cs, (uint32_t)(istart[k] * 8));
+      const int u0 = p.s.ri ? k * p.s.ri : 0;
+      const int u1 = p.s.ri && u0 + p.s.ri < p.s.nunits ? u0 + p.s.ri : p.s.nunits;
+      if (!decode_interval(g, p.s, t, b, (uint32_t)(istart[k + 1] * 8), coef, u0, u1)) bad = true;
+    }
+    delete[] cs;
+    delete[] istart;
+  }
+  uint8_t* smp = new uint8_t[g.nsamples]();
+  for (size_t blk = 0; blk < g.nblocks && !bad; blk++) {
+    int c, bx, by;
+    block_pos(g, (int)(blk / g.bpm), (int)(blk % g.bpm), c, bx, by);
+    if (!grey || c == 0) idct_islow(coef + 64 * blk, pg->q[c], smp + g.poff[c] + (size_t)8 * by * g.pw[c] + 8 * bx, g.pw[c]);
+  }
+  emit_frame(g, smp, out, grey, bad);
+  delete[] coef;
+  delete[] smp;
+  delete[] tbl;
+  delete pg;
   return bad ? 1 : OK;
 }
 #endif
